@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the capyCRYPT B200 batch engine (contract: see the task brief).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Metric (BASELINE.json): SHA3-256 GB/s (+ Ed448 scalar-mults/s in `extra`).  A step is one pass of the hot
@@ -39,6 +39,9 @@ MAC_EXEC_FIXED = 1.23e5
 MAC_EXEC_VAR = 6.86e5
 WARP_TIER_US_PER_PERM = 2.04  # chain speed of the fastest tier (one warp per message), profiles/README.md
 PEAK_FALLBACK = {"lop3": 18.52e12, "imad_wide": 8.67e12}  # profiles/r01_peaks_int_pipes.json
+# --dump-outputs writes a fixed, seeded sample of the digests: all 2^20 x 32 bytes would be 128 MiB as float32
+DUMP_ROWS = 1 << 18
+DUMP_SEED = 0
 
 
 def host_threads() -> int:
@@ -370,6 +373,18 @@ def emit_json_line(line: dict):
         os.write(_REAL_STDOUT, data)
 
 
+def dump_outputs(path: str, digests):
+    """Saves what the timed path returned in its last step, so that two builds can be compared output for output: the
+    SHA3-256 digests of DUMP_ROWS messages drawn with DUMP_SEED, in message order, one float32 per digest byte."""
+    import numpy as np
+    import torch
+
+    rows = np.sort(np.random.default_rng(DUMP_SEED).choice(N_MSGS, DUMP_ROWS, replace=False))
+    sample = digests.view(N_MSGS, DIGEST)[torch.from_numpy(rows).to(digests.device)].cpu().numpy()
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "sha3_256_digests.npy"), sample.astype(np.float32))
+
+
 def main():
     keep_stdout_for_the_json_line()
     ap = argparse.ArgumentParser()
@@ -379,7 +394,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--no-extras", action="store_true", help="skip the Ed448 / KMAC side measurements")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write a seeded sample of rank 0's last-step digests to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3)
     rank, world, local = _env_int("RANK", 0), _env_int("WORLD_SIZE", 1), _env_int("LOCAL_RANK", 0)
 
@@ -443,6 +464,8 @@ def main():
         ms = float(t.item())
     ms_per_step = ms / args.steps
     value = world * N_MSGS * MSG_LEN / (ms_per_step * 1e-3) / 1e9
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, outs[(args.steps - 1) % N_ROT])
 
     # ---- e2e: the same metric through the host-buffer C entry point (pinned host memory, H2D + D2H inside) ----
     k_e2e = max(5, min(args.steps, 100))

@@ -8,19 +8,28 @@ from __future__ import annotations
 import ctypes as C
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _u8p = C.POINTER(C.c_uint8)
 _u64p = C.POINTER(C.c_uint64)
+_NATIVE_DIR = None
 
 
 def build(native: bool = False, force: bool = False) -> str:
     """Compile ref_cpu.c.  native=True adds -march=native (bench CPU-baseline leg, built on
-    the machine that times it); the default x86-64-v3 build is portable to the GPU box."""
-    name = "libcapy_oracle_native.so" if native else "libcapy_oracle.so"
-    out = os.path.join(_HERE, "_build", name)
+    the machine that times it); the default x86-64-v3 build runs on any x86-64-v3 host.
+    The native build happens at benchmark time, when the tree may be read-only, so it goes to
+    a temporary directory that lives as long as the process."""
+    global _NATIVE_DIR
+    if native:
+        if _NATIVE_DIR is None:
+            _NATIVE_DIR = tempfile.TemporaryDirectory(prefix="capy_oracle_")
+        out = os.path.join(_NATIVE_DIR.name, "libcapy_oracle_native.so")
+    else:
+        out = os.path.join(_HERE, "_build", "libcapy_oracle.so")
     src = os.path.join(_HERE, "ref_cpu.c")
     if force or not os.path.exists(out) or os.path.getmtime(out) < os.path.getmtime(src):
         os.makedirs(os.path.dirname(out), exist_ok=True)
