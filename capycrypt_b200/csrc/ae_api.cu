@@ -120,16 +120,6 @@ static int dev_ae_open(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const AeCo
   return CAPY_OK;
 }
 
-// scratch slots of the AE pipelines (24..41 belong to ed448_api.cu and stay usable underneath)
-enum {
-  SA_KEYS = 56, SA_KEYOFF, SA_KEYMAT, SA_TNEW, SA_WX, SA_PROJ, SA_BAD, SA_KW, SA_SK, SA_FLAG,
-  SA_H0 = 66  // host staging: 66..79
-};
-
-#define CAPY_SCRATCH(var, type, slot, bytes)           \
-  type* var = (type*)scratch_get(dc, (slot), (bytes)); \
-  if (!var) return CAPY_ERR_OOM;
-
 static bool ae_customs(int variant, const char** ke, const char** ka) {
   if (variant == CAPY_AE_SHA3) {
     *ke = "SKE";  // sha3/encryptable.rs:41
@@ -147,9 +137,9 @@ static bool ae_customs(int variant, const char** ke, const char** ka) {
 // (ke || ka) <- KMACXOF(z || pw, "", 1024, "S")   sha3/encryptable.rs:33-37
 static int dev_sponge_keymat(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pws, const uint64_t* pw_off,
                              uint64_t pw_bytes, const uint8_t* nonces, uint64_t nonce_len, uint64_t n, uint8_t** keymat_out) {
-  CAPY_SCRATCH(keys, uint8_t, SA_KEYS, n * nonce_len + pw_bytes + 16);
-  CAPY_SCRATCH(koff, uint64_t, SA_KEYOFF, (n + 1) * 8);
-  CAPY_SCRATCH(keymat, uint8_t, SA_KEYMAT, n * 128);
+  CAPY_SCRATCH(keys, uint8_t, kAeKeys, n * nonce_len + pw_bytes + 16);
+  CAPY_SCRATCH(koff, uint64_t, kAeKeyOff, (n + 1) * 8);
+  CAPY_SCRATCH(keymat, uint8_t, kAeKeyMat, n * 128);
   ae_concat_kernel<<<grid_for(n * 32, 256), 256, 0, st>>>(nonces, nonce_len, pws, pw_off, keys, koff, n);
   ctx->launches++;
   CAPY_CUDA(ctx, cudaGetLastError());
@@ -196,7 +186,7 @@ static int dev_sponge_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int
   uint8_t* keymat;
   int rc = dev_sponge_keymat(ctx, dc, st, d, pws, pw_off, pw_bytes, nonces, nonce_len, n, &keymat);
   if (rc) return rc;
-  CAPY_SCRATCH(t_new, uint8_t, SA_TNEW, n * 64);
+  CAPY_SCRATCH(t_new, uint8_t, kAeTNew, n * 64);
   c.d = d;
   c.keymat = keymat;
   c.klen = 64;
@@ -207,7 +197,7 @@ static int dev_sponge_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int
 // (ke || ka) <- KMACXOF(W.x, "", 896, "PK")   ecc/encryptable.rs:40-41, 80-81
 static int dev_ecdhies_keymat(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* wx, uint64_t n,
                               uint8_t** keymat_out) {
-  CAPY_SCRATCH(keymat, uint8_t, SA_KEYMAT, n * 112);
+  CAPY_SCRATCH(keymat, uint8_t, kAeKeyMat, n * 112);
   KmacDevArgs a{};
   a.d_bits = d;
   a.keys = wx;
@@ -233,20 +223,15 @@ static AeCore ecdhies_core(int d, const uint8_t* keymat) {
   return c;
 }
 
-__global__ void ae_any_bad_kernel(const uint8_t* __restrict__ bad, int* bad_flag, uint64_t n) {
-  const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n && bad[i]) atomicOr(bad_flag, 1);
-}
-
 static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pub, const uint8_t* k_rand,
                            const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy,
                            int* d_bad_flag) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(proj, uint32_t, SA_PROJ, n * 256);
-  CAPY_SCRATCH(bad, uint8_t, SA_BAD, n);
-  CAPY_SCRATCH(wx, uint8_t, SA_WX, n * 56);
-  CAPY_SCRATCH(kw, uint32_t, SA_KW, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
+  CAPY_SCRATCH(bad, uint8_t, kAeBad, n);
+  CAPY_SCRATCH(wx, uint8_t, kAeWx, n * 56);
+  CAPY_SCRATCH(kw, uint32_t, kAeKw, n * 56);
   // k = 4 * BE(rand) mod r ; W = [k]V (:36-37)
   int rc = launch_var_base(ctx, dc, st, k_rand, 1, pub, nullptr, proj, bad, n, true);
   if (rc) return rc;
@@ -264,12 +249,7 @@ static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   if (rc) return rc;
   rc = dev_ae_seal(ctx, dc, st, ecdhies_core(d, keymat), msgs, off, n, ct, tag);
   if (rc) return rc;
-  if (d_bad_flag) {
-    ae_any_bad_kernel<<<grid_for(n, 256), 256, 0, st>>>(bad, d_bad_flag, n);
-    ctx->launches++;
-    CAPY_CUDA(ctx, cudaGetLastError());
-  }
-  return CAPY_OK;
+  return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
 
 static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pws, const uint64_t* pw_off,
@@ -277,11 +257,11 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
                            uint8_t* out, uint8_t* ok, int* d_bad_flag) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(proj, uint32_t, SA_PROJ, n * 256);
-  CAPY_SCRATCH(bad, uint8_t, SA_BAD, n);
-  CAPY_SCRATCH(wx, uint8_t, SA_WX, n * 56);
-  CAPY_SCRATCH(sk, uint8_t, SA_SK, n * 56);
-  CAPY_SCRATCH(t_new, uint8_t, SA_TNEW, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
+  CAPY_SCRATCH(bad, uint8_t, kAeBad, n);
+  CAPY_SCRATCH(wx, uint8_t, kAeWx, n * 56);
+  CAPY_SCRATCH(sk, uint8_t, kAeSk, n * 56);
+  CAPY_SCRATCH(t_new, uint8_t, kAeTNew, n * 56);
   // s = 4 * BE(KMACXOF(pw, "", 448, "SK")) mod r (:74-75)
   KmacDevArgs a{};
   a.d_bits = d;
@@ -306,36 +286,20 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   if (rc) return rc;
   rc = dev_ae_open(ctx, dc, st, ecdhies_core(d, keymat), ct, off, tag, bad, n, out, ok, t_new);
   if (rc) return rc;
-  if (d_bad_flag) {
-    ae_any_bad_kernel<<<grid_for(n, 256), 256, 0, st>>>(bad, d_bad_flag, n);
-    ctx->launches++;
-    CAPY_CUDA(ctx, cudaGetLastError());
-  }
-  return CAPY_OK;
+  return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
 
 // ---- host staging ------------------------------------------------------------------------------------
-static int h2d_fixed(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, const uint8_t* src, size_t bytes, uint8_t** out) {
-  uint8_t* d = (uint8_t*)scratch_get(dc, slot, bytes + 16);
-  if (!d) return CAPY_ERR_OOM;
-  if (bytes) {
-    const int rc = copy_in(ctx, dc, st, slot, d, src, bytes);
-    if (rc) return rc;
-  }
-  *out = d;
-  return CAPY_OK;
-}
-
-// output buffer for the byte range of items [i0, i1) of a packed batch, addressed with the caller's offsets
+// output buffer (scratch kHost5) for the byte range of items [i0, i1) of a packed batch, addressed with the caller's offsets
 struct StagedOut {
   uint8_t* d_raw;
   uint8_t* d_base;  // d_base + off[i] addresses item i
   uint64_t a0, bytes;
 };
-static int stage_out(DeviceCtx& dc, int slot, const uint64_t* off, uint64_t i0, uint64_t i1, StagedOut* o) {
+static int stage_out(DeviceCtx& dc, cudaStream_t st, const uint64_t* off, uint64_t i0, uint64_t i1, StagedOut* o) {
   o->a0 = off[i0] & ~(uint64_t)15;
   o->bytes = off[i1] - o->a0;
-  o->d_raw = (uint8_t*)scratch_get(dc, slot, (size_t)o->bytes + 16);
+  o->d_raw = (uint8_t*)scratch_get(dc, st, kHost5, (size_t)o->bytes + 16);
   if (!o->d_raw) return CAPY_ERR_OOM;
   o->d_base = reinterpret_cast<uint8_t*>(reinterpret_cast<uintptr_t>(o->d_raw) - (uintptr_t)o->a0);
   return CAPY_OK;
@@ -343,26 +307,13 @@ static int stage_out(DeviceCtx& dc, int slot, const uint64_t* off, uint64_t i0, 
 static int fetch_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const StagedOut& o, const uint64_t* off, uint64_t i0,
                      uint64_t i1, uint8_t* host) {
   const uint64_t b0 = off[i0], b1 = off[i1];
-  if (b1 > b0) return copy_out(ctx, dc, st, SA_H0 + 5, host + b0, o.d_base + b0, (size_t)(b1 - b0));
-  return CAPY_OK;
-}
-
-static int read_flag(capy_ctx* ctx, cudaStream_t st, int* d_flag, int* h_flag) {
-  CAPY_CUDA(ctx, cudaMemcpyAsync(h_flag, d_flag, sizeof(int), cudaMemcpyDeviceToHost, st));
-  CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+  if (b1 > b0) return copy_out(ctx, dc, st, kHost5, host + b0, o.d_base + b0, (size_t)(b1 - b0));
   return CAPY_OK;
 }
 
 }  // namespace capy
 
 using namespace capy;
-
-#define CAPY_DEV_PROLOGUE                                                                   \
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size()) return CAPY_ERR_BAD_ARG; \
-  DeviceCtx& dc = ctx->devs[dev_index];                                                     \
-  std::lock_guard<std::mutex> lk(*dc.mu); /* host-side state of this device (scratch slots, tables) */ \
-  DeviceGuard g(dc.dev);                                                                    \
-  cudaStream_t st = (cudaStream_t)stream;
 
 extern "C" {
 
@@ -397,30 +348,30 @@ int capy_sponge_encrypt_batch(capy_ctx* ctx, int d_bits, int variant, const uint
   if (variant != CAPY_AE_SHA3 && variant != CAPY_AE_KEM) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 2048);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    cudaStream_t st = dc.streams[0];
-    const uint64_t cnt = sh.i1 - sh.i0;
-    StagedPacked sp, sm;
-    uint8_t* d_nonce = nullptr;
-    int rc = stage_packed(ctx, dc, st, SA_H0, SA_H0 + 1, pws, pw_off, sh.i0, sh.i1, &sp);
-    if (rc) return rc;
-    rc = stage_packed(ctx, dc, st, SA_H0 + 2, SA_H0 + 3, msgs, msg_off, sh.i0, sh.i1, &sm);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 4, nonces + sh.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
-    if (rc) return rc;
-    StagedOut so;
-    rc = stage_out(dc, SA_H0 + 5, msg_off, sh.i0, sh.i1, &so);
-    if (rc) return rc;
-    uint8_t* d_tag = (uint8_t*)scratch_get(dc, SA_H0 + 6, cnt * 64);
-    if (!d_tag) return CAPY_ERR_OOM;
-    rc = dev_sponge_encrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[sh.i1] - pw_off[sh.i0], d_nonce,
-                            nonce_len, sm.d_base, sm.d_off, cnt, so.d_base, d_tag);
-    if (rc) return rc;
-    rc = fetch_out(ctx, dc, st, so, msg_off, sh.i0, sh.i1, ct);
-    if (rc) return rc;
-    CAPY_CUDA(ctx, cudaMemcpyAsync(tag64 + 64 * sh.i0, d_tag, cnt * 64, cudaMemcpyDeviceToHost, st));
-    CAPY_CUDA(ctx, cudaStreamSynchronize(st));
-    return CAPY_OK;
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sp, sm;
+      uint8_t* d_nonce = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
+      if (rc) return rc;
+      rc = stage_packed(ctx, dc, st, kHost2, kHost3, msgs, msg_off, ch.i0, ch.i1, &sm);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost4, nonces + ch.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
+      if (rc) return rc;
+      StagedOut so;
+      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
+      if (rc) return rc;
+      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 64);
+      if (!d_tag) return CAPY_ERR_OOM;
+      rc = dev_sponge_encrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[ch.i1] - pw_off[ch.i0], d_nonce,
+                              nonce_len, sm.d_base, sm.d_off, cnt, so.d_base, d_tag);
+      if (rc) return rc;
+      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
+      if (rc) return rc;
+      CAPY_CUDA(ctx, cudaMemcpyAsync(tag64 + 64 * ch.i0, d_tag, cnt * 64, cudaMemcpyDeviceToHost, st));
+      return CAPY_OK;
+    });
   });
 }
 
@@ -432,32 +383,32 @@ int capy_sponge_decrypt_batch(capy_ctx* ctx, int d_bits, int variant, const uint
   if (variant != CAPY_AE_SHA3 && variant != CAPY_AE_KEM) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(ct_off, 0, 0, n, ctx->devs.size(), 2048);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    cudaStream_t st = dc.streams[0];
-    const uint64_t cnt = sh.i1 - sh.i0;
-    StagedPacked sp, sc;
-    uint8_t *d_nonce = nullptr, *d_tag = nullptr;
-    int rc = stage_packed(ctx, dc, st, SA_H0, SA_H0 + 1, pws, pw_off, sh.i0, sh.i1, &sp);
-    if (rc) return rc;
-    rc = stage_packed(ctx, dc, st, SA_H0 + 2, SA_H0 + 3, ct, ct_off, sh.i0, sh.i1, &sc);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 4, nonces + sh.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 6, tag64 + 64 * sh.i0, (size_t)(cnt * 64), &d_tag);
-    if (rc) return rc;
-    StagedOut so;
-    rc = stage_out(dc, SA_H0 + 5, ct_off, sh.i0, sh.i1, &so);
-    if (rc) return rc;
-    uint8_t* d_ok = (uint8_t*)scratch_get(dc, SA_H0 + 7, cnt);
-    if (!d_ok) return CAPY_ERR_OOM;
-    rc = dev_sponge_decrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[sh.i1] - pw_off[sh.i0], d_nonce,
-                            nonce_len, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok);
-    if (rc) return rc;
-    rc = fetch_out(ctx, dc, st, so, ct_off, sh.i0, sh.i1, out);
-    if (rc) return rc;
-    CAPY_CUDA(ctx, cudaMemcpyAsync(ok + sh.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
-    CAPY_CUDA(ctx, cudaStreamSynchronize(st));
-    return CAPY_OK;
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sp, sc;
+      uint8_t *d_nonce = nullptr, *d_tag = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
+      if (rc) return rc;
+      rc = stage_packed(ctx, dc, st, kHost2, kHost3, ct, ct_off, ch.i0, ch.i1, &sc);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost4, nonces + ch.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost6, tag64 + 64 * ch.i0, (size_t)(cnt * 64), &d_tag);
+      if (rc) return rc;
+      StagedOut so;
+      rc = stage_out(dc, st, ct_off, ch.i0, ch.i1, &so);
+      if (rc) return rc;
+      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost7, cnt);
+      if (!d_ok) return CAPY_ERR_OOM;
+      rc = dev_sponge_decrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[ch.i1] - pw_off[ch.i0], d_nonce,
+                              nonce_len, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok);
+      if (rc) return rc;
+      rc = fetch_out(ctx, dc, st, so, ct_off, ch.i0, ch.i1, out);
+      if (rc) return rc;
+      CAPY_CUDA(ctx, cudaMemcpyAsync(ok + ch.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
+      return CAPY_OK;
+    });
   });
 }
 
@@ -488,39 +439,33 @@ int capy_ed448_key_encrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_x
   if (!ctx || (n && (!pub_xy112 || !k_rand56 || !msgs || !msg_off || !ct || !tag56 || !z_xy112))) return CAPY_ERR_BAD_ARG;
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  std::vector<int> flags(ctx->devs.size(), 0);
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 16384);
-  int rc = for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    cudaStream_t st = dc.streams[0];
-    const uint64_t cnt = sh.i1 - sh.i0;
-    StagedPacked sm;
-    uint8_t *d_pub = nullptr, *d_k = nullptr;
-    int rc = stage_packed(ctx, dc, st, SA_H0, SA_H0 + 1, msgs, msg_off, sh.i0, sh.i1, &sm);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 2, pub_xy112 + 112 * sh.i0, (size_t)cnt * 112, &d_pub);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 3, k_rand56 + 56 * sh.i0, (size_t)cnt * 56, &d_k);
-    if (rc) return rc;
-    StagedOut so;
-    rc = stage_out(dc, SA_H0 + 5, msg_off, sh.i0, sh.i1, &so);
-    if (rc) return rc;
-    uint8_t* d_tag = (uint8_t*)scratch_get(dc, SA_H0 + 6, cnt * 56);
-    uint8_t* d_z = (uint8_t*)scratch_get(dc, SA_H0 + 7, cnt * 112);
-    int* d_flag = (int*)scratch_get(dc, SA_FLAG, sizeof(int));
-    if (!d_tag || !d_z || !d_flag) return CAPY_ERR_OOM;
-    CAPY_CUDA(ctx, cudaMemsetAsync(d_flag, 0, sizeof(int), st));
-    rc = dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z, d_flag);
-    if (rc) return rc;
-    rc = fetch_out(ctx, dc, st, so, msg_off, sh.i0, sh.i1, ct);
-    if (rc) return rc;
-    CAPY_CUDA(ctx, cudaMemcpyAsync(tag56 + 56 * sh.i0, d_tag, cnt * 56, cudaMemcpyDeviceToHost, st));
-    CAPY_CUDA(ctx, cudaMemcpyAsync(z_xy112 + 112 * sh.i0, d_z, cnt * 112, cudaMemcpyDeviceToHost, st));
-    return read_flag(ctx, st, d_flag, &flags[dc.index]);
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, {sh}, bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sm;
+      uint8_t *d_pub = nullptr, *d_k = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost2, pub_xy112 + 112 * ch.i0, (size_t)cnt * 112, &d_pub);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost3, k_rand56 + 56 * ch.i0, (size_t)cnt * 56, &d_k);
+      if (rc) return rc;
+      StagedOut so;
+      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
+      if (rc) return rc;
+      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 56);
+      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost7, cnt * 112);
+      if (!d_tag || !d_z) return CAPY_ERR_OOM;
+      rc = dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z, d_flag);
+      if (rc) return rc;
+      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
+      if (rc) return rc;
+      CAPY_CUDA(ctx, cudaMemcpyAsync(tag56 + 56 * ch.i0, d_tag, cnt * 56, cudaMemcpyDeviceToHost, st));
+      CAPY_CUDA(ctx, cudaMemcpyAsync(z_xy112 + 112 * ch.i0, d_z, cnt * 112, cudaMemcpyDeviceToHost, st));
+      return CAPY_OK;
+    });
   });
-  if (rc) return rc;
-  for (int f : flags)
-    if (f) return CAPY_ERR_BAD_POINT;
-  return CAPY_OK;
 }
 
 int capy_ed448_key_decrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off,
@@ -529,40 +474,34 @@ int capy_ed448_key_decrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, 
   if (!ctx || (n && (!pws || !pw_off || !z_xy112 || !ct || !ct_off || !tag56 || !out || !ok))) return CAPY_ERR_BAD_ARG;
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  std::vector<int> flags(ctx->devs.size(), 0);
   auto shards = split_items(ct_off, 0, 0, n, ctx->devs.size(), 16384);
-  int rc = for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    cudaStream_t st = dc.streams[0];
-    const uint64_t cnt = sh.i1 - sh.i0;
-    StagedPacked sp, sc;
-    uint8_t *d_z = nullptr, *d_tag = nullptr;
-    int rc = stage_packed(ctx, dc, st, SA_H0, SA_H0 + 1, pws, pw_off, sh.i0, sh.i1, &sp);
-    if (rc) return rc;
-    rc = stage_packed(ctx, dc, st, SA_H0 + 2, SA_H0 + 3, ct, ct_off, sh.i0, sh.i1, &sc);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 4, z_xy112 + 112 * sh.i0, (size_t)cnt * 112, &d_z);
-    if (rc) return rc;
-    rc = h2d_fixed(ctx, dc, st, SA_H0 + 6, tag56 + 56 * sh.i0, (size_t)cnt * 56, &d_tag);
-    if (rc) return rc;
-    StagedOut so;
-    rc = stage_out(dc, SA_H0 + 5, ct_off, sh.i0, sh.i1, &so);
-    if (rc) return rc;
-    uint8_t* d_ok = (uint8_t*)scratch_get(dc, SA_H0 + 7, cnt);
-    int* d_flag = (int*)scratch_get(dc, SA_FLAG, sizeof(int));
-    if (!d_ok || !d_flag) return CAPY_ERR_OOM;
-    CAPY_CUDA(ctx, cudaMemsetAsync(d_flag, 0, sizeof(int), st));
-    rc = dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok,
-                         d_flag);
-    if (rc) return rc;
-    rc = fetch_out(ctx, dc, st, so, ct_off, sh.i0, sh.i1, out);
-    if (rc) return rc;
-    CAPY_CUDA(ctx, cudaMemcpyAsync(ok + sh.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
-    return read_flag(ctx, st, d_flag, &flags[dc.index]);
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, {sh}, bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sp, sc;
+      uint8_t *d_z = nullptr, *d_tag = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
+      if (rc) return rc;
+      rc = stage_packed(ctx, dc, st, kHost2, kHost3, ct, ct_off, ch.i0, ch.i1, &sc);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost4, z_xy112 + 112 * ch.i0, (size_t)cnt * 112, &d_z);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost6, tag56 + 56 * ch.i0, (size_t)cnt * 56, &d_tag);
+      if (rc) return rc;
+      StagedOut so;
+      rc = stage_out(dc, st, ct_off, ch.i0, ch.i1, &so);
+      if (rc) return rc;
+      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost7, cnt);
+      if (!d_ok) return CAPY_ERR_OOM;
+      rc = dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok,
+                           d_flag);
+      if (rc) return rc;
+      rc = fetch_out(ctx, dc, st, so, ct_off, ch.i0, ch.i1, out);
+      if (rc) return rc;
+      CAPY_CUDA(ctx, cudaMemcpyAsync(ok + ch.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
+      return CAPY_OK;
+    });
   });
-  if (rc) return rc;
-  for (int f : flags)
-    if (f) return CAPY_ERR_BAD_POINT;
-  return CAPY_OK;
 }
 
 }  // extern "C"

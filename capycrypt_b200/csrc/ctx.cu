@@ -17,8 +17,7 @@ int cuda_fail(capy_ctx* ctx, cudaError_t e, const char* what) {
   return e == cudaErrorMemoryAllocation ? CAPY_ERR_OOM : CAPY_ERR_CUDA;
 }
 
-void* scratch_get(DeviceCtx& dc, int slot, size_t bytes) {
-  Scratch& s = dc.scratch[slot];
+void* scratch_grow(Scratch& s, size_t bytes) {
   if (bytes == 0) bytes = 16;
   if (s.cap >= bytes) return s.p;
   if (s.p) {
@@ -170,13 +169,13 @@ static int stage_settle(capy_ctx* ctx, DeviceCtx& dc, StageSlot& ss, int h) {
   return CAPY_OK;
 }
 
-int copy_in(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* d_dst, const void* h_src, size_t bytes) {
+int copy_in(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, void* d_dst, const void* h_src, size_t bytes) {
   if (bytes == 0) return CAPY_OK;
-  if (bytes < kStageMinBytes || slot < 0 || slot >= kNumScratch || !host_is_pageable(h_src)) {
+  if (bytes < kStageMinBytes || !host_is_pageable(h_src)) {
     CAPY_CUDA(ctx, cudaMemcpyAsync(d_dst, h_src, bytes, cudaMemcpyHostToDevice, st));
     return CAPY_OK;
   }
-  StageSlot& ss = dc.stage[slot];
+  StageSlot& ss = dc.stage[stream_set(dc, st)][slot];
   int rc = stage_ready(ctx, dc, ss);
   if (rc) return rc;
   for (size_t at = 0; at < bytes; at += kStagePiece) {
@@ -194,13 +193,13 @@ int copy_in(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* d_dst
   return CAPY_OK;
 }
 
-int copy_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* h_dst, const void* d_src, size_t bytes) {
+int copy_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, void* h_dst, const void* d_src, size_t bytes) {
   if (bytes == 0) return CAPY_OK;
-  if (bytes < kStageMinBytes || slot < 0 || slot >= kNumScratch || !host_is_pageable(h_dst)) {
+  if (bytes < kStageMinBytes || !host_is_pageable(h_dst)) {
     CAPY_CUDA(ctx, cudaMemcpyAsync(h_dst, d_src, bytes, cudaMemcpyDeviceToHost, st));
     return CAPY_OK;
   }
-  StageSlot& ss = dc.stage[slot];
+  StageSlot& ss = dc.stage[stream_set(dc, st)][slot];
   int rc = stage_ready(ctx, dc, ss);
   if (rc) return rc;
   for (size_t at = 0; at < bytes; at += kStagePiece) {
@@ -221,22 +220,24 @@ int copy_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* h_ds
 
 int stage_drain(capy_ctx* ctx, DeviceCtx& dc) {
   int rc = CAPY_OK;
-  for (StageSlot& ss : dc.stage)
-    for (int h = 0; h < 2; h++)
-      if (ss.pending[h]) {
-        const int r = stage_settle(ctx, dc, ss, h);
-        if (r && !rc) rc = r;
-      }
+  for (auto& set : dc.stage)
+    for (StageSlot& ss : set)
+      for (int h = 0; h < 2; h++)
+        if (ss.pending[h]) {
+          const int r = stage_settle(ctx, dc, ss, h);
+          if (r && !rc) rc = r;
+        }
   return rc;
 }
 
 void stage_free(DeviceCtx& dc) {
-  for (StageSlot& ss : dc.stage) {
-    for (int h = 0; h < 2; h++)
-      if (ss.ev[h]) cudaEventDestroy(ss.ev[h]);
-    if (ss.p) cudaFreeHost(ss.p);
-    ss = StageSlot();
-  }
+  for (auto& set : dc.stage)
+    for (StageSlot& ss : set) {
+      for (int h = 0; h < 2; h++)
+        if (ss.ev[h]) cudaEventDestroy(ss.ev[h]);
+      if (ss.p) cudaFreeHost(ss.p);
+      ss = StageSlot();
+    }
   dc.copy_pool.reset();
 }
 
@@ -322,8 +323,10 @@ void capy_gpu_destroy(capy_ctx* ctx) {
     plan_cache_clear(dc);
     for (int s = 0; s < kNumStreams; s++)
       if (dc.streams[s]) cudaStreamDestroy(dc.streams[s]);
-    for (Scratch& sc : dc.scratch)
-      if (sc.p) cudaFree(sc.p);
+    for (auto& set : dc.scratch)
+      for (Scratch& sc : set)
+        if (sc.p) cudaFree(sc.p);
+    if (dc.vb_slabs.p) cudaFree(dc.vb_slabs.p);
     for (auto& kv : dc.prefix_cache) {
       if (kv.second.d_state) cudaFree(kv.second.d_state);
       if (kv.second.d_prefix) cudaFree(kv.second.d_prefix);
@@ -340,11 +343,14 @@ int capy_gpu_scrub(capy_ctx* ctx) {
     std::lock_guard<std::mutex> lk(*dc.mu);
     DeviceGuard g(dc.dev);
     CAPY_CUDA(ctx, cudaDeviceSynchronize());
-    for (Scratch& sc : dc.scratch)
-      if (sc.p) CAPY_CUDA(ctx, cudaMemset(sc.p, 0, sc.cap));
+    for (auto& set : dc.scratch)
+      for (Scratch& sc : set)
+        if (sc.p) CAPY_CUDA(ctx, cudaMemset(sc.p, 0, sc.cap));
+    if (dc.vb_slabs.p) CAPY_CUDA(ctx, cudaMemset(dc.vb_slabs.p, 0, dc.vb_slabs.cap));
     CAPY_CUDA(ctx, cudaDeviceSynchronize());
-    for (StageSlot& ss : dc.stage)  // the page-locked staging halves saw passwords and plaintexts too
-      if (ss.p) memset(ss.p, 0, 2 * kStagePiece);
+    for (auto& set : dc.stage)  // the page-locked staging halves saw passwords and plaintexts too
+      for (StageSlot& ss : set)
+        if (ss.p) memset(ss.p, 0, 2 * kStagePiece);
   }
   return CAPY_OK;
 }

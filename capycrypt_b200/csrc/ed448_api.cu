@@ -154,35 +154,19 @@ int launch_to_affine(capy_ctx* ctx, cudaStream_t st, const uint32_t* proj, uint6
   return CAPY_OK;
 }
 
-// scratch slots of the Ed448 pipelines
-enum {
-  SL_KWORDS = 24, SL_SWORDS, SL_PROJ, SL_PROJ2, SL_BAD, SL_TMP56A, SL_TMP56B, SL_TMP56C, SL_FLAG,
-  SL_H_IN0 = 36  // 36.. host staging
-};
-
-// The pipelines below keep their intermediates in fixed scratch slots.  A host entry point runs several chunks at once on
-// the device's internal streams, so every internal stream has its own copy of the slots 24..54 (stream 0: the slots
-// themselves, streams 1 and 2: shadow ranges behind the AE slots); a caller's stream (the _dev entry points) uses set 0.
-// Slot 55 (the per-SM table slabs of var_base_kernel) is shared: an SM runs one var_base block at a time.
-constexpr int kEdShadowBase = 80, kEdShadowStride = 32;
-static_assert(kEdShadowBase + (kNumStreams - 1) * kEdShadowStride <= kNumScratch, "scratch slots of the stream copies");
-static inline int ed_stream_index(const DeviceCtx& dc, cudaStream_t st) {
-  for (int k = 1; k < kNumStreams; k++)
-    if (dc.streams[k] == st) return k;
-  return 0;
+int launch_any_bad(capy_ctx* ctx, cudaStream_t st, const uint8_t* bad, int* bad_flag, uint64_t n) {
+  any_bad_kernel<<<grid_for(n, 256), 256, 0, st>>>(bad, bad_flag, n);
+  ctx->launches++;
+  CAPY_CUDA(ctx, cudaGetLastError());
+  return CAPY_OK;
 }
-static inline int ed_slot(int slot, int ss) { return ss == 0 ? slot : kEdShadowBase + (ss - 1) * kEdShadowStride + (slot - 24); }
-
-#define CAPY_SCRATCH(var, type, slot, bytes)                                                    \
-  type* var = (type*)scratch_get(dc, ed_slot((slot), ed_stream_index(dc, st)), (bytes));        \
-  if (!var) return CAPY_ERR_OOM;
 
 // ---- device pipelines (async on `st`) ----------------------------------------------------------------
 static int dev_fixed_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* d_scalars, uint64_t n,
                           uint8_t* d_out_xy) {
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(kw, uint32_t, SL_KWORDS, n * 56);
-  CAPY_SCRATCH(proj, uint32_t, SL_PROJ, n * 256);
+  CAPY_SCRATCH(kw, uint32_t, kEdKWords, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
   int rc = launch_scalar_prep(ctx, st, d_scalars, 0, kw, nullptr, n);
   if (rc) return rc;
   rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true);
@@ -193,18 +177,13 @@ static int dev_fixed_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const u
 static int dev_var_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* d_scalars, const uint8_t* d_points,
                         uint64_t n, uint8_t* d_out_xy, int* d_bad_flag) {
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(proj, uint32_t, SL_PROJ, n * 256);
-  CAPY_SCRATCH(bad, uint8_t, SL_BAD, n);
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
+  CAPY_SCRATCH(bad, uint8_t, kEdBad, n);
   int rc = launch_var_base(ctx, dc, st, d_scalars, 0, d_points, nullptr, proj, bad, n, true);
   if (rc) return rc;
   rc = launch_to_affine(ctx, st, proj, n, 0, bad, d_out_xy);
   if (rc) return rc;
-  if (d_bad_flag) {
-    any_bad_kernel<<<grid_for(n, 256), 256, 0, st>>>(bad, d_bad_flag, n);
-    ctx->launches++;
-    CAPY_CUDA(ctx, cudaGetLastError());
-  }
-  return CAPY_OK;
+  return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
 
 static KmacDevArgs kmac_args(int d, const uint8_t* keys, const uint64_t* key_off, uint64_t key_len, const uint8_t* data,
@@ -230,7 +209,7 @@ static KmacDevArgs kmac_args(int d, const uint8_t* keys, const uint64_t* key_off
 // s = 4 * BE(KMACXOF(pw, "", 448, "SK", d)) mod r  (ecc/keypair.rs:42-43): words + optional BE bytes
 int dev_secret_scalar(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pws,
                              const uint64_t* d_pw_off, uint64_t n, uint32_t* s_words, uint8_t* s_be) {
-  CAPY_SCRATCH(tmp, uint8_t, SL_TMP56A, n * 56);
+  CAPY_SCRATCH(tmp, uint8_t, kEdTmp56A, n * 56);
   int rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, d_pws, d_pw_off, 0, nullptr, nullptr, n, "SK", tmp));
   if (rc) return rc;
   return launch_scalar_prep(ctx, st, tmp, 1, s_words, s_be, n);
@@ -240,8 +219,8 @@ static int dev_keygen(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
                       uint64_t n, uint8_t* d_out_xy) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(sw, uint32_t, SL_SWORDS, n * 56);
-  CAPY_SCRATCH(proj, uint32_t, SL_PROJ, n * 256);
+  CAPY_SCRATCH(sw, uint32_t, kEdSWords, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
   int rc = dev_secret_scalar(ctx, dc, st, d, d_pws, d_pw_off, n, sw, nullptr);
   if (rc) return rc;
   rc = launch_fixed_base(ctx, dc, st, sw, proj, n, true);
@@ -253,11 +232,11 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
                     const uint8_t* d_msgs, const uint64_t* d_msg_off, uint64_t n, uint8_t* d_h, uint8_t* d_z) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(sw, uint32_t, SL_SWORDS, n * 56);
-  CAPY_SCRATCH(kw, uint32_t, SL_KWORDS, n * 56);
-  CAPY_SCRATCH(proj, uint32_t, SL_PROJ, n * 256);
-  CAPY_SCRATCH(s_be, uint8_t, SL_TMP56B, n * 56);
-  CAPY_SCRATCH(tmp, uint8_t, SL_TMP56C, n * 56);
+  CAPY_SCRATCH(sw, uint32_t, kEdSWords, n * 56);
+  CAPY_SCRATCH(kw, uint32_t, kEdKWords, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
+  CAPY_SCRATCH(s_be, uint8_t, kEdTmp56B, n * 56);
+  CAPY_SCRATCH(tmp, uint8_t, kEdTmp56C, n * 56);
   // s (signable.rs:41-43)
   int rc = dev_secret_scalar(ctx, dc, st, d, d_pws, d_pw_off, n, sw, s_be);
   if (rc) return rc;
@@ -286,12 +265,12 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
                       int* d_bad_flag) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  CAPY_SCRATCH(kw, uint32_t, SL_KWORDS, n * 56);
-  CAPY_SCRATCH(projA, uint32_t, SL_PROJ, n * 256);
-  CAPY_SCRATCH(projB, uint32_t, SL_PROJ2, n * 256);
-  CAPY_SCRATCH(bad, uint8_t, SL_BAD, n);
-  CAPY_SCRATCH(ux, uint8_t, SL_TMP56A, n * 56);
-  CAPY_SCRATCH(hp, uint8_t, SL_TMP56B, n * 56);
+  CAPY_SCRATCH(kw, uint32_t, kEdKWords, n * 56);
+  CAPY_SCRATCH(projA, uint32_t, kEdProj, n * 256);
+  CAPY_SCRATCH(projB, uint32_t, kEdProj2, n * 256);
+  CAPY_SCRATCH(bad, uint8_t, kEdBad, n);
+  CAPY_SCRATCH(ux, uint8_t, kEdTmp56A, n * 56);
+  CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
   // U = [z]G + [BE(h)]V with h unreduced (signable.rs:76-77, quirk Q10).  All inputs are public:
   // table lookups are direct, not scanned.
   int rc = launch_scalar_prep(ctx, st, d_z, 0, kw, nullptr, n);
@@ -312,65 +291,19 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
 }
 
 // ---- host wrappers -------------------------------------------------------------------------------------
-struct HostIn {
-  const void* p;
-  size_t bytes_per_item;  // fixed-size inputs
-};
-
-static int h2d(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, const void* src, size_t bytes, uint8_t** out) {
-  uint8_t* d = (uint8_t*)scratch_get(dc, slot, bytes + 16);
-  if (!d) return CAPY_ERR_OOM;
-  if (bytes) {
-    const int rc = copy_in(ctx, dc, st, slot, d, src, bytes);
-    if (rc) return rc;
-  }
-  *out = d;
-  return CAPY_OK;
-}
-
-// Runs `body(stream, slot set, chunk, d_flag)` for the chunks of one device's shard, rotating over the internal streams
-// (body enqueues the copies in, the pipeline and the copies out of its chunk and does not wait), then waits for the
-// streams.  flag_out (optional): the OR of what the chunks left in their stream's "bad point" flag.
-// Chunks of at least 2^18 items: the pipelines contain latency-bound steps (the batch inversion of to_affine_kernel runs
-// 16 items per thread, ~0.3 ms however few) that smaller chunks would repeat too often -- measured: four chunks of 2^16
-// through capy_ed448_fixed_base_batch 7.05 ms against 6.9 ms unchunked, although the copies (0.8 ms) were hidden.
-static size_t ed_chunk_count(uint64_t items) { return items < (1ull << 19) ? 1 : (size_t)std::min<uint64_t>(8, items >> 18); }
-
-template <class F>
-static int ed_host_chunks(capy_ctx* ctx, DeviceCtx& dc, Range sh, int* flag_out, F&& body) {
-  auto chunks = split_items(nullptr, 1, sh.i0, sh.i1, ed_chunk_count(sh.i1 - sh.i0), 0);
-  const int used = (int)std::min<size_t>(chunks.size(), kNumStreams);
-  int* d_flags[kNumStreams] = {};
-  for (int s = 0; s < used; s++) {
-    d_flags[s] = (int*)scratch_get(dc, ed_slot(SL_FLAG, s), sizeof(int));
-    if (!d_flags[s]) return CAPY_ERR_OOM;
-    CAPY_CUDA(ctx, cudaMemsetAsync(d_flags[s], 0, sizeof(int), dc.streams[s]));
-  }
-  for (size_t c = 0; c < chunks.size(); c++) {
-    const int s = (int)(c % kNumStreams);
-    int rc = body(dc.streams[s], s, chunks[c], d_flags[s]);
-    if (rc) return rc;
-  }
-  int h_flags[kNumStreams] = {};
-  for (int s = 0; s < used; s++) {
-    if (flag_out) CAPY_CUDA(ctx, cudaMemcpyAsync(&h_flags[s], d_flags[s], sizeof(int), cudaMemcpyDeviceToHost, dc.streams[s]));
-    CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
-  }
-  if (flag_out)
-    for (int s = 0; s < used; s++) *flag_out |= h_flags[s];
-  return CAPY_OK;
+// The chunks of one device's shard (run_chunks).  At least 2^18 items: the pipelines contain latency-bound steps (the
+// batch inversion of to_affine_kernel runs 16 items per thread, ~0.3 ms however few) that smaller chunks would repeat too
+// often -- measured: four chunks of 2^16 through capy_ed448_fixed_base_batch 7.05 ms against 6.9 ms unchunked, although
+// the copies (0.8 ms) were hidden.
+static std::vector<Range> ed_chunks(Range sh) {
+  const uint64_t items = sh.i1 - sh.i0;
+  const size_t count = items < (1ull << 19) ? 1 : (size_t)std::min<uint64_t>(8, items >> 18);
+  return split_items(nullptr, 1, sh.i0, sh.i1, count, 0);
 }
 
 }  // namespace capy
 
 using namespace capy;
-
-#define CAPY_DEV_PROLOGUE                                                                       \
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size()) return CAPY_ERR_BAD_ARG;     \
-  DeviceCtx& dc = ctx->devs[dev_index];                                                         \
-  std::lock_guard<std::mutex> lk(*dc.mu); /* host-side state of this device (scratch slots, tables) */ \
-  DeviceGuard g(dc.dev);                                                                        \
-  cudaStream_t st = (cudaStream_t)stream;
 
 extern "C" {
 
@@ -412,23 +345,23 @@ int capy_ed448_verify_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int 
 }
 
 // ---- host-buffer entry points: shard across the ctx devices by item count; inside a device the shard is cut into chunks
-// that rotate over the device's streams (own scratch slots per stream, ed_slot), so the copies of one chunk run under the
-// kernels of its neighbours ----
+// that rotate over the device's streams (run_chunks), so the copies of one chunk run under the kernels of its
+// neighbours ----
 int capy_ed448_fixed_base_batch(capy_ctx* ctx, const uint8_t* scalars_be56, uint64_t n, uint8_t* out_xy112) {
   if (!ctx || (n && (!scalars_be56 || !out_xy112))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, nullptr, [&](cudaStream_t st, int ss, Range ch, int*) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       uint8_t *d_sc = nullptr, *d_out = nullptr;
-      int rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0, ss), scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
+      int rc = h2d(ctx, dc, st, kHost0, scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
       if (rc) return rc;
-      d_out = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 1, ss), cnt * 112);
+      d_out = (uint8_t*)scratch_get(dc, st, kHost1, cnt * 112);
       if (!d_out) return CAPY_ERR_OOM;
       rc = dev_fixed_base(ctx, dc, st, d_sc, cnt, d_out);
       if (rc) return rc;
-      return copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 1, ss), out_xy112 + 112 * ch.i0, d_out, cnt * 112);
+      return copy_out(ctx, dc, st, kHost1, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
     });
   });
 }
@@ -437,27 +370,22 @@ int capy_ed448_var_base_batch(capy_ctx* ctx, const uint8_t* scalars_be56, const 
                               uint8_t* out_xy112) {
   if (!ctx || (n && (!scalars_be56 || !points_xy112 || !out_xy112))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
-  std::vector<int> flags(ctx->devs.size(), 0);
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  int rc = for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, &flags[dc.index], [&](cudaStream_t st, int ss, Range ch, int* d_flag) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       uint8_t *d_sc = nullptr, *d_pt = nullptr;
-      int rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0, ss), scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
+      int rc = h2d(ctx, dc, st, kHost0, scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
       if (rc) return rc;
-      rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0 + 1, ss), points_xy112 + 112 * ch.i0, cnt * 112, &d_pt);
+      rc = h2d(ctx, dc, st, kHost1, points_xy112 + 112 * ch.i0, cnt * 112, &d_pt);
       if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 2, ss), cnt * 112);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 112);
       if (!d_out) return CAPY_ERR_OOM;
       rc = dev_var_base(ctx, dc, st, d_sc, d_pt, cnt, d_out, d_flag);
       if (rc) return rc;
-      return copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 2, ss), out_xy112 + 112 * ch.i0, d_out, cnt * 112);
+      return copy_out(ctx, dc, st, kHost2, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
     });
   });
-  if (rc) return rc;
-  for (int f : flags)
-    if (f) return CAPY_ERR_BAD_POINT;
-  return CAPY_OK;
 }
 
 int capy_ed448_keygen_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off, uint64_t n,
@@ -466,17 +394,17 @@ int capy_ed448_keygen_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, nullptr, [&](cudaStream_t st, int ss, Range ch, int*) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, ed_slot(SL_H_IN0, ss), ed_slot(SL_H_IN0 + 1, ss), pws, pw_off, ch.i0, ch.i1, &sp);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
       if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 2, ss), cnt * 112);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 112);
       if (!d_out) return CAPY_ERR_OOM;
       rc = dev_keygen(ctx, dc, st, d_bits, sp.d_base, sp.d_off, cnt, d_out);
       if (rc) return rc;
-      return copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 2, ss), out_xy112 + 112 * ch.i0, d_out, cnt * 112);
+      return copy_out(ctx, dc, st, kHost2, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
     });
   });
 }
@@ -487,22 +415,22 @@ int capy_ed448_sign_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const u
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, nullptr, [&](cudaStream_t st, int ss, Range ch, int*) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       StagedPacked sp, sm;
-      int rc = stage_packed(ctx, dc, st, ed_slot(SL_H_IN0, ss), ed_slot(SL_H_IN0 + 1, ss), pws, pw_off, ch.i0, ch.i1, &sp);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
       if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, ed_slot(SL_H_IN0 + 2, ss), ed_slot(SL_H_IN0 + 3, ss), msgs, msg_off, ch.i0, ch.i1, &sm);
+      rc = stage_packed(ctx, dc, st, kHost2, kHost3, msgs, msg_off, ch.i0, ch.i1, &sm);
       if (rc) return rc;
-      uint8_t* d_h = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 4, ss), cnt * 56);
-      uint8_t* d_z = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 5, ss), cnt * 56);
+      uint8_t* d_h = (uint8_t*)scratch_get(dc, st, kHost4, cnt * 56);
+      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost5, cnt * 56);
       if (!d_h || !d_z) return CAPY_ERR_OOM;
       rc = dev_sign(ctx, dc, st, d_bits, sp.d_base, sp.d_off, sm.d_base, sm.d_off, cnt, d_h, d_z);
       if (rc) return rc;
-      rc = copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 4, ss), h56 + 56 * ch.i0, d_h, cnt * 56);
+      rc = copy_out(ctx, dc, st, kHost4, h56 + 56 * ch.i0, d_h, cnt * 56);
       if (rc) return rc;
-      return copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 5, ss), z_be56 + 56 * ch.i0, d_z, cnt * 56);
+      return copy_out(ctx, dc, st, kHost5, z_be56 + 56 * ch.i0, d_z, cnt * 56);
     });
   });
 }
@@ -512,65 +440,58 @@ int capy_ed448_verify_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112,
   if (!ctx || (n && (!pub_xy112 || !msgs || !msg_off || !h56 || !z_be56 || !ok))) return CAPY_ERR_BAD_ARG;
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
-  std::vector<int> flags(ctx->devs.size(), 0);
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
-  int rc = for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, &flags[dc.index], [&](cudaStream_t st, int ss, Range ch, int* d_flag) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       StagedPacked sm;
       uint8_t *d_pub = nullptr, *d_h = nullptr, *d_z = nullptr;
-      int rc = stage_packed(ctx, dc, st, ed_slot(SL_H_IN0, ss), ed_slot(SL_H_IN0 + 1, ss), msgs, msg_off, ch.i0, ch.i1, &sm);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
       if (rc) return rc;
-      rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0 + 2, ss), pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
+      rc = h2d(ctx, dc, st, kHost2, pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
       if (rc) return rc;
-      rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0 + 3, ss), h56 + 56 * ch.i0, cnt * 56, &d_h);
+      rc = h2d(ctx, dc, st, kHost3, h56 + 56 * ch.i0, cnt * 56, &d_h);
       if (rc) return rc;
-      rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0 + 4, ss), z_be56 + 56 * ch.i0, cnt * 56, &d_z);
+      rc = h2d(ctx, dc, st, kHost4, z_be56 + 56 * ch.i0, cnt * 56, &d_z);
       if (rc) return rc;
-      uint8_t* d_ok = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 5, ss), cnt);
+      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost5, cnt);
       if (!d_ok) return CAPY_ERR_OOM;
       rc = dev_verify(ctx, dc, st, d_bits, d_pub, sm.d_base, sm.d_off, d_h, d_z, cnt, d_ok, d_flag);
       if (rc) return rc;
-      return copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 5, ss), ok + ch.i0, d_ok, cnt);
+      return copy_out(ctx, dc, st, kHost5, ok + ch.i0, d_ok, cnt);
     });
   });
-  if (rc) return rc;
-  for (int f : flags)
-    if (f) return CAPY_ERR_BAD_POINT;
-  return CAPY_OK;
 }
 
 int capy_ed448_ecdh_batch(capy_ctx* ctx, const uint8_t* k_rand56, const uint8_t* pub_xy112, uint64_t n, uint8_t* wx56,
                           uint8_t* z_xy112) {
   if (!ctx || (n && (!k_rand56 || !pub_xy112 || !wx56))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
-  std::vector<int> flags(ctx->devs.size(), 0);
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  int rc = for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
-    return ed_host_chunks(ctx, dc, sh, &flags[dc.index], [&](cudaStream_t st, int ss, Range ch, int* d_flag) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       uint8_t *d_k = nullptr, *d_pub = nullptr;
-      int rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0, ss), k_rand56 + 56 * ch.i0, cnt * 56, &d_k);
+      int rc = h2d(ctx, dc, st, kHost0, k_rand56 + 56 * ch.i0, cnt * 56, &d_k);
       if (rc) return rc;
-      rc = h2d(ctx, dc, st, ed_slot(SL_H_IN0 + 1, ss), pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
+      rc = h2d(ctx, dc, st, kHost1, pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
       if (rc) return rc;
-      uint8_t* d_wx = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 2, ss), cnt * 56);
-      uint32_t* proj = (uint32_t*)scratch_get(dc, ed_slot(SL_PROJ, ss), cnt * 256);
-      uint8_t* bad = (uint8_t*)scratch_get(dc, ed_slot(SL_BAD, ss), cnt);
+      uint8_t* d_wx = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 56);
+      uint32_t* proj = (uint32_t*)scratch_get(dc, st, kEdProj, cnt * 256);
+      uint8_t* bad = (uint8_t*)scratch_get(dc, st, kEdBad, cnt);
       if (!d_wx || !proj || !bad) return CAPY_ERR_OOM;
       // W = [k]V with k = 4 * BE(rand) mod r (ecc/encryptable.rs:36-37); W.x
       rc = launch_var_base(ctx, dc, st, d_k, 1, d_pub, nullptr, proj, bad, cnt, true);
       if (rc) return rc;
       rc = launch_to_affine(ctx, st, proj, cnt, 1, bad, d_wx);
       if (rc) return rc;
-      any_bad_kernel<<<grid_for(cnt, 256), 256, 0, st>>>(bad, d_flag, cnt);
-      ctx->launches++;
-      CAPY_CUDA(ctx, cudaGetLastError());
-      rc = copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 2, ss), wx56 + 56 * ch.i0, d_wx, cnt * 56);
+      rc = launch_any_bad(ctx, st, bad, d_flag, cnt);
+      if (rc) return rc;
+      rc = copy_out(ctx, dc, st, kHost2, wx56 + 56 * ch.i0, d_wx, cnt * 56);
       if (rc) return rc;
       if (z_xy112) {  // Z = [k]G (:38)
-        uint32_t* kw = (uint32_t*)scratch_get(dc, ed_slot(SL_KWORDS, ss), cnt * 56);
-        uint8_t* d_z = (uint8_t*)scratch_get(dc, ed_slot(SL_H_IN0 + 3, ss), cnt * 112);
+        uint32_t* kw = (uint32_t*)scratch_get(dc, st, kEdKWords, cnt * 56);
+        uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost3, cnt * 112);
         if (!kw || !d_z) return CAPY_ERR_OOM;
         rc = launch_scalar_prep(ctx, st, d_k, 1, kw, nullptr, cnt);
         if (rc) return rc;
@@ -578,16 +499,12 @@ int capy_ed448_ecdh_batch(capy_ctx* ctx, const uint8_t* k_rand56, const uint8_t*
         if (rc) return rc;
         rc = launch_to_affine(ctx, st, proj, cnt, 0, nullptr, d_z);
         if (rc) return rc;
-        rc = copy_out(ctx, dc, st, ed_slot(SL_H_IN0 + 3, ss), z_xy112 + 112 * ch.i0, d_z, cnt * 112);
+        rc = copy_out(ctx, dc, st, kHost3, z_xy112 + 112 * ch.i0, d_z, cnt * 112);
         if (rc) return rc;
       }
       return CAPY_OK;
     });
   });
-  if (rc) return rc;
-  for (int f : flags)
-    if (f) return CAPY_ERR_BAD_POINT;
-  return CAPY_OK;
 }
 
 }  // extern "C"

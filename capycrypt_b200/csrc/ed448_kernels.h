@@ -5,8 +5,6 @@
 
 namespace capy {
 
-static inline unsigned grid_for(uint64_t n, unsigned block) { return (unsigned)((n + block - 1) / block); }
-
 // extended point of item i, limb-major SoA: word w at proj[w * n + i], w = 0..63 (X | Y | Z | T)
 __device__ __forceinline__ void store_ext(uint32_t* __restrict__ proj, uint64_t n, uint64_t i, const PtExt& p) {
 #pragma unroll
@@ -22,13 +20,14 @@ __device__ __forceinline__ void store_ext(uint32_t* __restrict__ proj, uint64_t 
 int launch_fixed_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint32_t* k_words, uint32_t* proj, uint64_t n,
                       bool constant_time);
 // ed448_var.cu
-constexpr int SL_VB_SLABS = 55;  // scratch slot of the per-SM table slabs (24..41 are the pipelines of ed448_api.cu, 56.. the AE ones)
 int launch_var_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* scalars, int mode4, const uint8_t* points,
                     const uint32_t* addend, uint32_t* proj, uint8_t* bad, uint64_t n, bool constant_time);
 
 // ed448_api.cu
 int launch_scalar_prep(capy_ctx* ctx, cudaStream_t st, const uint8_t* in, int mode, uint32_t* words, uint8_t* be, uint64_t n);
 int launch_to_affine(capy_ctx* ctx, cudaStream_t st, const uint32_t* proj, uint64_t n, int mode, const uint8_t* bad, uint8_t* out);
+// *bad_flag |= 1 when any of bad[0 .. n) is set
+int launch_any_bad(capy_ctx* ctx, cudaStream_t st, const uint8_t* bad, int* bad_flag, uint64_t n);
 int dev_secret_scalar(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pws, const uint64_t* d_pw_off,
                       uint64_t n, uint32_t* s_words, uint8_t* s_be);
 

@@ -84,7 +84,7 @@ __global__ void __launch_bounds__(VB_BLOCK, 1) var_base_kernel(const uint8_t* __
 int launch_var_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* scalars, int mode4, const uint8_t* points,
                     const uint32_t* addend, uint32_t* proj, uint8_t* bad, uint64_t n, bool constant_time) {
   // per-SM table slabs of the second half of every block (a fixed 34 MB per device, allocated once)
-  uint4* slabs = (uint4*)scratch_get(dc, SL_VB_SLABS, (size_t)dc.sm_count * VB_SLAB_BYTES);
+  uint4* slabs = (uint4*)scratch_grow(dc.vb_slabs, (size_t)dc.sm_count * VB_SLAB_BYTES);
   if (!slabs) return CAPY_ERR_OOM;
   CAPY_CUDA(ctx, cudaFuncSetAttribute(var_base_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)VB_SMEM));
   var_base_kernel<<<grid_for(n, VB_BLOCK), VB_BLOCK, VB_SMEM, st>>>(scalars, mode4, points, addend, proj, bad, n,

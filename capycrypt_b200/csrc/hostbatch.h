@@ -1,4 +1,4 @@
-// hostbatch.h -- host-buffer plumbing shared by the SHA3 and Ed448 entry points.
+// hostbatch.h -- host-buffer plumbing shared by the SHA3, Ed448 and AE entry points.
 #pragma once
 #include <algorithm>
 #include <condition_variable>
@@ -130,44 +130,88 @@ inline std::vector<DeviceShare> lpt_shares(const uint64_t* off, uint64_t n, size
   return sh;
 }
 
-// Runs fn(device, shard) for every shard: inline on the caller's thread for a single shard, else on the devices'
-// persistent worker threads (DeviceWorker), each holding its device's lock for the duration of its closure.
+// Runs fn(device, shard, bad_point) for every shard: inline on the caller's thread for a single shard, else on the
+// devices' persistent worker threads (DeviceWorker), each holding its device's lock for the duration of its closure.
+// fn may set *bad_point (an input point was not on the curve): the call then returns CAPY_ERR_BAD_POINT, unless a device
+// failed otherwise, and only after every device has handed its outputs to the caller's buffers.
 template <class F>
 inline int for_each_device(capy_ctx* ctx, const std::vector<Range>& shards, F&& fn) {
-  if (shards.size() <= 1) {
-    if (shards.empty()) return CAPY_OK;
+  if (shards.empty()) return CAPY_OK;
+  std::vector<int> rcs(shards.size(), CAPY_OK), bad(shards.size(), 0);
+  if (shards.size() == 1) {
     DeviceCtx& dc = ctx->devs[0];
     std::lock_guard<std::mutex> lk(*dc.mu);
     DeviceGuard g(dc.dev);
     HostOffScope hs(dc);
-    const int rc = fn(dc, shards[0]);
+    rcs[0] = fn(dc, shards[0], &bad[0]);
     const int rd = stage_drain(ctx, dc);  // staged device-to-host copies: hand the bytes to the caller's buffers
-    return rc ? rc : rd;
-  }
-  std::vector<int> rcs(shards.size(), CAPY_OK);
-  std::mutex m;
-  std::condition_variable cv;
-  size_t pending = shards.size();
-  for (size_t k = 0; k < shards.size(); k++) {
-    DeviceCtx& dc = ctx->devs[k];
-    dc.worker->post([&, k] {
-      {
-        std::lock_guard<std::mutex> lk(*ctx->devs[k].mu);
-        HostOffScope hs(ctx->devs[k]);
-        rcs[k] = fn(ctx->devs[k], shards[k]);
-        const int rd = stage_drain(ctx, ctx->devs[k]);
-        if (!rcs[k]) rcs[k] = rd;
-      }
-      std::lock_guard<std::mutex> lk(m);
-      if (--pending == 0) cv.notify_one();
-    });
-  }
-  {
+    if (!rcs[0]) rcs[0] = rd;
+  } else {
+    std::mutex m;
+    std::condition_variable cv;
+    size_t pending = shards.size();
+    for (size_t k = 0; k < shards.size(); k++) {
+      DeviceCtx& dc = ctx->devs[k];
+      dc.worker->post([&, k] {
+        {
+          std::lock_guard<std::mutex> lk(*ctx->devs[k].mu);
+          HostOffScope hs(ctx->devs[k]);
+          rcs[k] = fn(ctx->devs[k], shards[k], &bad[k]);
+          const int rd = stage_drain(ctx, ctx->devs[k]);
+          if (!rcs[k]) rcs[k] = rd;
+        }
+        std::lock_guard<std::mutex> lk(m);
+        if (--pending == 0) cv.notify_one();
+      });
+    }
     std::unique_lock<std::mutex> lk(m);
     cv.wait(lk, [&] { return pending == 0; });
   }
   for (int rc : rcs)
     if (rc) return rc;
+  for (int b : bad)
+    if (b) return CAPY_ERR_BAD_POINT;
+  return CAPY_OK;
+}
+
+// Runs body(stream, chunk, d_flag) for the chunks of one device's shard, rotating over the device's internal streams, then
+// waits for the streams it used.  body enqueues the copies in, the pipeline and the copies out of its chunk and does not
+// wait, so the copies of one chunk run under the kernels of its neighbours.  With bad_flag_out, every stream's kFlag is
+// zeroed first and passed as d_flag (else nullptr), and *bad_flag_out gets the OR of what the chunks left there.
+template <class F>
+inline int run_chunks(capy_ctx* ctx, DeviceCtx& dc, const std::vector<Range>& chunks, int* bad_flag_out, F&& body) {
+  const int used = (int)std::min<size_t>(chunks.size(), kNumStreams);
+  int* d_flags[kNumStreams] = {};
+  if (bad_flag_out)
+    for (int s = 0; s < used; s++) {
+      d_flags[s] = (int*)scratch_get(dc, dc.streams[s], kFlag, sizeof(int));
+      if (!d_flags[s]) return CAPY_ERR_OOM;
+      CAPY_CUDA(ctx, cudaMemsetAsync(d_flags[s], 0, sizeof(int), dc.streams[s]));
+    }
+  for (size_t c = 0; c < chunks.size(); c++) {
+    const int s = (int)(c % kNumStreams);
+    const int rc = body(dc.streams[s], chunks[c], d_flags[s]);
+    if (rc) return rc;
+  }
+  int h_flags[kNumStreams] = {};
+  for (int s = 0; s < used; s++) {
+    if (bad_flag_out) CAPY_CUDA(ctx, cudaMemcpyAsync(&h_flags[s], d_flags[s], sizeof(int), cudaMemcpyDeviceToHost, dc.streams[s]));
+    CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
+  }
+  if (bad_flag_out)
+    for (int s = 0; s < used; s++) *bad_flag_out |= h_flags[s];
+  return CAPY_OK;
+}
+
+// one host input of `bytes` bytes copied into scratch `slot` (16 bytes of slack)
+inline int h2d(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, const void* src, size_t bytes, uint8_t** out) {
+  uint8_t* d = (uint8_t*)scratch_get(dc, st, slot, bytes + 16);
+  if (!d) return CAPY_ERR_OOM;
+  if (bytes) {
+    const int rc = copy_in(ctx, dc, st, slot, d, src, bytes);
+    if (rc) return rc;
+  }
+  *out = d;
   return CAPY_OK;
 }
 
@@ -177,12 +221,12 @@ struct StagedPacked {
   const uint64_t* d_off = nullptr;  // device copy of off[i0 .. i1]
 };
 
-inline int stage_packed(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot_data, int slot_off, const uint8_t* data,
+inline int stage_packed(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot_data, Slot slot_off, const uint8_t* data,
                         const uint64_t* off, uint64_t i0, uint64_t i1, StagedPacked* out) {
   const uint64_t a0 = off[i0] & ~(uint64_t)15, a1 = off[i1];
   const size_t nbytes = (size_t)(a1 - a0);
-  uint8_t* d_data = (uint8_t*)scratch_get(dc, slot_data, nbytes + 16);
-  uint64_t* d_off = (uint64_t*)scratch_get(dc, slot_off, (size_t)(i1 - i0 + 1) * 8);
+  uint8_t* d_data = (uint8_t*)scratch_get(dc, st, slot_data, nbytes + 16);
+  uint64_t* d_off = (uint64_t*)scratch_get(dc, st, slot_off, (size_t)(i1 - i0 + 1) * 8);
   if (!d_data || !d_off) return CAPY_ERR_OOM;
   if (nbytes) {
     const int rc = copy_in(ctx, dc, st, slot_data, d_data, data + a0, nbytes);

@@ -19,10 +19,26 @@
 namespace capy {
 
 constexpr int kNumStreams = 3;
-constexpr int kNumScratch = 152;  // 0..23 sponge entry points, 24..55 Ed448 pipelines, 56..79 AE pipelines, 80..143 Ed448 slots of streams 1, 2,
-                                  // 144..151 chain hand-off (states, tickets) of the sponge entry points
 
-// grow-only device scratch slots; each API call uses a fixed set of slot ids
+// Device scratch slots.  Every internal stream has its own set of them (DeviceCtx::scratch[set][slot]): the chunks of a
+// host call run on the three streams at once, and scratch_get picks the set from the stream, so two streams never share
+// a buffer.  A caller's stream (the _dev entry points) uses set 0.
+enum Slot {
+  // device buffers of the inputs and outputs of a host entry point, in the order it stages them.  Shared by all host
+  // entry points: one host call holds a device at a time, waits for its streams and drains its staging before it returns,
+  // and no device pipeline uses these slots.
+  kHost0, kHost1, kHost2, kHost3, kHost4, kHost5, kHost6, kHost7,
+  kFlag,                    // "bad point" flag of run_chunks (hostbatch.h)
+  kPlanHist, kPlanOrder,    // plan_ragged: length histogram (+ summary), work order
+  kChainStates, kChainSync,  // chain hand-off of launch_sponge_chain / launch_chain_jobs: states, tickets
+  // Ed448 pipelines (ed448_api.cu)
+  kEdKWords, kEdSWords, kEdProj, kEdProj2, kEdBad, kEdTmp56A, kEdTmp56B, kEdTmp56C,
+  // AE pipelines (ae_api.cu)
+  kAeKeys, kAeKeyOff, kAeKeyMat, kAeTNew, kAeWx, kAeProj, kAeBad, kAeKw, kAeSk,
+  kSlotsPerStream
+};
+
+// grow-only device scratch
 struct Scratch {
   void* p = nullptr;
   size_t cap = 0;
@@ -120,7 +136,8 @@ struct DeviceCtx {
   int dev = 0;
   int index = 0;  // position in capy_ctx::devs
   cudaStream_t streams[kNumStreams] = {};
-  Scratch scratch[kNumScratch];
+  Scratch scratch[kNumStreams][kSlotsPerStream];
+  Scratch vb_slabs;  // per-SM table slabs of var_base_kernel: shared by all streams (an SM runs one var_base block at a time)
   std::map<std::string, PrefixState> prefix_cache;
   std::vector<PlanEntry> plans;
   // host copies of the offsets arrays a host entry point has staged into device scratch (stage_packed), keyed by the
@@ -140,7 +157,7 @@ struct DeviceCtx {
   std::unique_ptr<std::mutex> mu{new std::mutex()};
   std::unique_ptr<DeviceWorker> worker;  // only in a multi-device ctx
   // staging of pageable host buffers, one double buffer per scratch slot that needs it (created at first use)
-  std::vector<StageSlot> stage{(size_t)kNumScratch};
+  StageSlot stage[kNumStreams][kSlotsPerStream];
   std::unique_ptr<CopyPool> copy_pool;
 };
 
@@ -173,12 +190,40 @@ int cuda_fail(capy_ctx* ctx, cudaError_t e, const char* what);
     if (_e != cudaSuccess) return ::capy::cuda_fail((ctx), _e, #expr);   \
   } while (0)
 
-// returns nullptr on OOM
-void* scratch_get(DeviceCtx& dc, int slot, size_t bytes);
+inline bool dev_index_ok(const capy_ctx* ctx, int dev_index) {
+  return ctx && dev_index >= 0 && dev_index < (int)ctx->devs.size();
+}
+// The _dev entry points: checks ctx and dev_index, then holds the device's lock (host-side state of this device: scratch
+// slots, caches, tables) and makes it current; defines `dc` and `st` (the caller's stream).
+#define CAPY_DEV_PROLOGUE                                                                    \
+  if (!dev_index_ok(ctx, dev_index)) return CAPY_ERR_BAD_ARG;                                \
+  DeviceCtx& dc = ctx->devs[dev_index];                                                      \
+  std::lock_guard<std::mutex> lk(*dc.mu);                                                    \
+  DeviceGuard g(dc.dev);                                                                     \
+  cudaStream_t st = (cudaStream_t)stream;
+
+// k when st is the device's internal stream k; 0 for any other stream (a caller's stream)
+inline int stream_set(const DeviceCtx& dc, cudaStream_t st) {
+  for (int k = 1; k < kNumStreams; k++)
+    if (dc.streams[k] == st) return k;
+  return 0;
+}
+
+// grows `s` to at least `bytes`; returns nullptr on OOM
+void* scratch_grow(Scratch& s, size_t bytes);
+// the buffer of `slot` in the slot set of stream st; returns nullptr on OOM
+inline void* scratch_get(DeviceCtx& dc, cudaStream_t st, Slot slot, size_t bytes) {
+  return scratch_grow(dc.scratch[stream_set(dc, st)][slot], bytes);
+}
+#define CAPY_SCRATCH(var, type, slot, bytes)                    \
+  type* var = (type*)scratch_get(dc, st, (slot), (bytes));      \
+  if (!var) return CAPY_ERR_OOM;
+
+inline unsigned grid_for(uint64_t n, unsigned block) { return (unsigned)((n + block - 1) / block); }
 
 // host <-> device copies of the host entry points (hostbatch.h); `slot` = the scratch slot of the device buffer
-int copy_in(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* d_dst, const void* h_src, size_t bytes);
-int copy_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int slot, void* h_dst, const void* d_src, size_t bytes);
+int copy_in(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, void* d_dst, const void* h_src, size_t bytes);
+int copy_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, void* h_dst, const void* d_src, size_t bytes);
 // waits for the staged device-to-host copies of this device and hands their bytes to the caller's buffers
 int stage_drain(capy_ctx* ctx, DeviceCtx& dc);
 void stage_free(DeviceCtx& dc);

@@ -151,8 +151,6 @@ __global__ void prefix_state_kernel(const uint8_t* prefix, uint32_t nblocks, uin
   for (int k = 0; k < 25; k++) state[k] = ((uint64_t)a[k].hi << 32) | a[k].lo;
 }
 
-static inline unsigned grid_for(uint64_t n, unsigned block) { return (unsigned)((n + block - 1) / block); }
-
 // ------------------------------------------------------------------------------------------------
 // Mixed-length batches (BASELINE config 5): longest-processing-time-first order.
 // A sponge is sequential per message, so with one thread per message the job cannot finish before
@@ -384,10 +382,7 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
         return CAPY_OK;
       }
   }
-  int si = 0;  // scratch pair per internal stream (chunks on different streams overlap); callers' streams use pair 0
-  for (int k = 0; k < kNumStreams; k++)
-    if (dc.streams[k] == st) si = k;
-  uint32_t* hist = (uint32_t*)scratch_get(dc, 18 + 2 * si, (size_t)kLenBins * 4 + 64);
+  uint32_t* hist = (uint32_t*)scratch_get(dc, st, kPlanHist, (size_t)kLenBins * 4 + 64);
   uint32_t* order = nullptr;
   uint32_t* owned = nullptr;
   if (cached) {
@@ -397,7 +392,7 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
     }
     order = owned;
   } else {
-    order = (uint32_t*)scratch_get(dc, 19 + 2 * si, (size_t)n * 4);
+    order = (uint32_t*)scratch_get(dc, st, kPlanOrder, (size_t)n * 4);
   }
   if (!hist || !order) {
     if (owned) cudaFree(owned);
@@ -789,17 +784,11 @@ static int launch_chain_t(capy_ctx* ctx, cudaStream_t stream, const SpongeChain&
   return CAPY_OK;
 }
 
-static int chain_stream_index(const DeviceCtx& dc, cudaStream_t stream) {
-  for (int k = 1; k < kNumStreams; k++)
-    if (dc.streams[k] == stream) return k;
-  return 0;
-}
-
 // two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel)
 static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J0, const SpongeJob& J1,
                              bool data_dependent) {
   const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
-  uint32_t* sync = (uint32_t*)scratch_get(dc, 145 + 2 * chain_stream_index(dc, stream), ((size_t)nb + 1) * sizeof(uint32_t));
+  uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
   if (!sync) return CAPY_ERR_OOM;
   CAPY_CUDA(ctx, cudaMemsetAsync(sync, 0, ((size_t)nb + 1) * sizeof(uint32_t), stream));
   SpongeChain C;
@@ -821,7 +810,7 @@ static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, 
 
 // J (uniform batch, no order) as two dependent jobs cut after `cut` absorbed blocks
 static int launch_sponge_chain(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J, uint64_t cut) {
-  uint64_t* states = (uint64_t*)scratch_get(dc, 144 + 2 * chain_stream_index(dc, stream), (size_t)J.n * 25 * sizeof(uint64_t));
+  uint64_t* states = (uint64_t*)scratch_get(dc, stream, kChainStates, (size_t)J.n * 25 * sizeof(uint64_t));
   if (!states) return CAPY_ERR_OOM;
   SpongeJob J0 = J, J1 = J;
   J0.chain_out = states;
@@ -1057,21 +1046,16 @@ int capy_lpt_shares(const uint64_t* off, uint64_t n, uint32_t parts, uint32_t un
 // =================================================================================================
 int capy_sha3_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const uint8_t* d_data,
                         const uint64_t* d_off, uint64_t n, uint8_t* d_digests, uint32_t flags) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() || (n && (!d_data || !d_off || !d_digests)))
-    return CAPY_ERR_BAD_ARG;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceGuard g(ctx->devs[dev_index].dev);
-  return launch_sha3(ctx, ctx->devs[dev_index], (cudaStream_t)stream, d_bits, d_data, d_off, 0, 0, n, d_digests, flags);
+  if (n && (!d_data || !d_off || !d_digests)) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
+  return launch_sha3(ctx, dc, st, d_bits, d_data, d_off, 0, 0, n, d_digests, flags);
 }
 
 int capy_sha3_batch_fixed_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const uint8_t* d_data,
                               uint64_t msg_len, uint64_t stride, uint64_t n, uint8_t* d_digests, uint32_t) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() || (n && (!d_data || !d_digests)) || stride < msg_len)
-    return CAPY_ERR_BAD_ARG;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceGuard g(ctx->devs[dev_index].dev);
-  return launch_sha3(ctx, ctx->devs[dev_index], (cudaStream_t)stream, d_bits, d_data, nullptr, msg_len, stride, n, d_digests, 0,
-                     /*tail_readable=*/false);
+  if ((n && (!d_data || !d_digests)) || stride < msg_len) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
+  return launch_sha3(ctx, dc, st, d_bits, d_data, nullptr, msg_len, stride, n, d_digests, 0, /*tail_readable=*/false);
 }
 
 int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64_t* off, uint64_t n, uint8_t* digests,
@@ -1091,20 +1075,20 @@ int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64
     if (scattered) {
       std::vector<Range> slots;
       for (size_t k = 0; k < shares.size(); k++) slots.push_back({k, k + 1});  // for_each_device: one closure per device
-      return for_each_device(ctx, slots, [&](DeviceCtx& dc, Range slot) -> int {
+      return for_each_device(ctx, slots, [&](DeviceCtx& dc, Range slot, int*) -> int {
         const DeviceShare& sh = shares[slot.i0];
         if (sh.items == 0) return CAPY_OK;
         cudaStream_t st = dc.streams[0];
-        uint8_t* d_data = (uint8_t*)scratch_get(dc, 0, (size_t)sh.bytes + 16);
-        uint64_t* d_off = (uint64_t*)scratch_get(dc, 1, (size_t)(sh.items + 1) * 8);
-        uint8_t* d_out = (uint8_t*)scratch_get(dc, 2, (size_t)sh.items * ob);
+        uint8_t* d_data = (uint8_t*)scratch_get(dc, st, kHost0, (size_t)sh.bytes + 16);
+        uint64_t* d_off = (uint64_t*)scratch_get(dc, st, kHost1, (size_t)(sh.items + 1) * 8);
+        uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)sh.items * ob);
         if (!d_data || !d_off || !d_out) return CAPY_ERR_OOM;
         std::vector<uint64_t> loc(sh.items + 1);  // offsets of this device's items in its own packed buffer
         uint64_t at = 0, j = 0;
         for (const Run& r : sh.runs) {  // one copy per run of consecutive messages
           const uint64_t b0 = off[r.i0], b1 = off[r.i1];
           if (b1 > b0) {
-            const int rc = copy_in(ctx, dc, st, 0, d_data + at, data + b0, (size_t)(b1 - b0));
+            const int rc = copy_in(ctx, dc, st, kHost0, d_data + at, data + b0, (size_t)(b1 - b0));
             if (rc) return rc;
           }
           for (uint64_t i = r.i0; i < r.i1; i++) loc[j++] = at + (off[i] - b0);
@@ -1117,7 +1101,7 @@ int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64
         if (rc) return rc;
         j = 0;
         for (const Run& r : sh.runs) {  // the digests of a run are consecutive on both sides
-          rc = copy_out(ctx, dc, st, 2, digests + r.i0 * ob, d_out + j * ob, (size_t)(r.i1 - r.i0) * ob);
+          rc = copy_out(ctx, dc, st, kHost2, digests + r.i0 * ob, d_out + j * ob, (size_t)(r.i1 - r.i0) * ob);
           if (rc) return rc;
           j += r.i1 - r.i0;
         }
@@ -1127,26 +1111,19 @@ int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64
     }
   }
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 200);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
     // long messages: few big chunks, so that the longest-first schedule sees enough work beside them
-    const size_t nchunks = ragged_chunk_count(off, sh.i0, sh.i1, 0);
-    auto chunks = split_items(off, 0, sh.i0, sh.i1, nchunks, 200);
-    for (size_t c = 0; c < chunks.size(); c++) {
-      const int s = (int)(c % kNumStreams);
-      cudaStream_t st = dc.streams[s];
-      const Range ch = chunks[c];
+    auto chunks = split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, 0), 200);
+    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, 3 * s, 3 * s + 1, data, off, ch.i0, ch.i1, &sp);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sp);
       if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, 3 * s + 2, (size_t)(ch.i1 - ch.i0) * ob);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)(ch.i1 - ch.i0) * ob);
       if (!d_out) return CAPY_ERR_OOM;
       rc = launch_sha3(ctx, dc, st, d_bits, sp.d_base, sp.d_off, 0, 0, ch.i1 - ch.i0, d_out, flags);
       if (rc) return rc;
-      rc = copy_out(ctx, dc, st, 3 * s + 2, digests + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
-      if (rc) return rc;
-    }
-    for (int s = 0; s < kNumStreams; s++) CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
-    return CAPY_OK;
+      return copy_out(ctx, dc, st, kHost2, digests + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
+    });
   });
 }
 
@@ -1159,27 +1136,21 @@ int capy_sha3_batch_fixed(capy_ctx* ctx, int d_bits, const uint8_t* data, uint64
   // the uniform kernel wants 8-byte aligned rows; the copy lands on a 256-byte aligned buffer, so
   // only the stride matters
   auto shards = split_items(nullptr, stride, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
     auto chunks = split_items(nullptr, stride, sh.i0, sh.i1, chunk_count((sh.i1 - sh.i0) * stride, sh.i1 - sh.i0), 0);
-    for (size_t c = 0; c < chunks.size(); c++) {
-      const int s = (int)(c % kNumStreams);
-      cudaStream_t st = dc.streams[s];
-      const Range ch = chunks[c];
+    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       // last row may be shorter than the stride in the caller's buffer
       const size_t in_bytes = (size_t)((cnt - 1) * stride + msg_len);
-      uint8_t* d_in = (uint8_t*)scratch_get(dc, 3 * s, in_bytes + 16);
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, 3 * s + 2, (size_t)cnt * ob);
+      uint8_t* d_in = (uint8_t*)scratch_get(dc, st, kHost0, in_bytes + 16);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)cnt * ob);
       if (!d_in || !d_out) return CAPY_ERR_OOM;
-      int rc = copy_in(ctx, dc, st, 3 * s, d_in, data + ch.i0 * stride, in_bytes);
+      int rc = copy_in(ctx, dc, st, kHost0, d_in, data + ch.i0 * stride, in_bytes);
       if (rc) return rc;
       rc = launch_sha3(ctx, dc, st, d_bits, d_in, nullptr, msg_len, stride, cnt, d_out);
       if (rc) return rc;
-      rc = copy_out(ctx, dc, st, 3 * s + 2, digests + ch.i0 * ob, d_out, (size_t)cnt * ob);
-      if (rc) return rc;
-    }
-    for (int s = 0; s < kNumStreams; s++) CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
-    return CAPY_OK;
+      return copy_out(ctx, dc, st, kHost2, digests + ch.i0 * ob, d_out, (size_t)cnt * ob);
+    });
   });
 }
 
@@ -1189,14 +1160,9 @@ int capy_sha3_batch_fixed(capy_ctx* ctx, int d_bits, const uint8_t* data, uint64
 int capy_cshake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const uint8_t* d_data,
                           const uint64_t* d_off, uint64_t n, const uint8_t* fn_name, uint32_t fn_len,
                           const uint8_t* custom, uint32_t custom_len, uint64_t out_bits, uint8_t* d_out) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() || (n && (!d_data || !d_off || !d_out)) ||
-      (fn_len && !fn_name) || (custom_len && !custom))
-    return CAPY_ERR_BAD_ARG;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceCtx& dc = ctx->devs[dev_index];
-  DeviceGuard g(dc.dev);
-  return launch_cshake(ctx, dc, (cudaStream_t)stream, d_bits, d_data, d_off, n, fn_name, fn_len, custom, custom_len,
-                       out_bits, d_out);
+  if ((n && (!d_data || !d_off || !d_out)) || (fn_len && !fn_name) || (custom_len && !custom)) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
+  return launch_cshake(ctx, dc, st, d_bits, d_data, d_off, n, fn_name, fn_len, custom, custom_len, out_bits, d_out);
 }
 
 int capy_cshake_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64_t* off, uint64_t n,
@@ -1207,26 +1173,20 @@ int capy_cshake_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint
   const size_t ob = (size_t)(out_bits / 8);
   if (n == 0 || ob == 0) return CAPY_OK;
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 200 + ob);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
     auto chunks = split_items(off, 0, sh.i0, sh.i1,
                               ragged_chunk_count(off, sh.i0, sh.i1, (sh.i1 - sh.i0) * ob), 200 + ob);
-    for (size_t c = 0; c < chunks.size(); c++) {
-      const int s = (int)(c % kNumStreams);
-      cudaStream_t st = dc.streams[s];
-      const Range ch = chunks[c];
+    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, 3 * s, 3 * s + 1, data, off, ch.i0, ch.i1, &sp);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sp);
       if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, 3 * s + 2, (size_t)(ch.i1 - ch.i0) * ob);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)(ch.i1 - ch.i0) * ob);
       if (!d_out) return CAPY_ERR_OOM;
       rc = launch_cshake(ctx, dc, st, d_bits, sp.d_base, sp.d_off, ch.i1 - ch.i0, fn_name, fn_len, custom, custom_len,
                          out_bits, d_out);
       if (rc) return rc;
-      rc = copy_out(ctx, dc, st, 3 * s + 2, out + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
-      if (rc) return rc;
-    }
-    for (int s = 0; s < kNumStreams; s++) CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
-    return CAPY_OK;
+      return copy_out(ctx, dc, st, kHost2, out + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
+    });
   });
 }
 
@@ -1237,12 +1197,8 @@ int capy_kmac_xof_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bi
                             const uint64_t* d_key_off, const uint8_t* d_data, const uint64_t* d_off, uint64_t n,
                             const uint8_t* custom, uint32_t custom_len, uint64_t out_bits, const uint64_t* d_out_off,
                             uint8_t* d_out) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() ||
-      (n && (!d_keys || !d_key_off || !d_data || !d_off || !d_out)) || (custom_len && !custom))
-    return CAPY_ERR_BAD_ARG;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceCtx& dc = ctx->devs[dev_index];
-  DeviceGuard g(dc.dev);
+  if ((n && (!d_keys || !d_key_off || !d_data || !d_off || !d_out)) || (custom_len && !custom)) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
   KmacDevArgs a{};
   a.d_bits = d_bits;
   a.keys = d_keys;
@@ -1255,19 +1211,17 @@ int capy_kmac_xof_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bi
   a.out_bytes = a.out_stride = out_bits / 8;
   a.out_off = d_out_off;
   a.out = d_out;
-  return launch_kmac_xof(ctx, dc, (cudaStream_t)stream, a);
+  return launch_kmac_xof(ctx, dc, st, a);
 }
 
 int capy_kmac_xof_batch_fixed_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const uint8_t* d_keys,
                                   uint64_t key_len, uint64_t key_stride, const uint8_t* d_data, uint64_t msg_len,
                                   uint64_t msg_stride, uint64_t n, const uint8_t* custom, uint32_t custom_len,
                                   uint64_t out_bits, uint8_t* d_out) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() || (n && (!d_keys || !d_out)) ||
-      (n && msg_len && !d_data) || (custom_len && !custom) || key_stride < key_len || msg_stride < msg_len)
+  if ((n && (!d_keys || !d_out)) || (n && msg_len && !d_data) || (custom_len && !custom) || key_stride < key_len ||
+      msg_stride < msg_len)
     return CAPY_ERR_BAD_ARG;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceCtx& dc = ctx->devs[dev_index];
-  DeviceGuard g(dc.dev);
+  CAPY_DEV_PROLOGUE
   KmacDevArgs a{};
   a.d_bits = d_bits;
   a.keys = d_keys;
@@ -1281,7 +1235,7 @@ int capy_kmac_xof_batch_fixed_dev(capy_ctx* ctx, int dev_index, void* stream, in
   a.custom_len = custom_len;
   a.out_bytes = a.out_stride = out_bits / 8;
   a.out = d_out;
-  return launch_kmac_xof(ctx, dc, (cudaStream_t)stream, a);
+  return launch_kmac_xof(ctx, dc, st, a);
 }
 
 int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const uint64_t* key_off, const uint8_t* data,
@@ -1293,27 +1247,23 @@ int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const ui
   if (n == 0 || (!out_off && ob == 0)) return CAPY_OK;
   auto out_begin = [&](uint64_t i) -> uint64_t { return out_off ? out_off[i] : i * ob; };
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 400 + ob);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh) -> int {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
     const uint64_t tot = off[sh.i1] - off[sh.i0] + (out_begin(sh.i1) - out_begin(sh.i0));
     auto chunks = split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, tot - (off[sh.i1] - off[sh.i0])), 400 + ob);
-    // 5 scratch slots per stream: data, off, keys, key_off, out (+ out_off)
-    for (size_t c = 0; c < chunks.size(); c++) {
-      const int s = (int)(c % kNumStreams);
-      cudaStream_t st = dc.streams[s];
-      const Range ch = chunks[c];
+    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
       const uint64_t cnt = ch.i1 - ch.i0;
       StagedPacked sx, sk;
-      int rc = stage_packed(ctx, dc, st, 6 * s, 6 * s + 1, data, off, ch.i0, ch.i1, &sx);
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sx);
       if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, 6 * s + 2, 6 * s + 3, keys, key_off, ch.i0, ch.i1, &sk);
+      rc = stage_packed(ctx, dc, st, kHost2, kHost3, keys, key_off, ch.i0, ch.i1, &sk);
       if (rc) return rc;
       const uint64_t ob0 = out_begin(ch.i0), ob1 = out_begin(ch.i1);
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, 6 * s + 4, (size_t)(ob1 - ob0) + 16);
+      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost4, (size_t)(ob1 - ob0) + 16);
       if (!d_out) return CAPY_ERR_OOM;
       const uint64_t* d_out_off = nullptr;
       uint8_t* d_out_base = d_out;
       if (out_off) {
-        uint64_t* p = (uint64_t*)scratch_get(dc, 6 * s + 5, (size_t)(cnt + 1) * 8);
+        uint64_t* p = (uint64_t*)scratch_get(dc, st, kHost5, (size_t)(cnt + 1) * 8);
         if (!p) return CAPY_ERR_OOM;
         CAPY_CUDA(ctx, cudaMemcpyAsync(p, out_off + ch.i0, (size_t)(cnt + 1) * 8, cudaMemcpyHostToDevice, st));
         d_out_off = p;
@@ -1333,13 +1283,9 @@ int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const ui
       a.out = d_out_base;
       rc = launch_kmac_xof(ctx, dc, st, a);
       if (rc) return rc;
-      if (ob1 > ob0) {
-        rc = copy_out(ctx, dc, st, 6 * s + 4, out + ob0, d_out, (size_t)(ob1 - ob0));
-        if (rc) return rc;
-      }
-    }
-    for (int s = 0; s < kNumStreams; s++) CAPY_CUDA(ctx, cudaStreamSynchronize(dc.streams[s]));
-    return CAPY_OK;
+      if (ob1 > ob0) return copy_out(ctx, dc, st, kHost4, out + ob0, d_out, (size_t)(ob1 - ob0));
+      return CAPY_OK;
+    });
   });
 }
 
@@ -1348,12 +1294,10 @@ int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const ui
 // =================================================================================================
 int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int shake_bits, const uint8_t* d_data,
                               const uint64_t* d_off, uint64_t n, uint64_t out_bytes, uint8_t* d_out) {
-  if (!ctx || dev_index < 0 || dev_index >= (int)ctx->devs.size() || (n && (!d_data || !d_off || !d_out)) ||
-      (shake_bits != 128 && shake_bits != 256))
+  if (!dev_index_ok(ctx, dev_index) || (n && (!d_data || !d_off || !d_out)) || (shake_bits != 128 && shake_bits != 256))
     return CAPY_ERR_BAD_ARG;
   if (n == 0 || out_bytes == 0) return CAPY_OK;
-  std::lock_guard<std::mutex> lk(*ctx->devs[dev_index].mu);  // host-side state of this device (scratch slots, caches)
-  DeviceGuard g(ctx->devs[dev_index].dev);
+  CAPY_DEV_PROLOGUE
   SpongeJob J = empty_job();
   J.data = d_data;
   J.off = d_off;
@@ -1365,9 +1309,8 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
   J.out = d_out;
   J.out_stride = J.out_bytes = out_bytes;
   J.n = n;
-  DeviceCtx& dc = ctx->devs[dev_index];
   LaunchPlan plan;  // longest first, tiers for chain-bound batches, chains of a uniform batch cut in two: as for cSHAKE
-  int rc = plan_ragged(ctx, dc, (cudaStream_t)stream, d_off, n, J.rate, &plan);
+  int rc = plan_ragged(ctx, dc, st, d_off, n, J.rate, &plan);
   if (rc) return rc;
   J.order = plan.order;
   const int lanes = (int)J.rate / 8;
@@ -1375,9 +1318,9 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
     const uint64_t sq = 8ull * J.sq_lanes;
     uint64_t cut;
     if (chain_cut(dc.sm_count, n, plan.uniform_blocks, (out_bytes + sq - 1) / sq - 1, &cut))
-      return launch_sponge_chain(ctx, dc, (cudaStream_t)stream, lanes, J, cut);
+      return launch_sponge_chain(ctx, dc, st, lanes, J, cut);
   }
-  return launch_sponge(ctx, dc, (cudaStream_t)stream, lanes, J, plan);
+  return launch_sponge(ctx, dc, st, lanes, J, plan);
 }
 
 }  // extern "C"

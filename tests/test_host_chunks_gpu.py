@@ -1,7 +1,8 @@
 """GPU: the host-buffer Ed448 entry points cut a device's shard into chunks that run on the device's three streams at
-once, every stream with its own scratch slots (csrc/ed448_api.cu: ed_host_chunks, ed_slot).  Batches large enough to be
-chunked (>= 2^19 items) must give the bytes of the single-stream device-pointer pipelines -- which the other tests pin to
-the oracle -- and the oracle's on a seeded sample; a bad point in a late chunk must still be reported.
+once, every stream with its own scratch slots (csrc/hostbatch.h: run_chunks; csrc/internal.h: scratch_get).  Batches
+large enough to be chunked (>= 2^19 items) must give the bytes of the single-stream device-pointer pipelines -- which
+the other tests pin to the oracle -- and the oracle's on a seeded sample; a bad point in a late chunk must still be
+reported.
 
 Matches KeyPair::new (ecc/keypair.rs:41-51), sign / verify (ecc/signable.rs:40-86), the ECDH core of key_encrypt
 (ecc/encryptable.rs:36-38)."""
