@@ -29,7 +29,7 @@ enum Slot {
   // and no device pipeline uses these slots.
   kHost0, kHost1, kHost2, kHost3, kHost4, kHost5, kHost6, kHost7,
   kFlag,                    // "bad point" flag of run_chunks (hostbatch.h)
-  kPlanHist, kPlanOrder,    // plan_ragged: length histogram (+ summary), work order
+  kPlanHist, kPlanOrder,    // plan_ragged: device length histogram (+ summary), work order
   kChainStates, kChainSync,  // chain hand-off of launch_sponge_chain / launch_chain_jobs: states, tickets
   // Ed448 pipelines (ed448_api.cu)
   kEdKWords, kEdSWords, kEdProj, kEdProj2, kEdBad, kEdTmp56A, kEdTmp56B, kEdTmp56C,
@@ -53,13 +53,17 @@ struct PrefixState {
 };
 constexpr size_t kMaxPrefixEntries = 64;
 
-// How a ragged batch is launched (sha3_api.cu: plan_ragged).  `order` = work order (longest first) or nullptr.
+// How a ragged batch is launched (sha3_api.cu: plan_ragged builds it, run_sponge follows it).  `order` = work order
+// (longest first) or nullptr.
 struct LaunchPlan {
   const uint32_t* order = nullptr;
   int warps_per_smsp = 0;   // 0 = unthrottled
   uint64_t warp_items[3] = {0, 0, 0};  // one warp per item: [c - 1] of them run c chains per scheduler (ranks in this order)
   uint64_t pair_items = 0;             // the next ranks: two threads per item
-  uint64_t uniform_blocks = 0;         // != 0: every item holds this many whole blocks (+ a partial one): nothing to order
+  uint64_t uniform_blocks = 0;         // != 0: every item holds this many whole blocks (+ a partial one): nothing to order,
+                                       // and run_sponge may cut the chains
+  // chain-bound batch: one launch of the warp, pair and thread tiers (sponge_tiered_kernel)
+  bool tiered() const { return warp_items[0] || warp_items[1] || warp_items[2] || pair_items; }
 };
 
 // Cached plan of a ragged batch, keyed by the caller's offsets array (capy_gpu_set_plan_cache): a repeated call with the

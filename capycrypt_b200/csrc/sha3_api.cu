@@ -7,8 +7,9 @@
 #include <algorithm>
 #include <cmath>
 #include <cstdlib>
-#include <cstring>
+#include <memory>
 #include <thread>
+#include <type_traits>
 #include <vector>
 
 #include "internal.h"
@@ -329,7 +330,113 @@ static void plan_tiers(const std::vector<uint32_t>& cum, uint64_t n, uint32_t ma
   }
 }
 
-void plan_cache_clear(DeviceCtx& dc);  // ctx.cu
+// ---- small helpers of the launchers --------------------------------------------------------------------------------
+// Calls f(std::integral_constant<int, L>()) for the L of Ls that equals `lanes` (a lane count known at run time picks the
+// kernel instantiation) and returns its result; an unlisted value is CAPY_ERR_BAD_ARG.
+template <int... Ls, class F>
+static int with_lanes(int lanes, F&& f) {
+  int rc = CAPY_ERR_BAD_ARG;
+  (void)((lanes == Ls && ((rc = f(std::integral_constant<int, Ls>())), true)) || ...);
+  return rc;
+}
+
+// a device buffer that is freed when it goes out of scope, unless release() hands it to a cache entry
+struct CudaFree {
+  void operator()(void* p) const { cudaFree(p); }
+};
+template <class T>
+using DevPtr = std::unique_ptr<T, CudaFree>;
+template <class T>
+static cudaError_t dev_alloc(DevPtr<T>& p, size_t bytes) {
+  T* q = nullptr;
+  const cudaError_t e = cudaMalloc(&q, bytes);
+  if (e == cudaSuccess) p.reset(q);
+  return e;
+}
+
+// ---- plan of a ragged batch ----------------------------------------------------------------------------------------
+// Length histogram of a batch in whole blocks of `stride_bytes` (bin kLenBins - 1 holds every longer item)
+struct LenHist {
+  uint64_t total_blocks = 0;  // sum of (bin + 1) over the items
+  uint32_t max_bin = 0;       // largest non-empty bin
+  uint32_t bins = 0;          // number of non-empty bins
+  std::vector<uint32_t> cnt;  // items per bin when the histogram was taken on the host, else empty
+};
+
+// the histogram of a registered host offsets array
+static void host_len_hist(const uint64_t* h_off, uint64_t n, uint32_t stride_bytes, LenHist* h) {
+  h->cnt.assign(kLenBins, 0);
+  const double inv = 1.0 / (double)stride_bytes;
+  for (uint64_t i = 0; i < n; i++) {
+    const uint64_t len = h_off[i + 1] - h_off[i];
+    uint64_t q = (uint64_t)((double)len * inv);  // len / stride_bytes without a 64-bit division per item
+    if (q * stride_bytes > len) q--;
+    else if ((q + 1) * stride_bytes <= len) q++;
+    const uint32_t b = q < kLenBins - 1 ? (uint32_t)q : kLenBins - 1;
+    if (h->cnt[b]++ == 0) h->bins++;
+    if (b > h->max_bin) h->max_bin = b;
+    h->total_blocks += (uint64_t)b + 1;
+  }
+}
+
+// Enqueues the device histogram and its scan, which leaves hist[k] = number of items in bins > k (the cursors of the
+// scatter).  Without a host histogram the summary comes back to the host: a small copy and a stream synchronisation.
+static int device_len_hist(capy_ctx* ctx, cudaStream_t st, const uint64_t* d_off, uint64_t n, uint32_t stride_bytes,
+                           uint32_t* hist, LenHist* h) {
+  uint32_t* summary = hist + kLenBins;
+  CAPY_CUDA(ctx, cudaMemsetAsync(hist, 0, (size_t)kLenBins * 4 + 64, st));
+  len_hist_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, n, stride_bytes, hist);
+  len_scan_kernel<<<1, 1024, 0, st>>>(hist, summary);
+  ctx->launches += 2;
+  if (!h->cnt.empty()) return CAPY_OK;
+  uint32_t h_sum[4];
+  CAPY_CUDA(ctx, cudaMemcpyAsync(h_sum, summary, sizeof h_sum, cudaMemcpyDeviceToHost, st));
+  CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+  h->total_blocks = (uint64_t)h_sum[0] | ((uint64_t)h_sum[1] << 32);
+  h->max_bin = h_sum[2];
+  h->bins = h_sum[3];
+  return CAPY_OK;
+}
+
+// The plan a histogram gives: uniform block count, tiers of a chain-bound batch, occupancy throttle, and the scatter of
+// the items into `order`, longest first (hist = the scanned device histogram).
+static int plan_from_hist(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint64_t* d_off, uint64_t n,
+                          uint32_t stride_bytes, const LenHist& h, uint32_t* hist, uint32_t* order, bool allow_pair,
+                          int force_c, LaunchPlan* plan) {
+  const uint32_t max_blocks = h.max_bin + 1;
+  // time in units of one thread-per-state permutation on one scheduler: all work spread over every scheduler
+  // (32 states per warp, one warp per scheduler) vs the longest chain
+  const double ideal = (double)h.total_blocks / (32.0 * 4.0 * dc.sm_count);
+  // Chain-bound batch: the longest items go to the warp-per-item and the two-threads-per-item tiers
+  if (allow_pair && max_blocks > 64 && (double)max_blocks > 1.05 * ideal) {
+    std::vector<uint32_t> cum(kLenBins);  // number of items in bins > k
+    if (!h.cnt.empty()) {
+      uint32_t above = 0;
+      for (uint32_t k = kLenBins; k-- > 0;) {
+        cum[k] = above;
+        above += h.cnt[k];
+      }
+    } else {
+      CAPY_CUDA(ctx, cudaMemcpyAsync(cum.data(), hist, (size_t)kLenBins * 4, cudaMemcpyDeviceToHost, st));
+      CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+    }
+    plan_tiers(cum, n, max_blocks, (double)h.total_blocks, dc.sm_count, plan->warp_items, &plan->pair_items, force_c);
+  }
+  if (h.bins == 1) plan->uniform_blocks = max_blocks;
+  if (h.bins > 1) {  // (uniform lengths: nothing to order)
+    len_scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, n, stride_bytes, hist, order);
+    ctx->launches++;
+    CAPY_CUDA(ctx, cudaGetLastError());
+    plan->order = order;
+    plan->warps_per_smsp = 0;
+    if ((double)max_blocks * 4.0 > 0.7 * ideal) {
+      plan->warps_per_smsp = 3;
+      if ((double)max_blocks * 3.0 > 0.7 * ideal) plan->warps_per_smsp = 2;
+      if ((double)max_blocks * 2.0 > 0.7 * ideal) plan->warps_per_smsp = 1;
+    }
+  }
+  return CAPY_OK;
+}
 
 // builds the descending-length order for a ragged batch; decides the occupancy throttle and how many of the
 // longest items go to the warp-per-item and the two-threads-per-item tiers.
@@ -345,9 +452,7 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
   // The lengths are read there, so nothing comes back from the device and the chunk pipeline of the host call never
   // waits for a stream.  Uniform lengths (the bulk case: fixed-size records) need no device work at all.
   const uint64_t* h_off = host_off_find(dc, d_off, n);
-  std::vector<uint32_t> h_cnt;  // host histogram (non-uniform batches up to kHostPlanMaxItems)
-  uint64_t h_total = 0;
-  uint32_t h_max = 0, h_bins = 0;
+  LenHist h;
   if (h_off) {
     const uint64_t len0 = h_off[1] - h_off[0];
     bool uniform = true;
@@ -356,22 +461,8 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
       plan->uniform_blocks = len0 / stride_bytes + 1;
       return CAPY_OK;
     }
-    if (n > kHostPlanMaxItems) {
-      h_off = nullptr;  // a histogram of millions of items is cheaper on the device, round trip included
-    } else {
-      h_cnt.assign(kLenBins, 0);
-      const double inv = 1.0 / (double)stride_bytes;
-      for (uint64_t i = 0; i < n; i++) {
-        const uint64_t len = h_off[i + 1] - h_off[i];
-        uint64_t q = (uint64_t)((double)len * inv);  // len / stride_bytes without a 64-bit division per item
-        if (q * stride_bytes > len) q--;
-        else if ((q + 1) * stride_bytes <= len) q++;
-        const uint32_t b = q < kLenBins - 1 ? (uint32_t)q : kLenBins - 1;
-        if (h_cnt[b]++ == 0) h_bins++;
-        if (b > h_max) h_max = b;
-        h_total += (uint64_t)b + 1;
-      }
-    }
+    if (n > kHostPlanMaxItems) h_off = nullptr;  // a histogram of millions of items is cheaper on the device, round trip included
+    else host_len_hist(h_off, n, stride_bytes, &h);
   }
   const bool cached = ctx->plan_cache.load() != 0 && force_c == 0 && !h_off;
   if (cached) {
@@ -383,79 +474,19 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
       }
   }
   uint32_t* hist = (uint32_t*)scratch_get(dc, st, kPlanHist, (size_t)kLenBins * 4 + 64);
-  uint32_t* order = nullptr;
-  uint32_t* owned = nullptr;
-  if (cached) {
-    if (cudaMalloc(&owned, (size_t)n * 4) != cudaSuccess) {
-      cudaGetLastError();
-      return CAPY_ERR_OOM;
-    }
-    order = owned;
-  } else {
-    order = (uint32_t*)scratch_get(dc, st, kPlanOrder, (size_t)n * 4);
-  }
-  if (!hist || !order) {
-    if (owned) cudaFree(owned);
+  DevPtr<uint32_t> owned;  // the order of a cached plan lives as long as its cache entry
+  if (cached && dev_alloc(owned, (size_t)n * 4) != cudaSuccess) {
+    cudaGetLastError();
     return CAPY_ERR_OOM;
   }
-  auto fail = [&](cudaError_t e, const char* what) {
-    if (owned) cudaFree(owned);
-    return cuda_fail(ctx, e, what);
-  };
-#define PLAN_CUDA(expr)                                  \
-  do {                                                   \
-    cudaError_t _e = (expr);                             \
-    if (_e != cudaSuccess) return fail(_e, #expr);       \
-  } while (0)
-  uint32_t* summary = hist + kLenBins;
-  PLAN_CUDA(cudaMemsetAsync(hist, 0, (size_t)kLenBins * 4 + 64, st));
-  len_hist_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, n, stride_bytes, hist);
-  len_scan_kernel<<<1, 1024, 0, st>>>(hist, summary);
-  ctx->launches += 2;
-  uint32_t h_sum[4] = {(uint32_t)h_total, (uint32_t)(h_total >> 32), h_max, h_bins};
-  if (!h_off) {
-    PLAN_CUDA(cudaMemcpyAsync(h_sum, summary, sizeof h_sum, cudaMemcpyDeviceToHost, st));
-    PLAN_CUDA(cudaStreamSynchronize(st));
-  }
-  const uint64_t total_blocks = (uint64_t)h_sum[0] | ((uint64_t)h_sum[1] << 32);
-  const uint32_t max_blocks = h_sum[2] + 1, bins = h_sum[3];
-  // time in units of one thread-per-state permutation on one scheduler: all work spread over every scheduler
-  // (32 states per warp, one warp per scheduler) vs the longest chain
-  const double ideal = (double)total_blocks / (32.0 * 4.0 * dc.sm_count);
-  // Chain-bound batch: the longest items go to the warp-per-item and the two-threads-per-item tiers
-  if (allow_pair && max_blocks > 64 && (double)max_blocks > 1.05 * ideal) {
-    std::vector<uint32_t> cum(kLenBins);  // after the scan hist[k] = number of items in bins > k
-    if (h_off) {
-      uint32_t above = 0;
-      for (uint32_t k = kLenBins; k-- > 0;) {
-        cum[k] = above;
-        above += h_cnt[k];
-      }
-    } else {
-      PLAN_CUDA(cudaMemcpyAsync(cum.data(), hist, (size_t)kLenBins * 4, cudaMemcpyDeviceToHost, st));
-      PLAN_CUDA(cudaStreamSynchronize(st));
-    }
-    plan_tiers(cum, n, max_blocks, (double)total_blocks, dc.sm_count, plan->warp_items, &plan->pair_items, force_c);
-  }
-  if (bins == 1) plan->uniform_blocks = max_blocks;
-  if (bins > 1) {  // (uniform lengths: nothing to order)
-    len_scatter_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(d_off, n, stride_bytes, hist, order);
-    ctx->launches++;
-    PLAN_CUDA(cudaGetLastError());
-    plan->order = order;
-    plan->warps_per_smsp = 0;
-    if ((double)max_blocks * 4.0 > 0.7 * ideal) {
-      plan->warps_per_smsp = 3;
-      if ((double)max_blocks * 3.0 > 0.7 * ideal) plan->warps_per_smsp = 2;
-      if ((double)max_blocks * 2.0 > 0.7 * ideal) plan->warps_per_smsp = 1;
-    }
-  }
-#undef PLAN_CUDA
+  uint32_t* order = cached ? owned.get() : (uint32_t*)scratch_get(dc, st, kPlanOrder, (size_t)n * 4);
+  if (!hist || !order) return CAPY_ERR_OOM;
+  int rc = device_len_hist(ctx, st, d_off, n, stride_bytes, hist, &h);
+  if (rc) return rc;
+  rc = plan_from_hist(ctx, dc, st, d_off, n, stride_bytes, h, hist, order, allow_pair, force_c, plan);
+  if (rc) return rc;
   if (cached) {
-    if (!plan->order) {  // uniform batch: the entry records "nothing to do"
-      cudaFree(owned);
-      owned = nullptr;
-    }
+    if (!plan->order) owned.reset();  // uniform batch: the entry records "nothing to do"
     if (dc.plans.size() >= kMaxPlanEntries) {  // evict the least recently used plan
       size_t lru = 0;
       for (size_t k = 1; k < dc.plans.size(); k++)
@@ -469,20 +500,32 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
     e.unit = stride_bytes;
     e.allow_pair = allow_pair;
     e.plan = *plan;
-    e.owned_order = owned;
+    e.owned_order = owned.release();
     e.last_use = ++dc.use_clock;
     dc.plans.push_back(e);
   }
   return CAPY_OK;
 }
 
+// ---- one launch of a sponge job ------------------------------------------------------------------------------------
+// The occupancy throttle of a plan: warps_per_smsp = W in 1..3 launches 128-thread blocks (one warp per scheduler) with
+// a dynamic shared-memory footprint that lets W of them share an SM.
+template <class Kernel>
+static cudaError_t throttle(Kernel* kernel, const LaunchPlan& plan, unsigned* block, size_t* smem) {
+  *smem = 0;
+  if (plan.warps_per_smsp < 1 || plan.warps_per_smsp > 3) return cudaSuccess;
+  *block = 128;
+  *smem = (size_t)(227 * 1024 / plan.warps_per_smsp) - 1024;
+  return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024);
+}
+
 template <int LANES>
 static int launch_sponge_t(capy_ctx* ctx, cudaStream_t stream, SpongeJob J, unsigned block, const LaunchPlan& plan) {
-  const uint64_t warp_items = plan.warp_items[0] + plan.warp_items[1] + plan.warp_items[2], pair_items = plan.pair_items;
-  if (pair_items || warp_items) {
+  if (plan.tiered()) {
     // chain-bound batch: warp blocks (one, two, three chains per scheduler), then pair blocks, then thread-per-item
     // blocks, one block per SM.  A block has 384 threads: a warp-tier block of class c uses 4 c warps, the other tiers
     // the first four; the rest exit at once.
+    const uint64_t warp_items = plan.warp_items[0] + plan.warp_items[1] + plan.warp_items[2], pair_items = plan.pair_items;
     SpongeTiers tiers;
     uint32_t warp_blocks = 0;
     uint64_t rank = 0;
@@ -503,14 +546,8 @@ static int launch_sponge_t(capy_ctx* ctx, cudaStream_t stream, SpongeJob J, unsi
     CAPY_CUDA(ctx, cudaGetLastError());
     return CAPY_OK;
   }
-  size_t smem = 0;
-  const int warps_per_smsp = plan.warps_per_smsp;
-  if (warps_per_smsp >= 1 && warps_per_smsp <= 3) {
-    // one 128-thread block = one warp per scheduler; W blocks per SM via the shared-memory footprint
-    block = 128;
-    smem = (size_t)(227 * 1024 / warps_per_smsp) - 1024;
-    CAPY_CUDA(ctx, cudaFuncSetAttribute(sponge_kernel<LANES>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-  }
+  size_t smem;
+  CAPY_CUDA(ctx, throttle(sponge_kernel<LANES>, plan, &block, &smem));
   sponge_kernel<LANES><<<grid_for(J.n, block), block, smem, stream>>>(J);
   ctx->launches++;
   CAPY_CUDA(ctx, cudaGetLastError());
@@ -537,29 +574,112 @@ static unsigned pick_block(uint64_t n, int sm_count, int threads_per_sm) {
   return best;
 }
 
-static int launch_sponge(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J,
-                         const LaunchPlan& plan = LaunchPlan()) {
+// The kernels of a job are instantiated for the whole lanes of its rate: 21 for the 172-byte rate of D224 cSHAKE / KMAC
+// (quirk Q7), rate / 8 for every other rate.
+static int job_lanes(const SpongeJob& J) { return (int)(J.rate / 8); }
+
+static int launch_sponge(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J, const LaunchPlan& plan) {
   if (J.n == 0) return CAPY_OK;
   const unsigned block = pick_block(J.n, dc.sm_count, 384);
-  switch (lanes) {
-    case 9: return launch_sponge_t<9>(ctx, stream, J, block, plan);
-    case 13: return launch_sponge_t<13>(ctx, stream, J, block, plan);
-    case 17: return launch_sponge_t<17>(ctx, stream, J, block, plan);
-    case 18: return launch_sponge_t<18>(ctx, stream, J, block, plan);
-    case 19: return launch_sponge_t<19>(ctx, stream, J, block, plan);
-    case 21: return launch_sponge_t<21>(ctx, stream, J, block, plan);
-    default: return CAPY_ERR_BAD_ARG;
-  }
+  return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J), [&](auto L) {
+    return launch_sponge_t<decltype(L)::value>(ctx, stream, J, block, plan);
+  });
 }
 
-// chain cutting of uniform batches (defined with the cSHAKE / KMAC launchers below)
-static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t squeeze_extra, uint64_t* cut);
-static int launch_sponge_chain(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J, uint64_t cut);
+// two jobs one after the other, both in the order of `plan`
+static int launch_sponge_seq(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& A, const SpongeJob& B,
+                             const LaunchPlan& plan) {
+  const int rc = launch_sponge(ctx, dc, stream, A, plan);
+  if (rc) return rc;
+  return launch_sponge(ctx, dc, stream, B, plan);
+}
 
-static SpongeJob empty_job() {
-  SpongeJob J;
-  memset(&J, 0, sizeof J);
-  return J;
+// ---- chain splitting of uniform batches (sponge.cuh: sponge_chain_kernel) --------------------------------------------
+// Two dependent jobs in one launch need at least as many job-0 blocks as the GPU holds at once (CAPY_SPONGE_MINB per SM):
+// a job-1 block of a smaller batch could wait for its job-0 block.  CAPY_NO_CHAIN_SPLIT turns them off (A/B switch for
+// the probes).
+static bool chain_jobs_fit(int sm_count, uint64_t n) {
+  if (getenv("CAPY_NO_CHAIN_SPLIT") || sm_count < 1) return false;
+  return (n + 127) / 128 >= (uint64_t)CAPY_SPONGE_MINB * (uint64_t)sm_count;
+}
+
+// Where to cut: the batch must fill the schedulers unevenly, be large enough for two dependent jobs (chain_jobs_fit), and
+// leave the two halves about equally long; the cut lies inside -- or at the end of -- the absorb phase.  absorb_blocks
+// counts the blocks after skip_blocks, squeeze_extra the permutations between squeeze blocks.  (A wrong estimate costs
+// balance, never correctness: an item that is shorter than the cut simply has nothing left to absorb in job 1.)
+static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t squeeze_extra, uint64_t* cut) {
+  if (!chain_jobs_fit(sm_count, n)) return false;
+  const uint64_t warps = (n + 31) / 32, sched = 4ull * (uint64_t)sm_count;
+  if (warps > 8 * sched) return false;
+  auto fill = [&](uint64_t w) {
+    const double x = (double)w / (double)sched;
+    return x / std::ceil(x);
+  };
+  if (fill(2 * warps) < fill(warps) + 0.04) return false;
+  const uint64_t perms = absorb_blocks + squeeze_extra;
+  if (perms < 12) return false;
+  uint64_t k = (perms + 1) / 2;
+  if (k > absorb_blocks) k = absorb_blocks;
+  if (3 * k < perms) return false;  // the absorb phase is too short to carry a half
+  *cut = k;
+  return true;
+}
+
+// two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel)
+static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J0, const SpongeJob& J1,
+                             bool data_dependent) {
+  const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
+  uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
+  if (!sync) return CAPY_ERR_OOM;
+  CAPY_CUDA(ctx, cudaMemsetAsync(sync, 0, ((size_t)nb + 1) * sizeof(uint32_t), stream));
+  SpongeChain C;
+  C.j[0] = J0;
+  C.j[1] = J1;
+  C.sync = sync;
+  C.blocks_per_job = nb;
+  C.data_dependent = data_dependent ? 1u : 0u;
+  return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J0), [&](auto L) {
+    sponge_chain_kernel<decltype(L)::value><<<2 * nb, 128, 0, stream>>>(C);
+    ctx->launches++;
+    CAPY_CUDA(ctx, cudaGetLastError());
+    return CAPY_OK;
+  });
+}
+
+// J (uniform batch, no order) as two dependent jobs cut after `cut` absorbed blocks
+static int launch_sponge_chain(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J, uint64_t cut) {
+  uint64_t* states = (uint64_t*)scratch_get(dc, stream, kChainStates, (size_t)J.n * 25 * sizeof(uint64_t));
+  if (!states) return CAPY_ERR_OOM;
+  SpongeJob J0 = J, J1 = J;
+  J0.chain_out = states;
+  J0.stop_block = J.skip_blocks + cut;
+  J1.chain_in = states;
+  J1.skip_blocks = (uint32_t)(J.skip_blocks + cut);
+  return launch_chain_jobs(ctx, dc, stream, J0, J1, false);
+}
+
+// Whether a job is a uniform batch worth cutting along its chains, and where.  Uniform: a fixed-length job, or a plan
+// that found one block count.  Jobs that write at per-item offsets or XOR into a buffer are not cut, nor are rates that
+// are not lane-aligned (D224 cSHAKE / KMAC, quirk Q7).
+static bool uniform_cut(const DeviceCtx& dc, const SpongeJob& J, const LaunchPlan& plan, uint64_t* cut) {
+  if (J.out_off || J.xor_in || plan.order || (J.rate & 7u) != 0) return false;
+  const uint64_t msg_blocks = J.off ? plan.uniform_blocks : J.msg_len / J.rate + 1;  // the last one holds the trailer
+  if (!msg_blocks) return false;
+  // blocks absorbed after skip_blocks: the rest of the prefix, the key block bytepad(encode_string(K), w), the message
+  uint64_t absorb = msg_blocks;
+  if (J.keys) absorb += ((uint64_t)J.key_len + 8) / J.w + 1;
+  if (!J.skip_blocks) absorb += J.prefix_len / J.rate;
+  const uint64_t sq = 8ull * J.sq_lanes, squeeze_extra = J.out_bytes ? (J.out_bytes + sq - 1) / sq - 1 : 0;
+  return chain_cut(dc.sm_count, J.n, absorb, squeeze_extra, cut);
+}
+
+// Launches a built job in the order of `plan`: a uniform batch as two dependent jobs when uniform_cut says so, anything
+// else as one launch.
+static int run_sponge(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, SpongeJob J, const LaunchPlan& plan) {
+  J.order = plan.order;
+  uint64_t cut;
+  if (uniform_cut(dc, J, plan, &cut)) return launch_sponge_chain(ctx, dc, stream, J, cut);
+  return launch_sponge(ctx, dc, stream, J, plan);
 }
 
 // ---- SHA3-d ------------------------------------------------------------------------------------
@@ -588,49 +708,20 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
     const uint4* dq = reinterpret_cast<const uint4*>(data);
     uint4* oq = reinterpret_cast<uint4*>(out);
     const uint64_t s16 = stride / 16;
-#define CAPY_SHORT(L, M, OB) sha3_short_kernel<L, M><<<grid, block, 0, stream>>>(dq, s16, 0x06u, oq, OB, n)
-    if (d == 256) {
-      switch (msg_len / 8) {
-        case 2: CAPY_SHORT(17, 2, 32); break;
-        case 4: CAPY_SHORT(17, 4, 32); break;
-        case 6: CAPY_SHORT(17, 6, 32); break;
-        case 8: CAPY_SHORT(17, 8, 32); break;
-        case 10: CAPY_SHORT(17, 10, 32); break;
-        case 12: CAPY_SHORT(17, 12, 32); break;
-        case 14: CAPY_SHORT(17, 14, 32); break;
-        default: CAPY_SHORT(17, 16, 32); break;
-      }
-    } else {
-      switch (msg_len / 8) {
-        case 2: CAPY_SHORT(9, 2, 64); break;
-        case 4: CAPY_SHORT(9, 4, 64); break;
-        case 6: CAPY_SHORT(9, 6, 64); break;
-        default: CAPY_SHORT(9, 8, 64); break;
-      }
-    }
-#undef CAPY_SHORT
+    const int msg_lanes = (int)(msg_len / 8);  // 2, 4, .. 16 at D256; 2, 4, 6, 8 at D512
+    const int rc = d == 256 ? with_lanes<2, 4, 6, 8, 10, 12, 14, 16>(msg_lanes, [&](auto M) {
+      sha3_short_kernel<17, decltype(M)::value><<<grid, block, 0, stream>>>(dq, s16, 0x06u, oq, 32, n);
+      return CAPY_OK;
+    }) : with_lanes<2, 4, 6, 8>(msg_lanes, [&](auto M) {
+      sha3_short_kernel<9, decltype(M)::value><<<grid, block, 0, stream>>>(dq, s16, 0x06u, oq, 64, n);
+      return CAPY_OK;
+    });
+    if (rc) return rc;
     ctx->launches++;
     CAPY_CUDA(ctx, cudaGetLastError());
     return CAPY_OK;
   }
-  uint64_t cut = 0;
-  const bool cut_fixed = !off && chain_cut(dc.sm_count, n, msg_len / rate + 1, 0, &cut);  // long equal messages, uneven fill
-  // the uniform kernel stores 4-byte granules (28- and 48-byte digests) and reads whole 8-byte words
-  if (!off && !cut_fixed && (reinterpret_cast<uintptr_t>(data) & 7u) == 0 && (stride & 7u) == 0 &&
-      (reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (tail_readable || (msg_len & 7u) == 0)) {
-    const uint32_t suffix = (msg_len % 136u == 135u) ? 0x86u : 0x06u;  // shake_functions.rs:25-29 (Q2)
-    const unsigned block = 128, grid = grid_for(n, block);
-    switch (lanes) {
-      case 18: sha3_uniform_kernel<18><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n); break;
-      case 17: sha3_uniform_kernel<17><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n); break;
-      case 13: sha3_uniform_kernel<13><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n); break;
-      case 9: sha3_uniform_kernel<9><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n); break;
-    }
-    ctx->launches++;
-    CAPY_CUDA(ctx, cudaGetLastError());
-    return CAPY_OK;
-  }
-  SpongeJob J = empty_job();
+  SpongeJob J{};
   J.data = data;
   J.off = off;
   J.msg_len = msg_len;
@@ -642,17 +733,27 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
   J.out_stride = J.out_bytes = (uint64_t)d / 8;
   J.sq_lanes = (1600 - d) / 64;  // Rate::from(&d), sponge.rs:27 (first d/8 bytes are all that is kept)
   J.n = n;
+  // long equal messages that fill the GPU unevenly are cut along the chains (run_sponge), which the uniform kernel cannot
+  // do; the uniform kernel stores 4-byte granules (28- and 48-byte digests) and reads whole 8-byte words
+  uint64_t cut;
+  if (!off && !uniform_cut(dc, J, LaunchPlan(), &cut) && (reinterpret_cast<uintptr_t>(data) & 7u) == 0 &&
+      (stride & 7u) == 0 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (tail_readable || (msg_len & 7u) == 0)) {
+    const uint32_t suffix = (msg_len % 136u == 135u) ? 0x86u : 0x06u;  // shake_functions.rs:25-29 (Q2)
+    const unsigned block = 128, grid = grid_for(n, block);
+    return with_lanes<9, 13, 17, 18>(lanes, [&](auto L) {
+      sha3_uniform_kernel<decltype(L)::value><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n);
+      ctx->launches++;
+      CAPY_CUDA(ctx, cudaGetLastError());
+      return CAPY_OK;
+    });
+  }
   LaunchPlan plan;
   if (off && !(flags & CAPY_FLAG_NO_SORT)) {
     int rc = plan_ragged(ctx, dc, stream, off, n, rate, &plan, !(flags & CAPY_FLAG_NO_PAIR),
                          (int)((flags >> CAPY_FLAG_WARP_COSCHED_SHIFT) & 3u));
     if (rc) return rc;
   }
-  J.order = plan.order;
-  if (cut_fixed) return launch_sponge_chain(ctx, dc, stream, lanes, J, cut);
-  if (off && !plan.order && plan.uniform_blocks && chain_cut(dc.sm_count, n, plan.uniform_blocks, 0, &cut))
-    return launch_sponge_chain(ctx, dc, stream, lanes, J, cut);
-  return launch_sponge(ctx, dc, stream, lanes, J, plan);
+  return run_sponge(ctx, dc, stream, J, plan);
 }
 
 // ---- cSHAKE / KMAC prefix -----------------------------------------------------------------------
@@ -704,36 +805,28 @@ static int get_prefix(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d, 
   p.append(w - p.size() % w, '\0');  // aux_functions.rs:14-16 (quirk Q3)
   PrefixState ps;
   ps.prefix_len = (uint32_t)p.size();
-  auto fail = [&](cudaError_t e, const char* what) {  // nothing is cached on failure: free what was allocated
-    if (ps.d_prefix) cudaFree(ps.d_prefix);
-    if (ps.d_state) cudaFree(ps.d_state);
-    return cuda_fail(ctx, e, what);
-  };
-#define PREFIX_CUDA(expr)                          \
-  do {                                             \
-    cudaError_t _e = (expr);                       \
-    if (_e != cudaSuccess) return fail(_e, #expr); \
-  } while (0)
-  PREFIX_CUDA(cudaMalloc(&ps.d_prefix, p.size()));
-  PREFIX_CUDA(cudaMalloc(&ps.d_state, 25 * sizeof(uint64_t)));
-  PREFIX_CUDA(cudaMemcpyAsync(ps.d_prefix, p.data(), p.size(), cudaMemcpyHostToDevice, stream));
-  const int lanes = (int)(w * 8 / 64);  // 21 / 21 / 19 / 17
+  DevPtr<uint8_t> d_prefix;  // nothing is cached on failure: these free what was allocated
+  DevPtr<uint64_t> d_state;
+  CAPY_CUDA(ctx, dev_alloc(d_prefix, p.size()));
+  CAPY_CUDA(ctx, dev_alloc(d_state, 25 * sizeof(uint64_t)));
+  CAPY_CUDA(ctx, cudaMemcpyAsync(d_prefix.get(), p.data(), p.size(), cudaMemcpyHostToDevice, stream));
   if (w % 8 == 0) {
     // the prefix is a whole number of blocks: fold it into a cached state once
     ps.skip_blocks = ps.prefix_len / w;
-    switch (lanes) {
-      case 21: prefix_state_kernel<21><<<1, 32, 0, stream>>>(ps.d_prefix, ps.skip_blocks, ps.d_state); break;
-      case 19: prefix_state_kernel<19><<<1, 32, 0, stream>>>(ps.d_prefix, ps.skip_blocks, ps.d_state); break;
-      case 17: prefix_state_kernel<17><<<1, 32, 0, stream>>>(ps.d_prefix, ps.skip_blocks, ps.d_state); break;
-    }
-    ctx->launches++;
-    PREFIX_CUDA(cudaGetLastError());
+    const int rc = with_lanes<17, 19, 21>((int)(w / 8), [&](auto L) {
+      prefix_state_kernel<decltype(L)::value><<<1, 32, 0, stream>>>(d_prefix.get(), ps.skip_blocks, d_state.get());
+      ctx->launches++;
+      CAPY_CUDA(ctx, cudaGetLastError());
+      return CAPY_OK;
+    });
+    if (rc) return rc;
   } else {
     ps.skip_blocks = 0;  // D224: w = 172 is not lane aligned (quirk Q7), blocks straddle the prefix end
   }
   // the host string dies at return, and later calls may use the entry from other streams: wait for the build
-  PREFIX_CUDA(cudaStreamSynchronize(stream));
-#undef PREFIX_CUDA
+  CAPY_CUDA(ctx, cudaStreamSynchronize(stream));
+  ps.d_prefix = d_prefix.release();
+  ps.d_state = d_state.release();
   ps.last_use = ++dc.use_clock;
   auto ins = dc.prefix_cache.emplace(key, ps);
   *out = &ins.first->second;
@@ -751,83 +844,6 @@ static void fill_cshake_common(SpongeJob& J, int d, const PrefixState* ps) {
   J.sq_lanes = (1600 - d) / 64;
 }
 
-// ---- chain splitting of uniform batches (sponge.cuh: sponge_chain_kernel) --------------------------------------------
-// Where to cut: the batch must fill the schedulers unevenly, be large enough that no job-1 block has to wait for its
-// job-0 block (at least as many job-0 blocks as the GPU holds at once: CAPY_SPONGE_MINB per SM), and leave the two halves
-// about equally long; the cut lies inside -- or at the end of -- the absorb phase.  absorb_blocks counts the blocks after
-// skip_blocks, squeeze_extra the permutations between squeeze blocks.  (A wrong estimate costs balance, never
-// correctness: an item that is shorter than the cut simply has nothing left to absorb in job 1.)
-static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t squeeze_extra, uint64_t* cut) {
-  if (getenv("CAPY_NO_CHAIN_SPLIT")) return false;  // A/B switch for the probes
-  if (sm_count < 1) return false;
-  const uint64_t warps = (n + 31) / 32, sched = 4ull * (uint64_t)sm_count, blocks = (n + 127) / 128;
-  if (blocks < (uint64_t)CAPY_SPONGE_MINB * (uint64_t)sm_count || warps > 8 * sched) return false;
-  auto fill = [&](uint64_t w) {
-    const double x = (double)w / (double)sched;
-    return x / std::ceil(x);
-  };
-  if (fill(2 * warps) < fill(warps) + 0.04) return false;
-  const uint64_t perms = absorb_blocks + squeeze_extra;
-  if (perms < 12) return false;
-  uint64_t k = (perms + 1) / 2;
-  if (k > absorb_blocks) k = absorb_blocks;
-  if (3 * k < perms) return false;  // the absorb phase is too short to carry a half
-  *cut = k;
-  return true;
-}
-
-template <int LANES>
-static int launch_chain_t(capy_ctx* ctx, cudaStream_t stream, const SpongeChain& C, unsigned grid) {
-  sponge_chain_kernel<LANES><<<grid, 128, 0, stream>>>(C);
-  ctx->launches++;
-  CAPY_CUDA(ctx, cudaGetLastError());
-  return CAPY_OK;
-}
-
-// two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel)
-static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J0, const SpongeJob& J1,
-                             bool data_dependent) {
-  const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
-  uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
-  if (!sync) return CAPY_ERR_OOM;
-  CAPY_CUDA(ctx, cudaMemsetAsync(sync, 0, ((size_t)nb + 1) * sizeof(uint32_t), stream));
-  SpongeChain C;
-  C.j[0] = J0;
-  C.j[1] = J1;
-  C.sync = sync;
-  C.blocks_per_job = nb;
-  C.data_dependent = data_dependent ? 1u : 0u;
-  switch (lanes) {
-    case 9: return launch_chain_t<9>(ctx, stream, C, 2 * nb);
-    case 13: return launch_chain_t<13>(ctx, stream, C, 2 * nb);
-    case 17: return launch_chain_t<17>(ctx, stream, C, 2 * nb);
-    case 18: return launch_chain_t<18>(ctx, stream, C, 2 * nb);
-    case 19: return launch_chain_t<19>(ctx, stream, C, 2 * nb);
-    case 21: return launch_chain_t<21>(ctx, stream, C, 2 * nb);
-    default: return CAPY_ERR_BAD_ARG;
-  }
-}
-
-// J (uniform batch, no order) as two dependent jobs cut after `cut` absorbed blocks
-static int launch_sponge_chain(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int lanes, const SpongeJob& J, uint64_t cut) {
-  uint64_t* states = (uint64_t*)scratch_get(dc, stream, kChainStates, (size_t)J.n * 25 * sizeof(uint64_t));
-  if (!states) return CAPY_ERR_OOM;
-  SpongeJob J0 = J, J1 = J;
-  J0.chain_out = states;
-  J0.stop_block = J.skip_blocks + cut;
-  J1.chain_in = states;
-  J1.skip_blocks = (uint32_t)(J.skip_blocks + cut);
-  return launch_chain_jobs(ctx, dc, stream, lanes, J0, J1, false);
-}
-
-// blocks a uniform cSHAKE / KMAC item absorbs after the cached prefix, estimated from the message blocks of the plan
-static uint64_t absorb_blocks_estimate(const SpongeJob& J, uint64_t key_len, bool has_key, uint64_t msg_blocks_whole) {
-  uint64_t blocks = msg_blocks_whole + 1;  // the message and the block that holds its tail, the trailer and the pad
-  if (has_key) blocks += (key_len + 8) / J.w + 1;  // bytepad(encode_string(K), w)
-  if (!J.skip_blocks) blocks += J.prefix_len / J.rate;
-  return blocks;
-}
-
 static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d, const uint8_t* data,
                          const uint64_t* off, uint64_t n, const uint8_t* fn, uint32_t fn_len, const uint8_t* cs,
                          uint32_t cs_len, uint64_t out_bits, uint8_t* out) {
@@ -836,7 +852,7 @@ static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int 
   PrefixState* ps;
   int rc = get_prefix(ctx, dc, stream, d, fn, fn_len, cs, cs_len, &ps);
   if (rc) return rc;
-  SpongeJob J = empty_job();
+  SpongeJob J{};
   fill_cshake_common(J, d, ps);
   J.data = data;
   J.off = off;
@@ -847,19 +863,9 @@ static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int 
   J.out_stride = J.out_bytes = out_bits / 8;
   J.n = n;
   LaunchPlan plan;
-  if (off) {
-    rc = plan_ragged(ctx, dc, stream, off, n, J.rate & ~7u, &plan);
-    if (rc) return rc;
-  }
-  J.order = plan.order;
-  const int lanes = (int)(bytepad_value(d) * 8 / 64);
-  if (off && !plan.order && plan.uniform_blocks && (J.rate & 7u) == 0) {  // uniform batch: see launch_kmac_xof
-    const uint64_t absorb = absorb_blocks_estimate(J, 0, false, plan.uniform_blocks - 1);
-    const uint64_t sq = 8ull * J.sq_lanes, squeeze_extra = (J.out_bytes + sq - 1) / sq - 1;
-    uint64_t cut;
-    if (chain_cut(dc.sm_count, n, absorb, squeeze_extra, &cut)) return launch_sponge_chain(ctx, dc, stream, lanes, J, cut);
-  }
-  return launch_sponge(ctx, dc, stream, lanes, J, plan);
+  rc = plan_ragged(ctx, dc, stream, off, n, J.rate & ~7u, &plan);
+  if (rc) return rc;
+  return run_sponge(ctx, dc, stream, J, plan);
 }
 
 static int build_kmac_job(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a, SpongeJob* out) {
@@ -867,7 +873,7 @@ static int build_kmac_job(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, con
   PrefixState* ps;
   int rc = get_prefix(ctx, dc, stream, a.d_bits, kKmac, 4, a.custom, a.custom_len, &ps);
   if (rc) return rc;
-  SpongeJob J = empty_job();
+  SpongeJob J{};
   fill_cshake_common(J, a.d_bits, ps);
   J.keys = a.keys;
   J.key_off = a.key_off;
@@ -908,18 +914,7 @@ int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const Kma
   LaunchPlan plan;
   rc = plan_kmac(ctx, dc, stream, a, J, &plan);
   if (rc) return rc;
-  J.order = plan.order;
-  const int lanes = (int)(bytepad_value(a.d_bits) * 8 / 64);
-  // uniform batch (fixed-length call, or a plan that found one block count): cut the chains when that fills the GPU better
-  const uint64_t unit = J.rate & ~7u;
-  const uint64_t msg_blocks = a.off ? plan.uniform_blocks : a.msg_len / unit + 1;
-  if (!a.out_off && !a.xor_in && !plan.order && msg_blocks && (J.rate & 7u) == 0) {
-    const uint64_t absorb = absorb_blocks_estimate(J, a.key_len, a.keys != nullptr, msg_blocks - 1);
-    const uint64_t sq = 8ull * J.sq_lanes, squeeze_extra = a.out_bytes ? (a.out_bytes + sq - 1) / sq - 1 : 0;
-    uint64_t cut;
-    if (chain_cut(dc.sm_count, a.n, absorb, squeeze_extra, &cut)) return launch_sponge_chain(ctx, dc, stream, lanes, J, cut);
-  }
-  return launch_sponge(ctx, dc, stream, lanes, J, plan);
+  return run_sponge(ctx, dc, stream, J, plan);
 }
 
 // Two independent KMACXOF passes over the same items (same d, same n) as ONE launch: warps alternate between the two
@@ -933,12 +928,8 @@ static int launch_sponge2_t(capy_ctx* ctx, cudaStream_t stream, const SpongeJob&
   SpongeJob2 JJ;
   JJ.j[0] = A;
   JJ.j[1] = B;
-  size_t smem = 0;
-  if (plan.warps_per_smsp >= 1 && plan.warps_per_smsp <= 3) {
-    block = 128;
-    smem = (size_t)(227 * 1024 / plan.warps_per_smsp) - 1024;
-    CAPY_CUDA(ctx, cudaFuncSetAttribute(sponge_kernel2<LANES>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024));
-  }
+  size_t smem;
+  CAPY_CUDA(ctx, throttle(sponge_kernel2<LANES>, plan, &block, &smem));
   const uint64_t warps = 2 * ((A.n + 31) / 32);
   sponge_kernel2<LANES><<<grid_for(warps * 32, block), block, smem, stream>>>(JJ);
   ctx->launches++;
@@ -958,19 +949,11 @@ int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const Km
   rc = plan_kmac(ctx, dc, stream, a, JA, &plan);
   if (rc) return rc;
   JA.order = JB.order = plan.order;
-  const int lanes = (int)(bytepad_value(a.d_bits) * 8 / 64);
-  if (plan.warp_items[0] || plan.warp_items[1] || plan.warp_items[2] || plan.pair_items) {
-    rc = launch_sponge(ctx, dc, stream, lanes, JA, plan);
-    if (rc) return rc;
-    return launch_sponge(ctx, dc, stream, lanes, JB, plan);
-  }
+  if (plan.tiered()) return launch_sponge_seq(ctx, dc, stream, JA, JB, plan);
   const unsigned block = pick_block(2 * a.n, dc.sm_count, 384);
-  switch (lanes) {
-    case 17: return launch_sponge2_t<17>(ctx, stream, JA, JB, block, plan);
-    case 19: return launch_sponge2_t<19>(ctx, stream, JA, JB, block, plan);
-    case 21: return launch_sponge2_t<21>(ctx, stream, JA, JB, block, plan);
-    default: return CAPY_ERR_BAD_ARG;
-  }
+  return with_lanes<17, 19, 21>(job_lanes(JA), [&](auto L) {
+    return launch_sponge2_t<decltype(L)::value>(ctx, stream, JA, JB, block, plan);
+  });
 }
 
 // Two KMACXOF passes where the SECOND absorbs what the FIRST wrote for the same item (authenticated decryption: the
@@ -989,15 +972,9 @@ int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const
   rc = plan_kmac(ctx, dc, stream, second, J1, &plan);
   if (rc) return rc;
   J0.order = J1.order = plan.order;
-  const int lanes = (int)(bytepad_value(first.d_bits) * 8 / 64);
-  const bool tiers = plan.warp_items[0] || plan.warp_items[1] || plan.warp_items[2] || plan.pair_items;
-  const uint64_t blocks = (first.n + 127) / 128;
-  if (tiers || (J0.rate & 7u) != 0 || blocks < (uint64_t)CAPY_SPONGE_MINB * (uint64_t)dc.sm_count || getenv("CAPY_NO_CHAIN_SPLIT")) {
-    rc = launch_sponge(ctx, dc, stream, lanes, J0, plan);  // (a job-1 block of a small batch would wait for its job-0 block)
-    if (rc) return rc;
-    return launch_sponge(ctx, dc, stream, lanes, J1, plan);
-  }
-  return launch_chain_jobs(ctx, dc, stream, lanes, J0, J1, true);
+  if (plan.tiered() || (J0.rate & 7u) != 0 || !chain_jobs_fit(dc.sm_count, first.n))
+    return launch_sponge_seq(ctx, dc, stream, J0, J1, plan);
+  return launch_chain_jobs(ctx, dc, stream, J0, J1, true);
 }
 
 }  // namespace capy
@@ -1298,7 +1275,7 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
     return CAPY_ERR_BAD_ARG;
   if (n == 0 || out_bytes == 0) return CAPY_OK;
   CAPY_DEV_PROLOGUE
-  SpongeJob J = empty_job();
+  SpongeJob J{};
   J.data = d_data;
   J.off = d_off;
   J.trailer = 0x1F;
@@ -1312,15 +1289,7 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
   LaunchPlan plan;  // longest first, tiers for chain-bound batches, chains of a uniform batch cut in two: as for cSHAKE
   int rc = plan_ragged(ctx, dc, st, d_off, n, J.rate, &plan);
   if (rc) return rc;
-  J.order = plan.order;
-  const int lanes = (int)J.rate / 8;
-  if (!plan.order && plan.uniform_blocks) {
-    const uint64_t sq = 8ull * J.sq_lanes;
-    uint64_t cut;
-    if (chain_cut(dc.sm_count, n, plan.uniform_blocks, (out_bytes + sq - 1) / sq - 1, &cut))
-      return launch_sponge_chain(ctx, dc, st, lanes, J, cut);
-  }
-  return launch_sponge(ctx, dc, st, lanes, J, plan);
+  return run_sponge(ctx, dc, st, J, plan);
 }
 
 }  // extern "C"
