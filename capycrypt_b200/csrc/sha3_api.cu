@@ -14,6 +14,7 @@
 
 #include "internal.h"
 #include "hostbatch.h"
+#include "keccak_bs.cuh"
 #include "sponge.cuh"
 
 namespace capy {
@@ -95,41 +96,70 @@ __global__ void __launch_bounds__(128)
 
 // ------------------------------------------------------------------------------------------------
 // single-block SHA3-d of messages of exactly 8 * MSG_LANES bytes (MSG_LANES < LANES), 16-byte aligned
-// rows: the BASELINE cfg-1 shape (2^20 x 64 B).  Everything about the block layout is a compile-time
-// constant: message lanes come in with 128-bit loads, the suffix / 0x80 lanes are immediates, round 0 is
-// peeled so that the zero lanes fold away, and the remaining 23 rounds run two per loop iteration.
+// rows: the BASELINE cfg-1 shape (2^20 x 64 B).  Bitsliced (keccak_bs.cuh): a warp hashes its 32 messages together,
+// so the rotations run on the shuffle unit instead of the ALU pipe.  Each thread loads its own row with 128-bit loads;
+// a warp transpose turns the message words into bit-position words.  Everything about the block layout is a
+// compile-time constant: the zero lanes of the block fold away in the peeled round 0, the remaining 23 rounds run two
+// per loop iteration, and round 23 computes only the digest lanes.
+// Every thread of a warp that has a message takes part in every shuffle; threads past n hash zeros and store nothing.
+// The minimum of 4 blocks per SM lets ptxas use up to 128 registers: under the plain bound it chose 96 and spilled.
 // ------------------------------------------------------------------------------------------------
 template <int LANES, int MSG_LANES>
-__global__ void __launch_bounds__(128)
+__global__ void __launch_bounds__(128, 4)
     sha3_short_kernel(const uint4* __restrict__ data, uint64_t stride16, uint32_t suffix, uint4* __restrict__ out,
                       uint32_t out_bytes, uint64_t n) {
   static_assert(MSG_LANES % 2 == 0 && MSG_LANES < LANES, "whole 16-byte loads, one block");
+  constexpr int OUT_LANES = (200 - 8 * LANES) / 16;  // d / 64: 4 (SHA3-256) or 8 (SHA3-512)
+  const uint32_t lane = threadIdx.x & 31u;
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const uint4* q = data + i * stride16;
-  Lane a[25];
-  state_zero(a);
+  if (i - lane >= n) return;  // warp-uniform: the warp has no message
+  const bool live = i < n;
+  const BsTranspose transpose(lane);
+
+  uint32_t a[25][2];
+  {
+    const uint4* q = data + i * stride16;
+    uint32_t w[2 * MSG_LANES];
 #pragma unroll
-  for (int j = 0; j < MSG_LANES / 2; j++) {
-    const uint4 v = __ldg(q + j);
-    a[2 * j].lo = v.x;
-    a[2 * j].hi = v.y;
-    a[2 * j + 1].lo = v.z;
-    a[2 * j + 1].hi = v.w;
+    for (int j = 0; j < MSG_LANES / 2; j++) {
+      const uint4 v = live ? __ldg(q + j) : make_uint4(0u, 0u, 0u, 0u);
+      w[4 * j] = v.x;
+      w[4 * j + 1] = v.y;
+      w[4 * j + 2] = v.z;
+      w[4 * j + 3] = v.w;
+    }
+#pragma unroll
+    for (int j = 0; j < 2 * MSG_LANES; j++) w[j] = transpose(w[j]);
+#pragma unroll
+    for (int l = 0; l < MSG_LANES; l++) bs_gather(a[l], w[2 * l], w[2 * l + 1], lane);
   }
-  a[MSG_LANES].lo = suffix;  // 0x06 (0x86 can only occur for 135-byte messages, which are not 8-byte multiples)
-  a[LANES - 1].hi ^= 0x80000000u;  // 8 * MSG_LANES + 1 < rate always holds here: zeros then 0x80 (sponge.rs:89-95)
-  keccak_round(a, KECCAK_RC[0]);
+#pragma unroll
+  for (int l = MSG_LANES; l < 25; l++) a[l][0] = a[l][1] = 0u;
+  // 0x06 (0x86 can only occur for 135-byte messages, which are not 8-byte multiples): bits 2t, 2t+1 of the suffix
+  const uint32_t pad = (uint32_t)((uint64_t)suffix >> (2 * lane));
+  a[MSG_LANES][0] = 0u - (pad & 1u);
+  a[MSG_LANES][1] = 0u - ((pad >> 1) & 1u);
+  // 8 * MSG_LANES + 1 < rate always holds here: zeros then 0x80 (sponge.rs:89-95), bit 63 of the last lane
+  a[LANES - 1][1] ^= lane == 31 ? 0xFFFFFFFFu : 0u;
+
+  const uint2 rc = __ldg(&KECCAK_RC_BITS[lane]);
+  keccak_bs_round(a, lane, rc, 1u);
 #pragma unroll 1
   for (int r = 1; r < 23; r += 2) {
-    keccak_round(a, KECCAK_RC[r]);
-    keccak_round(a, KECCAK_RC[r + 1]);
+    keccak_bs_round(a, lane, rc, 1u << r);
+    keccak_bs_round(a, lane, rc, 2u << r);
   }
-  keccak_round(a, KECCAK_RC[23]);
+  keccak_bs_round(a, lane, rc, 1u << 23);
+
+  uint32_t w[2 * OUT_LANES];
+#pragma unroll
+  for (int l = 0; l < OUT_LANES; l++) bs_scatter(w[2 * l], w[2 * l + 1], a[l], lane);
+#pragma unroll
+  for (int j = 0; j < 2 * OUT_LANES; j++) w[j] = transpose(w[j]);
+  if (!live) return;
   uint4* o = out + i * (uint64_t)(out_bytes / 16);
 #pragma unroll
-  for (int j = 0; j < 4; j++)
-    if (16u * j < out_bytes) o[j] = make_uint4(a[2 * j].lo, a[2 * j].hi, a[2 * j + 1].lo, a[2 * j + 1].hi);
+  for (int j = 0; j < OUT_LANES / 2; j++) o[j] = make_uint4(w[4 * j], w[4 * j + 1], w[4 * j + 2], w[4 * j + 3]);
 }
 
 // one thread absorbs the whole-block part of a constant prefix into a cached state

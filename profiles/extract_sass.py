@@ -1,6 +1,6 @@
 """Writes the SASS of the hot loops to profiles/sass/ (cuobjdump of the objects build.py leaves under capycrypt_b200/_lib).
 usage: python profiles/extract_sass.py
-  keccak_round_x2.sass     the two-round loop body of sha3_short_kernel<17, 8> (headline): 244 LOP3 + 116 SHF
+  keccak_round_x2.sass     the two-round loop body of sha3_short_kernel<17, 8> (headline, bitsliced): 248 LOP3 + 104 SHFL
   keccak_pair_round.sass   one iteration (4 rounds) of the split-lane permutation inside sponge_tiered_kernel<9>
   keccak_warp_round.sass   the first rounds of the unrolled one-lane-per-thread permutation
   fe_mul.sass / fe_sqr.sass the out-of-line field multiplication / squaring of ed448_var.cu
