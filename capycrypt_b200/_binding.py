@@ -76,6 +76,13 @@ SIGNATURES = {
     "capy_ed448_key_decrypt_batch": (i32, [vp, i32, u8p, u64p, u8p, u8p, u64p, u8p, u64, u8p, u8p]),
     "capy_ed448_key_encrypt_batch_dev": (i32, [vp, i32, vp, i32, u8p, u8p, u8p, u64p, u64, u8p, u8p, u8p, vp]),
     "capy_ed448_key_decrypt_batch_dev": (i32, [vp, i32, vp, i32, u8p, u64p, u8p, u8p, u64p, u8p, u64, u8p, u8p, vp]),
+    "capy_ed448_pub_prepare": (i32, [vp, u8p, C.POINTER(vp)]),
+    "capy_ed448_pub_uses_comb": (i32, [vp]),
+    "capy_ed448_pub_free": (None, [vp]),
+    "capy_ed448_verify_prepared_batch": (i32, [vp, i32, vp, u8p, u64p, u8p, u8p, u64, u8p]),
+    "capy_ed448_verify_prepared_batch_dev": (i32, [vp, i32, vp, i32, vp, u8p, u64p, u8p, u8p, u64, u8p]),
+    "capy_ed448_key_encrypt_prepared_batch": (i32, [vp, i32, vp, u8p, u8p, u64p, u64, u8p, u8p, u8p]),
+    "capy_ed448_key_encrypt_prepared_batch_dev": (i32, [vp, i32, vp, i32, vp, u8p, u8p, u64p, u64, u8p, u8p, u8p]),
 }
 
 

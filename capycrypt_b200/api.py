@@ -23,7 +23,8 @@ from typing import Optional, Sequence
 
 import numpy as np
 
-from .engine import Engine, pack
+from ._binding import ERR_BAD_POINT, CapyError
+from .engine import Engine, PreparedPublicKey, pack
 
 
 class OperationError(Exception):
@@ -162,6 +163,58 @@ class Gpu:
                     res[i] = OperationError("SignatureVerificationFailure")
         return res
 
+    # ---- one signer / one recipient --------------------------------------------------------------------
+    def prepare_public_key(self, pub_key: bytes) -> PreparedPublicKey:
+        """Prepares one public key (affine x || y, 112 bytes) for verify_prepared / key_encrypt_prepared: worth it when
+        the key is used for many messages, over one call or several.  OperationError("InvalidPublicKey") when the point
+        is not on the curve.  Close the key (or use it in a `with` block) before the engine."""
+        if len(pub_key) != 112:
+            raise OperationError("InvalidPublicKey")
+        try:
+            return self.engine.ed448_pub_prepare(pub_key)
+        except CapyError as e:
+            if e.status == ERR_BAD_POINT:
+                raise OperationError("InvalidPublicKey") from None
+            raise
+
+    def verify_prepared(self, msgs: Sequence[Message], key: PreparedPublicKey) -> list[Optional[OperationError]]:
+        """verify() with key as every message's public key: the same result per message."""
+        res: list[Optional[OperationError]] = [None] * len(msgs)
+        groups: dict[int, list[int]] = {}
+        for i, m in enumerate(msgs):
+            if m.sig is None:
+                res[i] = OperationError("SignatureNotSet")
+            elif m.d is None:
+                res[i] = OperationError("SecurityParameterNotSet")
+            elif len(m.sig.h) != 56 or len(m.sig.z) != 56:
+                res[i] = OperationError("SignatureVerificationFailure")
+            else:
+                groups.setdefault(int(m.d), []).append(i)
+        for d, idx in groups.items():
+            md, mo = pack([msgs[i].msg for i in idx])
+            h = np.frombuffer(b"".join(msgs[i].sig.h for i in idx), dtype=np.uint8)
+            z = np.frombuffer(b"".join(msgs[i].sig.z for i in idx), dtype=np.uint8)
+            ok = self.engine.ed448_verify_prepared(key, md, mo, h, z, d)
+            for i, o in zip(idx, ok):
+                if not o:
+                    res[i] = OperationError("SignatureVerificationFailure")
+        return res
+
+    def key_encrypt_prepared(self, msgs: Sequence[Message], key: PreparedPublicKey, d: SecParam,
+                             k_rand: Optional[Sequence[bytes]] = None) -> None:
+        """key_encrypt() with key as every message's recipient: the same fields, the same bytes."""
+        d = SecParam.try_from(int(d))
+        if k_rand is None:
+            k_rand = [os.urandom(56) for _ in msgs]
+        if len(k_rand) != len(msgs) or any(len(k) != 56 for k in k_rand):
+            raise ValueError("key_encrypt_prepared: one 56-byte nonce per message")
+        md, mo = pack([m.msg for m in msgs])
+        ct, tag, z = self.engine.ed448_key_encrypt_prepared(key, b"".join(k_rand), md, mo, int(d))
+        for i, m in enumerate(msgs):
+            m.msg = bytearray(ct[int(mo[i]):int(mo[i + 1])].tobytes())
+            m.digest = tag[i].tobytes()
+            m.asym_nonce = z[i].tobytes()
+            m.d = d
 
     # ---- SpongeEncryptable ---------------------------------------------------------------------------
     def sha3_encrypt(self, msgs: Sequence[Message], pws: Sequence[bytes], d: SecParam,

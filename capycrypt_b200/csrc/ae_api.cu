@@ -223,6 +223,20 @@ static AeCore ecdhies_core(int d, const uint8_t* keymat) {
   return c;
 }
 
+// Z = [k]G (:38) with kw = k in SoA words ; (ke || ka) from W.x ; tag and ciphertext (:40-48)
+static int key_encrypt_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint32_t* kw, const uint8_t* wx,
+                              const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy) {
+  CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
+  int rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true);
+  if (rc) return rc;
+  rc = launch_to_affine(ctx, st, proj, n, 0, nullptr, z_xy);
+  if (rc) return rc;
+  uint8_t* keymat;
+  rc = dev_ecdhies_keymat(ctx, dc, st, d, wx, n, &keymat);
+  if (rc) return rc;
+  return dev_ae_seal(ctx, dc, st, ecdhies_core(d, keymat), msgs, off, n, ct, tag);
+}
+
 static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pub, const uint8_t* k_rand,
                            const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy,
                            int* d_bad_flag) {
@@ -237,19 +251,37 @@ static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   if (rc) return rc;
   rc = launch_to_affine(ctx, st, proj, n, 1, bad, wx);
   if (rc) return rc;
-  // Z = [k]G (:38)
   rc = launch_scalar_prep(ctx, st, k_rand, 1, kw, nullptr, n);
   if (rc) return rc;
-  rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true);
-  if (rc) return rc;
-  rc = launch_to_affine(ctx, st, proj, n, 0, nullptr, z_xy);
-  if (rc) return rc;
-  uint8_t* keymat;
-  rc = dev_ecdhies_keymat(ctx, dc, st, d, wx, n, &keymat);
-  if (rc) return rc;
-  rc = dev_ae_seal(ctx, dc, st, ecdhies_core(d, keymat), msgs, off, n, ct, tag);
+  rc = key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy);
   if (rc) return rc;
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
+}
+
+// W = [k]V for a prepared V through V's comb table (k is secret: constant-time scan), then as dev_key_encrypt
+static int dev_key_encrypt_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const capy_ed448_pub* key,
+                                    const uint8_t* k_rand, const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct,
+                                    uint8_t* tag, uint8_t* z_xy) {
+  if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
+  if (n == 0) return CAPY_OK;
+  const uint32_t* v_table = key->d_table[dc.index];
+  if (!v_table) {  // V has a torsion component: the variable-base pipeline with V repeated
+    CAPY_SCRATCH(pub, uint8_t, kEdPubRep, n * 112);
+    const int rc = broadcast_point(ctx, st, key->d_xy[dc.index], pub, n);
+    if (rc) return rc;
+    return dev_key_encrypt(ctx, dc, st, d, pub, k_rand, msgs, off, n, ct, tag, z_xy, nullptr);
+  }
+  CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
+  CAPY_SCRATCH(wx, uint8_t, kAeWx, n * 56);
+  CAPY_SCRATCH(kw, uint32_t, kAeKw, n * 56);
+  // k = 4 * BE(rand) mod r ; W = [k]V (:36-37)
+  int rc = launch_scalar_prep(ctx, st, k_rand, 1, kw, nullptr, n);
+  if (rc) return rc;
+  rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true, v_table);
+  if (rc) return rc;
+  rc = launch_to_affine(ctx, st, proj, n, 1, nullptr, wx);
+  if (rc) return rc;
+  return key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy);
 }
 
 static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pws, const uint64_t* pw_off,
@@ -458,6 +490,50 @@ int capy_ed448_key_encrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_x
       uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost7, cnt * 112);
       if (!d_tag || !d_z) return CAPY_ERR_OOM;
       rc = dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z, d_flag);
+      if (rc) return rc;
+      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
+      if (rc) return rc;
+      CAPY_CUDA(ctx, cudaMemcpyAsync(tag56 + 56 * ch.i0, d_tag, cnt * 56, cudaMemcpyDeviceToHost, st));
+      CAPY_CUDA(ctx, cudaMemcpyAsync(z_xy112 + 112 * ch.i0, d_z, cnt * 112, cudaMemcpyDeviceToHost, st));
+      return CAPY_OK;
+    });
+  });
+}
+
+int capy_ed448_key_encrypt_prepared_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits,
+                                              const capy_ed448_pub* key, const uint8_t* d_k_rand56, const uint8_t* d_msgs,
+                                              const uint64_t* d_msg_off, uint64_t n, uint8_t* d_ct, uint8_t* d_tag56,
+                                              uint8_t* d_z_xy112) {
+  if (pub_check(ctx, key)) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
+  if (n && (!d_k_rand56 || !d_msgs || !d_msg_off || !d_ct || !d_tag56 || !d_z_xy112)) return CAPY_ERR_BAD_ARG;
+  return dev_key_encrypt_prepared(ctx, dc, st, d_bits, key, d_k_rand56, d_msgs, d_msg_off, n, d_ct, d_tag56, d_z_xy112);
+}
+
+int capy_ed448_key_encrypt_prepared_batch(capy_ctx* ctx, int d_bits, const capy_ed448_pub* key, const uint8_t* k_rand56,
+                                          const uint8_t* msgs, const uint64_t* msg_off, uint64_t n, uint8_t* ct,
+                                          uint8_t* tag56, uint8_t* z_xy112) {
+  if (!ctx || pub_check(ctx, key) || (n && (!k_rand56 || !msgs || !msg_off || !ct || !tag56 || !z_xy112)))
+    return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (n == 0) return CAPY_OK;
+  auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 16384);
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sm;
+      uint8_t* d_k = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost3, k_rand56 + 56 * ch.i0, (size_t)cnt * 56, &d_k);
+      if (rc) return rc;
+      StagedOut so;
+      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
+      if (rc) return rc;
+      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 56);
+      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost7, cnt * 112);
+      if (!d_tag || !d_z) return CAPY_ERR_OOM;
+      rc = dev_key_encrypt_prepared(ctx, dc, st, d_bits, key, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z);
       if (rc) return rc;
       rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
       if (rc) return rc;

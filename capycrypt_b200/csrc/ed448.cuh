@@ -248,21 +248,28 @@ CAPY_HD void pt_dual_isogeny(PtExt& r, const PtExt& p) {
   fe_mul(r.T, xn, yn);   // 2 x 3
 }
 
-// r = [k]G (extended, on E) for k in [0, r) via the comb table of phi(G) read from global memory
-// (the CUDA kernel in ed448_fixed.cu runs the same loop with the table rows staged through shared memory)
-CAPY_HD void pt_fixed_base_mul(PtExt& r, const Sc& k, const uint32_t* __restrict__ table, bool CONSTANT_TIME) {
+// r = [k]P (extended, on E) for k in [0, r) via the comb table of phi(P) read from global memory; with table2 the
+// windows of k2 over table2 (the comb table of phi(Q)) run into the same accumulator: r = [k]P + [k2]Q.  Exact when
+// P and Q both have odd order r.  (The CUDA kernel in ed448_fixed.cu runs the same loop with the table rows staged
+// through shared memory.)
+CAPY_HD void pt_fixed_base_mul(PtExt& r, const Sc& k, const uint32_t* __restrict__ table, bool CONSTANT_TIME,
+                               const Sc* k2 = nullptr, const uint32_t* __restrict__ table2 = nullptr) {
   const Sc inv4 = {CAPY_INV4_LIMBS};
-  Sc kq;
-  sc_mul_mod(kq, k, inv4);  // k / 4 mod r
   PtExt acc;
   pt_identity(acc);  // (0, 1) is the identity of E' too
-  uint32_t carry = 0;
 #pragma unroll 1
-  for (int i = 0; i < FB_WINDOWS; i++) {
-    const int dgt = fb_digit(kq, i, carry);
-    PtNiels e;
-    fb_lookup_row<false>(e, table + (size_t)i * FB_ENTRIES * FB_ENTRY_WORDS, dgt, CONSTANT_TIME);
-    pt_madd_tw<true>(acc, acc, e);
+  for (int pass = 0; pass < (table2 ? 2 : 1); pass++) {
+    const uint32_t* tab = pass ? table2 : table;
+    Sc kq;
+    sc_mul_mod(kq, pass ? *k2 : k, inv4);  // k / 4 mod r
+    uint32_t carry = 0;
+#pragma unroll 1
+    for (int i = 0; i < FB_WINDOWS; i++) {
+      const int dgt = fb_digit(kq, i, carry);
+      PtNiels e;
+      fb_lookup_row<false>(e, tab + (size_t)i * FB_ENTRIES * FB_ENTRY_WORDS, dgt, CONSTANT_TIME);
+      pt_madd_tw<true>(acc, acc, e);
+    }
   }
   pt_dual_isogeny(r, acc);
 }
@@ -561,12 +568,70 @@ CAPY_HD void pt_generator(PtExt& g) {
   fe_mul(g.T, g.X, g.Y);
 }
 
-// writes the 16 entries of window i: (j+1) * 32^i * phi(G) as canonical Niels triples.  The multiples are
-// formed on E with the complete formulas, taken to affine, then pushed through the isogeny
+// table entry e := phi(P) as the canonical Niels triple (y' - x', y' + x', 2 d' x' y'), P projective on E:
+// P is taken to affine, then pushed through the isogeny
 //   phi(x, y) = ( 2xy / (y^2 - x^2),  (y^2 + x^2) / (2 - y^2 - x^2) )     (a homomorphism E -> E')
-CAPY_HD void fb_build_window(uint32_t* row /*[16 * 48]*/, int i) {
-  PtExt base;
-  pt_generator(base);
+// The denominators vanish only at points of even order: P must have odd order.
+CAPY_HD void fb_niels_entry(uint32_t* e /*[48]*/, const PtExt& acc) {
+  Fe zi, x, y, x2, y2, u, v, w, t, xt, yt, two;
+  fe_inv(zi, acc.Z);
+  fe_mul_call(&x, &acc.X, &zi);
+  fe_mul_call(&y, &acc.Y, &zi);
+  fe_sqr_call(&x2, &x);
+  fe_sqr_call(&y2, &y);
+  fe_sub(u, y2, x2);       // y^2 - x^2, alpha 3
+  fe_weak(u);
+  fe_add(t, y2, x2);       // y^2 + x^2, alpha 2
+  fe_zero(two);
+  two.v[0] = 2;
+  fe_weak(t);
+  fe_sub(v, two, t);       // 2 - y^2 - x^2
+  fe_weak(v);
+  fe_mul_call(&w, &u, &v);
+  fe_inv(w, w);            // 1 / (u v)
+  fe_mul_call(&xt, &x, &y);
+  fe_add(xt, xt, xt);      // 2xy, alpha 2
+  fe_weak(xt);
+  fe_mul_call(&xt, &xt, &v);
+  fe_mul_call(&xt, &xt, &w);  // x' = 2xy / u
+  fe_mul_call(&yt, &t, &u);
+  fe_mul_call(&yt, &yt, &w);  // y' = (y^2 + x^2) / v
+  Fe ymx, ypx, td;
+  fe_sub(ymx, yt, xt);
+  fe_add(ypx, yt, xt);
+  fe_mul_call(&td, &xt, &yt);
+  uint64_t R[16];
+  for (int k = 0; k < 16; k++) R[k] = (uint64_t)td.v[k] * EDW_2D_TW_ABS;
+  Fe td_abs;
+  fe_carry_wide(td_abs, R);
+  fe_neg(td, td_abs);      // 2 d' x' y' with d' = -39082
+  fe_canon(ymx);
+  fe_canon(ypx);
+  fe_canon(td);
+  for (int k = 0; k < 16; k++) {
+    e[k] = ymx.v[k];
+    e[16 + k] = ypx.v[k];
+    e[32 + k] = td.v[k];
+  }
+}
+
+// table entry e := phi(P) for P = (x, y) given as 112 affine bytes (x || y, little-endian), P of odd order
+CAPY_HD void fb_niels_entry_xy(uint32_t* e /*[48]*/, const uint8_t* xy) {
+  uint32_t w[14];
+  Fe x, y;
+  for (int j = 0; j < 14; j++) w[j] = (uint32_t)xy[4 * j] | ((uint32_t)xy[4 * j + 1] << 8) | ((uint32_t)xy[4 * j + 2] << 16) | ((uint32_t)xy[4 * j + 3] << 24);
+  fe_from_words(x, w);
+  for (int j = 0; j < 14; j++) w[j] = (uint32_t)xy[56 + 4 * j] | ((uint32_t)xy[57 + 4 * j] << 8) | ((uint32_t)xy[58 + 4 * j] << 16) | ((uint32_t)xy[59 + 4 * j] << 24);
+  fe_from_words(y, w);
+  PtExt p;
+  pt_from_affine(p, x, y);
+  fb_niels_entry(e, p);
+}
+
+// writes the 16 entries of window i of P's comb table: (j+1) * 32^i * phi(P), j < 16.  The multiples are formed on E
+// with the complete formulas (5i doublings, then additions of 32^i P).
+CAPY_HD void fb_build_window(uint32_t* row /*[16 * 48]*/, int i, const PtExt& p) {
+  PtExt base = p;
 #pragma unroll 1
   for (int k = 0; k < FB_WBITS * i; k++) pt_double<true>(base, base);
   PtCached cb;
@@ -575,48 +640,15 @@ CAPY_HD void fb_build_window(uint32_t* row /*[16 * 48]*/, int i) {
 #pragma unroll 1
   for (int j = 0; j < FB_ENTRIES; j++) {
     if (j > 0) pt_add_cached<true>(acc, acc, cb);
-    Fe zi, x, y, x2, y2, u, v, w, t, xt, yt, two;
-    fe_inv(zi, acc.Z);
-    fe_mul_call(&x, &acc.X, &zi);
-    fe_mul_call(&y, &acc.Y, &zi);
-    fe_sqr_call(&x2, &x);
-    fe_sqr_call(&y2, &y);
-    fe_sub(u, y2, x2);       // y^2 - x^2, alpha 3
-    fe_weak(u);
-    fe_add(t, y2, x2);       // y^2 + x^2, alpha 2
-    fe_zero(two);
-    two.v[0] = 2;
-    fe_weak(t);
-    fe_sub(v, two, t);       // 2 - y^2 - x^2
-    fe_weak(v);
-    fe_mul_call(&w, &u, &v);
-    fe_inv(w, w);            // 1 / (u v)
-    fe_mul_call(&xt, &x, &y);
-    fe_add(xt, xt, xt);      // 2xy, alpha 2
-    fe_weak(xt);
-    fe_mul_call(&xt, &xt, &v);
-    fe_mul_call(&xt, &xt, &w);  // x' = 2xy / u
-    fe_mul_call(&yt, &t, &u);
-    fe_mul_call(&yt, &yt, &w);  // y' = (y^2 + x^2) / v
-    Fe ymx, ypx, td;
-    fe_sub(ymx, yt, xt);
-    fe_add(ypx, yt, xt);
-    fe_mul_call(&td, &xt, &yt);
-    uint64_t R[16];
-    for (int k = 0; k < 16; k++) R[k] = (uint64_t)td.v[k] * EDW_2D_TW_ABS;
-    Fe td_abs;
-    fe_carry_wide(td_abs, R);
-    fe_neg(td, td_abs);      // 2 d' x' y' with d' = -39082
-    fe_canon(ymx);
-    fe_canon(ypx);
-    fe_canon(td);
-    uint32_t* e = row + j * FB_ENTRY_WORDS;
-    for (int k = 0; k < 16; k++) {
-      e[k] = ymx.v[k];
-      e[16 + k] = ypx.v[k];
-      e[32 + k] = td.v[k];
-    }
+    fb_niels_entry(row + j * FB_ENTRY_WORDS, acc);
   }
+}
+
+// window i of G's comb table
+CAPY_HD void fb_build_window(uint32_t* row /*[16 * 48]*/, int i) {
+  PtExt g;
+  pt_generator(g);
+  fb_build_window(row, i, g);
 }
 
 }  // namespace capy

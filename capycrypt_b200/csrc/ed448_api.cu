@@ -260,6 +260,22 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
   return CAPY_OK;
 }
 
+// ux = U.x ; h' = KMACXOF(ux, m, 448, "T") ; ok = (h' == h) && !bad   (signable.rs:78-85)
+static int verify_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint32_t* proj_u, const uint8_t* d_msgs,
+                         const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* bad, uint64_t n, uint8_t* d_ok,
+                         int* d_bad_flag) {
+  CAPY_SCRATCH(ux, uint8_t, kEdTmp56A, n * 56);
+  CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
+  int rc = launch_to_affine(ctx, st, proj_u, n, 1, nullptr, ux);
+  if (rc) return rc;
+  rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, ux, nullptr, 56, d_msgs, d_msg_off, n, "T", hp));
+  if (rc) return rc;
+  verify_compare_kernel<<<grid_for(n, 256), 256, 0, st>>>(hp, d_h, bad, d_ok, d_bad_flag, n);
+  ctx->launches++;
+  CAPY_CUDA(ctx, cudaGetLastError());
+  return CAPY_OK;
+}
+
 static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pub, const uint8_t* d_msgs,
                       const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* d_z, uint64_t n, uint8_t* d_ok,
                       int* d_bad_flag) {
@@ -269,8 +285,6 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
   CAPY_SCRATCH(projA, uint32_t, kEdProj, n * 256);
   CAPY_SCRATCH(projB, uint32_t, kEdProj2, n * 256);
   CAPY_SCRATCH(bad, uint8_t, kEdBad, n);
-  CAPY_SCRATCH(ux, uint8_t, kEdTmp56A, n * 56);
-  CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
   // U = [z]G + [BE(h)]V with h unreduced (signable.rs:76-77, quirk Q10).  All inputs are public:
   // table lookups are direct, not scanned.
   int rc = launch_scalar_prep(ctx, st, d_z, 0, kw, nullptr, n);
@@ -279,14 +293,117 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
   if (rc) return rc;
   rc = launch_var_base(ctx, dc, st, d_h, 0, d_pub, projA, projB, bad, n, false);
   if (rc) return rc;
-  rc = launch_to_affine(ctx, st, projB, n, 1, nullptr, ux);
+  return verify_finish(ctx, dc, st, d, projB, d_msgs, d_msg_off, d_h, bad, n, d_ok, d_bad_flag);
+}
+
+// ---- prepared public keys ------------------------------------------------------------------------------
+// out[0 .. n) := the 112 bytes at d_xy: one copy, then ceil(log2 n) copies that double what is there
+int broadcast_point(capy_ctx* ctx, cudaStream_t st, const uint8_t* d_xy, uint8_t* out, uint64_t n) {
+  if (n == 0) return CAPY_OK;
+  CAPY_CUDA(ctx, cudaMemcpyAsync(out, d_xy, 112, cudaMemcpyDeviceToDevice, st));
+  for (uint64_t have = 1; have < n; have *= 2)
+    CAPY_CUDA(ctx, cudaMemcpyAsync(out + 112 * have, out, 112 * std::min(have, n - have), cudaMemcpyDeviceToDevice, st));
+  return CAPY_OK;
+}
+
+// U = [z]G + [h]V for a prepared V, then as dev_verify
+static int dev_verify_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const capy_ed448_pub* key,
+                               const uint8_t* d_msgs, const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* d_z,
+                               uint64_t n, uint8_t* d_ok) {
+  if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
+  if (n == 0) return CAPY_OK;
+  const uint32_t* v_table = key->d_table[dc.index];
+  if (!v_table) {  // V has a torsion component: the variable-base pipeline with V repeated
+    CAPY_SCRATCH(pub, uint8_t, kEdPubRep, n * 112);
+    const int rc = broadcast_point(ctx, st, key->d_xy[dc.index], pub, n);
+    if (rc) return rc;
+    return dev_verify(ctx, dc, st, d, pub, d_msgs, d_msg_off, d_h, d_z, n, d_ok, nullptr);
+  }
+  CAPY_SCRATCH(zw, uint32_t, kEdKWords, n * 56);
+  CAPY_SCRATCH(hw, uint32_t, kEdSWords, n * 56);
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
+  // One joint comb over G's and V's tables.  The reference multiplies V by the unreduced integer h (quirk Q10); h mod r
+  // gives the same point only because V has order r, which preparation checked ([r]V = identity) before it built V's
+  // table.  All inputs are public: table lookups are direct, not scanned.
+  int rc = launch_scalar_prep(ctx, st, d_z, 0, zw, nullptr, n);
   if (rc) return rc;
-  // h' = KMACXOF(U.x, m, 448, "T") (:79)
-  rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, ux, nullptr, 56, d_msgs, d_msg_off, n, "T", hp));
+  rc = launch_scalar_prep(ctx, st, d_h, 0, hw, nullptr, n);
   if (rc) return rc;
-  verify_compare_kernel<<<grid_for(n, 256), 256, 0, st>>>(hp, d_h, bad, d_ok, d_bad_flag, n);
-  ctx->launches++;
-  CAPY_CUDA(ctx, cudaGetLastError());
+  rc = launch_fixed_base(ctx, dc, st, zw, proj, n, false, nullptr, hw, v_table);
+  if (rc) return rc;
+  return verify_finish(ctx, dc, st, d, proj, d_msgs, d_msg_off, d_h, nullptr, n, d_ok, nullptr);
+}
+
+int pub_check(const capy_ctx* ctx, const capy_ed448_pub* key) {
+  return key && key->ctx == ctx ? CAPY_OK : CAPY_ERR_BAD_ARG;
+}
+
+// the items of the table build: (j+1) * 32^i * V for i < FB_WINDOWS, j < FB_ENTRIES (item 16 i + j), then [r]V
+constexpr uint64_t kPubTableItems = (uint64_t)FB_WINDOWS * FB_ENTRIES;
+
+static std::vector<uint8_t> pub_table_scalars() {
+  std::vector<uint8_t> s((kPubTableItems + 1) * 56);
+  for (int i = 0; i < FB_WINDOWS; i++) {
+    Sc p = {};
+    p.w[(FB_WBITS * i) >> 5] = 1u << ((FB_WBITS * i) & 31);  // 32^i < r
+    for (int j = 0; j < FB_ENTRIES; j++) {
+      Sc m = {}, o;
+      m.w[0] = (uint32_t)(j + 1);
+      sc_mul_mod(o, p, m);
+      sc_to_be(&s[56 * (FB_ENTRIES * i + j)], o);
+    }
+  }
+  const Sc r = {CAPY_R_LIMBS};
+  sc_to_be(&s[56 * kPubTableItems], r);
+  return s;
+}
+
+struct DevTemp {  // cudaMalloc'ed for the duration of a scope
+  void* p = nullptr;
+  ~DevTemp() {
+    if (p) cudaFree(p);
+  }
+};
+
+// V's bytes on this device and, when *comb (on entry: still possible), its comb table: the multiples through the
+// variable-base pipeline (public scalars, direct lookups), to affine, into table entries (fb_table_kernel).  *comb is
+// cleared when [r]V is not the identity.
+static int pub_build_device(capy_ctx* ctx, DeviceCtx& dc, const std::vector<uint8_t>& scalars, capy_ed448_pub* key,
+                            bool* comb) {
+  const cudaStream_t st = dc.streams[0];
+  const int k = dc.index;
+  CAPY_CUDA(ctx, cudaMalloc(&key->d_xy[k], 112));
+  CAPY_CUDA(ctx, cudaMemcpy(key->d_xy[k], key->xy, 112, cudaMemcpyHostToDevice));
+  if (!*comb) return CAPY_OK;
+  const uint64_t m = kPubTableItems + 1;
+  DevTemp sc, pts, proj, aff;
+  CAPY_CUDA(ctx, cudaMalloc(&sc.p, m * 56));
+  CAPY_CUDA(ctx, cudaMalloc(&pts.p, m * 112));
+  CAPY_CUDA(ctx, cudaMalloc(&proj.p, m * 256));
+  CAPY_CUDA(ctx, cudaMalloc(&aff.p, m * 112));
+  CAPY_CUDA(ctx, cudaMemcpyAsync(sc.p, scalars.data(), m * 56, cudaMemcpyHostToDevice, st));
+  int rc = broadcast_point(ctx, st, key->d_xy[k], (uint8_t*)pts.p, m);
+  if (rc) return rc;
+  rc = launch_var_base(ctx, dc, st, (const uint8_t*)sc.p, 0, (const uint8_t*)pts.p, nullptr, (uint32_t*)proj.p, nullptr, m,
+                       false);
+  if (rc) return rc;
+  rc = launch_to_affine(ctx, st, (const uint32_t*)proj.p, m, 0, nullptr, (uint8_t*)aff.p);
+  if (rc) return rc;
+  uint8_t rv[112];
+  CAPY_CUDA(ctx, cudaMemcpyAsync(rv, (const uint8_t*)aff.p + 112 * kPubTableItems, 112, cudaMemcpyDeviceToHost, st));
+  CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+  bool identity = rv[56] == 1;  // (0, 1)
+  for (int b = 0; b < 112; b++)
+    if (b != 56 && rv[b]) identity = false;
+  if (!identity) {
+    *comb = false;
+    return CAPY_OK;
+  }
+  CAPY_CUDA(ctx, cudaMalloc(&key->d_table[k], kFbTableBytes));
+  rc = launch_fb_table_from_points(ctx, st, (const uint8_t*)aff.p, key->d_table[k]);
+  if (rc) return rc;
+  // later calls may launch on other (non-blocking) streams and must not see a half-built table
+  CAPY_CUDA(ctx, cudaStreamSynchronize(st));
   return CAPY_OK;
 }
 
@@ -461,6 +578,92 @@ int capy_ed448_verify_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112,
       return copy_out(ctx, dc, st, kHost5, ok + ch.i0, d_ok, cnt);
     });
   });
+}
+
+int capy_ed448_verify_prepared_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const capy_ed448_pub* key,
+                                         const uint8_t* d_msgs, const uint64_t* d_msg_off, const uint8_t* d_h56,
+                                         const uint8_t* d_z_be56, uint64_t n, uint8_t* d_ok) {
+  if (pub_check(ctx, key)) return CAPY_ERR_BAD_ARG;
+  CAPY_DEV_PROLOGUE
+  if (n && (!d_msgs || !d_msg_off || !d_h56 || !d_z_be56 || !d_ok)) return CAPY_ERR_BAD_ARG;
+  return dev_verify_prepared(ctx, dc, st, d_bits, key, d_msgs, d_msg_off, d_h56, d_z_be56, n, d_ok);
+}
+
+int capy_ed448_verify_prepared_batch(capy_ctx* ctx, int d_bits, const capy_ed448_pub* key, const uint8_t* msgs,
+                                     const uint64_t* msg_off, const uint8_t* h56, const uint8_t* z_be56, uint64_t n,
+                                     uint8_t* ok) {
+  if (!ctx || pub_check(ctx, key) || (n && (!msgs || !msg_off || !h56 || !z_be56 || !ok))) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (n == 0) return CAPY_OK;
+  auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
+    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
+      const uint64_t cnt = ch.i1 - ch.i0;
+      StagedPacked sm;
+      uint8_t *d_h = nullptr, *d_z = nullptr;
+      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost3, h56 + 56 * ch.i0, cnt * 56, &d_h);
+      if (rc) return rc;
+      rc = h2d(ctx, dc, st, kHost4, z_be56 + 56 * ch.i0, cnt * 56, &d_z);
+      if (rc) return rc;
+      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost5, cnt);
+      if (!d_ok) return CAPY_ERR_OOM;
+      rc = dev_verify_prepared(ctx, dc, st, d_bits, key, sm.d_base, sm.d_off, d_h, d_z, cnt, d_ok);
+      if (rc) return rc;
+      return copy_out(ctx, dc, st, kHost5, ok + ch.i0, d_ok, cnt);
+    });
+  });
+}
+
+int capy_ed448_pub_prepare(capy_ctx* ctx, const uint8_t* pub_xy112, capy_ed448_pub** out_key) {
+  if (!out_key) return CAPY_ERR_BAD_ARG;
+  *out_key = nullptr;
+  if (!ctx || !pub_xy112) return CAPY_ERR_BAD_ARG;
+  {  // on the curve?  (the decoding and the test of var_base_kernel)
+    uint32_t w[14];
+    Fe x, y;
+    PtExt p;
+    memcpy(w, pub_xy112, 56);
+    fe_from_words(x, w);
+    memcpy(w, pub_xy112 + 56, 56);
+    fe_from_words(y, w);
+    if (!pt_from_affine(p, x, y)) return CAPY_ERR_BAD_POINT;
+  }
+  capy_ed448_pub* key = new (std::nothrow) capy_ed448_pub();
+  if (!key) return CAPY_ERR_OOM;
+  key->ctx = ctx;
+  memcpy(key->xy, pub_xy112, 112);
+  const size_t nd = ctx->devs.size();
+  for (const DeviceCtx& dc : ctx->devs) key->dev.push_back(dc.dev);
+  key->d_xy.assign(nd, nullptr);
+  key->d_table.assign(nd, nullptr);
+  const std::vector<uint8_t> scalars = pub_table_scalars();
+  bool comb = true;
+  for (DeviceCtx& dc : ctx->devs) {
+    std::lock_guard<std::mutex> lk(*dc.mu);
+    DeviceGuard g(dc.dev);
+    const int rc = pub_build_device(ctx, dc, scalars, key, &comb);
+    if (rc) {
+      capy_ed448_pub_free(key);
+      return rc;
+    }
+  }
+  key->comb = comb;  // decided on the first device: the others run the same arithmetic
+  *out_key = key;
+  return CAPY_OK;
+}
+
+int capy_ed448_pub_uses_comb(const capy_ed448_pub* key) { return key && key->comb ? 1 : 0; }
+
+void capy_ed448_pub_free(capy_ed448_pub* key) {
+  if (!key) return;
+  for (size_t k = 0; k < key->dev.size(); k++) {
+    DeviceGuard g(key->dev[k]);
+    if (key->d_table[k]) cudaFree(key->d_table[k]);  // cudaFree waits for work that still reads it
+    if (key->d_xy[k]) cudaFree(key->d_xy[k]);
+  }
+  delete key;
 }
 
 int capy_ed448_ecdh_batch(capy_ctx* ctx, const uint8_t* k_rand56, const uint8_t* pub_xy112, uint64_t n, uint8_t* wx56,

@@ -17,8 +17,13 @@ __device__ __forceinline__ void store_ext(uint32_t* __restrict__ proj, uint64_t 
 }
 
 // ed448_fixed.cu
+// proj = [k]G, or [k]V with `table` = the comb table of V; with table2 also + [k2]V2 (joint comb, one launch)
 int launch_fixed_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint32_t* k_words, uint32_t* proj, uint64_t n,
-                      bool constant_time);
+                      bool constant_time, const uint32_t* table = nullptr, const uint32_t* k2_words = nullptr,
+                      const uint32_t* table2 = nullptr);
+// table := comb table of V from the FB_WINDOWS * FB_ENTRIES affine multiples (j+1) * 32^i * V, item 16 i + j
+int launch_fb_table_from_points(capy_ctx* ctx, cudaStream_t st, const uint8_t* points_xy, uint32_t* table);
+constexpr size_t kFbTableBytes = (size_t)FB_WINDOWS * FB_ENTRIES * FB_ENTRY_WORDS * sizeof(uint32_t);
 // ed448_var.cu
 int launch_var_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* scalars, int mode4, const uint8_t* points,
                     const uint32_t* addend, uint32_t* proj, uint8_t* bad, uint64_t n, bool constant_time);
@@ -28,6 +33,10 @@ int launch_scalar_prep(capy_ctx* ctx, cudaStream_t st, const uint8_t* in, int mo
 int launch_to_affine(capy_ctx* ctx, cudaStream_t st, const uint32_t* proj, uint64_t n, int mode, const uint8_t* bad, uint8_t* out);
 // *bad_flag |= 1 when any of bad[0 .. n) is set
 int launch_any_bad(capy_ctx* ctx, cudaStream_t st, const uint8_t* bad, int* bad_flag, uint64_t n);
+// out[0 .. n) := the 112 bytes at d_xy (device to device copies)
+int broadcast_point(capy_ctx* ctx, cudaStream_t st, const uint8_t* d_xy, uint8_t* out, uint64_t n);
+// CAPY_ERR_BAD_ARG unless key was prepared by ctx
+int pub_check(const capy_ctx* ctx, const capy_ed448_pub* key);
 int dev_secret_scalar(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pws, const uint64_t* d_pw_off,
                       uint64_t n, uint32_t* s_words, uint8_t* s_be);
 

@@ -33,6 +33,7 @@ enum Slot {
   kChainStates, kChainSync,  // chain hand-off of launch_sponge_chain / launch_chain_jobs: states, tickets
   // Ed448 pipelines (ed448_api.cu)
   kEdKWords, kEdSWords, kEdProj, kEdProj2, kEdBad, kEdTmp56A, kEdTmp56B, kEdTmp56C,
+  kEdPubRep,                // a prepared key's point repeated n times (the fallback of the prepared entry points)
   // AE pipelines (ae_api.cu)
   kAeKeys, kAeKeyOff, kAeKeyMat, kAeTNew, kAeWx, kAeProj, kAeBad, kAeKw, kAeSk,
   kSlotsPerStream
@@ -173,6 +174,17 @@ struct capy_ctx {
   std::string last_cuda_error;
   std::atomic<uint64_t> launches{0};
   std::atomic<int> plan_cache{0};
+};
+
+// A public key prepared for many operations (capy_ed448_pub_prepare, ed448_api.cu).  Owns, on every device of the ctx
+// that prepared it, V's affine bytes and -- when V has order r -- the comb table of phi(V).
+struct capy_ed448_pub {
+  const capy_ctx* ctx = nullptr;
+  uint8_t xy[112] = {};
+  bool comb = false;
+  std::vector<int> dev;            // CUDA device of every ctx device (frees without the ctx)
+  std::vector<uint8_t*> d_xy;      // [device index] V's 112 affine bytes
+  std::vector<uint32_t*> d_table;  // [device index] comb table of phi(V), or nullptr
 };
 
 namespace capy {

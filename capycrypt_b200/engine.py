@@ -73,6 +73,38 @@ def pack(items) -> tuple[np.ndarray, np.ndarray]:
     return data, off
 
 
+class PreparedPublicKey:
+    """A public key prepared on every device of one Engine (Engine.ed448_pub_prepare): the comb table of V that the
+    engine's *_prepared calls use.  Reuse it across calls; close() it (or leave the `with` block) before the engine."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, pub_xy112: bytes):
+        self._engine = engine
+        self.handle = handle
+        self.pub_xy112 = pub_xy112
+
+    @property
+    def uses_comb(self) -> bool:
+        """False when V has a torsion component: the prepared calls then run the variable-base pipelines"""
+        return self._engine.lib.capy_ed448_pub_uses_comb(self.handle) == 1
+
+    def close(self):
+        if self.handle is not None and self.handle.value:
+            self._engine.lib.capy_ed448_pub_free(self.handle)
+        self.handle = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Engine:
     """One capy_ctx.  devices=None -> current CUDA device."""
 
@@ -293,6 +325,40 @@ class Engine:
                                                                _hp(ct), _hp(tag), _hp(z)), allow=(B.ERR_BAD_POINT,))
         return rc, ct, tag, z
 
+    def ed448_pub_prepare(self, pub_xy112) -> PreparedPublicKey:
+        """capy_ed448_pub_prepare (blocking); CapyError(ERR_BAD_POINT) for an off-curve point."""
+        pub = _u8(pub_xy112)
+        if len(pub) != 112:
+            raise ValueError(f"pub_prepare: {len(pub)} bytes, need 112")
+        h = C.c_void_p()
+        self._check(self.lib.capy_ed448_pub_prepare(self._ctx, _hp(pub), C.byref(h)))
+        return PreparedPublicKey(self, h, pub.tobytes())
+
+    def ed448_verify_prepared(self, key: PreparedPublicKey, msgs, msg_off, h56, z_be56, d: int,
+                              ok_out: np.ndarray | None = None) -> np.ndarray:
+        """ed448_verify with every public key = the prepared one."""
+        msgs, msg_off, h, z = _u8(msgs), _u64(msg_off), _u8(h56), _u8(z_be56)
+        n = _need_packed(msgs, msg_off, "verify messages")
+        if len(h) != n * 56 or len(z) != n * 56:
+            raise ValueError(f"verify: h/z hold {len(h)}/{len(z)} bytes, need {n} x 56/56")
+        ok = _out(ok_out, (n,), "verify flags")
+        self._check(self.lib.capy_ed448_verify_prepared_batch(self._ctx, d, key.handle, _hp(msgs), _hp(msg_off), _hp(h),
+                                                              _hp(z), n, _hp(ok)))
+        return ok
+
+    def ed448_key_encrypt_prepared(self, key: PreparedPublicKey, k_rand56, msgs, msg_off, d: int):
+        """ed448_key_encrypt with every public key = the prepared one -> (ciphertext, tags n x 56, nonce points Z n x 112)."""
+        k, msgs, msg_off = _u8(k_rand56), _u8(msgs), _u64(msg_off)
+        n = _need_packed(msgs, msg_off, "key_encrypt messages")
+        if len(k) != n * 56:
+            raise ValueError(f"key_encrypt: k holds {len(k)} bytes, need {n} x 56")
+        ct = np.zeros(len(msgs), dtype=np.uint8)
+        tag = np.zeros((n, 56), dtype=np.uint8)
+        z = np.zeros((n, 112), dtype=np.uint8)
+        self._check(self.lib.capy_ed448_key_encrypt_prepared_batch(self._ctx, d, key.handle, _hp(k), _hp(msgs), _hp(msg_off),
+                                                                   n, _hp(ct), _hp(tag), _hp(z)))
+        return ct, tag, z
+
     def ed448_key_decrypt(self, pws, pw_off, z_xy112, ct, ct_off, tags, d: int):
         """-> (rc, buffer packed like ct, ok n)."""
         pws, pw_off, z, ct, ct_off, tags = _u8(pws), _u64(pw_off), _u8(z_xy112), _u8(ct), _u64(ct_off), _u8(tags)
@@ -420,3 +486,18 @@ class Engine:
             self._ctx, dev_index, self._stream(), d, t_pws.data_ptr(), t_pw_off.data_ptr(), t_z.data_ptr(),
             t_ct.data_ptr(), t_ct_off.data_ptr(), t_tag.data_ptr(), n, t_out.data_ptr(), t_ok.data_ptr(),
             t_bad.data_ptr() if t_bad is not None else None))
+
+    def ed448_verify_prepared_dev(self, key: PreparedPublicKey, t_msgs, t_msg_off, t_h, t_z, d: int, t_ok,
+                                  dev_index: int = 0):
+        n = t_msg_off.numel() - 1
+        self._check(self.lib.capy_ed448_verify_prepared_batch_dev(self._ctx, dev_index, self._stream(), d, key.handle,
+                                                                  t_msgs.data_ptr(), t_msg_off.data_ptr(), t_h.data_ptr(),
+                                                                  t_z.data_ptr(), n, t_ok.data_ptr()))
+        return t_ok
+
+    def ed448_key_encrypt_prepared_dev(self, key: PreparedPublicKey, t_k, t_msgs, t_msg_off, d: int, t_ct, t_tag, t_z,
+                                       dev_index: int = 0):
+        n = t_msg_off.numel() - 1
+        self._check(self.lib.capy_ed448_key_encrypt_prepared_batch_dev(
+            self._ctx, dev_index, self._stream(), d, key.handle, t_k.data_ptr(), t_msgs.data_ptr(), t_msg_off.data_ptr(),
+            n, t_ct.data_ptr(), t_tag.data_ptr(), t_z.data_ptr()))

@@ -95,6 +95,33 @@ inline void pack(const Items& items, GetBytes get, Bytes& data, std::vector<uint
 }
 }  // namespace detail
 
+// A public key prepared on every device of one Engine (Engine::prepare): the comb table of V that the verify /
+// key_encrypt overloads taking it use instead of the variable-base ladder.  Reuse it across calls; destroy it before
+// the Engine.
+class PreparedPublicKey {
+ public:
+  PreparedPublicKey(PreparedPublicKey&& o) noexcept : key_(o.key_) { o.key_ = nullptr; }
+  PreparedPublicKey& operator=(PreparedPublicKey&& o) noexcept {
+    if (this != &o) {
+      capy_ed448_pub_free(key_);
+      key_ = o.key_;
+      o.key_ = nullptr;
+    }
+    return *this;
+  }
+  PreparedPublicKey(const PreparedPublicKey&) = delete;
+  PreparedPublicKey& operator=(const PreparedPublicKey&) = delete;
+  ~PreparedPublicKey() { capy_ed448_pub_free(key_); }
+  // false when V has a torsion component: the prepared calls then run the generic pipelines (same results)
+  bool uses_comb() const { return capy_ed448_pub_uses_comb(key_) == 1; }
+  const capy_ed448_pub* raw() const { return key_; }
+
+ private:
+  friend class Engine;
+  explicit PreparedPublicKey(capy_ed448_pub* k) : key_(k) {}
+  capy_ed448_pub* key_ = nullptr;
+};
+
 class Engine {
  public:
   explicit Engine(const std::vector<int>& devices = {}) {
@@ -204,6 +231,70 @@ class Engine {
         if (!ok[k]) res[idx[k]] = OperationError::SignatureVerificationFailure;
     }
     return res;
+  }
+
+  // prepares V for many verify / key_encrypt calls (blocking); GpuError(CAPY_ERR_BAD_POINT) when V is off the curve
+  PreparedPublicKey prepare(const AffinePoint& pub) {
+    capy_ed448_pub* k = nullptr;
+    check(capy_ed448_pub_prepare(ctx_, pub.data(), &k));
+    return PreparedPublicKey(k);
+  }
+
+  // Signable::verify of every message against one signer: result[i] as verify() gives it with pubs[i] = the key
+  std::vector<std::optional<OperationError>> verify(const std::vector<Message>& msgs, const PreparedPublicKey& key) {
+    std::vector<std::optional<OperationError>> res(msgs.size());
+    for (int d_bits : {224, 256, 384, 512}) {
+      std::vector<size_t> idx;
+      for (size_t i = 0; i < msgs.size(); i++) {
+        if (!msgs[i].sig) res[i] = OperationError::SignatureNotSet;
+        else if (!msgs[i].d) res[i] = OperationError::SecurityParameterNotSet;
+        else if ((int)*msgs[i].d == d_bits) {
+          if (msgs[i].sig->h.size() != 56) res[i] = OperationError::SignatureVerificationFailure;
+          else idx.push_back(i);
+        }
+      }
+      if (idx.empty()) continue;
+      Bytes md, h, z;
+      std::vector<uint64_t> mo(1, 0);
+      for (size_t i : idx) {
+        md.insert(md.end(), msgs[i].msg.begin(), msgs[i].msg.end());
+        mo.push_back(md.size());
+        h.insert(h.end(), msgs[i].sig->h.begin(), msgs[i].sig->h.end());
+        z.insert(z.end(), msgs[i].sig->z.begin(), msgs[i].sig->z.end());
+      }
+      if (md.empty()) md.push_back(0);
+      Bytes ok(idx.size());
+      check(capy_ed448_verify_prepared_batch(ctx_, d_bits, key.raw(), md.data(), mo.data(), h.data(), z.data(), idx.size(),
+                                             ok.data()));
+      for (size_t k = 0; k < idx.size(); k++)
+        if (!ok[k]) res[idx[k]] = OperationError::SignatureVerificationFailure;
+    }
+    return res;
+  }
+
+  // KeyEncryptable::key_encrypt of every message to one recipient (as key_encrypt() with pubs[i] = the key)
+  std::optional<OperationError> key_encrypt(std::vector<Message>& msgs, const PreparedPublicKey& key, int d_bits,
+                                            const std::vector<std::array<uint8_t, 56>>* k_rand = nullptr) {
+    if (!sec_param_try_from(d_bits)) return OperationError::UnsupportedSecurityParameter;
+    const size_t n = msgs.size();
+    Bytes md, ks(n * 56 + 1);
+    std::vector<uint64_t> mo;
+    detail::pack(msgs, [](const Message& m) -> const Bytes& { return m.msg; }, md, mo);
+    std::random_device rd;
+    for (size_t i = 0; i < n; i++)
+      for (size_t k = 0; k < 56; k++) ks[56 * i + k] = k_rand ? (*k_rand)[i][k] : (uint8_t)rd();
+    Bytes ct(md.size()), tag(n * 56 + 1), z(n * 112 + 1);
+    check(capy_ed448_key_encrypt_prepared_batch(ctx_, d_bits, key.raw(), ks.data(), md.data(), mo.data(), n, ct.data(),
+                                                tag.data(), z.data()));
+    for (size_t i = 0; i < n; i++) {
+      msgs[i].msg.assign(ct.begin() + mo[i], ct.begin() + mo[i + 1]);
+      msgs[i].digest.assign(tag.begin() + 56 * i, tag.begin() + 56 * (i + 1));
+      AffinePoint zp;
+      std::copy(z.begin() + 112 * i, z.begin() + 112 * (i + 1), zp.begin());
+      msgs[i].asym_nonce = zp;
+      msgs[i].d = *sec_param_try_from(d_bits);
+    }
+    return std::nullopt;
   }
 
   // SpongeEncryptable::sha3_encrypt (sha3/encryptable.rs:29-45): msg <- ciphertext, digest <- tag, sym_nonce <- z.

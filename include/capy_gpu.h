@@ -267,6 +267,37 @@ int capy_ed448_key_decrypt_batch_dev(capy_ctx* ctx, int dev_index, void* stream,
                                      const uint64_t* d_ct_off, const uint8_t* d_tag56, uint64_t n, uint8_t* d_out,
                                      uint8_t* d_ok, int* d_bad_flag);
 
+/* ---- Prepared public keys: many verifications against one signer, many encryptions to one recipient ------------------
+ * Preparing V builds, on every device of the ctx, the comb table of phi(V) (270 KB per device, the layout of G's
+ * table).  Verification then computes [z]G + [h]V as one joint comb (two table walks into one accumulator, no
+ * doublings) and key_encrypt computes W = [k]V with a second comb instead of the variable-base ladder.  A key is
+ * reused across calls: the preparation (a few ms) pays for itself over all the items verified or encrypted with it.
+ * Results are byte for byte those of capy_ed448_verify_batch / capy_ed448_key_encrypt_batch with V repeated n times,
+ * for every on-curve V. */
+typedef struct capy_ed448_pub capy_ed448_pub;
+/* Blocking.  CAPY_ERR_BAD_POINT if V is off the curve (*out_key stays NULL).  A V outside the prime-order subgroup (a
+ * torsion component) gets no table: the prepared entry points then run the variable-base pipelines, same bytes. */
+int capy_ed448_pub_prepare(capy_ctx* ctx, const uint8_t* pub_xy112, capy_ed448_pub** out_key);
+/* 1 = V has a comb table, 0 = the prepared entry points fall back to the variable-base pipelines */
+int capy_ed448_pub_uses_comb(const capy_ed448_pub* key);
+/* Releases the key's device memory.  NULL is a no-op.  Call before capy_gpu_destroy of its ctx. */
+void capy_ed448_pub_free(capy_ed448_pub* key);
+/* capy_ed448_verify_batch with pub_xy112[i] = V for every i.  A key prepared by another ctx: CAPY_ERR_BAD_ARG. */
+int capy_ed448_verify_prepared_batch(capy_ctx* ctx, int d_bits, const capy_ed448_pub* key, const uint8_t* msgs,
+                                     const uint64_t* msg_off, const uint8_t* h56, const uint8_t* z_be56, uint64_t n,
+                                     uint8_t* ok);
+int capy_ed448_verify_prepared_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits, const capy_ed448_pub* key,
+                                         const uint8_t* d_msgs, const uint64_t* d_msg_off, const uint8_t* d_h56,
+                                         const uint8_t* d_z_be56, uint64_t n, uint8_t* d_ok);
+/* capy_ed448_key_encrypt_batch with pub_xy112[i] = V for every i */
+int capy_ed448_key_encrypt_prepared_batch(capy_ctx* ctx, int d_bits, const capy_ed448_pub* key, const uint8_t* k_rand56,
+                                          const uint8_t* msgs, const uint64_t* msg_off, uint64_t n, uint8_t* ct,
+                                          uint8_t* tag56, uint8_t* z_xy112);
+int capy_ed448_key_encrypt_prepared_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bits,
+                                              const capy_ed448_pub* key, const uint8_t* d_k_rand56, const uint8_t* d_msgs,
+                                              const uint64_t* d_msg_off, uint64_t n, uint8_t* d_ct, uint8_t* d_tag56,
+                                              uint8_t* d_z_xy112);
+
 #ifdef __cplusplus
 }
 #endif

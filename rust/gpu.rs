@@ -17,6 +17,11 @@ pub struct CapyCtx {
     _private: [u8; 0],
 }
 
+#[repr(C)]
+pub struct CapyEd448Pub {
+    _private: [u8; 0],
+}
+
 #[link(name = "capycrypt_gpu", kind = "static")]
 extern "C" {
     fn capy_gpu_init(devices: *const c_int, n_devices: c_int, out_ctx: *mut *mut CapyCtx) -> c_int;
@@ -111,6 +116,20 @@ extern "C" {
     fn capy_ed448_key_decrypt_batch_dev(ctx: *mut CapyCtx, dev_index: c_int, stream: *mut c_void, d_bits: c_int,
         d_pws: *const u8, d_pw_off: *const u64, d_z_xy112: *const u8, d_ct: *const u8, d_ct_off: *const u64,
         d_tag56: *const u8, n: u64, d_out: *mut u8, d_ok: *mut u8, d_bad_flag: *mut c_int) -> c_int;
+    fn capy_ed448_pub_prepare(ctx: *mut CapyCtx, pub_xy112: *const u8, out_key: *mut *mut CapyEd448Pub) -> c_int;
+    fn capy_ed448_pub_uses_comb(key: *const CapyEd448Pub) -> c_int;
+    fn capy_ed448_pub_free(key: *mut CapyEd448Pub);
+    fn capy_ed448_verify_prepared_batch(ctx: *mut CapyCtx, d_bits: c_int, key: *const CapyEd448Pub, msgs: *const u8,
+        msg_off: *const u64, h56: *const u8, z_be56: *const u8, n: u64, ok: *mut u8) -> c_int;
+    fn capy_ed448_verify_prepared_batch_dev(ctx: *mut CapyCtx, dev_index: c_int, stream: *mut c_void, d_bits: c_int,
+        key: *const CapyEd448Pub, d_msgs: *const u8, d_msg_off: *const u64, d_h56: *const u8, d_z_be56: *const u8,
+        n: u64, d_ok: *mut u8) -> c_int;
+    fn capy_ed448_key_encrypt_prepared_batch(ctx: *mut CapyCtx, d_bits: c_int, key: *const CapyEd448Pub,
+        k_rand56: *const u8, msgs: *const u8, msg_off: *const u64, n: u64, ct: *mut u8, tag56: *mut u8,
+        z_xy112: *mut u8) -> c_int;
+    fn capy_ed448_key_encrypt_prepared_batch_dev(ctx: *mut CapyCtx, dev_index: c_int, stream: *mut c_void,
+        d_bits: c_int, key: *const CapyEd448Pub, d_k_rand56: *const u8, d_msgs: *const u8, d_msg_off: *const u64,
+        n: u64, d_ct: *mut u8, d_tag56: *mut u8, d_z_xy112: *mut u8) -> c_int;
 }
 
 const CAPY_AE_SHA3: c_int = 0;
@@ -410,6 +429,100 @@ impl Gpu {
             }
         }
         res
+    }
+}
+
+/// A public key prepared on every device of one `Gpu` (`Gpu::prepare_public_key`): the comb table of V that
+/// `Gpu::verify_prepared` and `Gpu::key_encrypt_prepared` use instead of the variable-base ladder.  Reuse it across
+/// calls; drop it before the `Gpu` that prepared it.
+pub struct PreparedKey {
+    key: *mut CapyEd448Pub,
+}
+unsafe impl Send for PreparedKey {}
+
+impl PreparedKey {
+    /// false when V has a torsion component: the prepared calls then run the generic pipelines (same results)
+    pub fn uses_comb(&self) -> bool {
+        unsafe { capy_ed448_pub_uses_comb(self.key) == 1 }
+    }
+}
+
+impl Drop for PreparedKey {
+    fn drop(&mut self) {
+        unsafe { capy_ed448_pub_free(self.key) }
+    }
+}
+
+impl Gpu {
+    /// Prepares V for many `verify_prepared` / `key_encrypt_prepared` calls (blocking, a few ms per device).
+    pub fn prepare_public_key(&self, pub_key: &ExtendedPoint) -> Result<PreparedKey, OperationError> {
+        let xy = point_to_xy(pub_key);
+        let mut key = std::ptr::null_mut();
+        status(unsafe { capy_ed448_pub_prepare(self.ctx, xy.as_ptr(), &mut key) })?;
+        Ok(PreparedKey { key })
+    }
+
+    /// Batched `Signable::verify` of every message against one signer; same errors as `verify`.
+    pub fn verify_prepared(&self, msgs: &[Message], key: &PreparedKey) -> Vec<Result<(), OperationError>> {
+        let mut res: Vec<Result<(), OperationError>> = msgs.iter().map(|_| Ok(())).collect();
+        for d in [SecParam::D224, SecParam::D256, SecParam::D384, SecParam::D512] {
+            let mut idx = Vec::new();
+            for (i, m) in msgs.iter().enumerate() {
+                if m.sig.is_none() {
+                    res[i] = Err(OperationError::SignatureNotSet);
+                } else if m.d.is_none() {
+                    res[i] = Err(OperationError::SecurityParameterNotSet);
+                } else if m.d == Some(d) {
+                    if m.sig.as_ref().unwrap().h.len() == 56 {
+                        idx.push(i);
+                    } else {
+                        res[i] = Err(OperationError::SignatureVerificationFailure);
+                    }
+                }
+            }
+            if idx.is_empty() {
+                continue;
+            }
+            let (mut h, mut z) = (Vec::new(), Vec::new());
+            for &i in &idx {
+                let sig = msgs[i].sig.as_ref().unwrap();
+                h.extend_from_slice(&sig.h);
+                z.extend_from_slice(&sig.z.val.to_be_bytes());
+            }
+            let (md, mo) = pack(idx.iter().map(|&i| msgs[i].msg.as_slice()));
+            let mut ok = vec![0u8; idx.len()];
+            let rc = unsafe {
+                capy_ed448_verify_prepared_batch(self.ctx, d as c_int, key.key, md.as_ptr(), mo.as_ptr(), h.as_ptr(),
+                                                 z.as_ptr(), idx.len() as u64, ok.as_mut_ptr())
+            };
+            for (k, &i) in idx.iter().enumerate() {
+                if rc != 0 || ok[k] == 0 {
+                    res[i] = Err(OperationError::SignatureVerificationFailure);
+                }
+            }
+        }
+        res
+    }
+
+    /// Batched `KeyEncryptable::key_encrypt` of every message to one recipient.
+    pub fn key_encrypt_prepared(&self, msgs: &mut [Message], key: &PreparedKey, d: SecParam) -> Result<(), OperationError> {
+        use crate::sha3::aux_functions::byte_utils::get_random_bytes;
+        use tiny_ed448_goldilocks::curve::affine::AffinePoint;
+        let n = msgs.len();
+        let k_rand: Vec<u8> = (0..n).flat_map(|_| get_random_bytes(56)).collect();
+        let (md, mo) = pack(msgs.iter().map(|m| m.msg.as_slice()));
+        let (mut ct, mut tag, mut z) = (vec![0u8; md.len()], vec![0u8; n * 56], vec![0u8; n * 112]);
+        status(unsafe {
+            capy_ed448_key_encrypt_prepared_batch(self.ctx, d as c_int, key.key, k_rand.as_ptr(), md.as_ptr(),
+                                                  mo.as_ptr(), n as u64, ct.as_mut_ptr(), tag.as_mut_ptr(), z.as_mut_ptr())
+        })?;
+        for (i, m) in msgs.iter_mut().enumerate() {
+            m.msg = Box::new(ct[mo[i] as usize..mo[i + 1] as usize].to_vec());
+            m.digest = tag[56 * i..56 * i + 56].to_vec();
+            m.asym_nonce = Some(AffinePoint::from_xy_bytes(&z[112 * i..112 * i + 112]).to_extended());
+            m.d = Some(d);
+        }
+        Ok(())
     }
 }
 
