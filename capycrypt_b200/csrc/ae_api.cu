@@ -321,28 +321,6 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
 
-// ---- host staging ------------------------------------------------------------------------------------
-// output buffer (scratch kHost5) for the byte range of items [i0, i1) of a packed batch, addressed with the caller's offsets
-struct StagedOut {
-  uint8_t* d_raw;
-  uint8_t* d_base;  // d_base + off[i] addresses item i
-  uint64_t a0, bytes;
-};
-static int stage_out(DeviceCtx& dc, cudaStream_t st, const uint64_t* off, uint64_t i0, uint64_t i1, StagedOut* o) {
-  o->a0 = off[i0] & ~(uint64_t)15;
-  o->bytes = off[i1] - o->a0;
-  o->d_raw = (uint8_t*)scratch_get(dc, st, kHost5, (size_t)o->bytes + 16);
-  if (!o->d_raw) return CAPY_ERR_OOM;
-  o->d_base = reinterpret_cast<uint8_t*>(reinterpret_cast<uintptr_t>(o->d_raw) - (uintptr_t)o->a0);
-  return CAPY_OK;
-}
-static int fetch_out(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const StagedOut& o, const uint64_t* off, uint64_t i0,
-                     uint64_t i1, uint8_t* host) {
-  const uint64_t b0 = off[i0], b1 = off[i1];
-  if (b1 > b0) return copy_out(ctx, dc, st, kHost5, host + b0, o.d_base + b0, (size_t)(b1 - b0));
-  return CAPY_OK;
-}
-
 }  // namespace capy
 
 using namespace capy;
@@ -380,30 +358,14 @@ int capy_sponge_encrypt_batch(capy_ctx* ctx, int d_bits, int variant, const uint
   if (variant != CAPY_AE_SHA3 && variant != CAPY_AE_KEM) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 2048);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sp, sm;
-      uint8_t* d_nonce = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, kHost2, kHost3, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost4, nonces + ch.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
-      if (rc) return rc;
-      StagedOut so;
-      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
-      if (rc) return rc;
-      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 64);
-      if (!d_tag) return CAPY_ERR_OOM;
-      rc = dev_sponge_encrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[ch.i1] - pw_off[ch.i0], d_nonce,
-                              nonce_len, sm.d_base, sm.d_off, cnt, so.d_base, d_tag);
-      if (rc) return rc;
-      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
-      if (rc) return rc;
-      CAPY_CUDA(ctx, cudaMemcpyAsync(tag64 + 64 * ch.i0, d_tag, cnt * 64, cudaMemcpyDeviceToHost, st));
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(pws, pw_off), sm = io.in_packed(msgs, msg_off);
+    const uint8_t* d_nonce = io.in(nonces, nonce_len);
+    uint8_t* d_ct = io.out_packed(ct, msg_off);
+    uint8_t* d_tag = io.out(tag64, 64);
+    if (io.rc()) return io.rc();
+    return dev_sponge_encrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[io.i1()] - pw_off[io.i0()], d_nonce,
+                              nonce_len, sm.d_base, sm.d_off, io.n(), d_ct, d_tag);
   });
 }
 
@@ -415,32 +377,15 @@ int capy_sponge_decrypt_batch(capy_ctx* ctx, int d_bits, int variant, const uint
   if (variant != CAPY_AE_SHA3 && variant != CAPY_AE_KEM) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(ct_off, 0, 0, n, ctx->devs.size(), 2048);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sp, sc;
-      uint8_t *d_nonce = nullptr, *d_tag = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, kHost2, kHost3, ct, ct_off, ch.i0, ch.i1, &sc);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost4, nonces + ch.i0 * nonce_len, (size_t)(cnt * nonce_len), &d_nonce);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost6, tag64 + 64 * ch.i0, (size_t)(cnt * 64), &d_tag);
-      if (rc) return rc;
-      StagedOut so;
-      rc = stage_out(dc, st, ct_off, ch.i0, ch.i1, &so);
-      if (rc) return rc;
-      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost7, cnt);
-      if (!d_ok) return CAPY_ERR_OOM;
-      rc = dev_sponge_decrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[ch.i1] - pw_off[ch.i0], d_nonce,
-                              nonce_len, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok);
-      if (rc) return rc;
-      rc = fetch_out(ctx, dc, st, so, ct_off, ch.i0, ch.i1, out);
-      if (rc) return rc;
-      CAPY_CUDA(ctx, cudaMemcpyAsync(ok + ch.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(pws, pw_off), sc = io.in_packed(ct, ct_off);
+    const uint8_t* d_nonce = io.in(nonces, nonce_len);
+    const uint8_t* d_tag = io.in(tag64, 64);
+    uint8_t* d_out = io.out_packed(out, ct_off);
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return dev_sponge_decrypt(ctx, dc, st, d_bits, variant, sp.d_base, sp.d_off, pw_off[io.i1()] - pw_off[io.i0()], d_nonce,
+                              nonce_len, sc.d_base, sc.d_off, d_tag, io.n(), d_out, d_ok);
   });
 }
 
@@ -472,31 +417,15 @@ int capy_ed448_key_encrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_x
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 16384);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
-    return run_chunks(ctx, dc, {sh}, bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sm;
-      uint8_t *d_pub = nullptr, *d_k = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost2, pub_xy112 + 112 * ch.i0, (size_t)cnt * 112, &d_pub);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost3, k_rand56 + 56 * ch.i0, (size_t)cnt * 56, &d_k);
-      if (rc) return rc;
-      StagedOut so;
-      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
-      if (rc) return rc;
-      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 56);
-      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost7, cnt * 112);
-      if (!d_tag || !d_z) return CAPY_ERR_OOM;
-      rc = dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z, d_flag);
-      if (rc) return rc;
-      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
-      if (rc) return rc;
-      CAPY_CUDA(ctx, cudaMemcpyAsync(tag56 + 56 * ch.i0, d_tag, cnt * 56, cudaMemcpyDeviceToHost, st));
-      CAPY_CUDA(ctx, cudaMemcpyAsync(z_xy112 + 112 * ch.i0, d_z, cnt * 112, cudaMemcpyDeviceToHost, st));
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, one_chunk, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sm = io.in_packed(msgs, msg_off);
+    const uint8_t* d_pub = io.in(pub_xy112, 112);
+    const uint8_t* d_k = io.in(k_rand56, 56);
+    uint8_t* d_ct = io.out_packed(ct, msg_off);
+    uint8_t* d_tag = io.out(tag56, 56);
+    uint8_t* d_z = io.out(z_xy112, 112);
+    if (io.rc()) return io.rc();
+    return dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, sm.d_base, sm.d_off, io.n(), d_ct, d_tag, d_z, io.d_flag());
   });
 }
 
@@ -518,29 +447,14 @@ int capy_ed448_key_encrypt_prepared_batch(capy_ctx* ctx, int d_bits, const capy_
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 16384);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, {sh}, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sm;
-      uint8_t* d_k = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost3, k_rand56 + 56 * ch.i0, (size_t)cnt * 56, &d_k);
-      if (rc) return rc;
-      StagedOut so;
-      rc = stage_out(dc, st, msg_off, ch.i0, ch.i1, &so);
-      if (rc) return rc;
-      uint8_t* d_tag = (uint8_t*)scratch_get(dc, st, kHost6, cnt * 56);
-      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost7, cnt * 112);
-      if (!d_tag || !d_z) return CAPY_ERR_OOM;
-      rc = dev_key_encrypt_prepared(ctx, dc, st, d_bits, key, d_k, sm.d_base, sm.d_off, cnt, so.d_base, d_tag, d_z);
-      if (rc) return rc;
-      rc = fetch_out(ctx, dc, st, so, msg_off, ch.i0, ch.i1, ct);
-      if (rc) return rc;
-      CAPY_CUDA(ctx, cudaMemcpyAsync(tag56 + 56 * ch.i0, d_tag, cnt * 56, cudaMemcpyDeviceToHost, st));
-      CAPY_CUDA(ctx, cudaMemcpyAsync(z_xy112 + 112 * ch.i0, d_z, cnt * 112, cudaMemcpyDeviceToHost, st));
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sm = io.in_packed(msgs, msg_off);
+    const uint8_t* d_k = io.in(k_rand56, 56);
+    uint8_t* d_ct = io.out_packed(ct, msg_off);
+    uint8_t* d_tag = io.out(tag56, 56);
+    uint8_t* d_z = io.out(z_xy112, 112);
+    if (io.rc()) return io.rc();
+    return dev_key_encrypt_prepared(ctx, dc, st, d_bits, key, d_k, sm.d_base, sm.d_off, io.n(), d_ct, d_tag, d_z);
   });
 }
 
@@ -551,32 +465,15 @@ int capy_ed448_key_decrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, 
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(ct_off, 0, 0, n, ctx->devs.size(), 16384);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
-    return run_chunks(ctx, dc, {sh}, bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sp, sc;
-      uint8_t *d_z = nullptr, *d_tag = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, kHost2, kHost3, ct, ct_off, ch.i0, ch.i1, &sc);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost4, z_xy112 + 112 * ch.i0, (size_t)cnt * 112, &d_z);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost6, tag56 + 56 * ch.i0, (size_t)cnt * 56, &d_tag);
-      if (rc) return rc;
-      StagedOut so;
-      rc = stage_out(dc, st, ct_off, ch.i0, ch.i1, &so);
-      if (rc) return rc;
-      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost7, cnt);
-      if (!d_ok) return CAPY_ERR_OOM;
-      rc = dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, sc.d_base, sc.d_off, d_tag, cnt, so.d_base, d_ok,
-                           d_flag);
-      if (rc) return rc;
-      rc = fetch_out(ctx, dc, st, so, ct_off, ch.i0, ch.i1, out);
-      if (rc) return rc;
-      CAPY_CUDA(ctx, cudaMemcpyAsync(ok + ch.i0, d_ok, cnt, cudaMemcpyDeviceToHost, st));
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, one_chunk, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(pws, pw_off), sc = io.in_packed(ct, ct_off);
+    const uint8_t* d_z = io.in(z_xy112, 112);
+    const uint8_t* d_tag = io.in(tag56, 56);
+    uint8_t* d_out = io.out_packed(out, ct_off);
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, sc.d_base, sc.d_off, d_tag, io.n(), d_out, d_ok,
+                           io.d_flag());
   });
 }
 

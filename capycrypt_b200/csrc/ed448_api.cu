@@ -296,6 +296,29 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
   return verify_finish(ctx, dc, st, d, projB, d_msgs, d_msg_off, d_h, bad, n, d_ok, d_bad_flag);
 }
 
+// W = [k]V with k = 4 * BE(rand) mod r (ecc/encryptable.rs:36-37): W.x ; optionally Z = [k]G (:38)
+static int dev_ecdh(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint8_t* d_k, const uint8_t* d_pub, uint64_t n,
+                    uint8_t* d_wx, uint8_t* d_z_xy, int* d_bad_flag) {
+  if (n == 0) return CAPY_OK;
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, n * 256);
+  CAPY_SCRATCH(bad, uint8_t, kEdBad, n);
+  int rc = launch_var_base(ctx, dc, st, d_k, 1, d_pub, nullptr, proj, bad, n, true);
+  if (rc) return rc;
+  rc = launch_to_affine(ctx, st, proj, n, 1, bad, d_wx);
+  if (rc) return rc;
+  if (d_bad_flag) {
+    rc = launch_any_bad(ctx, st, bad, d_bad_flag, n);
+    if (rc) return rc;
+  }
+  if (!d_z_xy) return CAPY_OK;
+  CAPY_SCRATCH(kw, uint32_t, kEdKWords, n * 56);
+  rc = launch_scalar_prep(ctx, st, d_k, 1, kw, nullptr, n);
+  if (rc) return rc;
+  rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true);
+  if (rc) return rc;
+  return launch_to_affine(ctx, st, proj, n, 0, nullptr, d_z_xy);
+}
+
 // ---- prepared public keys ------------------------------------------------------------------------------
 // out[0 .. n) := the 112 bytes at d_xy: one copy, then ceil(log2 n) copies that double what is there
 int broadcast_point(capy_ctx* ctx, cudaStream_t st, const uint8_t* d_xy, uint8_t* out, uint64_t n) {
@@ -462,24 +485,17 @@ int capy_ed448_verify_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int 
 }
 
 // ---- host-buffer entry points: shard across the ctx devices by item count; inside a device the shard is cut into chunks
-// that rotate over the device's streams (run_chunks), so the copies of one chunk run under the kernels of its
+// that rotate over the device's streams (run_host_call), so the copies of one chunk run under the kernels of its
 // neighbours ----
 int capy_ed448_fixed_base_batch(capy_ctx* ctx, const uint8_t* scalars_be56, uint64_t n, uint8_t* out_xy112) {
   if (!ctx || (n && (!scalars_be56 || !out_xy112))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      uint8_t *d_sc = nullptr, *d_out = nullptr;
-      int rc = h2d(ctx, dc, st, kHost0, scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
-      if (rc) return rc;
-      d_out = (uint8_t*)scratch_get(dc, st, kHost1, cnt * 112);
-      if (!d_out) return CAPY_ERR_OOM;
-      rc = dev_fixed_base(ctx, dc, st, d_sc, cnt, d_out);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost1, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
-    });
+  return run_host_call(ctx, shards, ed_chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const uint8_t* d_sc = io.in(scalars_be56, 56);
+    uint8_t* d_out = io.out(out_xy112, 112);
+    if (io.rc()) return io.rc();
+    return dev_fixed_base(ctx, dc, st, d_sc, io.n(), d_out);
   });
 }
 
@@ -488,20 +504,12 @@ int capy_ed448_var_base_batch(capy_ctx* ctx, const uint8_t* scalars_be56, const 
   if (!ctx || (n && (!scalars_be56 || !points_xy112 || !out_xy112))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      uint8_t *d_sc = nullptr, *d_pt = nullptr;
-      int rc = h2d(ctx, dc, st, kHost0, scalars_be56 + 56 * ch.i0, cnt * 56, &d_sc);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost1, points_xy112 + 112 * ch.i0, cnt * 112, &d_pt);
-      if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 112);
-      if (!d_out) return CAPY_ERR_OOM;
-      rc = dev_var_base(ctx, dc, st, d_sc, d_pt, cnt, d_out, d_flag);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost2, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
-    });
+  return run_host_call(ctx, shards, ed_chunks, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const uint8_t* d_sc = io.in(scalars_be56, 56);
+    const uint8_t* d_pt = io.in(points_xy112, 112);
+    uint8_t* d_out = io.out(out_xy112, 112);
+    if (io.rc()) return io.rc();
+    return dev_var_base(ctx, dc, st, d_sc, d_pt, io.n(), d_out, io.d_flag());
   });
 }
 
@@ -511,18 +519,11 @@ int capy_ed448_keygen_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 112);
-      if (!d_out) return CAPY_ERR_OOM;
-      rc = dev_keygen(ctx, dc, st, d_bits, sp.d_base, sp.d_off, cnt, d_out);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost2, out_xy112 + 112 * ch.i0, d_out, cnt * 112);
-    });
+  return run_host_call(ctx, shards, ed_chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(pws, pw_off);
+    uint8_t* d_out = io.out(out_xy112, 112);
+    if (io.rc()) return io.rc();
+    return dev_keygen(ctx, dc, st, d_bits, sp.d_base, sp.d_off, io.n(), d_out);
   });
 }
 
@@ -532,23 +533,12 @@ int capy_ed448_sign_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, const u
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sp, sm;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, pws, pw_off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, kHost2, kHost3, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      uint8_t* d_h = (uint8_t*)scratch_get(dc, st, kHost4, cnt * 56);
-      uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost5, cnt * 56);
-      if (!d_h || !d_z) return CAPY_ERR_OOM;
-      rc = dev_sign(ctx, dc, st, d_bits, sp.d_base, sp.d_off, sm.d_base, sm.d_off, cnt, d_h, d_z);
-      if (rc) return rc;
-      rc = copy_out(ctx, dc, st, kHost4, h56 + 56 * ch.i0, d_h, cnt * 56);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost5, z_be56 + 56 * ch.i0, d_z, cnt * 56);
-    });
+  return run_host_call(ctx, shards, ed_chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(pws, pw_off), sm = io.in_packed(msgs, msg_off);
+    uint8_t* d_h = io.out(h56, 56);
+    uint8_t* d_z = io.out(z_be56, 56);
+    if (io.rc()) return io.rc();
+    return dev_sign(ctx, dc, st, d_bits, sp.d_base, sp.d_off, sm.d_base, sm.d_off, io.n(), d_h, d_z);
   });
 }
 
@@ -558,25 +548,14 @@ int capy_ed448_verify_batch(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112,
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sm;
-      uint8_t *d_pub = nullptr, *d_h = nullptr, *d_z = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost2, pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost3, h56 + 56 * ch.i0, cnt * 56, &d_h);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost4, z_be56 + 56 * ch.i0, cnt * 56, &d_z);
-      if (rc) return rc;
-      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost5, cnt);
-      if (!d_ok) return CAPY_ERR_OOM;
-      rc = dev_verify(ctx, dc, st, d_bits, d_pub, sm.d_base, sm.d_off, d_h, d_z, cnt, d_ok, d_flag);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost5, ok + ch.i0, d_ok, cnt);
-    });
+  return run_host_call(ctx, shards, ed_chunks, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sm = io.in_packed(msgs, msg_off);
+    const uint8_t* d_pub = io.in(pub_xy112, 112);
+    const uint8_t* d_h = io.in(h56, 56);
+    const uint8_t* d_z = io.in(z_be56, 56);
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return dev_verify(ctx, dc, st, d_bits, d_pub, sm.d_base, sm.d_off, d_h, d_z, io.n(), d_ok, io.d_flag());
   });
 }
 
@@ -596,23 +575,13 @@ int capy_ed448_verify_prepared_batch(capy_ctx* ctx, int d_bits, const capy_ed448
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(msg_off, 0, 0, n, ctx->devs.size(), 4096);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sm;
-      uint8_t *d_h = nullptr, *d_z = nullptr;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, msgs, msg_off, ch.i0, ch.i1, &sm);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost3, h56 + 56 * ch.i0, cnt * 56, &d_h);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost4, z_be56 + 56 * ch.i0, cnt * 56, &d_z);
-      if (rc) return rc;
-      uint8_t* d_ok = (uint8_t*)scratch_get(dc, st, kHost5, cnt);
-      if (!d_ok) return CAPY_ERR_OOM;
-      rc = dev_verify_prepared(ctx, dc, st, d_bits, key, sm.d_base, sm.d_off, d_h, d_z, cnt, d_ok);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost5, ok + ch.i0, d_ok, cnt);
-    });
+  return run_host_call(ctx, shards, ed_chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sm = io.in_packed(msgs, msg_off);
+    const uint8_t* d_h = io.in(h56, 56);
+    const uint8_t* d_z = io.in(z_be56, 56);
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return dev_verify_prepared(ctx, dc, st, d_bits, key, sm.d_base, sm.d_off, d_h, d_z, io.n(), d_ok);
   });
 }
 
@@ -671,42 +640,13 @@ int capy_ed448_ecdh_batch(capy_ctx* ctx, const uint8_t* k_rand56, const uint8_t*
   if (!ctx || (n && (!k_rand56 || !pub_xy112 || !wx56))) return CAPY_ERR_BAD_ARG;
   if (n == 0) return CAPY_OK;
   auto shards = split_items(nullptr, 1, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
-    return run_chunks(ctx, dc, ed_chunks(sh), bad_point, [&](cudaStream_t st, Range ch, int* d_flag) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      uint8_t *d_k = nullptr, *d_pub = nullptr;
-      int rc = h2d(ctx, dc, st, kHost0, k_rand56 + 56 * ch.i0, cnt * 56, &d_k);
-      if (rc) return rc;
-      rc = h2d(ctx, dc, st, kHost1, pub_xy112 + 112 * ch.i0, cnt * 112, &d_pub);
-      if (rc) return rc;
-      uint8_t* d_wx = (uint8_t*)scratch_get(dc, st, kHost2, cnt * 56);
-      uint32_t* proj = (uint32_t*)scratch_get(dc, st, kEdProj, cnt * 256);
-      uint8_t* bad = (uint8_t*)scratch_get(dc, st, kEdBad, cnt);
-      if (!d_wx || !proj || !bad) return CAPY_ERR_OOM;
-      // W = [k]V with k = 4 * BE(rand) mod r (ecc/encryptable.rs:36-37); W.x
-      rc = launch_var_base(ctx, dc, st, d_k, 1, d_pub, nullptr, proj, bad, cnt, true);
-      if (rc) return rc;
-      rc = launch_to_affine(ctx, st, proj, cnt, 1, bad, d_wx);
-      if (rc) return rc;
-      rc = launch_any_bad(ctx, st, bad, d_flag, cnt);
-      if (rc) return rc;
-      rc = copy_out(ctx, dc, st, kHost2, wx56 + 56 * ch.i0, d_wx, cnt * 56);
-      if (rc) return rc;
-      if (z_xy112) {  // Z = [k]G (:38)
-        uint32_t* kw = (uint32_t*)scratch_get(dc, st, kEdKWords, cnt * 56);
-        uint8_t* d_z = (uint8_t*)scratch_get(dc, st, kHost3, cnt * 112);
-        if (!kw || !d_z) return CAPY_ERR_OOM;
-        rc = launch_scalar_prep(ctx, st, d_k, 1, kw, nullptr, cnt);
-        if (rc) return rc;
-        rc = launch_fixed_base(ctx, dc, st, kw, proj, cnt, true);
-        if (rc) return rc;
-        rc = launch_to_affine(ctx, st, proj, cnt, 0, nullptr, d_z);
-        if (rc) return rc;
-        rc = copy_out(ctx, dc, st, kHost3, z_xy112 + 112 * ch.i0, d_z, cnt * 112);
-        if (rc) return rc;
-      }
-      return CAPY_OK;
-    });
+  return run_host_call(ctx, shards, ed_chunks, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const uint8_t* d_k = io.in(k_rand56, 56);
+    const uint8_t* d_pub = io.in(pub_xy112, 112);
+    uint8_t* d_wx = io.out(wx56, 56);
+    uint8_t* d_z = z_xy112 ? io.out(z_xy112, 112) : nullptr;
+    if (io.rc()) return io.rc();
+    return dev_ecdh(ctx, dc, st, d_k, d_pub, io.n(), d_wx, d_z, io.d_flag());
   });
 }
 

@@ -203,44 +203,131 @@ inline int run_chunks(capy_ctx* ctx, DeviceCtx& dc, const std::vector<Range>& ch
   return CAPY_OK;
 }
 
-// one host input of `bytes` bytes copied into scratch `slot` (16 bytes of slack)
-inline int h2d(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot, const void* src, size_t bytes, uint8_t** out) {
-  uint8_t* d = (uint8_t*)scratch_get(dc, st, slot, bytes + 16);
-  if (!d) return CAPY_ERR_OOM;
-  if (bytes) {
-    const int rc = copy_in(ctx, dc, st, slot, d, src, bytes);
-    if (rc) return rc;
-  }
-  *out = d;
-  return CAPY_OK;
-}
-
 // one packed host input staged per chunk: bytes [a0, off[i1]) with a0 = off[i0] rounded down to 16
 struct StagedPacked {
   const uint8_t* d_base = nullptr;  // device pointer such that d_base + off[i] addresses item i
   const uint64_t* d_off = nullptr;  // device copy of off[i0 .. i1]
 };
 
-inline int stage_packed(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Slot slot_data, Slot slot_off, const uint8_t* data,
-                        const uint64_t* off, uint64_t i0, uint64_t i1, StagedPacked* out) {
-  const uint64_t a0 = off[i0] & ~(uint64_t)15, a1 = off[i1];
-  const size_t nbytes = (size_t)(a1 - a0);
-  uint8_t* d_data = (uint8_t*)scratch_get(dc, st, slot_data, nbytes + 16);
-  uint64_t* d_off = (uint64_t*)scratch_get(dc, st, slot_off, (size_t)(i1 - i0 + 1) * 8);
-  if (!d_data || !d_off) return CAPY_ERR_OOM;
-  if (nbytes) {
-    const int rc = copy_in(ctx, dc, st, slot_data, d_data, data + a0, nbytes);
-    if (rc) return rc;
+// The device buffers of one chunk's inputs and outputs (run_host_call).  Every declaration takes the next kHost slot, so
+// two buffers of one call never share one, and a declaration past kHost7 is an error rather than a wrap-around.  Inputs
+// are copied in when declared; outputs are copied back to the caller's buffers, in the order declared, by copy_back.  A
+// failed declaration returns nullptr and makes rc() nonzero; the declarations after it do nothing.
+class HostChunk {
+ public:
+  HostChunk(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, Range r, int* d_flag)
+      : ctx_(ctx), dc_(dc), st_(st), r_(r), d_flag_(d_flag) {}
+  uint64_t i0() const { return r_.i0; }
+  uint64_t i1() const { return r_.i1; }
+  uint64_t n() const { return r_.i1 - r_.i0; }
+  int* d_flag() const { return d_flag_; }  // run_chunks' bad-point flag of this stream, or nullptr
+  int rc() const { return rc_; }
+
+  // n() rows of `row` bytes from host + row * i0 (`bytes` overrides the length, e.g. a short last row); 16 bytes of slack
+  const uint8_t* in(const void* host, size_t row, size_t bytes = ~size_t(0)) {
+    if (bytes == ~size_t(0)) bytes = row * n();
+    Slot s{};
+    uint8_t* d = grab(bytes + 16, &s);
+    if (d) note(copy_in(ctx_, dc_, st_, s, d, (const uint8_t*)host + row * r_.i0, bytes));
+    return rc_ ? nullptr : d;
   }
-  {
-    const int rc = copy_in(ctx, dc, st, slot_off, d_off, off + i0, (size_t)(i1 - i0 + 1) * 8);
-    if (rc) return rc;
+
+  // the items [i0, i1) of a packed input: bytes [a0, off[i1]) with a0 = off[i0] rounded down to 16, and off[i0 .. i1]
+  StagedPacked in_packed(const uint8_t* data, const uint64_t* off) {
+    const uint64_t a0 = off[r_.i0] & ~(uint64_t)15;
+    const size_t bytes = (size_t)(off[r_.i1] - a0), count = (size_t)n() + 1;
+    Slot sd{}, so{};
+    uint8_t* d_data = grab(bytes + 16, &sd);
+    uint64_t* d_off = (uint64_t*)grab(count * 8, &so);
+    if (!rc_) note(copy_in(ctx_, dc_, st_, sd, d_data, data + a0, bytes));
+    if (!rc_) note(copy_in(ctx_, dc_, st_, so, d_off, off + r_.i0, count * 8));
+    if (rc_) return {};
+    host_off_register(dc_, d_off, off + r_.i0, count);  // plan_ragged plans from the host copy: no device round trip
+    return {rebase(d_data, a0), d_off};
   }
-  out->d_base = reinterpret_cast<const uint8_t*>(reinterpret_cast<uintptr_t>(d_data) - (uintptr_t)a0);
-  out->d_off = d_off;
-  host_off_register(dc, d_off, off + i0, i1 - i0 + 1);  // plan_ragged plans from the host copy: no device round trip
-  return CAPY_OK;
+
+  // n() rows of `row` bytes, copied back to host + row * i0
+  uint8_t* out(void* host, size_t row) {
+    Slot s{};
+    uint8_t* d = grab(row * n(), &s);
+    if (d) outs_.push_back({s, (uint8_t*)host + row * r_.i0, d, row * n()});
+    return d;
+  }
+
+  // the items [i0, i1) of a packed output: d + off[i] addresses item i (laid out as in_packed); bytes [off[i0], off[i1])
+  // are copied back to the same offsets of host
+  uint8_t* out_packed(uint8_t* host, const uint64_t* off) {
+    const uint64_t a0 = off[r_.i0] & ~(uint64_t)15, b0 = off[r_.i0], b1 = off[r_.i1];
+    Slot s{};
+    uint8_t* d = grab((size_t)(b1 - a0) + 16, &s);
+    if (!d) return nullptr;
+    uint8_t* base = rebase(d, a0);
+    outs_.push_back({s, host + b0, base + b0, (size_t)(b1 - b0)});
+    return base;
+  }
+
+  // enqueues the copies of the outputs back to the caller's buffers (copy_out: pageable ones are staged)
+  int copy_back() {
+    if (rc_) return rc_;
+    for (const Out& o : outs_) {
+      const int rc = copy_out(ctx_, dc_, st_, o.slot, o.host, o.dev, o.bytes);
+      if (rc) return rc;
+    }
+    return CAPY_OK;
+  }
+
+ private:
+  struct Out {
+    Slot slot;
+    void* host;
+    const uint8_t* dev;
+    size_t bytes;
+  };
+  uint8_t* grab(size_t bytes, Slot* slot) {
+    if (rc_) return nullptr;
+    if (next_ > kHost7 - kHost0) {
+      rc_ = CAPY_ERR_BAD_ARG;
+      return nullptr;
+    }
+    *slot = (Slot)(kHost0 + next_++);
+    uint8_t* d = (uint8_t*)scratch_get(dc_, st_, *slot, bytes);
+    if (!d) rc_ = CAPY_ERR_OOM;
+    return d;
+  }
+  void note(int rc) {
+    if (!rc_) rc_ = rc;
+  }
+  static uint8_t* rebase(uint8_t* d, uint64_t a0) {
+    return reinterpret_cast<uint8_t*>(reinterpret_cast<uintptr_t>(d) - (uintptr_t)a0);
+  }
+  capy_ctx* ctx_;
+  DeviceCtx& dc_;
+  cudaStream_t st_;
+  Range r_;
+  int* d_flag_;
+  int next_ = 0, rc_ = CAPY_OK;
+  std::vector<Out> outs_;
+};
+
+// One host call: the shards go to the ctx devices (for_each_device), chunks_of_shard(shard) cuts a shard into the chunks
+// that rotate over the device's streams (run_chunks), and body(dc, st, io) declares a chunk's inputs and outputs on `io`
+// and enqueues its pipeline; the outputs are then copied back.  With bad_points the chunks get run_chunks' bad-point
+// flag (io.d_flag()), and a bad point anywhere makes the call return CAPY_ERR_BAD_POINT.
+template <class Chunks, class Body>
+inline int run_host_call(capy_ctx* ctx, const std::vector<Range>& shards, Chunks&& chunks_of_shard, bool bad_points,
+                         Body&& body) {
+  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int* bad_point) -> int {
+    return run_chunks(ctx, dc, chunks_of_shard(sh), bad_points ? bad_point : nullptr,
+                      [&](cudaStream_t st, Range ch, int* d_flag) -> int {
+                        HostChunk io(ctx, dc, st, ch, d_flag);
+                        const int rc = body(dc, st, io);
+                        return rc ? rc : io.copy_back();
+                      });
+  });
 }
+
+// the chunker of the calls that run a device's shard as one chunk
+inline std::vector<Range> one_chunk(Range sh) { return {sh}; }
 
 constexpr uint64_t kChunkBytes = 8ull << 20;
 

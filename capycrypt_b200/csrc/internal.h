@@ -24,9 +24,10 @@ constexpr int kNumStreams = 3;
 // host call run on the three streams at once, and scratch_get picks the set from the stream, so two streams never share
 // a buffer.  A caller's stream (the _dev entry points) uses set 0.
 enum Slot {
-  // device buffers of the inputs and outputs of a host entry point, in the order it stages them.  Shared by all host
-  // entry points: one host call holds a device at a time, waits for its streams and drains its staging before it returns,
-  // and no device pipeline uses these slots.
+  // device buffers of the inputs and outputs of a host entry point, handed out in declaration order by HostChunk
+  // (hostbatch.h); only the scattered multi-device path of capy_sha3_batch names them.  Shared by all host entry points:
+  // one host call holds a device at a time, waits for its streams and drains its staging before it returns, and no
+  // device pipeline uses these slots.
   kHost0, kHost1, kHost2, kHost3, kHost4, kHost5, kHost6, kHost7,
   kFlag,                    // "bad point" flag of run_chunks (hostbatch.h)
   kPlanHist, kPlanOrder,    // plan_ragged: device length histogram (+ summary), work order
@@ -145,9 +146,9 @@ struct DeviceCtx {
   Scratch vb_slabs;  // per-SM table slabs of var_base_kernel: shared by all streams (an SM runs one var_base block at a time)
   std::map<std::string, PrefixState> prefix_cache;
   std::vector<PlanEntry> plans;
-  // host copies of the offsets arrays a host entry point has staged into device scratch (stage_packed), keyed by the
-  // device address: plan_ragged reads the lengths from the host copy instead of fetching the histogram summary from the
-  // device (no stream synchronisation inside a host-buffer call).  Valid only while that host call runs (HostOffScope).
+  // host copies of the offsets arrays a host entry point has staged into device scratch (HostChunk::in_packed), keyed by
+  // the device address: plan_ragged reads the lengths from the host copy instead of fetching the histogram summary from
+  // the device (no stream synchronisation inside a host-buffer call).  Valid only while that host call runs (HostOffScope).
   struct HostOff {
     const uint64_t* d_off;
     const uint64_t* h_off;

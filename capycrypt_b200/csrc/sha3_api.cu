@@ -478,7 +478,7 @@ static int plan_ragged(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uint
                        uint32_t stride_bytes, LaunchPlan* plan, bool allow_pair = true, int force_c = 0) {
   *plan = LaunchPlan();
   if (n < 1 || n > 0xffffffffull) return CAPY_OK;
-  // Host-buffer entry points: the offsets were staged from a host array that is still alive (stage_packed registers it).
+  // Host-buffer entry points: the offsets were staged from a host array that is still alive (HostChunk::in_packed registers it).
   // The lengths are read there, so nothing comes back from the device and the chunk pipeline of the host call never
   // waits for a stream.  Uniform lengths (the bulk case: fixed-size records) need no device work at all.
   const uint64_t* h_off = host_off_find(dc, d_off, n);
@@ -1118,19 +1118,13 @@ int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64
     }
   }
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 200);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    // long messages: few big chunks, so that the longest-first schedule sees enough work beside them
-    auto chunks = split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, 0), 200);
-    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)(ch.i1 - ch.i0) * ob);
-      if (!d_out) return CAPY_ERR_OOM;
-      rc = launch_sha3(ctx, dc, st, d_bits, sp.d_base, sp.d_off, 0, 0, ch.i1 - ch.i0, d_out, flags);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost2, digests + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
-    });
+  // long messages: few big chunks, so that the longest-first schedule sees enough work beside them
+  auto chunks = [&](Range sh) { return split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, 0), 200); };
+  return run_host_call(ctx, shards, chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(data, off);
+    uint8_t* d_out = io.out(digests, ob);
+    if (io.rc()) return io.rc();
+    return launch_sha3(ctx, dc, st, d_bits, sp.d_base, sp.d_off, 0, 0, io.n(), d_out, flags);
   });
 }
 
@@ -1143,21 +1137,15 @@ int capy_sha3_batch_fixed(capy_ctx* ctx, int d_bits, const uint8_t* data, uint64
   // the uniform kernel wants 8-byte aligned rows; the copy lands on a 256-byte aligned buffer, so
   // only the stride matters
   auto shards = split_items(nullptr, stride, 0, n, ctx->devs.size(), 0);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    auto chunks = split_items(nullptr, stride, sh.i0, sh.i1, chunk_count((sh.i1 - sh.i0) * stride, sh.i1 - sh.i0), 0);
-    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      // last row may be shorter than the stride in the caller's buffer
-      const size_t in_bytes = (size_t)((cnt - 1) * stride + msg_len);
-      uint8_t* d_in = (uint8_t*)scratch_get(dc, st, kHost0, in_bytes + 16);
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)cnt * ob);
-      if (!d_in || !d_out) return CAPY_ERR_OOM;
-      int rc = copy_in(ctx, dc, st, kHost0, d_in, data + ch.i0 * stride, in_bytes);
-      if (rc) return rc;
-      rc = launch_sha3(ctx, dc, st, d_bits, d_in, nullptr, msg_len, stride, cnt, d_out);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost2, digests + ch.i0 * ob, d_out, (size_t)cnt * ob);
-    });
+  auto chunks = [&](Range sh) {
+    return split_items(nullptr, stride, sh.i0, sh.i1, chunk_count((sh.i1 - sh.i0) * stride, sh.i1 - sh.i0), 0);
+  };
+  return run_host_call(ctx, shards, chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    // the last row may be shorter than the stride in the caller's buffer
+    const uint8_t* d_in = io.in(data, stride, (size_t)((io.n() - 1) * stride + msg_len));
+    uint8_t* d_out = io.out(digests, ob);
+    if (io.rc()) return io.rc();
+    return launch_sha3(ctx, dc, st, d_bits, d_in, nullptr, msg_len, stride, io.n(), d_out);
   });
 }
 
@@ -1180,20 +1168,15 @@ int capy_cshake_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint
   const size_t ob = (size_t)(out_bits / 8);
   if (n == 0 || ob == 0) return CAPY_OK;
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 200 + ob);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    auto chunks = split_items(off, 0, sh.i0, sh.i1,
-                              ragged_chunk_count(off, sh.i0, sh.i1, (sh.i1 - sh.i0) * ob), 200 + ob);
-    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      StagedPacked sp;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sp);
-      if (rc) return rc;
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost2, (size_t)(ch.i1 - ch.i0) * ob);
-      if (!d_out) return CAPY_ERR_OOM;
-      rc = launch_cshake(ctx, dc, st, d_bits, sp.d_base, sp.d_off, ch.i1 - ch.i0, fn_name, fn_len, custom, custom_len,
-                         out_bits, d_out);
-      if (rc) return rc;
-      return copy_out(ctx, dc, st, kHost2, out + ch.i0 * ob, d_out, (size_t)(ch.i1 - ch.i0) * ob);
-    });
+  auto chunks = [&](Range sh) {
+    return split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, (sh.i1 - sh.i0) * ob), 200 + ob);
+  };
+  return run_host_call(ctx, shards, chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(data, off);
+    uint8_t* d_out = io.out(out, ob);
+    if (io.rc()) return io.rc();
+    return launch_cshake(ctx, dc, st, d_bits, sp.d_base, sp.d_off, io.n(), fn_name, fn_len, custom, custom_len, out_bits,
+                         d_out);
   });
 }
 
@@ -1254,45 +1237,30 @@ int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const ui
   if (n == 0 || (!out_off && ob == 0)) return CAPY_OK;
   auto out_begin = [&](uint64_t i) -> uint64_t { return out_off ? out_off[i] : i * ob; };
   auto shards = split_items(off, 0, 0, n, ctx->devs.size(), 400 + ob);
-  return for_each_device(ctx, shards, [&](DeviceCtx& dc, Range sh, int*) -> int {
-    const uint64_t tot = off[sh.i1] - off[sh.i0] + (out_begin(sh.i1) - out_begin(sh.i0));
-    auto chunks = split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, tot - (off[sh.i1] - off[sh.i0])), 400 + ob);
-    return run_chunks(ctx, dc, chunks, nullptr, [&](cudaStream_t st, Range ch, int*) -> int {
-      const uint64_t cnt = ch.i1 - ch.i0;
-      StagedPacked sx, sk;
-      int rc = stage_packed(ctx, dc, st, kHost0, kHost1, data, off, ch.i0, ch.i1, &sx);
-      if (rc) return rc;
-      rc = stage_packed(ctx, dc, st, kHost2, kHost3, keys, key_off, ch.i0, ch.i1, &sk);
-      if (rc) return rc;
-      const uint64_t ob0 = out_begin(ch.i0), ob1 = out_begin(ch.i1);
-      uint8_t* d_out = (uint8_t*)scratch_get(dc, st, kHost4, (size_t)(ob1 - ob0) + 16);
-      if (!d_out) return CAPY_ERR_OOM;
-      const uint64_t* d_out_off = nullptr;
-      uint8_t* d_out_base = d_out;
-      if (out_off) {
-        uint64_t* p = (uint64_t*)scratch_get(dc, st, kHost5, (size_t)(cnt + 1) * 8);
-        if (!p) return CAPY_ERR_OOM;
-        CAPY_CUDA(ctx, cudaMemcpyAsync(p, out_off + ch.i0, (size_t)(cnt + 1) * 8, cudaMemcpyHostToDevice, st));
-        d_out_off = p;
-        d_out_base = reinterpret_cast<uint8_t*>(reinterpret_cast<uintptr_t>(d_out) - (uintptr_t)ob0);
-      }
-      KmacDevArgs a{};
-      a.d_bits = d_bits;
-      a.keys = sk.d_base;
-      a.key_off = sk.d_off;
-      a.data = sx.d_base;
-      a.off = sx.d_off;
-      a.n = cnt;
-      a.custom = custom;
-      a.custom_len = custom_len;
-      a.out_bytes = a.out_stride = ob;
-      a.out_off = d_out_off;
-      a.out = d_out_base;
-      rc = launch_kmac_xof(ctx, dc, st, a);
-      if (rc) return rc;
-      if (ob1 > ob0) return copy_out(ctx, dc, st, kHost4, out + ob0, d_out, (size_t)(ob1 - ob0));
-      return CAPY_OK;
-    });
+  auto chunks = [&](Range sh) {
+    return split_items(off, 0, sh.i0, sh.i1, ragged_chunk_count(off, sh.i0, sh.i1, out_begin(sh.i1) - out_begin(sh.i0)),
+                       400 + ob);
+  };
+  return run_host_call(ctx, shards, chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sx = io.in_packed(data, off), sk = io.in_packed(keys, key_off);
+    KmacDevArgs a{};
+    a.d_bits = d_bits;
+    a.keys = sk.d_base;
+    a.key_off = sk.d_off;
+    a.data = sx.d_base;
+    a.off = sx.d_off;
+    a.n = io.n();
+    a.custom = custom;
+    a.custom_len = custom_len;
+    a.out_bytes = a.out_stride = ob;
+    if (out_off) {
+      a.out_off = (const uint64_t*)io.in(out_off, 8, (size_t)(io.n() + 1) * 8);
+      a.out = io.out_packed(out, out_off);
+    } else {
+      a.out = io.out(out, ob);
+    }
+    if (io.rc()) return io.rc();
+    return launch_kmac_xof(ctx, dc, st, a);
   });
 }
 

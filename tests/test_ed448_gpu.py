@@ -201,6 +201,23 @@ def test_ecdh_agreement(engine, oracle):
     assert rc == 0 and np.array_equal(W2[:, :56], wx)
 
 
+def test_ecdh_without_z(engine):
+    """capy_ed448_ecdh_batch with z_xy112 == NULL: the same W.x as with Z requested, and a bad point is still reported."""
+    rnd = random.Random(31)
+    n = 64
+    pd, po = pack([rnd.randbytes(16) for _ in range(n)])
+    pub = engine.ed448_keygen(pd, po, 512)
+    k = np.frombuffer(rnd.randbytes(56 * n), dtype=np.uint8)
+    rc, wx, Z = engine.ed448_ecdh(k, pub)
+    assert rc == 0 and Z is not None
+    rc, wx_only, Z_none = engine.ed448_ecdh(k, pub, want_z=False)
+    assert rc == 0 and Z_none is None and np.array_equal(wx_only, wx)
+    pub[5] = np.frombuffer(E.point_to_bytes((5, 7)), dtype=np.uint8)
+    rc, wx_bad, _ = engine.ed448_ecdh(k, pub, want_z=False)
+    keep = np.arange(n) != 5
+    assert rc == B.ERR_BAD_POINT and not wx_bad[5].any() and np.array_equal(wx_bad[keep], wx[keep])
+
+
 def test_unsupported_security_parameter(engine):
     pd, po = pack([b"pw"])
     with pytest.raises(B.CapyError) as e:
