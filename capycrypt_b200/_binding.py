@@ -83,6 +83,14 @@ SIGNATURES = {
     "capy_ed448_verify_prepared_batch_dev": (i32, [vp, i32, vp, i32, vp, u8p, u64p, u8p, u8p, u64, u8p]),
     "capy_ed448_key_encrypt_prepared_batch": (i32, [vp, i32, vp, u8p, u8p, u64p, u64, u8p, u8p, u8p]),
     "capy_ed448_key_encrypt_prepared_batch_dev": (i32, [vp, i32, vp, i32, vp, u8p, u8p, u64p, u64, u8p, u8p, u8p]),
+    "capy_sha3_hasher_new": (i32, [vp, i32, u64, C.POINTER(vp)]),
+    "capy_kmac_xof_hasher_new": (i32, [vp, i32, u8p, u64p, u64, u8p, u32, C.POINTER(vp)]),
+    "capy_hasher_device_range": (i32, [vp, i32, C.POINTER(u64), C.POINTER(u64)]),
+    "capy_hasher_update": (i32, [vp, vp, u8p, u64p]),
+    "capy_hasher_update_dev": (i32, [vp, vp, i32, vp, u8p, u64p]),
+    "capy_hasher_final": (i32, [vp, vp, u64, u64p, u8p]),
+    "capy_hasher_final_dev": (i32, [vp, vp, i32, vp, u64, u64p, u8p]),
+    "capy_hasher_free": (None, [vp]),
 }
 
 

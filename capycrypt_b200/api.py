@@ -24,7 +24,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from ._binding import ERR_BAD_POINT, CapyError
-from .engine import Engine, PreparedPublicKey, pack
+from .engine import Engine, Hasher, PreparedPublicKey, pack
 
 
 class OperationError(Exception):
@@ -118,6 +118,22 @@ class Gpu:
         kd, ko = pack(keys)
         xd, xo = pack(xs)
         return [r.tobytes() for r in self.engine.kmac_xof(kd, ko, xd, xo, l, s, int(d))]
+
+    # ---- messages in pieces ----------------------------------------------------------------------------
+    def sha3_stream(self, n: int, d: SecParam) -> "SpongeStream":
+        """n compute_sha3_hash streams fed in pieces: finish() gives the digests of the concatenated pieces."""
+        d = SecParam.try_from(int(d))
+        return SpongeStream(self.engine.sha3_hasher(n, int(d)), int(d))
+
+    def kmac_xof_stream(self, keys: Sequence[bytes], s: str | bytes, d: SecParam) -> "SpongeStream":
+        """one kmac_xof stream per key, fed in pieces: finish(l) gives kmac_xof(key, concatenated pieces, l, s, d);
+        compute_tagged_hash is finish(d).  D224 is refused (ValueError): see capy_gpu.h."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("kmac_xof_stream: D224 is not resumable (quirk Q7)")
+        s = s.encode() if isinstance(s, str) else s
+        kd, ko = pack(keys)
+        return SpongeStream(self.engine.kmac_xof_hasher(kd, ko, s, int(d)), int(d))
 
     # ---- KeyPair::new ----------------------------------------------------------------------------------
     def new_keypairs(self, pws: Sequence[bytes], owner: str, d: SecParam) -> list[KeyPair]:
@@ -311,6 +327,33 @@ class Gpu:
                 else:
                     res[i] = OperationError("KeyDecryptionError")
         return res
+
+
+class SpongeStream:
+    """Streams of Gpu.sha3_stream / Gpu.kmac_xof_stream: update() appends one piece per stream, finish() ends them.
+    Use it in a `with` block (or call close()) to release its device memory before the engine."""
+
+    def __init__(self, hasher: Hasher, d: int):
+        self.hasher = hasher
+        self.d = d
+
+    def update(self, pieces: Sequence[bytes]) -> None:
+        data, off = pack(pieces)
+        self.hasher.update(data, off)
+
+    def finish(self, l: Optional[int] = None) -> list[bytes]:
+        """SHA3-d: the digests (l must be None or d).  KMACXOF: l output bits per stream (default d)."""
+        out = self.hasher.final(self.d if l is None else l)
+        return [r.tobytes() for r in out]
+
+    def close(self) -> None:
+        self.hasher.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
 
 
 def _append_reference_padding(msg: bytearray, d: int) -> None:

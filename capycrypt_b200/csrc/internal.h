@@ -188,6 +188,26 @@ struct capy_ed448_pub {
   std::vector<uint32_t*> d_table;  // [device index] comb table of phi(V), or nullptr
 };
 
+// A batch of resumable SHA3-d / KMACXOF streams (capy_sha3_hasher_new / capy_kmac_xof_hasher_new, sha3_api.cu).  Items
+// [first[k], first[k + 1]) live on device k of the ctx that created it, in buffers of their own: they are not scratch
+// slots, so the one-shot calls between two updates never touch them.  On device k, item j (counted from first[k]) has
+//   d_state[k]  25 lanes at [l * items_k + j]: every whole block of its stream so far (200 B per item)
+//   d_carry[k]  the bytes behind the last whole block at [j * rate ..), total % rate of them
+//   d_total[k]  [j] = message bytes absorbed so far (uint64)
+struct capy_hasher {
+  const capy_ctx* ctx = nullptr;
+  int d_bits = 0;
+  bool kmac = false;
+  uint32_t rate = 0;
+  uint64_t n = 0;
+  std::vector<uint64_t> first;     // [device index] first item; first[devices] = n
+  std::vector<int> dev;            // CUDA device of every ctx device (frees without the ctx)
+  std::vector<uint64_t*> d_state;  // [device index], nullptr when the device holds no item
+  std::vector<uint8_t*> d_carry;
+  std::vector<uint64_t*> d_total;
+  std::vector<char> finished;      // [device index] its items were finalised
+};
+
 namespace capy {
 
 // RAII device switch

@@ -655,9 +655,10 @@ static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t
   return true;
 }
 
-// two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel)
+// two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel); with
+// jobs = 1, J0 alone (and, with `resume`, as resumable streams)
 static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J0, const SpongeJob& J1,
-                             bool data_dependent) {
+                             bool data_dependent, uint32_t jobs = 2, const SpongeResume* resume = nullptr) {
   const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
   uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
   if (!sync) return CAPY_ERR_OOM;
@@ -668,8 +669,9 @@ static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, 
   C.sync = sync;
   C.blocks_per_job = nb;
   C.data_dependent = data_dependent ? 1u : 0u;
+  C.resume = resume ? *resume : SpongeResume{};
   return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J0), [&](auto L) {
-    sponge_chain_kernel<decltype(L)::value><<<2 * nb, 128, 0, stream>>>(C);
+    sponge_chain_kernel<decltype(L)::value><<<jobs * nb, 128, 0, stream>>>(C);
     ctx->launches++;
     CAPY_CUDA(ctx, cudaGetLastError());
     return CAPY_OK;
@@ -1007,6 +1009,108 @@ int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const
   return launch_chain_jobs(ctx, dc, stream, J0, J1, true);
 }
 
+// ---- resumable streams (capy_hasher) -------------------------------------------------------------------------------
+// Every update and final is ONE single-job launch of sponge_chain_kernel over a range of the hasher's items on one device
+// (thread per item, no order, no cut); SpongeJob::carry switches sponge_item to the resumed stream.
+static int hasher_check(const capy_ctx* ctx, const capy_hasher* h) { return h && ctx && h->ctx == ctx ? CAPY_OK : CAPY_ERR_BAD_ARG; }
+static uint64_t hasher_items(const capy_hasher* h, int k) { return h->first[k + 1] - h->first[k]; }
+static bool hasher_any_finished(const capy_hasher* h) {
+  for (char f : h->finished)
+    if (f) return true;
+  return false;
+}
+static std::vector<Range> hasher_shards(const capy_hasher* h) {  // one per device, in device order (for_each_device)
+  std::vector<Range> s;
+  for (size_t k = 0; k + 1 < h->first.size(); k++) s.push_back({h->first[k], h->first[k + 1]});
+  return s;
+}
+
+// the job of an update or a final over the items [j0, j0 + n) of device k (indices on that device), and its streams
+static SpongeJob hasher_job(const capy_hasher* h, int k, uint64_t j0, uint64_t n, SpongeResume* R) {
+  SpongeJob J{};
+  J.rate = h->rate;
+  J.sq_lanes = (1600 - h->d_bits) / 64;
+  if (h->kmac) {
+    J.trailer = 0x040100u;  // right_encode(0) = 00 01 (shake_functions.rs:86) then 04 (:57)
+    J.trailer_len = 3;
+  } else {
+    J.sha3_suffix = 1;  // 06 | 86 from the total length (Q2)
+    J.trailer_len = 1;
+  }
+  J.chain_in = h->d_state[k] + j0;
+  J.n = n;
+  R->carry = h->d_carry[k] + j0 * h->rate;
+  R->totals = h->d_total[k] + j0;
+  R->state_n = hasher_items(h, k);
+  return J;
+}
+
+static int hasher_update_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, uint64_t j0, uint64_t n,
+                               const uint8_t* d_data, const uint64_t* d_off) {
+  if (n == 0) return CAPY_OK;
+  SpongeResume R;
+  SpongeJob J = hasher_job(h, dc.index, j0, n, &R);
+  J.chain_out = h->d_state[dc.index] + j0;
+  J.stop_block = ~0ull;
+  J.data = d_data;
+  J.off = d_off;
+  return launch_chain_jobs(ctx, dc, st, J, J, false, 1, &R);
+}
+
+static int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
+                              uint64_t out_bytes, const uint64_t* d_out_off, uint8_t* d_out) {
+  if (n == 0 || (!d_out_off && out_bytes == 0)) return CAPY_OK;
+  SpongeResume R;
+  SpongeJob J = hasher_job(h, dc.index, j0, n, &R);
+  J.out = d_out;
+  J.out_off = d_out_off;
+  J.out_stride = J.out_bytes = out_bytes;
+  return launch_chain_jobs(ctx, dc, st, J, J, false, 1, &R);
+}
+
+// A hasher with zeroed buffers on every device that holds items (blocking).  Items are dealt out in equal contiguous
+// ranges.
+static int hasher_create(capy_ctx* ctx, int d_bits, bool kmac, uint64_t n, capy_hasher** out) {
+  capy_hasher* h = new (std::nothrow) capy_hasher();
+  if (!h) return CAPY_ERR_OOM;
+  h->ctx = ctx;
+  h->d_bits = d_bits;
+  h->kmac = kmac;
+  h->rate = kmac ? (uint32_t)(1600 - d_bits) / 8 : (1600 - sha3_capacity(d_bits)) / 8;
+  h->n = n;
+  const uint64_t nd = ctx->devs.size();
+  for (uint64_t k = 0; k <= nd; k++) h->first.push_back((n / nd) * k + std::min(k, n % nd));
+  for (const DeviceCtx& dc : ctx->devs) h->dev.push_back(dc.dev);
+  h->d_state.assign(nd, nullptr);
+  h->d_carry.assign(nd, nullptr);
+  h->d_total.assign(nd, nullptr);
+  h->finished.assign(nd, 0);
+  for (DeviceCtx& dc : ctx->devs) {
+    const uint64_t m = hasher_items(h, dc.index);
+    if (m == 0) continue;
+    std::lock_guard<std::mutex> lk(*dc.mu);
+    DeviceGuard g(dc.dev);
+    const cudaStream_t st = dc.streams[0];
+    const int rc = [&]() -> int {
+      CAPY_CUDA(ctx, cudaMalloc(&h->d_state[dc.index], (size_t)m * 200));
+      CAPY_CUDA(ctx, cudaMalloc(&h->d_carry[dc.index], (size_t)m * h->rate));
+      CAPY_CUDA(ctx, cudaMalloc(&h->d_total[dc.index], (size_t)m * 8));
+      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_state[dc.index], 0, (size_t)m * 200, st));
+      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_carry[dc.index], 0, (size_t)m * h->rate, st));
+      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_total[dc.index], 0, (size_t)m * 8, st));
+      CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+      return CAPY_OK;
+    }();
+    if (rc) {
+      cudaGetLastError();
+      capy_hasher_free(h);
+      return rc;
+    }
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
 }  // namespace capy
 
 using namespace capy;
@@ -1288,6 +1392,144 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
   int rc = plan_ragged(ctx, dc, st, d_off, n, J.rate, &plan);
   if (rc) return rc;
   return run_sponge(ctx, dc, st, J, plan);
+}
+
+// =================================================================================================
+// resumable SHA3-d / KMACXOF streams
+// =================================================================================================
+int capy_sha3_hasher_new(capy_ctx* ctx, int d_bits, uint64_t n, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  return hasher_create(ctx, d_bits, false, n, out);
+}
+
+int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, const uint64_t* key_off, uint64_t n,
+                             const uint8_t* custom, uint32_t custom_len, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx || (n && (!keys || !key_off)) || (custom_len && !custom)) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // the 172-byte rate is read as 168 (Q7): see the header
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, true, n, &h);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  // P | KB: the cached prefix state, then the key block of every item -- a KMAC job with no message and no trailer ends
+  // exactly there; its states are the hasher's starting states (one chunk per device: the states are stored at [k * n + i])
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    const StagedPacked sk = io.in_packed(keys, key_off);
+    if (io.rc()) return io.rc();
+    KmacDevArgs a{};
+    a.d_bits = d_bits;
+    a.keys = sk.d_base;
+    a.key_off = sk.d_off;
+    a.data = sk.d_base;  // (no message: never read)
+    a.n = io.n();
+    a.custom = custom;
+    a.custom_len = custom_len;
+    SpongeJob J;
+    const int rj = build_kmac_job(ctx, dc, st, a, &J);
+    if (rj) return rj;
+    J.trailer = 0;
+    J.trailer_len = 0;
+    J.chain_out = h->d_state[dc.index];
+    J.stop_block = ~0ull;
+    return launch_chain_jobs(ctx, dc, st, J, J, false, 1);
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+int capy_hasher_device_range(const capy_hasher* h, int dev_index, uint64_t* i0, uint64_t* i1) {
+  if (!h || !i0 || !i1 || dev_index < 0 || dev_index >= (int)h->dev.size()) return CAPY_ERR_BAD_ARG;
+  *i0 = h->first[dev_index];
+  *i1 = h->first[dev_index + 1];
+  return CAPY_OK;
+}
+
+int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off) {
+  if (hasher_check(ctx, h) || hasher_any_finished(h) || (h->n && (!data || !off))) return CAPY_ERR_BAD_ARG;
+  if (h->n == 0) return CAPY_OK;
+  auto chunks = [&](Range sh) {
+    return split_items(off, 0, sh.i0, sh.i1, chunk_count(off[sh.i1] - off[sh.i0], sh.i1 - sh.i0), 200);
+  };
+  return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(data, off);
+    if (io.rc()) return io.rc();
+    return hasher_update_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), sp.d_base, sp.d_off);
+  });
+}
+
+int capy_hasher_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_data,
+                           const uint64_t* d_off) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || h->finished[dev_index]) return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && (!d_data || !d_off)) return CAPY_ERR_BAD_ARG;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return hasher_update_items(ctx, dc, st, h, 0, m, d_data, d_off);
+}
+
+int capy_hasher_final(capy_ctx* ctx, capy_hasher* h, uint64_t out_bits, const uint64_t* out_off, uint8_t* out) {
+  if (hasher_check(ctx, h) || hasher_any_finished(h) || (h->n && !out)) return CAPY_ERR_BAD_ARG;
+  if (!h->kmac && (out_bits != (uint64_t)h->d_bits || out_off)) return CAPY_ERR_BAD_ARG;
+  for (char& f : h->finished) f = 1;
+  const size_t ob = (size_t)(out_bits / 8);
+  if (h->n == 0 || (!out_off && ob == 0)) return CAPY_OK;
+  auto out_begin = [&](uint64_t i) -> uint64_t { return out_off ? out_off[i] : i * ob; };
+  auto chunks = [&](Range sh) {
+    return split_items(out_off, ob, sh.i0, sh.i1, chunk_count(out_begin(sh.i1) - out_begin(sh.i0), sh.i1 - sh.i0), 0);
+  };
+  return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const uint64_t* d_out_off = nullptr;
+    uint8_t* d_out;
+    if (out_off) {
+      d_out_off = (const uint64_t*)io.in(out_off, 8, (size_t)(io.n() + 1) * 8);
+      d_out = io.out_packed(out, out_off);
+    } else {
+      d_out = io.out(out, ob);
+    }
+    if (io.rc()) return io.rc();
+    return hasher_final_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), ob, d_out_off, d_out);
+  });
+}
+
+int capy_hasher_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint64_t out_bits,
+                          const uint64_t* d_out_off, uint8_t* d_out) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || h->finished[dev_index]) return CAPY_ERR_BAD_ARG;
+  if (!h->kmac && (out_bits != (uint64_t)h->d_bits || d_out_off)) return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && !d_out) return CAPY_ERR_BAD_ARG;
+  h->finished[dev_index] = 1;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return hasher_final_items(ctx, dc, st, h, 0, m, out_bits / 8, d_out_off, d_out);
+}
+
+void capy_hasher_free(capy_hasher* h) {
+  if (!h) return;
+  for (size_t k = 0; k < h->dev.size(); k++) {
+    if (!h->d_state[k] && !h->d_carry[k] && !h->d_total[k]) continue;
+    DeviceGuard g(h->dev[k]);
+    cudaDeviceSynchronize();  // work still queued on a caller's stream may read them
+    // after the key block a KMAC state is key material: zeroed before the memory goes back
+    if (h->d_state[k]) cudaMemset(h->d_state[k], 0, (size_t)hasher_items(h, (int)k) * 200);
+    if (h->d_carry[k]) cudaMemset(h->d_carry[k], 0, (size_t)hasher_items(h, (int)k) * h->rate);
+    cudaDeviceSynchronize();
+    if (h->d_state[k]) cudaFree(h->d_state[k]);
+    if (h->d_carry[k]) cudaFree(h->d_carry[k]);
+    if (h->d_total[k]) cudaFree(h->d_total[k]);
+  }
+  delete h;
 }
 
 }  // extern "C"

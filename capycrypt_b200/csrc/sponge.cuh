@@ -77,6 +77,17 @@ struct SpongeJob {
   uint64_t stop_block;
 };
 
+// Resumable streams (capy_hasher; a job of sponge_chain_kernel with order == nullptr, so rank = item i).  Item i's state
+// at chain_in[k * state_n + i] holds every whole block of its stream before the carry bytes carry[i * rate ..), whose
+// count is totals[i] % rate.  With chain_out the job is an update (absorbs the whole blocks of carry | X, stores the
+// state, keeps the rest as the new carry, adds |X| to totals[i]); without, the final (carry | T | pad, then squeeze).
+// Kept out of SpongeJob, so that the kernels without a hand-off compile to what they were.
+struct SpongeResume {
+  uint8_t* carry;    // nullptr: not a resumable job
+  uint64_t* totals;
+  uint64_t state_n;  // stride of the lane-major states (the items of the device; a job may cover a part of them)
+};
+
 __device__ __forceinline__ uint32_t left_encode_nbytes(uint64_t v) {
   uint32_t nb = 1;
   while (nb < 8 && (v >> (8 * nb)) != 0) nb++;
@@ -186,6 +197,35 @@ struct SpongeGeom {
     if (J.fips_pad && !has_pad) trailer |= 0x80u << (8 * (trailer_len - 1));
   }
 
+  // The stream of a resumable item (SpongeResume): the carry stands in the place of P, so this job absorbs  carry | X  (an
+  // update: whole blocks only, no trailer, no pad) or  carry | T | pad  (the final job).  Everything before the carry was
+  // block-aligned, so the carry and T alone decide whether there is a pad block (Q1), and the SHA3-d suffix comes from
+  // the total length (Q2).  RATE is lane-aligned: D224 KMAC (Q7) is not resumable.
+  template <uint32_t RATE>
+  __device__ __forceinline__ void init_resume(const SpongeJob& J, const SpongeResume& R, uint64_t i) {
+    const uint64_t total = R.totals[i];
+    const bool update = J.chain_out != nullptr;
+    prefix = R.carry + i * RATE;
+    prefix_len = (uint32_t)(total % RATE);
+    key = nullptr;
+    hdr_len = 0;
+    k0 = k1 = x0 = prefix_len;
+    x = prefix;
+    uint64_t xlen = 0;
+    if (update) {
+      x = J.data + J.off[i];
+      xlen = J.off[i + 1] - J.off[i];
+    }
+    x1 = x0 + xlen;
+    trailer = update ? 0u : J.sha3_suffix ? ((total % 136u == 135u) ? 0x86u : 0x06u) : J.trailer;
+    t1 = p1 = x1 + (update ? 0u : J.trailer_len);
+    has_pad1 = false;
+    const uint64_t rem = t1 % RATE;
+    has_pad = !update && rem != 0;
+    padded = has_pad ? t1 + (RATE - rem) : t1;
+    nblocks = padded / RATE;  // an update: the whole blocks of carry | X
+  }
+
   // bytes of the segment [seg0, seg1) (stream offsets; base[0] sits at seg0) that fall into the lane at o
   template <bool COH = false>
   static __device__ __forceinline__ uint64_t piece(const uint8_t* base, uint64_t seg0, uint64_t seg1, uint64_t o) {
@@ -238,15 +278,22 @@ struct SpongeGeom {
 // CHAIN: the item may start from / stop at a handed-over state (rank = its slot in the hand-off arrays); the plain
 // kernels instantiate CHAIN = false and compile to what they were.
 // COH: the message was written earlier in this launch (dependent job): see ld_u8.
-template <int LANES, bool CHAIN = false, bool COH = false>
-__device__ __forceinline__ void sponge_item(const SpongeJob& J, uint64_t i, uint64_t rank = 0) {
+// RESUME (with CHAIN): the item is the resumable stream R describes (SpongeGeom::init_resume); an update also leaves the
+// new carry and total behind.
+template <int LANES, bool CHAIN = false, bool COH = false, bool RESUME = false>
+__device__ __forceinline__ void sponge_item(const SpongeJob& J, uint64_t i, uint64_t rank = 0, const SpongeResume* R = nullptr) {
   SpongeGeom g;
-  g.template init<8u * LANES>(J, i);
+  uint64_t state_n = J.n;
+  if constexpr (RESUME) {
+    g.template init_resume<8u * LANES>(J, *R, i);
+    state_n = R->state_n;
+  }
+  else g.template init<8u * LANES>(J, i);
   Lane a[25];
   if (CHAIN && J.chain_in) {
 #pragma unroll
     for (int k = 0; k < 25; k++) {
-      const uint64_t v = __ldcg(J.chain_in + (uint64_t)k * J.n + rank);  // written by another SM in this launch: L2, not L1
+      const uint64_t v = __ldcg(J.chain_in + (uint64_t)k * state_n + rank);  // written by another SM in this launch: L2, not L1
       a[k].lo = (uint32_t)v;
       a[k].hi = (uint32_t)(v >> 32);
     }
@@ -406,7 +453,14 @@ __device__ __forceinline__ void sponge_item(const SpongeJob& J, uint64_t i, uint
 
   if (CHAIN && J.chain_out) {  // hand the state to the next segment (coalesced: lane k of rank r at [k * n + r])
 #pragma unroll
-    for (int k = 0; k < 25; k++) J.chain_out[(uint64_t)k * J.n + rank] = ((uint64_t)a[k].hi << 32) | a[k].lo;
+    for (int k = 0; k < 25; k++) J.chain_out[(uint64_t)k * state_n + rank] = ((uint64_t)a[k].hi << 32) | a[k].lo;
+    if constexpr (RESUME) {  // an update: the bytes behind the last whole block are the new carry (the old one was read above)
+      uint8_t* cb = R->carry + i * STRIDE;
+      const uint64_t s0 = nblocks * STRIDE;
+#pragma unroll 1
+      for (uint64_t q = s0 > g.x0 ? s0 : g.x0; q < g.x1; q++) cb[q - s0] = g.x[q - g.x0];
+      R->totals[i] += g.x1 - g.x0;
+    }
     return;
   }
 
@@ -732,7 +786,8 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_kernel2(const __
 // each: 6.92 per scheduler.  Both jobs are ONE launch; a block takes a ticket when it starts, the first `blocks_per_job`
 // tickets work on job 0, the others on job 1, and a job-1 block waits for the job-0 block of the same items (which holds a
 // smaller ticket, so it is running or done: no deadlock).  The launcher only cuts batches with at least as many job-0
-// blocks as the GPU holds at once, so in practice nobody waits.
+// blocks as the GPU holds at once, so in practice nobody waits.  A launch of only `blocks_per_job` blocks runs job 0 alone
+// (every ticket is a job-0 ticket, nobody waits): the updates and finals of resumable streams (SpongeJob::carry).
 struct SpongeChain {
   SpongeJob j[2];
   uint32_t* sync;  // [0] ticket counter, [1 + b] warps of job-0 block b that have stored their states; zeroed before the launch
@@ -740,7 +795,14 @@ struct SpongeChain {
   // job 1 reads, as its message, bytes that job 0 wrote for the same item (the two passes of an authenticated
   // decryption: keystream XOR, then the tag over the plaintext): its message loads go to the L2
   uint32_t data_dependent;
+  SpongeResume resume;  // carry == nullptr: the jobs are not resumable streams
 };
+// resumable streams (order == nullptr: rank = item), out of line: the cut chains keep their own register allocation
+template <int LANES>
+__device__ __noinline__ void sponge_item_resume_ool(const SpongeJob& J, const SpongeResume* R, uint64_t i) {
+  sponge_item<LANES, true, false, true>(J, i, i, R);
+}
+
 template <int LANES>
 __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(const __grid_constant__ SpongeChain C) {
   __shared__ uint32_t ticket_s;
@@ -757,6 +819,7 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(con
   const uint64_t r = (uint64_t)b * 128 + threadIdx.x;
   if (r < J.n) {
     if (job && C.data_dependent) sponge_item<LANES, true, true>(J, sponge_rank_item(J, r), r);
+    else if (C.resume.carry) sponge_item_resume_ool<LANES>(J, &C.resume, r);
     else sponge_item<LANES, true>(J, sponge_rank_item(J, r), r);
   }
   if (!job) {

@@ -105,6 +105,78 @@ class PreparedPublicKey:
             pass
 
 
+class Hasher:
+    """A batch of n resumable SHA3-d or KMACXOF streams on one Engine (Engine.sha3_hasher / Engine.kmac_xof_hasher).
+    update() appends one piece per stream; final() returns what Engine.sha3 / Engine.kmac_xof return for the concatenated
+    pieces.  close() it (or leave the `with` block) before the engine."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, n: int, d: int, kmac: bool):
+        self._engine = engine
+        self.handle = handle
+        self.n = n
+        self.d = d
+        self.kmac = kmac
+
+    def device_range(self, dev_index: int = 0) -> tuple[int, int]:
+        """the items [i0, i1) that live on device dev_index of the engine"""
+        i0, i1 = C.c_uint64(0), C.c_uint64(0)
+        self._engine._check(self._engine.lib.capy_hasher_device_range(self.handle, dev_index, C.byref(i0), C.byref(i1)))
+        return int(i0.value), int(i1.value)
+
+    def update(self, data, off) -> None:
+        """capy_hasher_update: stream i appends data[off[i] .. off[i+1]) (blocking)"""
+        data, off = _u8(data), _u64(off)
+        if _need_packed(data, off, "hasher pieces") != self.n:
+            raise ValueError(f"hasher update: {off.size - 1} pieces for {self.n} streams")
+        self._engine._check(self._engine.lib.capy_hasher_update(self._engine._ctx, self.handle, _hp(data), _hp(off)))
+
+    def final(self, out_bits: int | None = None, out_off=None, out: np.ndarray | None = None) -> np.ndarray:
+        """capy_hasher_final: SHA3-d -> n x d/8 digests; KMACXOF -> n x out_bits/8, or packed by out_off"""
+        out_bits = self.d if out_bits is None else out_bits
+        if out_off is None:
+            out = _out(out, (self.n, out_bits // 8), "hasher output")
+            oo = None
+        else:
+            out_off = _u64(out_off)
+            if out_off.size != self.n + 1 or bool(np.any(out_off[1:] < out_off[:-1])):
+                raise ValueError("hasher final: out_off needs n + 1 non-decreasing entries")
+            out = _out(out, (int(out_off[-1]),), "hasher output")
+            oo = _hp(out_off)
+        self._engine._check(self._engine.lib.capy_hasher_final(self._engine._ctx, self.handle, out_bits, oo, _hp(out)))
+        return out
+
+    def update_dev(self, t_data, t_off, dev_index: int = 0) -> None:
+        """capy_hasher_update_dev on torch's current stream: t_off holds i1 - i0 + 1 offsets (device_range)"""
+        self._engine._check(self._engine.lib.capy_hasher_update_dev(self._engine._ctx, self.handle, dev_index,
+                                                                    self._engine._stream(), t_data.data_ptr(),
+                                                                    t_off.data_ptr()))
+
+    def final_dev(self, t_out, out_bits: int | None = None, t_out_off=None, dev_index: int = 0):
+        """capy_hasher_final_dev on torch's current stream (the items of device_range(dev_index))"""
+        out_bits = self.d if out_bits is None else out_bits
+        self._engine._check(self._engine.lib.capy_hasher_final_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), out_bits,
+            t_out_off.data_ptr() if t_out_off is not None else None, t_out.data_ptr()))
+        return t_out
+
+    def close(self):
+        if self.handle is not None and self.handle.value:
+            self._engine.lib.capy_hasher_free(self.handle)
+        self.handle = C.c_void_p()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
 class Engine:
     """One capy_ctx.  devices=None -> current CUDA device."""
 
@@ -224,6 +296,22 @@ class Engine:
         self._check(self.lib.capy_kmac_xof_batch(self._ctx, d, _hp(keys), _hp(key_off), _hp(data), _hp(off), n,
                                                  _hp(cs_a), len(cs_a), out_bits, oo, _hp(out)))
         return out
+
+    def sha3_hasher(self, n: int, d: int) -> Hasher:
+        """capy_sha3_hasher_new: n resumable SHA3-d streams (blocking)"""
+        h = C.c_void_p()
+        self._check(self.lib.capy_sha3_hasher_new(self._ctx, d, n, C.byref(h)))
+        return Hasher(self, h, n, d, False)
+
+    def kmac_xof_hasher(self, keys, key_off, custom: bytes, d: int) -> Hasher:
+        """capy_kmac_xof_hasher_new: one resumable KMACXOF stream per key, customisation string `custom` (blocking)"""
+        keys, key_off = _u8(keys), _u64(key_off)
+        n = _need_packed(keys, key_off, "hasher keys")
+        cs_a = _u8(custom)
+        h = C.c_void_p()
+        self._check(self.lib.capy_kmac_xof_hasher_new(self._ctx, d, _hp(keys), _hp(key_off), n, _hp(cs_a), len(cs_a),
+                                                      C.byref(h)))
+        return Hasher(self, h, n, d, True)
 
     def ed448_fixed_base(self, scalars_be56, out: np.ndarray | None = None) -> np.ndarray:
         sc = _u8(scalars_be56)

@@ -122,6 +122,58 @@ class PreparedPublicKey {
   capy_ed448_pub* key_ = nullptr;
 };
 
+// A batch of resumable SHA3-d or KMACXOF streams (Engine::sha3_hasher / Engine::kmac_xof_hasher): update() appends one
+// piece per stream, final() returns what compute_sha3_hash / kmac_xof return for the concatenated pieces.  Destroy it
+// before the Engine.
+class Hasher {
+ public:
+  Hasher(Hasher&& o) noexcept : ctx_(o.ctx_), h_(o.h_), n_(o.n_), d_bits_(o.d_bits_) { o.h_ = nullptr; }
+  Hasher& operator=(Hasher&& o) noexcept {
+    if (this != &o) {
+      capy_hasher_free(h_);
+      ctx_ = o.ctx_;
+      h_ = o.h_;
+      n_ = o.n_;
+      d_bits_ = o.d_bits_;
+      o.h_ = nullptr;
+    }
+    return *this;
+  }
+  Hasher(const Hasher&) = delete;
+  Hasher& operator=(const Hasher&) = delete;
+  ~Hasher() { capy_hasher_free(h_); }
+
+  // pieces[i] is appended to stream i
+  void update(const std::vector<Bytes>& pieces) {
+    if (pieces.size() != n_) throw GpuError(CAPY_ERR_BAD_ARG, "Hasher::update: one piece per stream");
+    Bytes data;
+    std::vector<uint64_t> off;
+    detail::pack(pieces, [](const Bytes& b) -> const Bytes& { return b; }, data, off);
+    check(capy_hasher_update(ctx_, h_, data.data(), off.data()));
+  }
+  // SHA3-d: out_bits = d_bits (0 = d_bits); KMACXOF: out_bits per stream
+  std::vector<Bytes> final(uint64_t out_bits = 0) {
+    if (out_bits == 0) out_bits = (uint64_t)d_bits_;
+    const size_t ob = (size_t)(out_bits / 8);
+    Bytes out(n_ * ob + 1);
+    check(capy_hasher_final(ctx_, h_, out_bits, nullptr, out.data()));
+    std::vector<Bytes> res(n_);
+    for (size_t i = 0; i < n_; i++) res[i].assign(out.begin() + i * ob, out.begin() + (i + 1) * ob);
+    return res;
+  }
+
+ private:
+  friend class Engine;
+  Hasher(capy_ctx* ctx, capy_hasher* h, size_t n, int d_bits) : ctx_(ctx), h_(h), n_(n), d_bits_(d_bits) {}
+  void check(int rc) {
+    if (rc != CAPY_OK) throw GpuError(rc, rc == CAPY_ERR_CUDA ? capy_last_cuda_error(ctx_) : capy_strerror(rc));
+  }
+  capy_ctx* ctx_ = nullptr;
+  capy_hasher* h_ = nullptr;
+  size_t n_ = 0;
+  int d_bits_ = 0;
+};
+
 class Engine {
  public:
   explicit Engine(const std::vector<int>& devices = {}) {
@@ -168,6 +220,24 @@ class Engine {
     std::vector<Bytes> res(msgs.size());
     for (size_t i = 0; i < msgs.size(); i++) res[i].assign(out.begin() + i * ob, out.begin() + (i + 1) * ob);
     return res;
+  }
+
+  // n SHA3-d streams fed in pieces (blocking)
+  Hasher sha3_hasher(size_t n, int d_bits) {
+    capy_hasher* h = nullptr;
+    check(capy_sha3_hasher_new(ctx_, d_bits, n, &h));
+    return Hasher(ctx_, h, n, d_bits);
+  }
+
+  // one KMACXOF stream per key, customisation string s (blocking); d_bits = 224 is refused (CAPY_ERR_BAD_ARG)
+  Hasher kmac_xof_hasher(const std::vector<Bytes>& keys, const std::string& s, int d_bits) {
+    Bytes kd;
+    std::vector<uint64_t> ko;
+    detail::pack(keys, [](const Bytes& b) -> const Bytes& { return b; }, kd, ko);
+    capy_hasher* h = nullptr;
+    check(capy_kmac_xof_hasher_new(ctx_, d_bits, kd.data(), ko.data(), keys.size(),
+                                   reinterpret_cast<const uint8_t*>(s.data()), (uint32_t)s.size(), &h));
+    return Hasher(ctx_, h, keys.size(), d_bits);
   }
 
   // KeyPair::new for every password

@@ -298,6 +298,43 @@ int capy_ed448_key_encrypt_prepared_batch_dev(capy_ctx* ctx, int dev_index, void
                                               const uint64_t* d_msg_off, uint64_t n, uint8_t* d_ct, uint8_t* d_tag56,
                                               uint8_t* d_z_xy112);
 
+/* ---- Resumable SHA3-d and KMACXOF: messages fed in pieces ------------------------------------------------------------
+ * A hasher is a batch of n independent streams, one per item, for one operator: SHA3-d (compute_sha3_hash) or KMACXOF
+ * (kmac_xof / compute_tagged_hash, one key per item and one customisation string S for the batch).  Each update appends
+ * one piece to every stream (item i: data[off[i] .. off[i+1]), empty pieces allowed); the final returns, byte for byte,
+ * what capy_sha3_batch / capy_kmac_xof_batch return for the concatenated pieces (Q1, Q2 and Q3 included).  Nothing is
+ * packed or kept whole: the device holds per stream its 200-byte state, up to rate - 1 bytes not yet absorbed and the
+ * running length.  So a caller whose data arrives in blocks (files, records, logs) needs no concatenated copy, and
+ * with the _dev calls can copy piece k + 1 to the device while piece k is absorbed.
+ *  - the items are dealt out over the ctx's devices in equal contiguous ranges when the hasher is created
+ *    (capy_hasher_device_range); host calls shard by those ranges, a _dev call covers the items [i0, i1) of its device
+ *    (d_off: i1 - i0 + 1 offsets into d_data; d_out_off likewise, absolute offsets into d_out).
+ *  - the _dev calls of one hasher go, per device, in order on one stream, under the one-stream-at-a-time rule above.
+ *  - after final (or final_dev on a device) the hasher is finished: a later update or final (of those items) returns
+ *    CAPY_ERR_BAD_ARG.  A hasher of another ctx: CAPY_ERR_BAD_ARG.  n == 0 gives a hasher whose calls do nothing.
+ *  - KMACXOF at d_bits = 224 is refused (CAPY_ERR_BAD_ARG): under quirk Q7 its 172-byte rate is counted by 172 but read
+ *    by 168, so which bytes are absorbed depends on the final length (the last 4 x blocks bytes of the stream are never
+ *    read) and a resumable stream would have to keep about 2.3 % of every message until the final.  SHA3-224 is fine. */
+typedef struct capy_hasher capy_hasher;
+/* zeroed streams; blocking */
+int capy_sha3_hasher_new(capy_ctx* ctx, int d_bits, uint64_t n, capy_hasher** out);
+/* absorbs P | bytepad(encode_string(K_i), w) for every item; blocking */
+int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, const uint64_t* key_off, uint64_t n,
+                             const uint8_t* custom, uint32_t custom_len, capy_hasher** out);
+int capy_hasher_device_range(const capy_hasher* h, int dev_index, uint64_t* i0, uint64_t* i1);
+/* off: n + 1 offsets into data */
+int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off);
+int capy_hasher_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_data,
+                           const uint64_t* d_off);
+/* SHA3-d: out_bits == d_bits and out_off == NULL, n x d_bits/8 digests.  KMACXOF: as capy_kmac_xof_batch (out_bits for
+ * every item, or out_off with n + 1 offsets for per-item lengths). */
+int capy_hasher_final(capy_ctx* ctx, capy_hasher* h, uint64_t out_bits, const uint64_t* out_off, uint8_t* out);
+int capy_hasher_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint64_t out_bits,
+                          const uint64_t* d_out_off, uint8_t* d_out);
+/* zeroes and releases the hasher's device memory (a KMAC state holds key material).  NULL is a no-op.  Call before
+ * capy_gpu_destroy of its ctx. */
+void capy_hasher_free(capy_hasher* h);
+
 #ifdef __cplusplus
 }
 #endif

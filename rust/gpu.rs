@@ -22,6 +22,11 @@ pub struct CapyEd448Pub {
     _private: [u8; 0],
 }
 
+#[repr(C)]
+pub struct CapyHasher {
+    _private: [u8; 0],
+}
+
 #[link(name = "capycrypt_gpu", kind = "static")]
 extern "C" {
     fn capy_gpu_init(devices: *const c_int, n_devices: c_int, out_ctx: *mut *mut CapyCtx) -> c_int;
@@ -130,6 +135,18 @@ extern "C" {
     fn capy_ed448_key_encrypt_prepared_batch_dev(ctx: *mut CapyCtx, dev_index: c_int, stream: *mut c_void,
         d_bits: c_int, key: *const CapyEd448Pub, d_k_rand56: *const u8, d_msgs: *const u8, d_msg_off: *const u64,
         n: u64, d_ct: *mut u8, d_tag56: *mut u8, d_z_xy112: *mut u8) -> c_int;
+    fn capy_sha3_hasher_new(ctx: *mut CapyCtx, d_bits: c_int, n: u64, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_kmac_xof_hasher_new(ctx: *mut CapyCtx, d_bits: c_int, keys: *const u8, key_off: *const u64, n: u64,
+        custom: *const u8, custom_len: u32, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_hasher_device_range(h: *const CapyHasher, dev_index: c_int, i0: *mut u64, i1: *mut u64) -> c_int;
+    fn capy_hasher_update(ctx: *mut CapyCtx, h: *mut CapyHasher, data: *const u8, off: *const u64) -> c_int;
+    fn capy_hasher_update_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_data: *const u8, d_off: *const u64) -> c_int;
+    fn capy_hasher_final(ctx: *mut CapyCtx, h: *mut CapyHasher, out_bits: u64, out_off: *const u64,
+        out: *mut u8) -> c_int;
+    fn capy_hasher_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        out_bits: u64, d_out_off: *const u64, d_out: *mut u8) -> c_int;
+    fn capy_hasher_free(h: *mut CapyHasher);
 }
 
 const CAPY_AE_SHA3: c_int = 0;
@@ -523,6 +540,62 @@ impl Gpu {
             m.d = Some(d);
         }
         Ok(())
+    }
+}
+
+/// A batch of resumable SHA3-d or KMACXOF streams (`Gpu::sha3_hasher`, `Gpu::kmac_xof_hasher`): `update` appends one
+/// piece per stream, `finish` returns what `compute_sha3_hash` / `kmac_xof` give for the concatenated pieces.  Drop it
+/// before the `Gpu` that created it.
+pub struct Hasher {
+    ctx: *mut CapyCtx,
+    h: *mut CapyHasher,
+    n: usize,
+}
+unsafe impl Send for Hasher {}
+
+impl Hasher {
+    /// `pieces[i]` is appended to stream i.
+    pub fn update(&mut self, pieces: &[&[u8]]) -> Result<(), OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        status(unsafe { capy_hasher_update(self.ctx, self.h, data.as_ptr(), off.as_ptr()) })
+    }
+
+    /// SHA3-d: the digests (`l_bits` = d).  KMACXOF: `l_bits` output bits per stream.  The hasher is finished after it.
+    pub fn finish(&mut self, l_bits: u64) -> Result<Vec<Vec<u8>>, OperationError> {
+        let ob = (l_bits / 8) as usize;
+        let mut out = vec![0u8; self.n * ob + 1];
+        status(unsafe { capy_hasher_final(self.ctx, self.h, l_bits, std::ptr::null(), out.as_mut_ptr()) })?;
+        Ok((0..self.n).map(|i| out[i * ob..(i + 1) * ob].to_vec()).collect())
+    }
+}
+
+impl Drop for Hasher {
+    fn drop(&mut self) {
+        unsafe { capy_hasher_free(self.h) }
+    }
+}
+
+impl Gpu {
+    /// n `compute_sha3_hash` streams fed in pieces (blocking).
+    pub fn sha3_hasher(&self, n: usize, d: SecParam) -> Result<Hasher, OperationError> {
+        let mut h = std::ptr::null_mut();
+        status(unsafe { capy_sha3_hasher_new(self.ctx, d as c_int, n as u64, &mut h) })?;
+        Ok(Hasher { ctx: self.ctx, h, n })
+    }
+
+    /// One `kmac_xof` stream per key with customisation string `s` (blocking); `compute_tagged_hash` is
+    /// `finish(d as u64)`.  D224 is refused (capy_gpu.h: quirk Q7).
+    pub fn kmac_xof_hasher(&self, keys: &[&[u8]], s: &str, d: SecParam) -> Result<Hasher, OperationError> {
+        let (kd, ko) = pack(keys.iter().copied());
+        let mut h = std::ptr::null_mut();
+        status(unsafe {
+            capy_kmac_xof_hasher_new(self.ctx, d as c_int, kd.as_ptr(), ko.as_ptr(), keys.len() as u64, s.as_ptr(),
+                                     s.len() as u32, &mut h)
+        })?;
+        Ok(Hasher { ctx: self.ctx, h, n: keys.len() })
     }
 }
 

@@ -14,7 +14,7 @@ RUST = os.path.join(ROOT, "rust", "gpu.rs")
 
 C_INT_TYPES = {"int": "c_int", "uint32_t": "u32", "uint64_t": "u64", "size_t": "usize", "double": "f64"}
 C_PTR_BASE = {"void": "c_void", "uint8_t": "u8", "uint32_t": "u32", "uint64_t": "u64", "int": "c_int", "char": "c_char",
-              "capy_ctx": "CapyCtx", "capy_ed448_pub": "CapyEd448Pub", "double": "f64"}
+              "capy_ctx": "CapyCtx", "capy_ed448_pub": "CapyEd448Pub", "capy_hasher": "CapyHasher", "double": "f64"}
 
 
 def _strip_comments(src: str) -> str:
