@@ -10,8 +10,6 @@
 //   c          <- KMACXOF(ke, "", |m|, S_KE) xor m           keystream, squeezed straight into the XOR
 // Decrypt recomputes t' over the recovered plaintext and, on mismatch, hands the ciphertext back unchanged
 // (the reference XORs the keystream a second time, encryptable.rs:77-82).  No RNG inside: nonces are inputs.
-#include <cstring>
-
 #include "ed448_kernels.h"
 #include "hostbatch.h"
 
@@ -64,33 +62,26 @@ struct AeCore {
   uint32_t tag_bytes;
 };
 
-static KmacDevArgs ae_kmac_args(const AeCore& c, const uint8_t* key0, uint64_t n, const char* custom) {
-  KmacDevArgs a{};
-  a.d_bits = c.d;
-  a.keys = key0;
-  a.key_len = c.klen;
-  a.key_stride = 2ull * c.klen;
-  a.data = key0;  // replaced by the caller when the message is absorbed
-  a.n = n;
-  a.custom = reinterpret_cast<const uint8_t*>(custom);
-  a.custom_len = (uint32_t)strlen(custom);
-  return a;
-}
-
 // t = KMACXOF(ka, m, tag, KA) ; c = KMACXOF(ke, "", |m|, KE) ^ m.  `ct` may alias `msgs` (in place): then the tag
 // pass has to finish before the keystream overwrites the message; otherwise the two passes are independent and go
 // out as ONE launch (launch_kmac_xof2: twice the warps, so the last wave of the grid is full).
 static int dev_ae_seal(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const AeCore& c, const uint8_t* msgs,
                        const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag) {
-  KmacDevArgs a = ae_kmac_args(c, c.keymat + c.klen, n, c.ka_custom);
-  a.data = msgs;
-  a.off = off;
-  a.out_bytes = a.out_stride = c.tag_bytes;
-  a.out = tag;
-  KmacDevArgs k = ae_kmac_args(c, c.keymat, n, c.ke_custom);
-  k.out_off = off;
-  k.out = ct;
-  k.xor_in = msgs;
+  KmacPass a(c.d, c.ka_custom, n);
+  a.job.keys = c.keymat + c.klen;
+  a.job.key_len = c.klen;
+  a.job.key_stride = 2ull * c.klen;
+  a.job.data = msgs;
+  a.job.off = off;
+  a.job.out_bytes = a.job.out_stride = c.tag_bytes;
+  a.job.out = tag;
+  KmacPass k(c.d, c.ke_custom, n);
+  k.job.keys = c.keymat;
+  k.job.key_len = c.klen;
+  k.job.key_stride = 2ull * c.klen;
+  k.job.out_off = off;
+  k.job.out = ct;
+  k.job.xor_in = msgs;
   if (ct != msgs) return launch_kmac_xof2(ctx, dc, st, a, k);
   int rc = launch_kmac_xof(ctx, dc, st, a);
   if (rc) return rc;
@@ -102,15 +93,21 @@ static int dev_ae_open(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const AeCo
                        const uint64_t* off, const uint8_t* tag, const uint8_t* bad, uint64_t n, uint8_t* out, uint8_t* ok,
                        uint8_t* t_new) {
   if (out == ct) return CAPY_ERR_BAD_ARG;  // the ciphertext must survive for the restore-on-failure path
-  KmacDevArgs k = ae_kmac_args(c, c.keymat, n, c.ke_custom);
-  k.out_off = off;
-  k.out = out;
-  k.xor_in = ct;
-  KmacDevArgs a = ae_kmac_args(c, c.keymat + c.klen, n, c.ka_custom);
-  a.data = out;
-  a.off = off;
-  a.out_bytes = a.out_stride = c.tag_bytes;
-  a.out = t_new;
+  KmacPass k(c.d, c.ke_custom, n);
+  k.job.keys = c.keymat;
+  k.job.key_len = c.klen;
+  k.job.key_stride = 2ull * c.klen;
+  k.job.out_off = off;
+  k.job.out = out;
+  k.job.xor_in = ct;
+  KmacPass a(c.d, c.ka_custom, n);
+  a.job.keys = c.keymat + c.klen;
+  a.job.key_len = c.klen;
+  a.job.key_stride = 2ull * c.klen;
+  a.job.data = out;
+  a.job.off = off;
+  a.job.out_bytes = a.job.out_stride = c.tag_bytes;
+  a.job.out = t_new;
   // the tag pass reads what the keystream pass writes: dependent jobs of one launch when the batch is large enough
   int rc = launch_kmac_xof_dep(ctx, dc, st, k, a);
   if (rc) return rc;
@@ -143,16 +140,11 @@ static int dev_sponge_keymat(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int 
   ae_concat_kernel<<<grid_for(n * 32, 256), 256, 0, st>>>(nonces, nonce_len, pws, pw_off, keys, koff, n);
   ctx->launches++;
   CAPY_CUDA(ctx, cudaGetLastError());
-  KmacDevArgs a{};
-  a.d_bits = d;
-  a.keys = keys;
-  a.key_off = koff;
-  a.data = keys;
-  a.n = n;
-  a.custom = reinterpret_cast<const uint8_t*>("S");
-  a.custom_len = 1;
-  a.out_bytes = a.out_stride = 128;
-  a.out = keymat;
+  KmacPass a(d, "S", n);
+  a.job.keys = keys;
+  a.job.key_off = koff;
+  a.job.out_bytes = a.job.out_stride = 128;
+  a.job.out = keymat;
   a.no_sort = true;
   *keymat_out = keymat;
   return launch_kmac_xof(ctx, dc, st, a);
@@ -198,16 +190,11 @@ static int dev_sponge_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int
 static int dev_ecdhies_keymat(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* wx, uint64_t n,
                               uint8_t** keymat_out) {
   CAPY_SCRATCH(keymat, uint8_t, kAeKeyMat, n * 112);
-  KmacDevArgs a{};
-  a.d_bits = d;
-  a.keys = wx;
-  a.key_len = a.key_stride = 56;
-  a.data = wx;
-  a.n = n;
-  a.custom = reinterpret_cast<const uint8_t*>("PK");
-  a.custom_len = 2;
-  a.out_bytes = a.out_stride = 112;
-  a.out = keymat;
+  KmacPass a(d, "PK", n);
+  a.job.keys = wx;
+  a.job.key_stride = a.job.key_len = 56;
+  a.job.out_bytes = a.job.out_stride = 112;
+  a.job.out = keymat;
   *keymat_out = keymat;
   return launch_kmac_xof(ctx, dc, st, a);
 }
@@ -295,16 +282,11 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   CAPY_SCRATCH(sk, uint8_t, kAeSk, n * 56);
   CAPY_SCRATCH(t_new, uint8_t, kAeTNew, n * 56);
   // s = 4 * BE(KMACXOF(pw, "", 448, "SK")) mod r (:74-75)
-  KmacDevArgs a{};
-  a.d_bits = d;
-  a.keys = pws;
-  a.key_off = pw_off;
-  a.data = pws;
-  a.n = n;
-  a.custom = reinterpret_cast<const uint8_t*>("SK");
-  a.custom_len = 2;
-  a.out_bytes = a.out_stride = 56;
-  a.out = sk;
+  KmacPass a(d, "SK", n);
+  a.job.keys = pws;
+  a.job.key_off = pw_off;
+  a.job.out_bytes = a.job.out_stride = 56;
+  a.job.out = sk;
   a.no_sort = true;
   int rc = launch_kmac_xof(ctx, dc, st, a);
   if (rc) return rc;

@@ -186,31 +186,16 @@ static int dev_var_base(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const uin
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
 
-static KmacDevArgs kmac_args(int d, const uint8_t* keys, const uint64_t* key_off, uint64_t key_len, const uint8_t* data,
-                             const uint64_t* off, uint64_t n, const char* custom, uint8_t* out) {
-  KmacDevArgs a{};
-  a.d_bits = d;
-  a.keys = keys;
-  a.key_off = key_off;
-  a.key_len = key_len;
-  a.key_stride = key_len;
-  a.data = data ? data : keys;
-  a.off = off;
-  a.msg_len = 0;
-  a.msg_stride = 0;
-  a.n = n;
-  a.custom = reinterpret_cast<const uint8_t*>(custom);
-  a.custom_len = (uint32_t)strlen(custom);
-  a.out_bytes = a.out_stride = 56;  // 448 bits
-  a.out = out;
-  return a;
-}
-
 // s = 4 * BE(KMACXOF(pw, "", 448, "SK", d)) mod r  (ecc/keypair.rs:42-43): words + optional BE bytes
 int dev_secret_scalar(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pws,
                              const uint64_t* d_pw_off, uint64_t n, uint32_t* s_words, uint8_t* s_be) {
   CAPY_SCRATCH(tmp, uint8_t, kEdTmp56A, n * 56);
-  int rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, d_pws, d_pw_off, 0, nullptr, nullptr, n, "SK", tmp));
+  KmacPass a(d, "SK", n);
+  a.job.keys = d_pws;
+  a.job.key_off = d_pw_off;
+  a.job.out_bytes = a.job.out_stride = 56;  // 448 bits
+  a.job.out = tmp;
+  int rc = launch_kmac_xof(ctx, dc, st, a);
   if (rc) return rc;
   return launch_scalar_prep(ctx, st, tmp, 1, s_words, s_be, n);
 }
@@ -241,7 +226,14 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
   int rc = dev_secret_scalar(ctx, dc, st, d, d_pws, d_pw_off, n, sw, s_be);
   if (rc) return rc;
   // k = 4 * BE(KMACXOF(s_bytes, m, 448, "N")) mod r (:45-46)
-  rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, s_be, nullptr, 56, d_msgs, d_msg_off, n, "N", tmp));
+  KmacPass k(d, "N", n);
+  k.job.keys = s_be;
+  k.job.key_stride = k.job.key_len = 56;
+  k.job.data = d_msgs;
+  k.job.off = d_msg_off;
+  k.job.out_bytes = k.job.out_stride = 56;
+  k.job.out = tmp;
+  rc = launch_kmac_xof(ctx, dc, st, k);
   if (rc) return rc;
   rc = launch_scalar_prep(ctx, st, tmp, 1, kw, nullptr, n);
   if (rc) return rc;
@@ -250,8 +242,12 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
   if (rc) return rc;
   rc = launch_to_affine(ctx, st, proj, n, 1, nullptr, tmp);
   if (rc) return rc;
-  // h = KMACXOF(ux, m, 448, "T") (:51)
-  rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, tmp, nullptr, 56, d_msgs, d_msg_off, n, "T", d_h));
+  // h = KMACXOF(ux, m, 448, "T") (:51): the pass of k with another key, output and customisation string
+  KmacPass h = k;
+  h.custom = "T";
+  h.job.keys = tmp;
+  h.job.out = d_h;
+  rc = launch_kmac_xof(ctx, dc, st, h);
   if (rc) return rc;
   // z = k - h * s mod r (:52-54)
   sign_finish_kernel<<<grid_for(n, 128), 128, 0, st>>>(kw, sw, d_h, d_z, n);
@@ -268,7 +264,14 @@ static int verify_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, c
   CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
   int rc = launch_to_affine(ctx, st, proj_u, n, 1, nullptr, ux);
   if (rc) return rc;
-  rc = launch_kmac_xof(ctx, dc, st, kmac_args(d, ux, nullptr, 56, d_msgs, d_msg_off, n, "T", hp));
+  KmacPass h(d, "T", n);
+  h.job.keys = ux;
+  h.job.key_stride = h.job.key_len = 56;
+  h.job.data = d_msgs;
+  h.job.off = d_msg_off;
+  h.job.out_bytes = h.job.out_stride = 56;
+  h.job.out = hp;
+  rc = launch_kmac_xof(ctx, dc, st, h);
   if (rc) return rc;
   verify_compare_kernel<<<grid_for(n, 256), 256, 0, st>>>(hp, d_h, bad, d_ok, d_bad_flag, n);
   ctx->launches++;

@@ -11,10 +11,12 @@
 #include <memory>
 #include <mutex>
 #include <string>
+#include <string_view>
 #include <thread>
 #include <vector>
 
 #include "../../include/capy_gpu.h"
+#include "sponge_job.h"
 
 namespace capy {
 
@@ -287,35 +289,21 @@ inline const uint64_t* host_off_find(const DeviceCtx& dc, const uint64_t* d_off,
 }
 
 inline bool valid_secparam(int d) { return d == 224 || d == 256 || d == 384 || d == 512; }
-inline uint32_t bytepad_value(int d) { return d == 224 ? 172u : d == 256 ? 168u : d == 384 ? 152u : 136u; }  // lib.rs:137-144
-inline uint32_t sha3_capacity(int d) {  // constants.rs:38-45
-  int x = d * 2;
-  return x <= 448 ? 448u : x <= 512 ? 512u : x <= 768 ? 768u : 1024u;
-}
 
 // ---- device-level launchers (async on `stream`), implemented in sha3_api.cu -----------------
-struct KmacDevArgs {
+// One KMACXOF pass over job.n items.  The caller fills in the per-item fields of `job`: keys, messages (none: data stays
+// nullptr and msg_len 0), outputs, xor_in.  The launchers add the operator fields and the prefix of (d_bits, custom).
+struct KmacPass {
   int d_bits;
-  const uint8_t* keys;
-  const uint64_t* key_off;  // nullptr -> fixed
-  uint64_t key_len, key_stride;
-  const uint8_t* data;
-  const uint64_t* off;  // nullptr -> fixed
-  uint64_t msg_len, msg_stride;
-  uint64_t n;
-  const uint8_t* custom;
-  uint32_t custom_len;
-  uint64_t out_bytes;
-  const uint64_t* out_off;
-  uint64_t out_stride;
-  uint8_t* out;
-  const uint8_t* xor_in = nullptr;  // out = keystream ^ xor_in (same layout as out)
+  std::string_view custom;
   bool no_sort = false;  // keep the caller's order (skips the length bucketing and its tiny D2H sync)
+  SpongeJob job{};
+  KmacPass(int d, std::string_view s, uint64_t n) : d_bits(d), custom(s) { job.n = n; }
 };
-int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a);
+int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a);
 // two passes over the same items (same d, same n) as one launch; the plan (work order) is taken from `a`
-int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a, const KmacDevArgs& b);
+int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, const KmacPass& b);
 // two passes where `second` absorbs what `first` wrote for the same item: one launch of dependent jobs when the batch is large
-int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& first, const KmacDevArgs& second);
+int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& first, const KmacPass& second);
 
 }  // namespace capy

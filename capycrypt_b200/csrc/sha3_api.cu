@@ -714,6 +714,55 @@ static int run_sponge(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, SpongeJ
   return launch_sponge(ctx, dc, stream, J, plan);
 }
 
+// ---- the operators: rate, squeeze width, trailer and pad of each; callers add their data and output fields ------------
+static SpongeJob sha3_job(int d) {
+  SpongeJob J{};
+  J.trailer_len = 1;
+  J.sha3_suffix = 1;  // 06 | 86 from the message length (Q2)
+  J.rate = sha3_rate(d);
+  J.sq_lanes = squeeze_lanes(d);  // the first d/8 bytes are all that is kept
+  return J;
+}
+
+// q4: N = S = "" (quirk Q4, shake_functions.rs:59-61)
+static SpongeJob cshake_job(int d, bool q4) {
+  SpongeJob J{};
+  J.trailer = 0x04;  // shake_functions.rs:57
+  J.trailer_len = 1;
+  if (q4) J.q4_rate = sha3_rate(d);
+  J.rate = cshake_rate(d);
+  J.sq_lanes = squeeze_lanes(d);
+  return J;
+}
+
+// on top of J, the caller's per-item fields
+static SpongeJob kmac_job(int d, SpongeJob J = SpongeJob{}) {
+  J.trailer = 0x040100u;  // right_encode(0) = 00 01 (shake_functions.rs:86) then 04 (:57)
+  J.trailer_len = 3;
+  J.rate = cshake_rate(d);
+  J.sq_lanes = squeeze_lanes(d);
+  return J;
+}
+
+static SpongeJob shake_job(int shake_bits) {
+  SpongeJob J{};
+  J.trailer = 0x1F;
+  J.trailer_len = 1;
+  J.fips_pad = 1;
+  J.rate = shake_rate(shake_bits);
+  J.sq_lanes = squeeze_lanes(2 * shake_bits);
+  return J;
+}
+
+// the cached prefix P of a cSHAKE / KMAC job (get_prefix); its bytepad width is the rate
+static void set_prefix(SpongeJob& J, const PrefixState* ps) {
+  J.prefix = ps->d_prefix;
+  J.prefix_len = ps->prefix_len;
+  J.init_state = ps->skip_blocks ? ps->d_state : nullptr;
+  J.skip_blocks = ps->skip_blocks;
+  J.w = J.rate;
+}
+
 // ---- SHA3-d ------------------------------------------------------------------------------------
 // tail_readable: the 8-byte word that holds the last message byte of the LAST row may be read in full (the host entry
 // points stage into buffers with slack; a caller-owned device buffer may end with the last message byte)
@@ -731,10 +780,9 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
     return launch_sha3(ctx, dc, stream, d, data + (n - 1) * stride, nullptr, msg_len, stride, 1, out + (n - 1) * (uint64_t)(d / 8),
                        flags, false);
   }
-  const uint32_t rate = (1600 - sha3_capacity(d)) / 8;  // 144 / 136 / 104 / 72
-  const int lanes = (int)rate / 8;
+  SpongeJob J = sha3_job(d);
   if (!off && (reinterpret_cast<uintptr_t>(data) & 15u) == 0 && (reinterpret_cast<uintptr_t>(out) & 15u) == 0 &&
-      (stride & 15u) == 0 && (d == 256 || d == 512) && msg_len >= 16 && (msg_len & 15u) == 0 && msg_len < rate) {
+      (stride & 15u) == 0 && (d == 256 || d == 512) && msg_len >= 16 && (msg_len & 15u) == 0 && msg_len < J.rate) {
     // compile-time block layout: single-block messages of a whole number of 16-byte rows (cfg 1 is 64 B at D256)
     const unsigned block = 128, grid = grid_for(n, block);
     const uint4* dq = reinterpret_cast<const uint4*>(data);
@@ -753,17 +801,12 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
     CAPY_CUDA(ctx, cudaGetLastError());
     return CAPY_OK;
   }
-  SpongeJob J{};
   J.data = data;
   J.off = off;
   J.msg_len = msg_len;
   J.msg_stride = stride;
-  J.trailer_len = 1;
-  J.sha3_suffix = 1;
-  J.rate = rate;
   J.out = out;
   J.out_stride = J.out_bytes = (uint64_t)d / 8;
-  J.sq_lanes = (1600 - d) / 64;  // Rate::from(&d), sponge.rs:27 (first d/8 bytes are all that is kept)
   J.n = n;
   // long equal messages that fill the GPU unevenly are cut along the chains (run_sponge), which the uniform kernel cannot
   // do; the uniform kernel stores 4-byte granules (28- and 48-byte digests) and reads whole 8-byte words
@@ -772,7 +815,7 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
       (stride & 7u) == 0 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0 && (tail_readable || (msg_len & 7u) == 0)) {
     const uint32_t suffix = (msg_len % 136u == 135u) ? 0x86u : 0x06u;  // shake_functions.rs:25-29 (Q2)
     const unsigned block = 128, grid = grid_for(n, block);
-    return with_lanes<9, 13, 17, 18>(lanes, [&](auto L) {
+    return with_lanes<9, 13, 17, 18>(job_lanes(J), [&](auto L) {
       sha3_uniform_kernel<decltype(L)::value><<<grid, block, 0, stream>>>(data, stride, msg_len, suffix, out, d / 8, n);
       ctx->launches++;
       CAPY_CUDA(ctx, cudaGetLastError());
@@ -781,7 +824,7 @@ static int launch_sha3(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d,
   }
   LaunchPlan plan;
   if (off && !(flags & CAPY_FLAG_NO_SORT)) {
-    int rc = plan_ragged(ctx, dc, stream, off, n, rate, &plan, !(flags & CAPY_FLAG_NO_PAIR),
+    int rc = plan_ragged(ctx, dc, stream, off, n, J.rate, &plan, !(flags & CAPY_FLAG_NO_PAIR),
                          (int)((flags >> CAPY_FLAG_WARP_COSCHED_SHIFT) & 3u));
     if (rc) return rc;
   }
@@ -829,7 +872,7 @@ static int get_prefix(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d, 
     if (lru->second.d_prefix) cudaFree(lru->second.d_prefix);
     dc.prefix_cache.erase(lru);
   }
-  const uint32_t w = bytepad_value(d);
+  const uint32_t w = cshake_rate(d);  // the bytepad width
   std::string p;  // bytepad(encode_string(N) || encode_string(S), w)   shake_functions.rs:50-55
   host_left_encode(p, w);
   host_encode_string(p, fn, fn_len);
@@ -865,17 +908,6 @@ static int get_prefix(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d, 
   return CAPY_OK;
 }
 
-static void fill_cshake_common(SpongeJob& J, int d, const PrefixState* ps) {
-  const uint32_t w = bytepad_value(d);
-  J.prefix = ps->d_prefix;
-  J.prefix_len = ps->prefix_len;
-  J.init_state = ps->skip_blocks ? ps->d_state : nullptr;
-  J.skip_blocks = ps->skip_blocks;
-  J.w = w;
-  J.rate = (1600 - d) / 8;  // capacity = d bits (shake_functions.rs:63, quirk Q7)
-  J.sq_lanes = (1600 - d) / 64;
-}
-
 static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int d, const uint8_t* data,
                          const uint64_t* off, uint64_t n, const uint8_t* fn, uint32_t fn_len, const uint8_t* cs,
                          uint32_t cs_len, uint64_t out_bits, uint8_t* out) {
@@ -884,13 +916,10 @@ static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int 
   PrefixState* ps;
   int rc = get_prefix(ctx, dc, stream, d, fn, fn_len, cs, cs_len, &ps);
   if (rc) return rc;
-  SpongeJob J{};
-  fill_cshake_common(J, d, ps);
+  SpongeJob J = cshake_job(d, fn_len == 0 && cs_len == 0);
+  set_prefix(J, ps);
   J.data = data;
   J.off = off;
-  J.trailer = 0x04;  // shake_functions.rs:57
-  J.trailer_len = 1;
-  if (fn_len == 0 && cs_len == 0) J.q4_rate = (1600 - sha3_capacity(d)) / 8;  // quirk Q4, :59-61
   J.out = out;
   J.out_stride = J.out_bytes = out_bits / 8;
   J.n = n;
@@ -900,46 +929,33 @@ static int launch_cshake(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, int 
   return run_sponge(ctx, dc, stream, J, plan);
 }
 
-static int build_kmac_job(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a, SpongeJob* out) {
+// the pass's own per-item fields, with the KMAC operator fields and the prefix of (d, custom)
+static int build_kmac_job(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, SpongeJob* out) {
   static const uint8_t kKmac[4] = {'K', 'M', 'A', 'C'};
   PrefixState* ps;
-  int rc = get_prefix(ctx, dc, stream, a.d_bits, kKmac, 4, a.custom, a.custom_len, &ps);
+  int rc = get_prefix(ctx, dc, stream, a.d_bits, kKmac, 4, reinterpret_cast<const uint8_t*>(a.custom.data()),
+                      (uint32_t)a.custom.size(), &ps);
   if (rc) return rc;
-  SpongeJob J{};
-  fill_cshake_common(J, a.d_bits, ps);
-  J.keys = a.keys;
-  J.key_off = a.key_off;
-  J.key_len = (uint32_t)a.key_len;
-  J.key_stride = a.key_stride;
-  J.data = a.data;
-  J.off = a.off;
-  J.msg_len = a.msg_len;
-  J.msg_stride = a.msg_stride;
-  J.trailer = 0x040100u;  // right_encode(0) = 00 01 (shake_functions.rs:86) then 04 (:57)
-  J.trailer_len = 3;
-  J.out = a.out;
-  J.out_off = a.out_off;
-  J.out_stride = a.out_stride;
-  J.out_bytes = a.out_bytes;
-  J.xor_in = a.xor_in;
-  J.n = a.n;
+  SpongeJob J = kmac_job(a.d_bits, a.job);
+  set_prefix(J, ps);
+  if (!J.data) J.data = J.keys;  // no message: never read, but the kernels still offset it per item
   *out = J;
   return CAPY_OK;
 }
 
-static int plan_kmac(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a, const SpongeJob& J, LaunchPlan* plan) {
+static int plan_kmac(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, const SpongeJob& J, LaunchPlan* plan) {
   *plan = LaunchPlan();
   if (a.no_sort) return CAPY_OK;
-  if (a.off) return plan_ragged(ctx, dc, stream, a.off, a.n, J.rate & ~7u, plan);
+  if (J.off) return plan_ragged(ctx, dc, stream, J.off, J.n, J.rate & ~7u, plan);
   // keystream shape (sha3/encryptable.rs:41): the work of an item is its squeeze length
-  if (a.out_off) return plan_ragged(ctx, dc, stream, a.out_off, a.n, 8u * J.sq_lanes, plan);
+  if (J.out_off) return plan_ragged(ctx, dc, stream, J.out_off, J.n, 8u * J.sq_lanes, plan);
   return CAPY_OK;
 }
 
-int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a) {
+int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a) {
   if (!valid_secparam(a.d_bits)) return CAPY_ERR_BAD_SECPARAM;
-  if (a.n == 0) return CAPY_OK;
-  if (!a.out_off && a.out_bytes == 0) return CAPY_OK;
+  if (a.job.n == 0) return CAPY_OK;
+  if (!a.job.out_off && a.job.out_bytes == 0) return CAPY_OK;
   SpongeJob J;
   int rc = build_kmac_job(ctx, dc, stream, a, &J);
   if (rc) return rc;
@@ -969,9 +985,9 @@ static int launch_sponge2_t(capy_ctx* ctx, cudaStream_t stream, const SpongeJob&
   return CAPY_OK;
 }
 
-int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& a, const KmacDevArgs& b) {
-  if (!valid_secparam(a.d_bits) || a.d_bits != b.d_bits || a.n != b.n) return CAPY_ERR_BAD_ARG;
-  if (a.n == 0) return CAPY_OK;
+int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, const KmacPass& b) {
+  if (!valid_secparam(a.d_bits) || a.d_bits != b.d_bits || a.job.n != b.job.n) return CAPY_ERR_BAD_ARG;
+  if (a.job.n == 0) return CAPY_OK;
   SpongeJob JA, JB;
   int rc = build_kmac_job(ctx, dc, stream, a, &JA);
   if (rc) return rc;
@@ -982,7 +998,7 @@ int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const Km
   if (rc) return rc;
   JA.order = JB.order = plan.order;
   if (plan.tiered()) return launch_sponge_seq(ctx, dc, stream, JA, JB, plan);
-  const unsigned block = pick_block(2 * a.n, dc.sm_count, 384);
+  const unsigned block = pick_block(2 * JA.n, dc.sm_count, 384);
   return with_lanes<17, 19, 21>(job_lanes(JA), [&](auto L) {
     return launch_sponge2_t<decltype(L)::value>(ctx, stream, JA, JB, block, plan);
   });
@@ -992,9 +1008,9 @@ int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const Km
 // keystream pass recovers the plaintext, the tag pass runs over it -- sha3/encryptable.rs:66-75): one launch of
 // dependent jobs instead of two kernels, so the partial wave of the first pass is filled by the second.  Both follow the
 // plan (work order) of `second`.  Small or chain-bound batches run the two passes one after the other.
-int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacDevArgs& first, const KmacDevArgs& second) {
-  if (!valid_secparam(first.d_bits) || first.d_bits != second.d_bits || first.n != second.n) return CAPY_ERR_BAD_ARG;
-  if (first.n == 0) return CAPY_OK;
+int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& first, const KmacPass& second) {
+  if (!valid_secparam(first.d_bits) || first.d_bits != second.d_bits || first.job.n != second.job.n) return CAPY_ERR_BAD_ARG;
+  if (first.job.n == 0) return CAPY_OK;
   SpongeJob J0, J1;
   int rc = build_kmac_job(ctx, dc, stream, first, &J0);
   if (rc) return rc;
@@ -1004,7 +1020,7 @@ int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const
   rc = plan_kmac(ctx, dc, stream, second, J1, &plan);
   if (rc) return rc;
   J0.order = J1.order = plan.order;
-  if (plan.tiered() || (J0.rate & 7u) != 0 || !chain_jobs_fit(dc.sm_count, first.n))
+  if (plan.tiered() || (J0.rate & 7u) != 0 || !chain_jobs_fit(dc.sm_count, J0.n))
     return launch_sponge_seq(ctx, dc, stream, J0, J1, plan);
   return launch_chain_jobs(ctx, dc, stream, J0, J1, true);
 }
@@ -1025,18 +1041,12 @@ static std::vector<Range> hasher_shards(const capy_hasher* h) {  // one per devi
   return s;
 }
 
+// the operator of the hasher's streams; its prefix and keys are already in their states
+static SpongeJob hasher_operator(const capy_hasher* h) { return h->kmac ? kmac_job(h->d_bits) : sha3_job(h->d_bits); }
+
 // the job of an update or a final over the items [j0, j0 + n) of device k (indices on that device), and its streams
 static SpongeJob hasher_job(const capy_hasher* h, int k, uint64_t j0, uint64_t n, SpongeResume* R) {
-  SpongeJob J{};
-  J.rate = h->rate;
-  J.sq_lanes = (1600 - h->d_bits) / 64;
-  if (h->kmac) {
-    J.trailer = 0x040100u;  // right_encode(0) = 00 01 (shake_functions.rs:86) then 04 (:57)
-    J.trailer_len = 3;
-  } else {
-    J.sha3_suffix = 1;  // 06 | 86 from the total length (Q2)
-    J.trailer_len = 1;
-  }
+  SpongeJob J = hasher_operator(h);
   J.chain_in = h->d_state[k] + j0;
   J.n = n;
   R->carry = h->d_carry[k] + j0 * h->rate;
@@ -1076,7 +1086,7 @@ static int hasher_create(capy_ctx* ctx, int d_bits, bool kmac, uint64_t n, capy_
   h->ctx = ctx;
   h->d_bits = d_bits;
   h->kmac = kmac;
-  h->rate = kmac ? (uint32_t)(1600 - d_bits) / 8 : (1600 - sha3_capacity(d_bits)) / 8;
+  h->rate = hasher_operator(h).rate;
   h->n = n;
   const uint64_t nd = ctx->devs.size();
   for (uint64_t k = 0; k <= nd; k++) h->first.push_back((n / nd) * k + std::min(k, n % nd));
@@ -1179,8 +1189,7 @@ int capy_sha3_batch(capy_ctx* ctx, int d_bits, const uint8_t* data, const uint64
     // several devices: the outliers of the batch (long chains) are dealt out longest first, the rest follows in
     // contiguous ranges (lpt_shares).  When nothing had to be dealt out every share is one run and the plain path
     // below does the same thing with pipelined chunks.
-    const uint32_t rate = (1600 - sha3_capacity(d_bits)) / 8;
-    auto shares = lpt_shares(off, n, ctx->devs.size(), rate, 2);
+    auto shares = lpt_shares(off, n, ctx->devs.size(), sha3_rate(d_bits), 2);
     bool scattered = false;
     for (const DeviceShare& s : shares) scattered |= s.runs.size() > 1;
     if (scattered) {
@@ -1293,18 +1302,14 @@ int capy_kmac_xof_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int d_bi
                             uint8_t* d_out) {
   if ((n && (!d_keys || !d_key_off || !d_data || !d_off || !d_out)) || (custom_len && !custom)) return CAPY_ERR_BAD_ARG;
   CAPY_DEV_PROLOGUE
-  KmacDevArgs a{};
-  a.d_bits = d_bits;
-  a.keys = d_keys;
-  a.key_off = d_key_off;
-  a.data = d_data;
-  a.off = d_off;
-  a.n = n;
-  a.custom = custom;
-  a.custom_len = custom_len;
-  a.out_bytes = a.out_stride = out_bits / 8;
-  a.out_off = d_out_off;
-  a.out = d_out;
+  KmacPass a(d_bits, {reinterpret_cast<const char*>(custom), custom_len}, n);
+  a.job.keys = d_keys;
+  a.job.key_off = d_key_off;
+  a.job.data = d_data;
+  a.job.off = d_off;
+  a.job.out_bytes = a.job.out_stride = out_bits / 8;
+  a.job.out_off = d_out_off;
+  a.job.out = d_out;
   return launch_kmac_xof(ctx, dc, st, a);
 }
 
@@ -1316,19 +1321,15 @@ int capy_kmac_xof_batch_fixed_dev(capy_ctx* ctx, int dev_index, void* stream, in
       msg_stride < msg_len)
     return CAPY_ERR_BAD_ARG;
   CAPY_DEV_PROLOGUE
-  KmacDevArgs a{};
-  a.d_bits = d_bits;
-  a.keys = d_keys;
-  a.key_len = key_len;
-  a.key_stride = key_stride;
-  a.data = d_data ? d_data : d_keys;  // never dereferenced when msg_len == 0
-  a.msg_len = msg_len;
-  a.msg_stride = msg_stride;
-  a.n = n;
-  a.custom = custom;
-  a.custom_len = custom_len;
-  a.out_bytes = a.out_stride = out_bits / 8;
-  a.out = d_out;
+  KmacPass a(d_bits, {reinterpret_cast<const char*>(custom), custom_len}, n);
+  a.job.keys = d_keys;
+  a.job.key_len = (uint32_t)key_len;
+  a.job.key_stride = key_stride;
+  a.job.data = d_data;
+  a.job.msg_len = msg_len;
+  a.job.msg_stride = msg_stride;
+  a.job.out_bytes = a.job.out_stride = out_bits / 8;
+  a.job.out = d_out;
   return launch_kmac_xof(ctx, dc, st, a);
 }
 
@@ -1347,21 +1348,17 @@ int capy_kmac_xof_batch(capy_ctx* ctx, int d_bits, const uint8_t* keys, const ui
   };
   return run_host_call(ctx, shards, chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
     const StagedPacked sx = io.in_packed(data, off), sk = io.in_packed(keys, key_off);
-    KmacDevArgs a{};
-    a.d_bits = d_bits;
-    a.keys = sk.d_base;
-    a.key_off = sk.d_off;
-    a.data = sx.d_base;
-    a.off = sx.d_off;
-    a.n = io.n();
-    a.custom = custom;
-    a.custom_len = custom_len;
-    a.out_bytes = a.out_stride = ob;
+    KmacPass a(d_bits, {reinterpret_cast<const char*>(custom), custom_len}, io.n());
+    a.job.keys = sk.d_base;
+    a.job.key_off = sk.d_off;
+    a.job.data = sx.d_base;
+    a.job.off = sx.d_off;
+    a.job.out_bytes = a.job.out_stride = ob;
     if (out_off) {
-      a.out_off = (const uint64_t*)io.in(out_off, 8, (size_t)(io.n() + 1) * 8);
-      a.out = io.out_packed(out, out_off);
+      a.job.out_off = (const uint64_t*)io.in(out_off, 8, (size_t)(io.n() + 1) * 8);
+      a.job.out = io.out_packed(out, out_off);
     } else {
-      a.out = io.out(out, ob);
+      a.job.out = io.out(out, ob);
     }
     if (io.rc()) return io.rc();
     return launch_kmac_xof(ctx, dc, st, a);
@@ -1377,14 +1374,9 @@ int capy_fips_shake_batch_dev(capy_ctx* ctx, int dev_index, void* stream, int sh
     return CAPY_ERR_BAD_ARG;
   if (n == 0 || out_bytes == 0) return CAPY_OK;
   CAPY_DEV_PROLOGUE
-  SpongeJob J{};
+  SpongeJob J = shake_job(shake_bits);
   J.data = d_data;
   J.off = d_off;
-  J.trailer = 0x1F;
-  J.trailer_len = 1;
-  J.fips_pad = 1;
-  J.rate = (1600 - 2 * shake_bits) / 8;
-  J.sq_lanes = J.rate / 8;
   J.out = d_out;
   J.out_stride = J.out_bytes = out_bytes;
   J.n = n;
@@ -1424,14 +1416,9 @@ int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, con
     if (io.n() == 0) return CAPY_OK;  // (a device without items)
     const StagedPacked sk = io.in_packed(keys, key_off);
     if (io.rc()) return io.rc();
-    KmacDevArgs a{};
-    a.d_bits = d_bits;
-    a.keys = sk.d_base;
-    a.key_off = sk.d_off;
-    a.data = sk.d_base;  // (no message: never read)
-    a.n = io.n();
-    a.custom = custom;
-    a.custom_len = custom_len;
+    KmacPass a(d_bits, {reinterpret_cast<const char*>(custom), custom_len}, io.n());
+    a.job.keys = sk.d_base;
+    a.job.key_off = sk.d_off;
     SpongeJob J;
     const int rj = build_kmac_job(ctx, dc, st, a, &J);
     if (rj) return rj;

@@ -15,78 +15,13 @@
 #pragma once
 #include "keccak.cuh"
 #include "keccak_pair.cuh"
+#include "sponge_job.h"
 
 #ifndef CAPY_SPONGE_MINB
 #define CAPY_SPONGE_MINB 3
 #endif
 
 namespace capy {
-
-struct SpongeJob {
-  // constant prefix segment
-  const uint8_t* prefix;
-  uint32_t prefix_len;
-  // state after the first skip_blocks blocks (all inside P) were absorbed; nullptr = zero state
-  const uint64_t* init_state;
-  uint32_t skip_blocks;
-  // per-item keys (nullptr = no key block).  key_off == nullptr -> fixed key_len at key_stride
-  const uint8_t* keys;
-  const uint64_t* key_off;
-  uint64_t key_stride;
-  uint32_t key_len;
-  uint32_t w;  // bytepad width (SecParam::bytepad_value, lib.rs:137-144)
-  // per-item messages.  off == nullptr -> fixed msg_len at msg_stride
-  const uint8_t* data;
-  const uint64_t* off;
-  uint64_t msg_stride;
-  uint64_t msg_len;
-  // trailer bytes, little-endian packed, trailer_len <= 4.  sha3_suffix: trailer is 0x86 when
-  // len % 136 == 135 else 0x06 (rate 136 hard-coded for every d, quirk Q2)
-  uint32_t trailer;
-  uint32_t trailer_len;
-  uint32_t sha3_suffix;
-  // fips_pad: FIPS 202 pad10*1 (0x80 is ORed into the last byte even when already aligned);
-  // only used by the SHAKE extras that have no reference counterpart
-  uint32_t fips_pad;
-  // q4_rate != 0: reference quirk Q4 (cshake with N = S = ""): after the 0x04 trailer the buffer
-  // was run through shake(): a 06|86 suffix chosen from (len % 136) and a first pad to q4_rate
-  uint32_t q4_rate;
-  // rate in bytes as the reference computes it ((1600 - c) / 8; 172 for D224 cSHAKE, quirk Q7)
-  uint32_t rate;
-  // output: out_off == nullptr -> out_bytes per item at out_stride
-  uint8_t* out;
-  const uint64_t* out_off;
-  uint64_t out_stride;
-  uint64_t out_bytes;
-  uint32_t sq_lanes;  // lanes emitted per squeeze block = (1600 - d) / 64
-  // optional: out = squeeze XOR xor_in (same layout as out): keystream applied in place of a second pass
-  // (c = m ^ kmac_xof(ke, "", |m|, ...), sha3/encryptable.rs:41-42, ecc/encryptable.rs:45)
-  const uint8_t* xor_in;
-  uint64_t n;
-  // optional permutation of work: item index = order ? order[r] : r for rank r (length-sorted launch)
-  const uint32_t* order;
-  // tiers of a chain-bound batch (sponge_tiered_kernel): ranks [0, warp_items) one warp per item,
-  // [warp_items, first) two threads per item, [first, n) one thread per item
-  uint64_t warp_items;
-  uint64_t first;
-  // chain hand-off (sponge_chain_kernel): the chains of a uniform batch are cut in two segments that run as dependent jobs.
-  //   chain_out != nullptr: absorb blocks [skip_blocks, stop_block) only, then store the 25 lanes at chain_out[k * n + rank]
-  //   chain_in  != nullptr: start from the lanes another segment stored there (instead of init_state), at block skip_blocks
-  uint64_t* chain_out;
-  const uint64_t* chain_in;
-  uint64_t stop_block;
-};
-
-// Resumable streams (capy_hasher; a job of sponge_chain_kernel with order == nullptr, so rank = item i).  Item i's state
-// at chain_in[k * state_n + i] holds every whole block of its stream before the carry bytes carry[i * rate ..), whose
-// count is totals[i] % rate.  With chain_out the job is an update (absorbs the whole blocks of carry | X, stores the
-// state, keeps the rest as the new carry, adds |X| to totals[i]); without, the final (carry | T | pad, then squeeze).
-// Kept out of SpongeJob, so that the kernels without a hand-off compile to what they were.
-struct SpongeResume {
-  uint8_t* carry;    // nullptr: not a resumable job
-  uint64_t* totals;
-  uint64_t state_n;  // stride of the lane-major states (the items of the device; a job may cover a part of them)
-};
 
 __device__ __forceinline__ uint32_t left_encode_nbytes(uint64_t v) {
   uint32_t nb = 1;

@@ -1,13 +1,14 @@
-"""Checks that the plain sponge kernels compile to the same instructions in two builds.
+"""Checks that the kernels of two builds compile to the same instructions.
 
     python tools/compare_sass.py OLD NEW [--kernels sponge_kernel,sponge_tiered_kernel,sponge_kernel2]
 
-OLD and NEW are each an object or library with sm_100a code (e.g. capycrypt_b200/_lib/obj_*/sha3_api.o) or a source tree
-of this project, whose csrc/sha3_api.cu is then compiled with the flags of capycrypt_b200/build.py into a temporary
-directory.  Every instantiation of the named kernels is disassembled (cuobjdump -sass) and compared instruction by
-instruction after constant-bank offsets (c[0x0][0x...], where kernel parameters live) are masked: a kernel whose parameter
-struct grew at its end reads the same fields at the same offsets, and a second struct behind it moves.  Prints one line
-per kernel and exits 1 when any of them differs in anything else, or is missing in one build.  No GPU needed.
+OLD and NEW are each an object or library with sm_100a code (e.g. capycrypt_b200/_lib/libcapycrypt_gpu.so) or a source
+tree of this project, whose csrc/ sources are then compiled with the flags of capycrypt_b200/build.py into a temporary
+directory.  Every kernel -- or, with --kernels, every instantiation of the named ones -- is disassembled
+(cuobjdump -sass), paired with its namesake by mangled name, and compared instruction by instruction after constant-bank
+offsets (c[0x0][0x...], where kernel parameters live) are masked: a kernel whose parameter struct grew at its end reads
+the same fields at the same offsets, and a second struct behind it moves.  Prints one line per kernel and exits 1 when
+any of them differs in anything else, or is missing in one build.  No GPU needed.
 """
 from __future__ import annotations
 
@@ -22,15 +23,17 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.join(HERE, ".."))
 
 
-def _object(path: str, tmp: str, tag: str) -> str:
+def _objects(path: str, tmp: str, tag: str) -> list[str]:
     if os.path.isfile(path):
-        return path
-    from capycrypt_b200.build import BASE_FLAGS, NVCC
+        return [path]
+    from capycrypt_b200.build import BASE_FLAGS, NVCC, SOURCES
 
-    obj = os.path.join(tmp, f"{tag}_sha3_api.o")
-    src = os.path.join(path, "capycrypt_b200", "csrc", "sha3_api.cu")
-    subprocess.run([NVCC, *BASE_FLAGS, "-c", src, "-o", obj], check=True)
-    return obj
+    objs = []
+    for src in SOURCES:
+        obj = os.path.join(tmp, f"{tag}_{src.replace('.cu', '.o')}")
+        subprocess.run([NVCC, *BASE_FLAGS, "-c", os.path.join(path, "capycrypt_b200", "csrc", src), "-o", obj], check=True)
+        objs.append(obj)
+    return objs
 
 
 def _functions(obj: str) -> dict[str, list[str]]:
@@ -49,18 +52,26 @@ def _functions(obj: str) -> dict[str, list[str]]:
     return funcs
 
 
+def _build(path: str, tmp: str, tag: str) -> dict[str, list[str]]:
+    funcs: dict[str, list[str]] = {}
+    for obj in _objects(path, tmp, tag):
+        funcs.update(_functions(obj))
+    return funcs
+
+
 def main() -> int:
     ap = argparse.ArgumentParser()
     ap.add_argument("old")
     ap.add_argument("new")
-    ap.add_argument("--kernels", default="sponge_kernel,sponge_tiered_kernel,sponge_kernel2")
+    ap.add_argument("--kernels", help="comma-separated kernel templates to compare (default: every kernel)")
     args = ap.parse_args()
-    names = args.kernels.split(",")
     with tempfile.TemporaryDirectory() as tmp:
-        old = _functions(_object(args.old, tmp, "old"))
-        new = _functions(_object(args.new, tmp, "new"))
-    pick = lambda fs: {k: v for k, v in fs.items() if any(re.match(rf"_ZN4capy{len(n)}{n}ILi\d+EEEv", k) for n in names)}
-    old, new = pick(old), pick(new)
+        old = _build(args.old, tmp, "old")
+        new = _build(args.new, tmp, "new")
+    if args.kernels:
+        names = args.kernels.split(",")
+        pick = lambda fs: {k: v for k, v in fs.items() if any(re.match(rf"_ZN4capy{len(n)}{n}ILi\d+EEEv", k) for n in names)}
+        old, new = pick(old), pick(new)
     bad = 0
     for k in sorted(set(old) | set(new)):
         if k not in old or k not in new:
@@ -74,6 +85,7 @@ def main() -> int:
     if not old:
         print("no matching kernels found")
         return 1
+    print(f"{len(set(old) | set(new))} kernels, {bad} differ or are missing")
     return 1 if bad else 0
 
 
