@@ -91,6 +91,13 @@ SIGNATURES = {
     "capy_hasher_final": (i32, [vp, vp, u64, u64p, u8p]),
     "capy_hasher_final_dev": (i32, [vp, vp, i32, vp, u64, u64p, u8p]),
     "capy_hasher_free": (None, [vp]),
+    "capy_sponge_encrypt_stream_new": (i32, [vp, i32, i32, u8p, u64p, u8p, u64, u64, C.POINTER(vp)]),
+    "capy_ed448_key_encrypt_stream_new": (i32, [vp, i32, u8p, vp, u8p, u64, u8p, C.POINTER(vp)]),
+    "capy_ed448_verify_stream_new": (i32, [vp, i32, u8p, vp, u8p, u8p, u64, C.POINTER(vp)]),
+    "capy_hasher_encrypt_update": (i32, [vp, vp, u8p, u64p, u8p]),
+    "capy_hasher_encrypt_update_dev": (i32, [vp, vp, i32, vp, u8p, u64p, u8p]),
+    "capy_hasher_verify_final": (i32, [vp, vp, u8p]),
+    "capy_hasher_verify_final_dev": (i32, [vp, vp, i32, vp, u8p, vp]),
 }
 
 

@@ -135,6 +135,73 @@ class Gpu:
         kd, ko = pack(keys)
         return SpongeStream(self.engine.kmac_xof_hasher(kd, ko, s, int(d)), int(d))
 
+    def sha3_encrypt_stream(self, pws: Sequence[bytes], d: SecParam,
+                            nonces: Optional[Sequence[bytes]] = None) -> "EncryptStream":
+        """one sha3_encrypt per password whose plaintext arrives in pieces: update() returns the ciphertext pieces,
+        finish() the tags; together they are the .msg and .digest sha3_encrypt gives for the concatenated plaintext, and
+        .nonces its .sym_nonce.  D224 is refused (ValueError): see capy_gpu.h."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("sha3_encrypt_stream: D224 is not resumable (quirk Q7)")
+        if nonces is None:
+            nonces = [os.urandom(512) for _ in pws]
+        if len(nonces) != len(pws) or any(len(z) != 512 for z in nonces):
+            raise ValueError("sha3_encrypt_stream: one 512-byte nonce per password")
+        pd, po = pack(pws)
+        st = self.engine.sponge_encrypt_stream(pd, po, b"".join(nonces), 512, int(d))
+        return EncryptStream(st, nonces=[bytes(z) for z in nonces])
+
+    def key_encrypt_stream(self, pub_keys: Sequence[bytes] | PreparedPublicKey, d: SecParam,
+                           k_rand: Optional[Sequence[bytes]] = None, n: Optional[int] = None) -> "EncryptStream":
+        """one key_encrypt per recipient (or n to one prepared key) whose plaintext arrives in pieces: as
+        sha3_encrypt_stream, with .asym_nonces the Z of each message.  OperationError("InvalidPublicKey") for an
+        off-curve key; D224 is refused (ValueError)."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("key_encrypt_stream: D224 is not resumable (quirk Q7)")
+        prepared = isinstance(pub_keys, PreparedPublicKey)
+        if n is None:
+            n = len(k_rand) if k_rand is not None else (None if prepared else len(pub_keys))
+        if n is None:
+            raise ValueError("key_encrypt_stream: a prepared key needs n or k_rand")
+        if k_rand is None:
+            k_rand = [os.urandom(56) for _ in range(n)]
+        if len(k_rand) != n or any(len(k) != 56 for k in k_rand):
+            raise ValueError("key_encrypt_stream: one 56-byte nonce per message")
+        if not prepared and (len(pub_keys) != n or any(len(p) != 112 for p in pub_keys)):
+            raise ValueError("key_encrypt_stream: one 112-byte public key per message")
+        pub = pub_keys if prepared else b"".join(pub_keys)
+        try:
+            st, z = self.engine.ed448_key_encrypt_stream(pub, b"".join(k_rand), int(d))
+        except CapyError as e:
+            if e.status == ERR_BAD_POINT:
+                raise OperationError("InvalidPublicKey") from None
+            raise
+        return EncryptStream(st, asym_nonces=[r.tobytes() for r in z])
+
+    def verify_stream(self, sigs: Sequence[Optional[Signature]], pub_keys: Sequence[bytes] | PreparedPublicKey,
+                      d: SecParam) -> "VerifyStream":
+        """verify() of signatures whose messages arrive in pieces: update() appends one piece per message, finish() gives
+        what verify() gives for the concatenated pieces.  A missing signature (SignatureNotSet) or a malformed signature
+        or key (SignatureVerificationFailure) fails on its own.  D224 is refused (ValueError)."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("verify_stream: D224 is not resumable (quirk Q7)")
+        prepared = isinstance(pub_keys, PreparedPublicKey)
+        res: list[Optional[OperationError]] = [None] * len(sigs)
+        idx = []
+        for i, sg in enumerate(sigs):
+            if sg is None:
+                res[i] = OperationError("SignatureNotSet")
+            elif len(sg.h) != 56 or len(sg.z) != 56 or (not prepared and len(pub_keys[i]) != 112):
+                res[i] = OperationError("SignatureVerificationFailure")
+            else:
+                idx.append(i)
+        h = b"".join(sigs[i].h for i in idx)
+        z = b"".join(sigs[i].z for i in idx)
+        pub = pub_keys if prepared else b"".join(pub_keys[i] for i in idx)
+        return VerifyStream(self.engine.ed448_verify_stream(pub, h, z, int(d)), idx, res)
+
     # ---- KeyPair::new ----------------------------------------------------------------------------------
     def new_keypairs(self, pws: Sequence[bytes], owner: str, d: SecParam) -> list[KeyPair]:
         d = SecParam.try_from(int(d))
@@ -348,6 +415,65 @@ class SpongeStream:
 
     def close(self) -> None:
         self.hasher.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class EncryptStream:
+    """Streams of Gpu.sha3_encrypt_stream / Gpu.key_encrypt_stream: update() encrypts one piece per message, finish()
+    returns the tags.  Use it in a `with` block (or call close()) to release its device memory before the engine."""
+
+    def __init__(self, stream, nonces: Optional[list[bytes]] = None, asym_nonces: Optional[list[bytes]] = None):
+        self.stream = stream
+        self.nonces = nonces
+        self.asym_nonces = asym_nonces
+
+    def update(self, pieces: Sequence[bytes]) -> list[bytes]:
+        data, off = pack(pieces)
+        ct = self.stream.update(data, off)
+        return [ct[int(off[i]):int(off[i + 1])].tobytes() for i in range(len(pieces))]
+
+    def finish(self) -> list[bytes]:
+        return [r.tobytes() for r in self.stream.final()]
+
+    def close(self) -> None:
+        self.stream.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class VerifyStream:
+    """Streams of Gpu.verify_stream: update() appends one piece per message (all of them, the failed ones included),
+    finish() gives verify()'s result per message."""
+
+    def __init__(self, stream, idx: list[int], res: list[Optional[OperationError]]):
+        self.stream = stream
+        self.idx = idx
+        self.res = res
+
+    def update(self, pieces: Sequence[bytes]) -> None:
+        if len(pieces) != len(self.res):
+            raise ValueError(f"verify_stream update: {len(pieces)} pieces for {len(self.res)} messages")
+        data, off = pack([pieces[i] for i in self.idx])
+        self.stream.update(data, off)
+
+    def finish(self) -> list[Optional[OperationError]]:
+        _, ok = self.stream.final()
+        for i, o in zip(self.idx, ok):
+            if not o:
+                self.res[i] = OperationError("SignatureVerificationFailure")
+        return self.res
+
+    def close(self) -> None:
+        self.stream.close()
 
     def __enter__(self):
         return self

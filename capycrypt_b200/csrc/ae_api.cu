@@ -210,9 +210,11 @@ static AeCore ecdhies_core(int d, const uint8_t* keymat) {
   return c;
 }
 
-// Z = [k]G (:38) with kw = k in SoA words ; (ke || ka) from W.x ; tag and ciphertext (:40-48)
+// Z = [k]G (:38) with kw = k in SoA words ; (ke || ka) from W.x ; tag and ciphertext (:40-48).  With keymat_out, no
+// message: (ke || ka) is handed back for an encryption stream instead.
 static int key_encrypt_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint32_t* kw, const uint8_t* wx,
-                              const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy) {
+                              const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy,
+                              uint8_t** keymat_out) {
   CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
   int rc = launch_fixed_base(ctx, dc, st, kw, proj, n, true);
   if (rc) return rc;
@@ -221,12 +223,16 @@ static int key_encrypt_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int
   uint8_t* keymat;
   rc = dev_ecdhies_keymat(ctx, dc, st, d, wx, n, &keymat);
   if (rc) return rc;
+  if (keymat_out) {
+    *keymat_out = keymat;
+    return CAPY_OK;
+  }
   return dev_ae_seal(ctx, dc, st, ecdhies_core(d, keymat), msgs, off, n, ct, tag);
 }
 
 static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pub, const uint8_t* k_rand,
                            const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct, uint8_t* tag, uint8_t* z_xy,
-                           int* d_bad_flag) {
+                           int* d_bad_flag, uint8_t** keymat_out = nullptr) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
@@ -240,7 +246,7 @@ static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   if (rc) return rc;
   rc = launch_scalar_prep(ctx, st, k_rand, 1, kw, nullptr, n);
   if (rc) return rc;
-  rc = key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy);
+  rc = key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy, keymat_out);
   if (rc) return rc;
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
 }
@@ -248,7 +254,7 @@ static int dev_key_encrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
 // W = [k]V for a prepared V through V's comb table (k is secret: constant-time scan), then as dev_key_encrypt
 static int dev_key_encrypt_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const capy_ed448_pub* key,
                                     const uint8_t* k_rand, const uint8_t* msgs, const uint64_t* off, uint64_t n, uint8_t* ct,
-                                    uint8_t* tag, uint8_t* z_xy) {
+                                    uint8_t* tag, uint8_t* z_xy, uint8_t** keymat_out = nullptr) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   const uint32_t* v_table = key->d_table[dc.index];
@@ -256,7 +262,7 @@ static int dev_key_encrypt_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t s
     CAPY_SCRATCH(pub, uint8_t, kEdPubRep, n * 112);
     const int rc = broadcast_point(ctx, st, key->d_xy[dc.index], pub, n);
     if (rc) return rc;
-    return dev_key_encrypt(ctx, dc, st, d, pub, k_rand, msgs, off, n, ct, tag, z_xy, nullptr);
+    return dev_key_encrypt(ctx, dc, st, d, pub, k_rand, msgs, off, n, ct, tag, z_xy, nullptr, keymat_out);
   }
   CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
   CAPY_SCRATCH(wx, uint8_t, kAeWx, n * 56);
@@ -268,7 +274,7 @@ static int dev_key_encrypt_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t s
   if (rc) return rc;
   rc = launch_to_affine(ctx, st, proj, n, 1, nullptr, wx);
   if (rc) return rc;
-  return key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy);
+  return key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy, keymat_out);
 }
 
 static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pws, const uint64_t* pw_off,
@@ -301,6 +307,22 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   rc = dev_ae_open(ctx, dc, st, ecdhies_core(d, keymat), ct, off, tag, bad, n, out, ok, t_new);
   if (rc) return rc;
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
+}
+
+// The two sponges of an encryption stream (capy_hasher) from (ke || ka) on the device, for the items of device dc: the tag
+// stream KMAC(ka, ., KA) after P | KB, and the keystream KMAC(ke, "", ., KE) at the start of its first squeeze block
+static int ae_stream_start(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const AeCore& c, capy_hasher* h, uint64_t n) {
+  KmacPass a(c.d, c.ka_custom, n);
+  a.job.keys = c.keymat + c.klen;
+  a.job.key_len = c.klen;
+  a.job.key_stride = 2ull * c.klen;
+  int rc = launch_kmac_state(ctx, dc, st, a, false, h->d_state[dc.index]);
+  if (rc) return rc;
+  KmacPass k(c.d, c.ke_custom, n);
+  k.job.keys = c.keymat;
+  k.job.key_len = c.klen;
+  k.job.key_stride = 2ull * c.klen;
+  return launch_kmac_state(ctx, dc, st, k, true, h->d_ks_state[dc.index]);
 }
 
 }  // namespace capy
@@ -457,6 +479,83 @@ int capy_ed448_key_decrypt_batch(capy_ctx* ctx, int d_bits, const uint8_t* pws, 
     return dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, sc.d_base, sc.d_off, d_tag, io.n(), d_out, d_ok,
                            io.d_flag());
   });
+}
+
+// =================================================================================================
+// encryption streams: the plaintext fed in pieces (capy_hasher_encrypt_update), the tag from capy_hasher_final
+// =================================================================================================
+// one chunk per device: the states are stored at [l * items + j]
+int capy_sponge_encrypt_stream_new(capy_ctx* ctx, int d_bits, int variant, const uint8_t* pws, const uint64_t* pw_off,
+                                   const uint8_t* nonces, uint64_t nonce_len, uint64_t n, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  AeCore c{};
+  if (!ctx || (n && (!pws || !pw_off || !nonces)) || !ae_customs(variant, &c.ke_custom, &c.ka_custom)) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // the tag stream absorbs at the 172-byte rate (Q7): see the header
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kEncryptStream, n, &h, 512);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    const StagedPacked sp = io.in_packed(pws, pw_off);
+    const uint8_t* d_nonce = io.in(nonces, nonce_len);
+    if (io.rc()) return io.rc();
+    uint8_t* keymat;
+    const int r = dev_sponge_keymat(ctx, dc, st, d_bits, sp.d_base, sp.d_off, pw_off[io.i1()] - pw_off[io.i0()], d_nonce,
+                                    nonce_len, io.n(), &keymat);
+    if (r) return r;
+    AeCore cc = c;
+    cc.d = d_bits;
+    cc.keymat = keymat;
+    cc.klen = 64;  // ke_ka.split_at(64)
+    return ae_stream_start(ctx, dc, st, cc, h, io.n());
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+int capy_ed448_key_encrypt_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112, const capy_ed448_pub* key,
+                                      const uint8_t* k_rand56, uint64_t n, uint8_t* z_xy112, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx || !pub_xy112 == !key || (key && pub_check(ctx, key)) || (n && (!k_rand56 || !z_xy112))) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kEncryptStream, n, &h, 448);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, pub_xy112 != nullptr,
+                     [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;
+    const uint8_t* d_pub = pub_xy112 ? io.in(pub_xy112, 112) : nullptr;
+    const uint8_t* d_k = io.in(k_rand56, 56);
+    uint8_t* d_z = io.out(z_xy112, 112);
+    if (io.rc()) return io.rc();
+    uint8_t* keymat;
+    const int r = d_pub ? dev_key_encrypt(ctx, dc, st, d_bits, d_pub, d_k, nullptr, nullptr, io.n(), nullptr, nullptr, d_z,
+                                          io.d_flag(), &keymat)
+                        : dev_key_encrypt_prepared(ctx, dc, st, d_bits, key, d_k, nullptr, nullptr, io.n(), nullptr, nullptr,
+                                                   d_z, &keymat);
+    if (r) return r;
+    return ae_stream_start(ctx, dc, st, ecdhies_core(d_bits, keymat), h, io.n());
+  });
+  if (rc) {  // CAPY_ERR_BAD_POINT included: no stream for a batch with an off-curve key
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
 }
 
 }  // extern "C"

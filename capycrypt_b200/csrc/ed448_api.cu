@@ -154,6 +154,14 @@ int launch_to_affine(capy_ctx* ctx, cudaStream_t st, const uint32_t* proj, uint6
   return CAPY_OK;
 }
 
+int launch_verify_compare(capy_ctx* ctx, cudaStream_t st, const uint8_t* hp, const uint8_t* h, const uint8_t* bad, uint8_t* ok,
+                          int* bad_flag, uint64_t n) {
+  verify_compare_kernel<<<grid_for(n, 256), 256, 0, st>>>(hp, h, bad, ok, bad_flag, n);
+  ctx->launches++;
+  CAPY_CUDA(ctx, cudaGetLastError());
+  return CAPY_OK;
+}
+
 int launch_any_bad(capy_ctx* ctx, cudaStream_t st, const uint8_t* bad, int* bad_flag, uint64_t n) {
   any_bad_kernel<<<grid_for(n, 256), 256, 0, st>>>(bad, bad_flag, n);
   ctx->launches++;
@@ -256,14 +264,27 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
   return CAPY_OK;
 }
 
-// ux = U.x ; h' = KMACXOF(ux, m, 448, "T") ; ok = (h' == h) && !bad   (signable.rs:78-85)
+// Where a verification stream (capy_ed448_verify_stream_new) starts: U'.x and the off-curve flags (nullptr: none), in
+// scratch of the stream that computed them
+struct VerifyStart {
+  const uint8_t* ux = nullptr;
+  const uint8_t* bad = nullptr;
+};
+
+// ux = U.x ; h' = KMACXOF(ux, m, 448, "T") ; ok = (h' == h) && !bad   (signable.rs:78-85).  With `start`, only ux: the
+// rest is the verification stream's.
 static int verify_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint32_t* proj_u, const uint8_t* d_msgs,
                          const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* bad, uint64_t n, uint8_t* d_ok,
-                         int* d_bad_flag) {
+                         int* d_bad_flag, VerifyStart* start = nullptr) {
   CAPY_SCRATCH(ux, uint8_t, kEdTmp56A, n * 56);
   CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
   int rc = launch_to_affine(ctx, st, proj_u, n, 1, nullptr, ux);
   if (rc) return rc;
+  if (start) {
+    start->ux = ux;
+    start->bad = bad;
+    return CAPY_OK;
+  }
   KmacPass h(d, "T", n);
   h.job.keys = ux;
   h.job.key_stride = h.job.key_len = 56;
@@ -281,7 +302,7 @@ static int verify_finish(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, c
 
 static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* d_pub, const uint8_t* d_msgs,
                       const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* d_z, uint64_t n, uint8_t* d_ok,
-                      int* d_bad_flag) {
+                      int* d_bad_flag, VerifyStart* start = nullptr) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   CAPY_SCRATCH(kw, uint32_t, kEdKWords, n * 56);
@@ -296,7 +317,7 @@ static int dev_verify(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, cons
   if (rc) return rc;
   rc = launch_var_base(ctx, dc, st, d_h, 0, d_pub, projA, projB, bad, n, false);
   if (rc) return rc;
-  return verify_finish(ctx, dc, st, d, projB, d_msgs, d_msg_off, d_h, bad, n, d_ok, d_bad_flag);
+  return verify_finish(ctx, dc, st, d, projB, d_msgs, d_msg_off, d_h, bad, n, d_ok, d_bad_flag, start);
 }
 
 // W = [k]V with k = 4 * BE(rand) mod r (ecc/encryptable.rs:36-37): W.x ; optionally Z = [k]G (:38)
@@ -335,7 +356,7 @@ int broadcast_point(capy_ctx* ctx, cudaStream_t st, const uint8_t* d_xy, uint8_t
 // U = [z]G + [h]V for a prepared V, then as dev_verify
 static int dev_verify_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const capy_ed448_pub* key,
                                const uint8_t* d_msgs, const uint64_t* d_msg_off, const uint8_t* d_h, const uint8_t* d_z,
-                               uint64_t n, uint8_t* d_ok) {
+                               uint64_t n, uint8_t* d_ok, VerifyStart* start = nullptr) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   const uint32_t* v_table = key->d_table[dc.index];
@@ -343,7 +364,7 @@ static int dev_verify_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, in
     CAPY_SCRATCH(pub, uint8_t, kEdPubRep, n * 112);
     const int rc = broadcast_point(ctx, st, key->d_xy[dc.index], pub, n);
     if (rc) return rc;
-    return dev_verify(ctx, dc, st, d, pub, d_msgs, d_msg_off, d_h, d_z, n, d_ok, nullptr);
+    return dev_verify(ctx, dc, st, d, pub, d_msgs, d_msg_off, d_h, d_z, n, d_ok, nullptr, start);
   }
   CAPY_SCRATCH(zw, uint32_t, kEdKWords, n * 56);
   CAPY_SCRATCH(hw, uint32_t, kEdSWords, n * 56);
@@ -357,7 +378,7 @@ static int dev_verify_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, in
   if (rc) return rc;
   rc = launch_fixed_base(ctx, dc, st, zw, proj, n, false, nullptr, hw, v_table);
   if (rc) return rc;
-  return verify_finish(ctx, dc, st, d, proj, d_msgs, d_msg_off, d_h, nullptr, n, d_ok, nullptr);
+  return verify_finish(ctx, dc, st, d, proj, d_msgs, d_msg_off, d_h, nullptr, n, d_ok, nullptr, start);
 }
 
 int pub_check(const capy_ctx* ctx, const capy_ed448_pub* key) {
@@ -636,6 +657,49 @@ void capy_ed448_pub_free(capy_ed448_pub* key) {
     if (key->d_xy[k]) cudaFree(key->d_xy[k]);
   }
   delete key;
+}
+
+// The front end of verify up to U'.x (per-item keys: dev_verify; a prepared key: dev_verify_prepared), then KMAC streams
+// keyed by U'.x with S = "T" (one chunk per device: the states are stored at [l * items + j]).  h and the off-curve flags
+// stay with the streams for capy_hasher_verify_final.
+int capy_ed448_verify_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112, const capy_ed448_pub* key,
+                                 const uint8_t* h56, const uint8_t* z_be56, uint64_t n, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx || !pub_xy112 == !key || (key && pub_check(ctx, key)) || (n && (!h56 || !z_be56))) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // the "T" stream absorbs at the 172-byte rate (Q7): see the header
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kVerifyStream, n, &h, 448);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    const uint8_t* d_pub = pub_xy112 ? io.in(pub_xy112, 112) : nullptr;
+    const uint8_t* d_h = io.in(h56, 56);
+    const uint8_t* d_z = io.in(z_be56, 56);
+    if (io.rc()) return io.rc();
+    const int k = dc.index;
+    const uint64_t m = io.n();
+    VerifyStart vs;
+    int r = d_pub ? dev_verify(ctx, dc, st, d_bits, d_pub, nullptr, nullptr, d_h, d_z, m, nullptr, nullptr, &vs)
+                  : dev_verify_prepared(ctx, dc, st, d_bits, key, nullptr, nullptr, d_h, d_z, m, nullptr, &vs);
+    if (r) return r;
+    CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_h[k], d_h, m * 56, cudaMemcpyDeviceToDevice, st));
+    if (vs.bad) CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_bad[k], vs.bad, m, cudaMemcpyDeviceToDevice, st));
+    KmacPass a(d_bits, "T", m);
+    a.job.keys = vs.ux;
+    a.job.key_stride = a.job.key_len = 56;
+    return launch_kmac_state(ctx, dc, st, a, false, h->d_state[k]);
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
 }
 
 int capy_ed448_ecdh_batch(capy_ctx* ctx, const uint8_t* k_rand56, const uint8_t* pub_xy112, uint64_t n, uint8_t* wx56,

@@ -329,6 +329,9 @@ inline int run_host_call(capy_ctx* ctx, const std::vector<Range>& shards, Chunks
 // the chunker of the calls that run a device's shard as one chunk
 inline std::vector<Range> one_chunk(Range sh) { return {sh}; }
 
+// the items of a stream batch (capy_hasher) on each device of its ctx, one shard per device in device order (sha3_api.cu)
+std::vector<Range> hasher_shards(const capy_hasher* h);
+
 constexpr uint64_t kChunkBytes = 8ull << 20;
 
 // Ragged batches: a chunk is one launch, and a launch cannot finish before the longest message in it has (a sponge

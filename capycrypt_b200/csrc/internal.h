@@ -196,17 +196,32 @@ struct capy_ed448_pub {
 //   d_state[k]  25 lanes at [l * items_k + j]: every whole block of its stream so far (200 B per item)
 //   d_carry[k]  the bytes behind the last whole block at [j * rate ..), total % rate of them
 //   d_total[k]  [j] = message bytes absorbed so far (uint64)
+// Encryption streams (capy_sponge_encrypt_stream_new / capy_ed448_key_encrypt_stream_new, ae_api.cu) are KMAC streams
+// keyed by ka -- the tag -- with a keystream sponge beside each (SpongeSqueeze):
+//   d_ks_state[k]  25 lanes at [l * items_k + j]: the keystream sponge at the start of its current squeeze block
+//   d_ks_pos[k]    [j] = keystream bytes used so far
+// Verification streams (capy_ed448_verify_stream_new, ed448_api.cu) are KMAC streams keyed by U'.x with S = "T", and keep
+//   d_h[k]    [j * 56 ..) the signature's h ;  d_bad[k]  [j] = V_j is off the curve
+namespace capy {
+enum HasherKind { kSha3Stream, kKmacStream, kEncryptStream, kVerifyStream };
+}
 struct capy_hasher {
   const capy_ctx* ctx = nullptr;
   int d_bits = 0;
-  bool kmac = false;
+  int kind = capy::kSha3Stream;
+  bool kmac = false;  // every kind but kSha3Stream
   uint32_t rate = 0;
+  uint32_t tag_bits = 0;           // encryption and verification streams: the width of the final
   uint64_t n = 0;
   std::vector<uint64_t> first;     // [device index] first item; first[devices] = n
   std::vector<int> dev;            // CUDA device of every ctx device (frees without the ctx)
   std::vector<uint64_t*> d_state;  // [device index], nullptr when the device holds no item
   std::vector<uint8_t*> d_carry;
   std::vector<uint64_t*> d_total;
+  std::vector<uint64_t*> d_ks_state;  // encryption streams only
+  std::vector<uint64_t*> d_ks_pos;
+  std::vector<uint8_t*> d_h;          // verification streams only
+  std::vector<uint8_t*> d_bad;
   std::vector<char> finished;      // [device index] its items were finalised
 };
 
@@ -305,5 +320,14 @@ int launch_kmac_xof(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const Kma
 int launch_kmac_xof2(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, const KmacPass& b);
 // two passes where `second` absorbs what `first` wrote for the same item: one launch of dependent jobs when the batch is large
 int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& first, const KmacPass& second);
+// The state of a KMAC pass without message (a.job: keys, n) before its first squeeze, stored at states[l * n + i]: with
+// the trailer, after P | KB | 00 01 04 | pad (a keystream at position 0); without, exactly after P | KB (the start of a
+// KMAC stream)
+int launch_kmac_state(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, bool trailer, uint64_t* states);
+// a stream batch of `kind` (HasherKind) with zeroed buffers on every device that holds items (blocking; sha3_api.cu)
+int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher** out, uint32_t tag_bits = 0);
+// ok[i] = (hp_i == h_i) && !bad[i] over 56-byte rows; *bad_flag |= 1 when a bad[i] is set (ed448_api.cu)
+int launch_verify_compare(capy_ctx* ctx, cudaStream_t st, const uint8_t* hp, const uint8_t* h, const uint8_t* bad, uint8_t* ok,
+                          int* bad_flag, uint64_t n);
 
 }  // namespace capy

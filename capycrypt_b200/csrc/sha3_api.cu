@@ -658,7 +658,8 @@ static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t
 // two jobs over the same ranks in one launch, job 1 of an item after job 0 of that item (sponge_chain_kernel); with
 // jobs = 1, J0 alone (and, with `resume`, as resumable streams)
 static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J0, const SpongeJob& J1,
-                             bool data_dependent, uint32_t jobs = 2, const SpongeResume* resume = nullptr) {
+                             bool data_dependent, uint32_t jobs = 2, const SpongeResume* resume = nullptr,
+                             const SpongeSqueeze* squeeze = nullptr) {
   const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
   uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
   if (!sync) return CAPY_ERR_OOM;
@@ -670,6 +671,7 @@ static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, 
   C.blocks_per_job = nb;
   C.data_dependent = data_dependent ? 1u : 0u;
   C.resume = resume ? *resume : SpongeResume{};
+  C.squeeze = squeeze ? *squeeze : SpongeSqueeze{};
   return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J0), [&](auto L) {
     sponge_chain_kernel<decltype(L)::value><<<jobs * nb, 128, 0, stream>>>(C);
     ctx->launches++;
@@ -1035,10 +1037,21 @@ static bool hasher_any_finished(const capy_hasher* h) {
     if (f) return true;
   return false;
 }
-static std::vector<Range> hasher_shards(const capy_hasher* h) {  // one per device, in device order (for_each_device)
+std::vector<Range> hasher_shards(const capy_hasher* h) {
   std::vector<Range> s;
   for (size_t k = 0; k + 1 < h->first.size(); k++) s.push_back({h->first[k], h->first[k + 1]});
   return s;
+}
+
+// the outputs capy_hasher_final takes: SHA3-d digests, any KMACXOF output, the tag of encryption streams; verification
+// streams end in capy_hasher_verify_final
+static bool hasher_final_fits(const capy_hasher* h, uint64_t out_bits, const uint64_t* out_off) {
+  switch (h->kind) {
+    case kSha3Stream: return out_bits == (uint64_t)h->d_bits && !out_off;
+    case kKmacStream: return true;
+    case kEncryptStream: return out_bits == h->tag_bits && !out_off;
+    default: return false;
+  }
 }
 
 // the operator of the hasher's streams; its prefix and keys are already in their states
@@ -1067,6 +1080,28 @@ static int hasher_update_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, ca
   return launch_chain_jobs(ctx, dc, st, J, J, false, 1, &R);
 }
 
+// an update of encryption streams: job 0 absorbs the plaintext into the tag streams, job 1 XORs the keystream into it.
+// Job 1 of a block starts after job 0 of that block, so the tag has read the plaintext when `ct == data` overwrites it.
+static int hasher_encrypt_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, uint64_t j0, uint64_t n,
+                                const uint8_t* d_data, const uint64_t* d_off, uint8_t* d_ct) {
+  if (n == 0) return CAPY_OK;
+  const int k = dc.index;
+  SpongeResume R;
+  SpongeJob J0 = hasher_job(h, k, j0, n, &R);
+  J0.chain_out = h->d_state[k] + j0;
+  J0.stop_block = ~0ull;
+  J0.data = d_data;
+  J0.off = d_off;
+  SpongeJob J1 = hasher_operator(h);
+  J1.chain_in = J1.chain_out = h->d_ks_state[k] + j0;
+  J1.data = d_data;
+  J1.off = d_off;
+  J1.out = d_ct;
+  J1.n = n;
+  const SpongeSqueeze S{h->d_ks_pos[k] + j0, hasher_items(h, k)};
+  return launch_chain_jobs(ctx, dc, st, J0, J1, false, 2, &R, &S);
+}
+
 static int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
                               uint64_t out_bytes, const uint64_t* d_out_off, uint8_t* d_out) {
   if (n == 0 || (!d_out_off && out_bytes == 0)) return CAPY_OK;
@@ -1078,14 +1113,38 @@ static int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, con
   return launch_chain_jobs(ctx, dc, st, J, J, false, 1, &R);
 }
 
-// A hasher with zeroed buffers on every device that holds items (blocking).  Items are dealt out in equal contiguous
-// ranges.
-static int hasher_create(capy_ctx* ctx, int d_bits, bool kmac, uint64_t n, capy_hasher** out) {
+// the final of verification streams: h' through the tag final, then ok = (h' == h) && !bad
+static int hasher_verify_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
+                               uint8_t* d_ok, int* d_bad_flag) {
+  if (n == 0) return CAPY_OK;
+  CAPY_SCRATCH(hp, uint8_t, kEdTmp56B, n * 56);
+  const int rc = hasher_final_items(ctx, dc, st, h, j0, n, 56, nullptr, hp);
+  if (rc) return rc;
+  return launch_verify_compare(ctx, st, hp, h->d_h[dc.index] + 56 * j0, h->d_bad[dc.index] + j0, d_ok, d_bad_flag, n);
+}
+
+int launch_kmac_state(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, bool trailer, uint64_t* states) {
+  SpongeJob J;
+  const int rc = build_kmac_job(ctx, dc, stream, a, &J);
+  if (rc) return rc;
+  if (!trailer) {
+    J.trailer = 0;
+    J.trailer_len = 0;
+  }
+  J.chain_out = states;
+  J.stop_block = ~0ull;
+  return launch_chain_jobs(ctx, dc, stream, J, J, false, 1);
+}
+
+// Items are dealt out in equal contiguous ranges.
+int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher** out, uint32_t tag_bits) {
   capy_hasher* h = new (std::nothrow) capy_hasher();
   if (!h) return CAPY_ERR_OOM;
   h->ctx = ctx;
   h->d_bits = d_bits;
-  h->kmac = kmac;
+  h->kind = kind;
+  h->kmac = kind != kSha3Stream;
+  h->tag_bits = tag_bits;
   h->rate = hasher_operator(h).rate;
   h->n = n;
   const uint64_t nd = ctx->devs.size();
@@ -1094,6 +1153,10 @@ static int hasher_create(capy_ctx* ctx, int d_bits, bool kmac, uint64_t n, capy_
   h->d_state.assign(nd, nullptr);
   h->d_carry.assign(nd, nullptr);
   h->d_total.assign(nd, nullptr);
+  h->d_ks_state.assign(nd, nullptr);
+  h->d_ks_pos.assign(nd, nullptr);
+  h->d_h.assign(nd, nullptr);
+  h->d_bad.assign(nd, nullptr);
   h->finished.assign(nd, 0);
   for (DeviceCtx& dc : ctx->devs) {
     const uint64_t m = hasher_items(h, dc.index);
@@ -1102,12 +1165,20 @@ static int hasher_create(capy_ctx* ctx, int d_bits, bool kmac, uint64_t n, capy_
     DeviceGuard g(dc.dev);
     const cudaStream_t st = dc.streams[0];
     const int rc = [&]() -> int {
-      CAPY_CUDA(ctx, cudaMalloc(&h->d_state[dc.index], (size_t)m * 200));
-      CAPY_CUDA(ctx, cudaMalloc(&h->d_carry[dc.index], (size_t)m * h->rate));
-      CAPY_CUDA(ctx, cudaMalloc(&h->d_total[dc.index], (size_t)m * 8));
-      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_state[dc.index], 0, (size_t)m * 200, st));
-      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_carry[dc.index], 0, (size_t)m * h->rate, st));
-      CAPY_CUDA(ctx, cudaMemsetAsync(h->d_total[dc.index], 0, (size_t)m * 8, st));
+      auto zeroed = [&](auto*& p, size_t bytes) -> int {
+        CAPY_CUDA(ctx, cudaMalloc(&p, bytes));
+        CAPY_CUDA(ctx, cudaMemsetAsync(p, 0, bytes, st));
+        return CAPY_OK;
+      };
+      const int k = dc.index;
+      int r = zeroed(h->d_state[k], (size_t)m * 200);
+      if (!r) r = zeroed(h->d_carry[k], (size_t)m * h->rate);
+      if (!r) r = zeroed(h->d_total[k], (size_t)m * 8);
+      if (!r && kind == kEncryptStream) r = zeroed(h->d_ks_state[k], (size_t)m * 200);
+      if (!r && kind == kEncryptStream) r = zeroed(h->d_ks_pos[k], (size_t)m * 8);
+      if (!r && kind == kVerifyStream) r = zeroed(h->d_h[k], (size_t)m * 56);
+      if (!r && kind == kVerifyStream) r = zeroed(h->d_bad[k], (size_t)m);
+      if (r) return r;
       CAPY_CUDA(ctx, cudaStreamSynchronize(st));
       return CAPY_OK;
     }();
@@ -1394,7 +1465,7 @@ int capy_sha3_hasher_new(capy_ctx* ctx, int d_bits, uint64_t n, capy_hasher** ou
   *out = nullptr;
   if (!ctx) return CAPY_ERR_BAD_ARG;
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
-  return hasher_create(ctx, d_bits, false, n, out);
+  return hasher_create(ctx, d_bits, kSha3Stream, n, out);
 }
 
 int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, const uint64_t* key_off, uint64_t n,
@@ -1405,13 +1476,13 @@ int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, con
   if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
   if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // the 172-byte rate is read as 168 (Q7): see the header
   capy_hasher* h = nullptr;
-  int rc = hasher_create(ctx, d_bits, true, n, &h);
+  int rc = hasher_create(ctx, d_bits, kKmacStream, n, &h);
   if (rc || n == 0) {
     *out = h;
     return rc;
   }
-  // P | KB: the cached prefix state, then the key block of every item -- a KMAC job with no message and no trailer ends
-  // exactly there; its states are the hasher's starting states (one chunk per device: the states are stored at [k * n + i])
+  // P | KB: the cached prefix state, then the key block of every item (one chunk per device: the states are stored at
+  // [k * n + i])
   rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
     if (io.n() == 0) return CAPY_OK;  // (a device without items)
     const StagedPacked sk = io.in_packed(keys, key_off);
@@ -1419,14 +1490,7 @@ int capy_kmac_xof_hasher_new(capy_ctx* ctx, int d_bits, const uint8_t* keys, con
     KmacPass a(d_bits, {reinterpret_cast<const char*>(custom), custom_len}, io.n());
     a.job.keys = sk.d_base;
     a.job.key_off = sk.d_off;
-    SpongeJob J;
-    const int rj = build_kmac_job(ctx, dc, st, a, &J);
-    if (rj) return rj;
-    J.trailer = 0;
-    J.trailer_len = 0;
-    J.chain_out = h->d_state[dc.index];
-    J.stop_block = ~0ull;
-    return launch_chain_jobs(ctx, dc, st, J, J, false, 1);
+    return launch_kmac_state(ctx, dc, st, a, false, h->d_state[dc.index]);
   });
   if (rc) {
     capy_hasher_free(h);
@@ -1444,7 +1508,8 @@ int capy_hasher_device_range(const capy_hasher* h, int dev_index, uint64_t* i0, 
 }
 
 int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off) {
-  if (hasher_check(ctx, h) || hasher_any_finished(h) || (h->n && (!data || !off))) return CAPY_ERR_BAD_ARG;
+  if (hasher_check(ctx, h) || h->kind == kEncryptStream || hasher_any_finished(h) || (h->n && (!data || !off)))
+    return CAPY_ERR_BAD_ARG;
   if (h->n == 0) return CAPY_OK;
   auto chunks = [&](Range sh) {
     return split_items(off, 0, sh.i0, sh.i1, chunk_count(off[sh.i1] - off[sh.i0], sh.i1 - sh.i0), 200);
@@ -1458,7 +1523,8 @@ int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const
 
 int capy_hasher_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_data,
                            const uint64_t* d_off) {
-  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || h->finished[dev_index]) return CAPY_ERR_BAD_ARG;
+  if (hasher_check(ctx, h) || h->kind == kEncryptStream || !dev_index_ok(ctx, dev_index) || h->finished[dev_index])
+    return CAPY_ERR_BAD_ARG;
   const uint64_t m = hasher_items(h, dev_index);
   if (m && (!d_data || !d_off)) return CAPY_ERR_BAD_ARG;
   if (m == 0) return CAPY_OK;
@@ -1468,7 +1534,7 @@ int capy_hasher_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* s
 
 int capy_hasher_final(capy_ctx* ctx, capy_hasher* h, uint64_t out_bits, const uint64_t* out_off, uint8_t* out) {
   if (hasher_check(ctx, h) || hasher_any_finished(h) || (h->n && !out)) return CAPY_ERR_BAD_ARG;
-  if (!h->kmac && (out_bits != (uint64_t)h->d_bits || out_off)) return CAPY_ERR_BAD_ARG;
+  if (!hasher_final_fits(h, out_bits, out_off)) return CAPY_ERR_BAD_ARG;
   for (char& f : h->finished) f = 1;
   const size_t ob = (size_t)(out_bits / 8);
   if (h->n == 0 || (!out_off && ob == 0)) return CAPY_OK;
@@ -1493,7 +1559,7 @@ int capy_hasher_final(capy_ctx* ctx, capy_hasher* h, uint64_t out_bits, const ui
 int capy_hasher_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint64_t out_bits,
                           const uint64_t* d_out_off, uint8_t* d_out) {
   if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || h->finished[dev_index]) return CAPY_ERR_BAD_ARG;
-  if (!h->kmac && (out_bits != (uint64_t)h->d_bits || d_out_off)) return CAPY_ERR_BAD_ARG;
+  if (!hasher_final_fits(h, out_bits, d_out_off)) return CAPY_ERR_BAD_ARG;
   const uint64_t m = hasher_items(h, dev_index);
   if (m && !d_out) return CAPY_ERR_BAD_ARG;
   h->finished[dev_index] = 1;
@@ -1502,19 +1568,72 @@ int capy_hasher_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* st
   return hasher_final_items(ctx, dc, st, h, 0, m, out_bits / 8, d_out_off, d_out);
 }
 
+// ---- encryption and verification streams (created in ae_api.cu and ed448_api.cu) -------------------------------------
+int capy_hasher_encrypt_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off, uint8_t* ct) {
+  if (hasher_check(ctx, h) || h->kind != kEncryptStream || hasher_any_finished(h) || (h->n && (!data || !off || !ct)))
+    return CAPY_ERR_BAD_ARG;
+  if (h->n == 0) return CAPY_OK;
+  auto chunks = [&](Range sh) {
+    return split_items(off, 0, sh.i0, sh.i1, chunk_count(off[sh.i1] - off[sh.i0], sh.i1 - sh.i0), 400);
+  };
+  return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(data, off);
+    uint8_t* d_ct = io.out_packed(ct, off);
+    if (io.rc()) return io.rc();
+    return hasher_encrypt_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), sp.d_base, sp.d_off, d_ct);
+  });
+}
+
+int capy_hasher_encrypt_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_data,
+                                   const uint64_t* d_off, uint8_t* d_ct) {
+  if (hasher_check(ctx, h) || h->kind != kEncryptStream || !dev_index_ok(ctx, dev_index) || h->finished[dev_index])
+    return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && (!d_data || !d_off || !d_ct)) return CAPY_ERR_BAD_ARG;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return hasher_encrypt_items(ctx, dc, st, h, 0, m, d_data, d_off, d_ct);
+}
+
+int capy_hasher_verify_final(capy_ctx* ctx, capy_hasher* h, uint8_t* ok) {
+  if (hasher_check(ctx, h) || h->kind != kVerifyStream || hasher_any_finished(h) || (h->n && !ok)) return CAPY_ERR_BAD_ARG;
+  for (char& f : h->finished) f = 1;
+  if (h->n == 0) return CAPY_OK;
+  return run_host_call(ctx, hasher_shards(h), one_chunk, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return hasher_verify_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), d_ok, io.d_flag());
+  });
+}
+
+int capy_hasher_verify_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag) {
+  if (hasher_check(ctx, h) || h->kind != kVerifyStream || !dev_index_ok(ctx, dev_index) || h->finished[dev_index])
+    return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && !d_ok) return CAPY_ERR_BAD_ARG;
+  h->finished[dev_index] = 1;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return hasher_verify_items(ctx, dc, st, h, 0, m, d_ok, d_bad_flag);
+}
+
 void capy_hasher_free(capy_hasher* h) {
   if (!h) return;
   for (size_t k = 0; k < h->dev.size(); k++) {
-    if (!h->d_state[k] && !h->d_carry[k] && !h->d_total[k]) continue;
+    void* bufs[] = {h->d_state[k], h->d_carry[k], h->d_total[k], h->d_ks_state[k], h->d_ks_pos[k], h->d_h[k], h->d_bad[k]};
+    bool any = false;
+    for (void* p : bufs) any = any || p;
+    if (!any) continue;
+    const size_t m = (size_t)hasher_items(h, (int)k);
     DeviceGuard g(h->dev[k]);
     cudaDeviceSynchronize();  // work still queued on a caller's stream may read them
-    // after the key block a KMAC state is key material: zeroed before the memory goes back
-    if (h->d_state[k]) cudaMemset(h->d_state[k], 0, (size_t)hasher_items(h, (int)k) * 200);
-    if (h->d_carry[k]) cudaMemset(h->d_carry[k], 0, (size_t)hasher_items(h, (int)k) * h->rate);
+    // after the key block a KMAC state is key material, and so is a keystream state: zeroed before the memory goes back
+    if (h->d_state[k]) cudaMemset(h->d_state[k], 0, m * 200);
+    if (h->d_carry[k]) cudaMemset(h->d_carry[k], 0, m * h->rate);
+    if (h->d_ks_state[k]) cudaMemset(h->d_ks_state[k], 0, m * 200);
     cudaDeviceSynchronize();
-    if (h->d_state[k]) cudaFree(h->d_state[k]);
-    if (h->d_carry[k]) cudaFree(h->d_carry[k]);
-    if (h->d_total[k]) cudaFree(h->d_total[k]);
+    for (void* p : bufs)
+      if (p) cudaFree(p);
   }
   delete h;
 }

@@ -722,7 +722,9 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_kernel2(const __
 // tickets work on job 0, the others on job 1, and a job-1 block waits for the job-0 block of the same items (which holds a
 // smaller ticket, so it is running or done: no deadlock).  The launcher only cuts batches with at least as many job-0
 // blocks as the GPU holds at once, so in practice nobody waits.  A launch of only `blocks_per_job` blocks runs job 0 alone
-// (every ticket is a job-0 ticket, nobody waits): the updates and finals of resumable streams (SpongeJob::carry).
+// (every ticket is a job-0 ticket, nobody waits): the updates and finals of resumable streams (SpongeResume).  An update
+// of encryption streams runs both jobs at any size -- the tag stream's update, then its keystream (SpongeSqueeze) -- and
+// its job-1 blocks wait only for job-0 blocks that took their tickets earlier.
 struct SpongeChain {
   SpongeJob j[2];
   uint32_t* sync;  // [0] ticket counter, [1 + b] warps of job-0 block b that have stored their states; zeroed before the launch
@@ -731,11 +733,56 @@ struct SpongeChain {
   // decryption: keystream XOR, then the tag over the plaintext): its message loads go to the L2
   uint32_t data_dependent;
   SpongeResume resume;  // carry == nullptr: the jobs are not resumable streams
+  SpongeSqueeze squeeze;  // resumable streams with two jobs: job 1 is the keystream update of encryption streams
 };
 // resumable streams (order == nullptr: rank = item), out of line: the cut chains keep their own register allocation
 template <int LANES>
 __device__ __noinline__ void sponge_item_resume_ool(const SpongeJob& J, const SpongeResume* R, uint64_t i) {
   sponge_item<LANES, true, false, true>(J, i, i, R);
+}
+
+// Keystream update of item i (SpongeSqueeze): squeeze blocks of 8 LANES bytes (the cSHAKE / KMAC squeeze width equals the
+// rate at D256 / 384 / 512), entered at any byte of a block.  Lane j of a block is keystream bytes [8 j, 8 j + 8) of it; a
+// lane wholly inside the piece is one 8-byte load and store when data and out put keystream lanes on 8-byte boundaries
+// (pieces whose offsets and positions agree mod 8: the usual packed batch), any other lane goes byte by byte.  Out of line
+// like the resume path.
+template <int LANES>
+__device__ __noinline__ void sponge_squeeze_resume_ool(const SpongeJob& J, const SpongeSqueeze* S, uint64_t i) {
+  constexpr uint64_t SQ = 8ull * LANES;
+  const uint64_t state_n = S->state_n;
+  Lane a[25];
+#pragma unroll
+  for (int k = 0; k < 25; k++) {
+    const uint64_t v = J.chain_in[(uint64_t)k * state_n + i];
+    a[k].lo = (uint32_t)v;
+    a[k].hi = (uint32_t)(v >> 32);
+  }
+  const uint64_t p0 = S->pos[i], a0 = J.off[i], p1 = p0 + (J.off[i + 1] - a0);
+  const uint8_t* x = J.data + a0;  // keystream byte p goes with x[p - p0] and o[p - p0]
+  uint8_t* o = J.out + a0;
+  const bool al = ((reinterpret_cast<uintptr_t>(x) - p0) & 7u) == 0 && ((reinterpret_cast<uintptr_t>(o) - p0) & 7u) == 0;
+#pragma unroll 1
+  for (uint64_t b = p0 - p0 % SQ; b < p1;) {
+#pragma unroll
+    for (int j = 0; j < LANES; j++) {
+      const uint64_t l0 = b + 8ull * j, lo = l0 > p0 ? l0 : p0, hi = l0 + 8 < p1 ? l0 + 8 : p1;
+      if (lo < hi) {
+        if (al && hi - lo == 8) {
+          const uint2 m = *reinterpret_cast<const uint2*>(x + (lo - p0));
+          *reinterpret_cast<uint2*>(o + (lo - p0)) = make_uint2(a[j].lo ^ m.x, a[j].hi ^ m.y);
+        } else {
+          const uint64_t v = ((uint64_t)a[j].hi << 32) | a[j].lo;
+#pragma unroll 1
+          for (uint64_t q = lo; q < hi; q++) o[q - p0] = x[q - p0] ^ (uint8_t)(v >> (8 * (uint32_t)(q - l0)));
+        }
+      }
+    }
+    b += SQ;
+    if (b <= p1) keccak_f1600(a);  // this block is used up: the next byte comes from the next one
+  }
+#pragma unroll
+  for (int k = 0; k < 25; k++) J.chain_out[(uint64_t)k * state_n + i] = ((uint64_t)a[k].hi << 32) | a[k].lo;
+  S->pos[i] = p1;
 }
 
 template <int LANES>
@@ -754,6 +801,7 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(con
   const uint64_t r = (uint64_t)b * 128 + threadIdx.x;
   if (r < J.n) {
     if (job && C.data_dependent) sponge_item<LANES, true, true>(J, sponge_rank_item(J, r), r);
+    else if (C.resume.carry && job) sponge_squeeze_resume_ool<LANES>(J, &C.squeeze, r);  // (only encryption streams have a job 1)
     else if (C.resume.carry) sponge_item_resume_ool<LANES>(J, &C.resume, r);
     else sponge_item<LANES, true>(J, sponge_rank_item(J, r), r);
   }

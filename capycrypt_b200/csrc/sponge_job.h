@@ -71,6 +71,18 @@ struct SpongeResume {
   uint64_t state_n;  // stride of the lane-major states (the items of the device; a job may cover a part of them)
 };
 
+// Resumable keystreams (the keystream sponge of a capy_hasher encryption stream: job 1 of sponge_chain_kernel, beside the
+// update of its tag stream in job 0).  Item i's state at chain_in[k * state_n + i] is the sponge at the start of squeeze
+// block pos[i] / (8 LANES): the keystream is prefix-consistent, so piece X takes keystream bytes [pos[i], pos[i] + |X|).
+// The job writes out[off[i] ..) = those bytes ^ data[off[i] ..), permutes at every block end it reaches (eagerly: a piece
+// that ends on a block boundary leaves the state of the next block), stores the state at chain_out and advances pos[i].
+// A position of its own, not the tag stream's total: job 0 of the same launch advances that.  Kept out of SpongeJob, like
+// SpongeResume.
+struct SpongeSqueeze {
+  uint64_t* pos;
+  uint64_t state_n;
+};
+
 // ---- rates in bytes, as the reference computes them ------------------------------------------------------------------
 // SHA3-d capacity in bits: 2d rounded up to the reference's buckets (constants.rs:38-45)
 inline uint32_t sha3_capacity(int d) {

@@ -177,6 +177,68 @@ class Hasher:
             pass
 
 
+class EncryptStream(Hasher):
+    """n seal streams (Engine.sponge_encrypt_stream / Engine.ed448_key_encrypt_stream): update() encrypts one piece per
+    stream, final() returns the tags.  The concatenated ciphertext pieces and the tags are what the one-shot call gives
+    for the concatenated plaintext."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, n: int, d: int, tag_bytes: int):
+        super().__init__(engine, handle, n, d, True)
+        self.tag_bytes = tag_bytes
+
+    def update(self, data, off, out: np.ndarray | None = None) -> np.ndarray:
+        """capy_hasher_encrypt_update: the ciphertext of data[off[i] .. off[i+1]) at the same offsets of the result
+        (out may be data itself: in place)"""
+        data, off = _u8(data), _u64(off)
+        if _need_packed(data, off, "stream pieces") != self.n:
+            raise ValueError(f"stream update: {off.size - 1} pieces for {self.n} streams")
+        out = _out(out, (data.size,), "stream ciphertext")
+        self._engine._check(self._engine.lib.capy_hasher_encrypt_update(self._engine._ctx, self.handle, _hp(data), _hp(off),
+                                                                        _hp(out)))
+        return out
+
+    def final(self, out: np.ndarray | None = None) -> np.ndarray:
+        """the tags, n x tag_bytes"""
+        return super().final(8 * self.tag_bytes, None, out)
+
+    def update_dev(self, t_data, t_off, t_ct, dev_index: int = 0) -> None:
+        """capy_hasher_encrypt_update_dev on torch's current stream (t_ct may be t_data)"""
+        self._engine._check(self._engine.lib.capy_hasher_encrypt_update_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), t_data.data_ptr(), t_off.data_ptr(),
+            t_ct.data_ptr()))
+
+    def final_dev(self, t_out, dev_index: int = 0):
+        return super().final_dev(t_out, 8 * self.tag_bytes, None, dev_index)
+
+
+class VerifyStream(Hasher):
+    """n signature checks whose messages arrive in pieces (Engine.ed448_verify_stream): update() as Hasher, final()
+    -> (rc, ok) as Engine.ed448_verify."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, n: int, d: int):
+        super().__init__(engine, handle, n, d, True)
+
+    def final(self, ok_out: np.ndarray | None = None) -> tuple[int, np.ndarray]:
+        ok = _out(ok_out, (self.n,), "verify flags")
+        rc = self._engine._check(self._engine.lib.capy_hasher_verify_final(self._engine._ctx, self.handle, _hp(ok)),
+                                 allow=(B.ERR_BAD_POINT,))
+        return rc, ok
+
+    def final_dev(self, t_ok, t_bad=None, dev_index: int = 0):
+        """capy_hasher_verify_final_dev on torch's current stream; t_bad (one int32) gets 1 when a key was off the curve"""
+        self._engine._check(self._engine.lib.capy_hasher_verify_final_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), t_ok.data_ptr(),
+            t_bad.data_ptr() if t_bad is not None else None))
+        return t_ok
+
+
+def _pub_or_key(pub):
+    """(pub_xy112 bytes or None, prepared key handle or None) of a PreparedPublicKey or n x 112 key bytes"""
+    if isinstance(pub, PreparedPublicKey):
+        return None, pub.handle
+    return _u8(pub), None
+
+
 class Engine:
     """One capy_ctx.  devices=None -> current CUDA device."""
 
@@ -312,6 +374,42 @@ class Engine:
         self._check(self.lib.capy_kmac_xof_hasher_new(self._ctx, d, _hp(keys), _hp(key_off), n, _hp(cs_a), len(cs_a),
                                                       C.byref(h)))
         return Hasher(self, h, n, d, True)
+
+    def sponge_encrypt_stream(self, pws, pw_off, nonces, nonce_len: int, d: int, variant: int = B.AE_SHA3) -> EncryptStream:
+        """capy_sponge_encrypt_stream_new: one seal stream per password (blocking); tags of 64 bytes"""
+        pws, pw_off, nonces = _u8(pws), _u64(pw_off), _u8(nonces)
+        n = _need_packed(pws, pw_off, "stream passwords")
+        if len(nonces) != n * nonce_len:
+            raise ValueError(f"sponge_encrypt_stream: need {n} x {nonce_len} nonce bytes")
+        h = C.c_void_p()
+        self._check(self.lib.capy_sponge_encrypt_stream_new(self._ctx, d, variant, _hp(pws), _hp(pw_off), _hp(nonces),
+                                                            nonce_len, n, C.byref(h)))
+        return EncryptStream(self, h, n, d, 64)
+
+    def ed448_key_encrypt_stream(self, pub, k_rand56, d: int) -> tuple[EncryptStream, np.ndarray]:
+        """capy_ed448_key_encrypt_stream_new against n x 112 key bytes or a PreparedPublicKey (blocking) -> (streams with
+        tags of 56 bytes, nonce points Z n x 112).  CapyError(ERR_BAD_POINT) for an off-curve key."""
+        pub_b, key = _pub_or_key(pub)
+        k = _u8(k_rand56)
+        n = len(k) // 56
+        if len(k) != n * 56 or (pub_b is not None and len(pub_b) != n * 112):
+            raise ValueError(f"key_encrypt_stream: k holds {len(k)} bytes, need n x 56 and n x 112 key bytes")
+        z = np.zeros((n, 112), dtype=np.uint8)
+        h = C.c_void_p()
+        self._check(self.lib.capy_ed448_key_encrypt_stream_new(self._ctx, d, _hp(pub_b), key, _hp(k), n, _hp(z),
+                                                               C.byref(h)))
+        return EncryptStream(self, h, n, d, 56), z
+
+    def ed448_verify_stream(self, pub, h56, z_be56, d: int) -> VerifyStream:
+        """capy_ed448_verify_stream_new against n x 112 key bytes or a PreparedPublicKey (blocking)"""
+        pub_b, key = _pub_or_key(pub)
+        hb, zb = _u8(h56), _u8(z_be56)
+        n = len(hb) // 56
+        if len(hb) != n * 56 or len(zb) != n * 56 or (pub_b is not None and len(pub_b) != n * 112):
+            raise ValueError(f"verify_stream: h/z hold {len(hb)}/{len(zb)} bytes, need n x 56 and n x 112 key bytes")
+        h = C.c_void_p()
+        self._check(self.lib.capy_ed448_verify_stream_new(self._ctx, d, _hp(pub_b), key, _hp(hb), _hp(zb), n, C.byref(h)))
+        return VerifyStream(self, h, n, d)
 
     def ed448_fixed_base(self, scalars_be56, out: np.ndarray | None = None) -> np.ndarray:
         sc = _u8(scalars_be56)

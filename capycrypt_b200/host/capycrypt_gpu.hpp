@@ -162,6 +162,30 @@ class Hasher {
     return res;
   }
 
+  // encryption streams (Engine::sha3_encrypt_stream / key_encrypt_stream): the ciphertext of pieces[i] for every stream;
+  // final(512) (sponge AE) or final(448) (key_encrypt) then returns the tags
+  std::vector<Bytes> encrypt_update(const std::vector<Bytes>& pieces) {
+    if (pieces.size() != n_) throw GpuError(CAPY_ERR_BAD_ARG, "Hasher::encrypt_update: one piece per stream");
+    Bytes data;
+    std::vector<uint64_t> off;
+    detail::pack(pieces, [](const Bytes& b) -> const Bytes& { return b; }, data, off);
+    Bytes ct(data.size());
+    check(capy_hasher_encrypt_update(ctx_, h_, data.data(), off.data(), ct.data()));
+    std::vector<Bytes> res(n_);
+    for (size_t i = 0; i < n_; i++) res[i].assign(ct.begin() + off[i], ct.begin() + off[i + 1]);
+    return res;
+  }
+
+  // verification streams (Engine::verify_stream): ok per stream; *bad_point = a key was off the curve
+  Bytes verify_final(bool* bad_point = nullptr) {
+    Bytes ok(n_ + 1);
+    const int rc = capy_hasher_verify_final(ctx_, h_, ok.data());
+    if (rc != CAPY_ERR_BAD_POINT) check(rc);
+    if (bad_point) *bad_point = rc == CAPY_ERR_BAD_POINT;
+    ok.resize(n_);
+    return ok;
+  }
+
  private:
   friend class Engine;
   Hasher(capy_ctx* ctx, capy_hasher* h, size_t n, int d_bits) : ctx_(ctx), h_(h), n_(n), d_bits_(d_bits) {}
@@ -238,6 +262,51 @@ class Engine {
     check(capy_kmac_xof_hasher_new(ctx_, d_bits, kd.data(), ko.data(), keys.size(),
                                    reinterpret_cast<const uint8_t*>(s.data()), (uint32_t)s.size(), &h));
     return Hasher(ctx_, h, keys.size(), d_bits);
+  }
+
+  // sha3_encrypt of plaintexts fed in pieces (Hasher::encrypt_update, then final(512) for the tags): one stream per
+  // password, nonces[i] its 512-byte z (blocking); d_bits = 224 is refused (CAPY_ERR_BAD_ARG)
+  Hasher sha3_encrypt_stream(const std::vector<Bytes>& pws, const std::vector<Bytes>& nonces, int d_bits) {
+    Bytes pd, zs;
+    std::vector<uint64_t> po;
+    detail::pack(pws, [](const Bytes& b) -> const Bytes& { return b; }, pd, po);
+    for (const Bytes& z : nonces) {
+      if (z.size() != 512) throw GpuError(CAPY_ERR_BAD_ARG, "sha3_encrypt_stream: 512-byte nonces");
+      zs.insert(zs.end(), z.begin(), z.end());
+    }
+    if (nonces.size() != pws.size()) throw GpuError(CAPY_ERR_BAD_ARG, "sha3_encrypt_stream: one nonce per password");
+    zs.push_back(0);
+    capy_hasher* h = nullptr;
+    check(capy_sponge_encrypt_stream_new(ctx_, d_bits, CAPY_AE_SHA3, pd.data(), po.data(), zs.data(), 512, pws.size(), &h));
+    return Hasher(ctx_, h, pws.size(), d_bits);
+  }
+
+  // key_encrypt of plaintexts fed in pieces to one prepared key (then final(448) for the tags); z[i] <- Z_i (blocking)
+  Hasher key_encrypt_stream(const PreparedPublicKey& key, const std::vector<std::array<uint8_t, 56>>& k_rand, int d_bits,
+                            std::vector<AffinePoint>& z) {
+    const size_t n = k_rand.size();
+    Bytes ks(n * 56 + 1), zb(n * 112 + 1);
+    for (size_t i = 0; i < n; i++) std::copy(k_rand[i].begin(), k_rand[i].end(), ks.begin() + 56 * i);
+    capy_hasher* h = nullptr;
+    check(capy_ed448_key_encrypt_stream_new(ctx_, d_bits, nullptr, key.raw(), ks.data(), n, zb.data(), &h));
+    z.resize(n);
+    for (size_t i = 0; i < n; i++) std::copy(zb.begin() + 112 * i, zb.begin() + 112 * (i + 1), z[i].begin());
+    return Hasher(ctx_, h, n, d_bits);
+  }
+
+  // verify of messages fed in pieces (Hasher::update, then Hasher::verify_final) against one prepared key (blocking)
+  Hasher verify_stream(const std::vector<Signature>& sigs, const PreparedPublicKey& key, int d_bits) {
+    Bytes h, z;
+    for (const Signature& s : sigs) {
+      if (s.h.size() != 56) throw GpuError(CAPY_ERR_BAD_ARG, "verify_stream: 56-byte h");
+      h.insert(h.end(), s.h.begin(), s.h.end());
+      z.insert(z.end(), s.z.begin(), s.z.end());
+    }
+    h.push_back(0);
+    z.push_back(0);
+    capy_hasher* hs = nullptr;
+    check(capy_ed448_verify_stream_new(ctx_, d_bits, nullptr, key.raw(), h.data(), z.data(), sigs.size(), &hs));
+    return Hasher(ctx_, hs, sigs.size(), d_bits);
   }
 
   // KeyPair::new for every password

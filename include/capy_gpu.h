@@ -335,6 +335,38 @@ int capy_hasher_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* st
  * capy_gpu_destroy of its ctx. */
 void capy_hasher_free(capy_hasher* h);
 
+/* ---- Encrypting and verifying in pieces ------------------------------------------------------------------------------
+ * Two more kinds of hasher, for the operators that read their message once.  The concatenated pieces give, byte for
+ * byte, what the one-shot calls give.  Sign and the decryptions stay one-shot: sign reads the message twice, and a
+ * decryption must not release plaintext before the tag is checked.
+ *  - encryption streams (sha3_encrypt, the KEM symmetric half, key_encrypt): each stream holds the tag sponge, a KMAC
+ *    stream keyed by ka, and the keystream sponge KMACXOF(ke, "", ., KE), whose first |m| bytes do not depend on |m|.
+ *    ke || ka is derived on the device and never leaves it.  capy_hasher_encrypt_update writes the ciphertext of each
+ *    piece at the piece's own offsets; capy_hasher_final with out_bits = 512 (sponge AE) or 448 (key_encrypt) and no
+ *    out_off returns the tags.  capy_hasher_update on an encryption stream: CAPY_ERR_BAD_ARG.
+ *  - verification streams: U' = [z]G + [h]V is computed at creation, the message goes through capy_hasher_update, and
+ *    capy_hasher_verify_final compares h' with h.  capy_hasher_final on a verification stream: CAPY_ERR_BAD_ARG.
+ *  - d_bits = 224 is refused (CAPY_ERR_BAD_ARG) for both kinds: the message is absorbed at the 172-byte KMAC rate, as in
+ *    capy_kmac_xof_hasher_new.  The one-shot D224 calls are unaffected.
+ *  - a prepared key of another ctx, both or neither of pub_xy112 and key: CAPY_ERR_BAD_ARG. */
+/* sponge AE seal streams (variant CAPY_AE_SHA3 | CAPY_AE_KEM); nonces: n * nonce_len bytes; blocking */
+int capy_sponge_encrypt_stream_new(capy_ctx* ctx, int d_bits, int variant, const uint8_t* pws, const uint64_t* pw_off,
+                                   const uint8_t* nonces, uint64_t nonce_len, uint64_t n, capy_hasher** out);
+/* key_encrypt seal streams against n keys pub_xy112 or one prepared key; z_xy112 <- Z_i = [k_i]G; blocking.  An off-curve
+ * V_i: CAPY_ERR_BAD_POINT and no stream. */
+int capy_ed448_key_encrypt_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112, const capy_ed448_pub* key,
+                                      const uint8_t* k_rand56, uint64_t n, uint8_t* z_xy112, capy_hasher** out);
+/* verification streams against n keys pub_xy112 or one prepared key; blocking.  An off-curve V_i is reported by the final. */
+int capy_ed448_verify_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pub_xy112, const capy_ed448_pub* key,
+                                 const uint8_t* h56, const uint8_t* z_be56, uint64_t n, capy_hasher** out);
+/* ct[off[i] .. off[i+1]) = keystream ^ data[off[i] .. off[i+1]); ct may alias data */
+int capy_hasher_encrypt_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off, uint8_t* ct);
+int capy_hasher_encrypt_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_data,
+                                   const uint64_t* d_off, uint8_t* d_ct);
+/* ok[i] = 1 iff h' == h and V_i is on the curve; CAPY_ERR_BAD_POINT if any V_i was off the curve (_dev: *d_bad_flag |= 1) */
+int capy_hasher_verify_final(capy_ctx* ctx, capy_hasher* h, uint8_t* ok);
+int capy_hasher_verify_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag);
+
 #ifdef __cplusplus
 }
 #endif

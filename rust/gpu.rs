@@ -147,6 +147,19 @@ extern "C" {
     fn capy_hasher_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
         out_bits: u64, d_out_off: *const u64, d_out: *mut u8) -> c_int;
     fn capy_hasher_free(h: *mut CapyHasher);
+    fn capy_sponge_encrypt_stream_new(ctx: *mut CapyCtx, d_bits: c_int, variant: c_int, pws: *const u8,
+        pw_off: *const u64, nonces: *const u8, nonce_len: u64, n: u64, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_ed448_key_encrypt_stream_new(ctx: *mut CapyCtx, d_bits: c_int, pub_xy112: *const u8,
+        key: *const CapyEd448Pub, k_rand56: *const u8, n: u64, z_xy112: *mut u8, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_ed448_verify_stream_new(ctx: *mut CapyCtx, d_bits: c_int, pub_xy112: *const u8, key: *const CapyEd448Pub,
+        h56: *const u8, z_be56: *const u8, n: u64, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_hasher_encrypt_update(ctx: *mut CapyCtx, h: *mut CapyHasher, data: *const u8, off: *const u64,
+        ct: *mut u8) -> c_int;
+    fn capy_hasher_encrypt_update_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_data: *const u8, d_off: *const u64, d_ct: *mut u8) -> c_int;
+    fn capy_hasher_verify_final(ctx: *mut CapyCtx, h: *mut CapyHasher, ok: *mut u8) -> c_int;
+    fn capy_hasher_verify_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_ok: *mut u8, d_bad_flag: *mut c_int) -> c_int;
 }
 
 const CAPY_AE_SHA3: c_int = 0;
@@ -596,6 +609,132 @@ impl Gpu {
                                      s.len() as u32, &mut h)
         })?;
         Ok(Hasher { ctx: self.ctx, h, n: keys.len() })
+    }
+}
+
+/// Encryption streams (`Gpu::sha3_encrypt_stream`, `Gpu::key_encrypt_stream_prepared`): `update` returns the ciphertext of
+/// one piece per message, `finish` the tags; together they are the `.msg` and `.digest` of the one-shot call on the
+/// concatenated plaintext.  `nonces` holds each message's `sym_nonce` (512 bytes) or `asym_nonce` (Z, affine x || y).
+/// Drop it before the `Gpu` that created it.
+pub struct EncryptStream {
+    ctx: *mut CapyCtx,
+    h: *mut CapyHasher,
+    n: usize,
+    tag_bytes: usize,
+    pub nonces: Vec<Vec<u8>>,
+}
+unsafe impl Send for EncryptStream {}
+
+impl EncryptStream {
+    pub fn update(&mut self, pieces: &[&[u8]]) -> Result<Vec<Vec<u8>>, OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        let mut ct = vec![0u8; data.len()];
+        status(unsafe { capy_hasher_encrypt_update(self.ctx, self.h, data.as_ptr(), off.as_ptr(), ct.as_mut_ptr()) })?;
+        Ok((0..self.n).map(|i| ct[off[i] as usize..off[i + 1] as usize].to_vec()).collect())
+    }
+
+    /// The tags (64 bytes for sha3_encrypt, 56 for key_encrypt).  The streams are finished after it.
+    pub fn finish(&mut self) -> Result<Vec<Vec<u8>>, OperationError> {
+        let tb = self.tag_bytes;
+        let mut out = vec![0u8; self.n * tb + 1];
+        status(unsafe { capy_hasher_final(self.ctx, self.h, 8 * tb as u64, std::ptr::null(), out.as_mut_ptr()) })?;
+        Ok((0..self.n).map(|i| out[i * tb..(i + 1) * tb].to_vec()).collect())
+    }
+}
+
+impl Drop for EncryptStream {
+    fn drop(&mut self) {
+        unsafe { capy_hasher_free(self.h) }
+    }
+}
+
+/// Verification streams (`Gpu::verify_stream_prepared`): `update` appends one piece per message, `finish` gives what
+/// `verify_prepared` gives for the concatenated pieces.  Drop it before the `Gpu` that created it.
+pub struct VerifyStream {
+    ctx: *mut CapyCtx,
+    h: *mut CapyHasher,
+    n: usize,
+}
+unsafe impl Send for VerifyStream {}
+
+impl VerifyStream {
+    pub fn update(&mut self, pieces: &[&[u8]]) -> Result<(), OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        status(unsafe { capy_hasher_update(self.ctx, self.h, data.as_ptr(), off.as_ptr()) })
+    }
+
+    pub fn finish(&mut self) -> Vec<Result<(), OperationError>> {
+        let mut ok = vec![0u8; self.n + 1];
+        let rc = unsafe { capy_hasher_verify_final(self.ctx, self.h, ok.as_mut_ptr()) };
+        (0..self.n)
+            .map(|i| if rc != 0 || ok[i] == 0 { Err(OperationError::SignatureVerificationFailure) } else { Ok(()) })
+            .collect()
+    }
+}
+
+impl Drop for VerifyStream {
+    fn drop(&mut self) {
+        unsafe { capy_hasher_free(self.h) }
+    }
+}
+
+impl Gpu {
+    /// One `sha3_encrypt` per password whose plaintext arrives in pieces (blocking); the 512 nonce bytes per message are
+    /// drawn with the reference's `get_random_bytes`.  D224 is refused (capy_gpu.h: quirk Q7).
+    pub fn sha3_encrypt_stream(&self, pws: &[&[u8]], d: SecParam) -> Result<EncryptStream, OperationError> {
+        use crate::sha3::aux_functions::byte_utils::get_random_bytes;
+        let n = pws.len();
+        let nonces: Vec<Vec<u8>> = (0..n).map(|_| get_random_bytes(512)).collect();
+        let z: Vec<u8> = nonces.iter().flatten().copied().collect();
+        let (pd, po) = pack(pws.iter().copied());
+        let mut h = std::ptr::null_mut();
+        status(unsafe {
+            capy_sponge_encrypt_stream_new(self.ctx, d as c_int, CAPY_AE_SHA3, pd.as_ptr(), po.as_ptr(), z.as_ptr(), 512,
+                                           n as u64, &mut h)
+        })?;
+        Ok(EncryptStream { ctx: self.ctx, h, n, tag_bytes: 64, nonces })
+    }
+
+    /// n `key_encrypt`s to one prepared key whose plaintexts arrive in pieces (blocking); `nonces` holds each Z.
+    pub fn key_encrypt_stream_prepared(&self, n: usize, key: &PreparedKey, d: SecParam)
+                                       -> Result<EncryptStream, OperationError> {
+        use crate::sha3::aux_functions::byte_utils::get_random_bytes;
+        let k_rand: Vec<u8> = (0..n).flat_map(|_| get_random_bytes(56)).collect();
+        let mut z = vec![0u8; n * 112 + 1];
+        let mut h = std::ptr::null_mut();
+        status(unsafe {
+            capy_ed448_key_encrypt_stream_new(self.ctx, d as c_int, std::ptr::null(), key.key, k_rand.as_ptr(), n as u64,
+                                              z.as_mut_ptr(), &mut h)
+        })?;
+        let nonces = (0..n).map(|i| z[112 * i..112 * (i + 1)].to_vec()).collect();
+        Ok(EncryptStream { ctx: self.ctx, h, n, tag_bytes: 56, nonces })
+    }
+
+    /// `verify_prepared` of signatures whose messages arrive in pieces (blocking).
+    pub fn verify_stream_prepared(&self, sigs: &[Signature], key: &PreparedKey, d: SecParam)
+                                  -> Result<VerifyStream, OperationError> {
+        let (mut h, mut z) = (Vec::new(), Vec::new());
+        for sig in sigs {
+            if sig.h.len() != 56 {
+                return Err(OperationError::SignatureVerificationFailure);
+            }
+            h.extend_from_slice(&sig.h);
+            z.extend_from_slice(&sig.z.val.to_be_bytes());
+        }
+        h.push(0);
+        z.push(0);
+        let mut hs = std::ptr::null_mut();
+        status(unsafe {
+            capy_ed448_verify_stream_new(self.ctx, d as c_int, std::ptr::null(), key.key, h.as_ptr(), z.as_ptr(),
+                                         sigs.len() as u64, &mut hs)
+        })?;
+        Ok(VerifyStream { ctx: self.ctx, h: hs, n: sigs.len() })
     }
 }
 
