@@ -98,6 +98,17 @@ SIGNATURES = {
     "capy_hasher_encrypt_update_dev": (i32, [vp, vp, i32, vp, u8p, u64p, u8p]),
     "capy_hasher_verify_final": (i32, [vp, vp, u8p]),
     "capy_hasher_verify_final_dev": (i32, [vp, vp, i32, vp, u8p, vp]),
+    "capy_ed448_sign_stream_new": (i32, [vp, i32, u8p, u64p, u64, C.POINTER(vp)]),
+    "capy_sponge_decrypt_stream_new": (i32, [vp, i32, i32, u8p, u64p, u8p, u64, u8p, u64, C.POINTER(vp)]),
+    "capy_ed448_key_decrypt_stream_new": (i32, [vp, i32, u8p, u64p, u8p, u8p, u64, C.POINTER(vp)]),
+    "capy_hasher_next_pass": (i32, [vp, vp, u8p]),
+    "capy_hasher_next_pass_dev": (i32, [vp, vp, i32, vp, u8p, vp]),
+    "capy_hasher_decrypt_update": (i32, [vp, vp, u8p, u64p, u8p]),
+    "capy_hasher_decrypt_update_dev": (i32, [vp, vp, i32, vp, u8p, u64p, u8p]),
+    "capy_hasher_decrypt_final": (i32, [vp, vp, u8p]),
+    "capy_hasher_decrypt_final_dev": (i32, [vp, vp, i32, vp, u8p, vp]),
+    "capy_hasher_sign_final": (i32, [vp, vp, u8p, u8p, u8p]),
+    "capy_hasher_sign_final_dev": (i32, [vp, vp, i32, vp, u8p, u8p, u8p]),
 }
 
 

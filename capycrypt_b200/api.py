@@ -202,6 +202,49 @@ class Gpu:
         pub = pub_keys if prepared else b"".join(pub_keys[i] for i in idx)
         return VerifyStream(self.engine.ed448_verify_stream(pub, h, z, int(d)), idx, res)
 
+    # ---- messages fed twice in pieces -------------------------------------------------------------------
+    def sign_stream(self, keys: Sequence[KeyPair] | Sequence[bytes], d: SecParam) -> "SignStream":
+        """one sign() per key pair (or password) whose message is fed twice: update() in pass 1, next_pass(), the same
+        bytes again through update(), then finish() -> a Signature per message, as sign() gives for the concatenated
+        pieces, or OperationError("OperationResultNotSet") where pass 2 carried other bytes than pass 1.  D224 is refused
+        (ValueError)."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("sign_stream: D224 is not resumable (quirk Q7)")
+        pd, po = pack([k.priv_key if isinstance(k, KeyPair) else bytes(k) for k in keys])
+        return SignStream(self.engine.ed448_sign_stream(pd, po, int(d)))
+
+    def sha3_decrypt_stream(self, pws: Sequence[bytes], nonces: Sequence[bytes], tags: Sequence[bytes],
+                            d: SecParam) -> "DecryptStream":
+        """one sha3_decrypt per password whose ciphertext is fed twice: update() in pass 1 releases nothing, next_pass()
+        gives the verdicts (None or SHA3DecryptionFailure), decrypt() takes the same bytes again and returns the plaintext
+        pieces (the ciphertext for a failed message), finish() the final result, which also checks that both passes
+        carried the same bytes.  All nonces have one length.  D224 is refused (ValueError)."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("sha3_decrypt_stream: D224 is not resumable (quirk Q7)")
+        nl = len(nonces[0]) if nonces else 0
+        if len(nonces) != len(pws) or len(tags) != len(pws) or any(len(z) != nl for z in nonces):
+            raise ValueError("sha3_decrypt_stream: one nonce (all of one length) and one tag per password")
+        pd, po = pack(pws)
+        tb = b"".join(bytes(t).ljust(64, b"\0")[:64] for t in tags)
+        st = self.engine.sponge_decrypt_stream(pd, po, b"".join(nonces), nl, tb, int(d))
+        return DecryptStream(st, "SHA3DecryptionFailure", [len(t) != 64 for t in tags])
+
+    def key_decrypt_stream(self, pws: Sequence[bytes], asym_nonces: Sequence[bytes], tags: Sequence[bytes],
+                           d: SecParam) -> "DecryptStream":
+        """as sha3_decrypt_stream for key_decrypt: asym_nonces are the Z of the messages (112 bytes each); failures are
+        KeyDecryptionError, an off-curve Z included."""
+        d = SecParam.try_from(int(d))
+        if d == SecParam.D224:
+            raise ValueError("key_decrypt_stream: D224 is not resumable (quirk Q7)")
+        if len(asym_nonces) != len(pws) or len(tags) != len(pws) or any(len(z) != 112 for z in asym_nonces):
+            raise ValueError("key_decrypt_stream: one 112-byte Z and one tag per password")
+        pd, po = pack(pws)
+        tb = b"".join(bytes(t).ljust(56, b"\0")[:56] for t in tags)
+        st = self.engine.ed448_key_decrypt_stream(pd, po, b"".join(asym_nonces), tb, int(d))
+        return DecryptStream(st, "KeyDecryptionError", [len(t) != 56 for t in tags])
+
     # ---- KeyPair::new ----------------------------------------------------------------------------------
     def new_keypairs(self, pws: Sequence[bytes], owner: str, d: SecParam) -> list[KeyPair]:
         d = SecParam.try_from(int(d))
@@ -471,6 +514,70 @@ class VerifyStream:
             if not o:
                 self.res[i] = OperationError("SignatureVerificationFailure")
         return self.res
+
+    def close(self) -> None:
+        self.stream.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class SignStream:
+    """Streams of Gpu.sign_stream: update() one piece per message in each pass, next_pass() between the passes,
+    finish() the signatures."""
+
+    def __init__(self, stream):
+        self.stream = stream
+
+    def update(self, pieces: Sequence[bytes]) -> None:
+        self.stream.update(*pack(pieces))
+
+    def next_pass(self) -> None:
+        self.stream.next_pass()
+
+    def finish(self) -> list[Signature | OperationError]:
+        h, z, ok = self.stream.final()
+        return [Signature(h=hr.tobytes(), z=zr.tobytes()) if o else OperationError("OperationResultNotSet")
+                for hr, zr, o in zip(h, z, ok)]
+
+    def close(self) -> None:
+        self.stream.close()
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, *exc):
+        self.close()
+
+
+class DecryptStream:
+    """Streams of Gpu.sha3_decrypt_stream / Gpu.key_decrypt_stream: update() the ciphertext pieces of pass 1,
+    next_pass() -> verdicts, decrypt() the same pieces again -> plaintext pieces, finish() -> the results."""
+
+    def __init__(self, stream, error: str, bad_tag: list[bool]):
+        self.stream = stream
+        self.error = error
+        self.bad_tag = bad_tag  # a tag of the wrong length fails, as in the one-shot calls
+
+    def _results(self, ok) -> list[Optional[OperationError]]:
+        return [None if o and not b else OperationError(self.error) for o, b in zip(ok, self.bad_tag)]
+
+    def update(self, pieces: Sequence[bytes]) -> None:
+        self.stream.update(*pack(pieces))
+
+    def next_pass(self) -> list[Optional[OperationError]]:
+        return self._results(self.stream.next_pass()[1])
+
+    def decrypt(self, pieces: Sequence[bytes]) -> list[bytes]:
+        data, off = pack(pieces)
+        out = self.stream.decrypt(data, off)
+        return [out[int(off[i]):int(off[i + 1])].tobytes() for i in range(len(pieces))]
+
+    def finish(self) -> list[Optional[OperationError]]:
+        return self._results(self.stream.final()[1])
 
     def close(self) -> None:
         self.stream.close()

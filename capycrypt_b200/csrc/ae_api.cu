@@ -33,18 +33,20 @@ __global__ void __launch_bounds__(256) ae_concat_kernel(const uint8_t* __restric
   for (uint64_t k = lane; k < b - a; k += 32) keys[o + nonce_len + k] = pws[a + k];
 }
 
-// ok[i] = (t'_i == t_i) [&& !bad[i]]; on failure the output buffer of item i gets the ciphertext back.
+// ok[i] = (t'_i == t_i) [&& !bad[i]] [&& ok_in[i]]; on failure the output buffer of item i gets the ciphertext back.
 // one warp per item
 __global__ void __launch_bounds__(256) ae_finish_kernel(const uint8_t* __restrict__ t_new, const uint8_t* __restrict__ t_in,
                                                         uint32_t tag_bytes, const uint8_t* __restrict__ bad,
                                                         const uint8_t* __restrict__ ct, const uint64_t* __restrict__ off,
-                                                        uint8_t* __restrict__ out, uint8_t* __restrict__ ok, uint64_t n) {
+                                                        uint8_t* __restrict__ out, uint8_t* __restrict__ ok, uint64_t n,
+                                                        const uint8_t* __restrict__ ok_in) {
   const uint64_t i = ((uint64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const uint32_t lane = threadIdx.x & 31u;
   if (i >= n) return;
   uint32_t diff = 0;
   for (uint32_t k = lane; k < tag_bytes; k += 32) diff |= (uint32_t)(t_new[i * tag_bytes + k] ^ t_in[i * tag_bytes + k]);
   if (bad && bad[i]) diff = 1;
+  if (ok_in && !ok_in[i]) diff = 1;
   const bool good = !__any_sync(0xffffffffu, diff != 0);
   if (lane == 0) ok[i] = good ? 1 : 0;
   if (!good && out != ct) {
@@ -111,7 +113,7 @@ static int dev_ae_open(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const AeCo
   // the tag pass reads what the keystream pass writes: dependent jobs of one launch when the batch is large enough
   int rc = launch_kmac_xof_dep(ctx, dc, st, k, a);
   if (rc) return rc;
-  ae_finish_kernel<<<grid_for(n * 32, 256), 256, 0, st>>>(t_new, tag, c.tag_bytes, bad, ct, off, out, ok, n);
+  ae_finish_kernel<<<grid_for(n * 32, 256), 256, 0, st>>>(t_new, tag, c.tag_bytes, bad, ct, off, out, ok, n, nullptr);
   ctx->launches++;
   CAPY_CUDA(ctx, cudaGetLastError());
   return CAPY_OK;
@@ -277,9 +279,11 @@ static int dev_key_encrypt_prepared(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t s
   return key_encrypt_finish(ctx, dc, st, d, kw, wx, msgs, off, n, ct, tag, z_xy, keymat_out);
 }
 
+// With keymat_out, no ciphertext: (ke || ka) and the off-curve flags are handed back for a decryption stream instead.
 static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const uint8_t* pws, const uint64_t* pw_off,
                            const uint8_t* z_xy, const uint8_t* ct, const uint64_t* off, const uint8_t* tag, uint64_t n,
-                           uint8_t* out, uint8_t* ok, int* d_bad_flag) {
+                           uint8_t* out, uint8_t* ok, int* d_bad_flag, uint8_t** keymat_out = nullptr,
+                           const uint8_t** bad_out = nullptr) {
   if (!valid_secparam(d)) return CAPY_ERR_BAD_SECPARAM;
   if (n == 0) return CAPY_OK;
   CAPY_SCRATCH(proj, uint32_t, kAeProj, n * 256);
@@ -304,6 +308,11 @@ static int dev_key_decrypt(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d,
   uint8_t* keymat;
   rc = dev_ecdhies_keymat(ctx, dc, st, d, wx, n, &keymat);
   if (rc) return rc;
+  if (keymat_out) {
+    *keymat_out = keymat;
+    *bad_out = bad;
+    return CAPY_OK;
+  }
   rc = dev_ae_open(ctx, dc, st, ecdhies_core(d, keymat), ct, off, tag, bad, n, out, ok, t_new);
   if (rc) return rc;
   return d_bad_flag ? launch_any_bad(ctx, st, bad, d_bad_flag, n) : CAPY_OK;
@@ -323,6 +332,43 @@ static int ae_stream_start(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const 
   k.job.key_len = c.klen;
   k.job.key_stride = 2ull * c.klen;
   return launch_kmac_state(ctx, dc, st, k, true, h->d_ks_state[dc.index]);
+}
+
+// A decryption stream after ae_stream_start: keeps both start states for pass 2, the expected tags and the off-curve flags
+static int decrypt_stream_keep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, const uint8_t* d_tag,
+                               const uint8_t* bad, uint64_t n) {
+  const int k = dc.index;
+  CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_state0[k], h->d_state[k], n * 200, cudaMemcpyDeviceToDevice, st));
+  CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_ks_state0[k], h->d_ks_state[k], n * 200, cudaMemcpyDeviceToDevice, st));
+  CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_h[k], d_tag, n * (h->tag_bits / 8), cudaMemcpyDeviceToDevice, st));
+  if (bad) CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_bad[k], bad, n, cudaMemcpyDeviceToDevice, st));
+  return CAPY_OK;
+}
+
+// The tag over the plaintext of the pass that just ended, compared with the expected tag (ae_finish_kernel, no restore).
+// Pass 1: the verdict goes to d_verdict (and d_ok), and both sponges go back to their start states.  Pass 2: ok = the
+// verdict && this comparison.  key_decrypt: an off-curve Z_i fails, and sets *d_bad_flag as the one-shot call does.
+int decrypt_stream_check(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, bool second, uint8_t* d_ok,
+                         int* d_bad_flag) {
+  const int k = dc.index;
+  const uint64_t m = h->first[k + 1] - h->first[k];
+  const uint32_t tb = h->tag_bits / 8;
+  CAPY_SCRATCH(t_new, uint8_t, kAeTNew, m * tb);
+  int rc = hasher_final_items(ctx, dc, st, h, 0, m, tb, nullptr, t_new);
+  if (rc) return rc;
+  uint8_t* ok = second ? d_ok : h->d_verdict[k];
+  ae_finish_kernel<<<grid_for(m * 32, 256), 256, 0, st>>>(t_new, h->d_h[k], tb, h->d_bad[k], nullptr, nullptr, nullptr, ok, m,
+                                                          second ? h->d_verdict[k] : nullptr);
+  ctx->launches++;
+  CAPY_CUDA(ctx, cudaGetLastError());
+  if (!second) {
+    if (d_ok) CAPY_CUDA(ctx, cudaMemcpyAsync(d_ok, ok, m, cudaMemcpyDeviceToDevice, st));
+    CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_state[k], h->d_state0[k], m * 200, cudaMemcpyDeviceToDevice, st));
+    CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_ks_state[k], h->d_ks_state0[k], m * 200, cudaMemcpyDeviceToDevice, st));
+    rc = hasher_restart(ctx, dc, st, h);
+    if (rc) return rc;
+  }
+  return h->d_bad[k] && d_bad_flag ? launch_any_bad(ctx, st, h->d_bad[k], d_bad_flag, m) : CAPY_OK;
 }
 
 }  // namespace capy
@@ -513,6 +559,88 @@ int capy_sponge_encrypt_stream_new(capy_ctx* ctx, int d_bits, int variant, const
     cc.keymat = keymat;
     cc.klen = 64;  // ke_ka.split_at(64)
     return ae_stream_start(ctx, dc, st, cc, h, io.n());
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+// Decryption streams: (ke || ka) as capy_sponge_decrypt_batch derives it, the sponges of ae_stream_start, and the expected
+// tags (one chunk per device: the states are stored at [l * items + j])
+int capy_sponge_decrypt_stream_new(capy_ctx* ctx, int d_bits, int variant, const uint8_t* pws, const uint64_t* pw_off,
+                                   const uint8_t* nonces, uint64_t nonce_len, const uint8_t* tag64, uint64_t n,
+                                   capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  AeCore c{};
+  if (!ctx || (n && (!pws || !pw_off || !nonces || !tag64)) || !ae_customs(variant, &c.ke_custom, &c.ka_custom))
+    return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // the tag stream absorbs at the 172-byte rate (Q7): see the header
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kDecryptStream, n, &h, 512);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    const StagedPacked sp = io.in_packed(pws, pw_off);
+    const uint8_t* d_nonce = io.in(nonces, nonce_len);
+    const uint8_t* d_tag = io.in(tag64, 64);
+    if (io.rc()) return io.rc();
+    uint8_t* keymat;
+    int r = dev_sponge_keymat(ctx, dc, st, d_bits, sp.d_base, sp.d_off, pw_off[io.i1()] - pw_off[io.i0()], d_nonce, nonce_len,
+                              io.n(), &keymat);
+    if (r) return r;
+    AeCore cc = c;
+    cc.d = d_bits;
+    cc.keymat = keymat;
+    cc.klen = 64;  // ke_ka.split_at(64)
+    r = ae_stream_start(ctx, dc, st, cc, h, io.n());
+    if (r) return r;
+    return decrypt_stream_keep(ctx, dc, st, h, d_tag, nullptr, io.n());
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+// key_decrypt streams: s, W = [s]Z and (ke || ka) as capy_ed448_key_decrypt_batch computes them; an off-curve Z_i is
+// reported by capy_hasher_next_pass
+int capy_ed448_key_decrypt_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off,
+                                      const uint8_t* z_xy112, const uint8_t* tag56, uint64_t n, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx || (n && (!pws || !pw_off || !z_xy112 || !tag56))) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kDecryptStream, n, &h, 448);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;
+    const StagedPacked sp = io.in_packed(pws, pw_off);
+    const uint8_t* d_z = io.in(z_xy112, 112);
+    const uint8_t* d_tag = io.in(tag56, 56);
+    if (io.rc()) return io.rc();
+    uint8_t* keymat;
+    const uint8_t* bad;
+    int r = dev_key_decrypt(ctx, dc, st, d_bits, sp.d_base, sp.d_off, d_z, nullptr, nullptr, nullptr, io.n(), nullptr, nullptr,
+                            nullptr, &keymat, &bad);
+    if (r) return r;
+    r = ae_stream_start(ctx, dc, st, ecdhies_core(d_bits, keymat), h, io.n());
+    if (r) return r;
+    return decrypt_stream_keep(ctx, dc, st, h, d_tag, bad, io.n());
   });
   if (rc) {
     capy_hasher_free(h);

@@ -31,13 +31,18 @@ __global__ void __launch_bounds__(128) scalar_prep_kernel(const uint8_t* __restr
   if (out_be56) sc_to_be(out_be56 + 56 * i, o);
 }
 
-// z = k - (BE(h) * s mod r) mod r   (ecc/signable.rs:52-54)
+// z = k - (BE(h) * s mod r) mod r   (ecc/signable.rs:52-54).  With `keep` (sign streams), an item with keep[i] == 0 gets
+// h = z = 0: nothing derived from its k leaves the device.
 __global__ void __launch_bounds__(128) sign_finish_kernel(const uint32_t* __restrict__ k_words,
                                                           const uint32_t* __restrict__ s_words,
-                                                          const uint8_t* __restrict__ h56, uint8_t* __restrict__ z_be56,
-                                                          uint64_t n) {
+                                                          uint8_t* __restrict__ h56, uint8_t* __restrict__ z_be56,
+                                                          uint64_t n, const uint8_t* __restrict__ keep) {
   const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= n) return;
+  if (keep && !keep[i]) {
+    for (int j = 0; j < 56; j++) h56[56 * i + j] = z_be56[56 * i + j] = 0;
+    return;
+  }
   Sc k, s, h, hs, z;
 #pragma unroll
   for (int j = 0; j < 14; j++) {
@@ -258,7 +263,7 @@ static int dev_sign(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, int d, const 
   rc = launch_kmac_xof(ctx, dc, st, h);
   if (rc) return rc;
   // z = k - h * s mod r (:52-54)
-  sign_finish_kernel<<<grid_for(n, 128), 128, 0, st>>>(kw, sw, d_h, d_z, n);
+  sign_finish_kernel<<<grid_for(n, 128), 128, 0, st>>>(kw, sw, d_h, d_z, n, nullptr);
   ctx->launches++;
   CAPY_CUDA(ctx, cudaGetLastError());
   return CAPY_OK;
@@ -463,6 +468,52 @@ static std::vector<Range> ed_chunks(Range sh) {
   const uint64_t items = sh.i1 - sh.i0;
   const size_t count = items < (1ull << 19) ? 1 : (size_t)std::min<uint64_t>(8, items >> 18);
   return split_items(nullptr, 1, sh.i0, sh.i1, count, 0);
+}
+
+// End of pass 1 as dev_sign goes on after its "N" pass: N1 -> k = 4 * BE(N1) mod r, U = [k]G, then the "T" stream keyed by
+// U.x and a second "N" stream keyed by BE56(s), both from the first byte again
+int sign_stream_next(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h) {
+  const int k = dc.index;
+  const uint64_t m = h->first[k + 1] - h->first[k];
+  CAPY_SCRATCH(proj, uint32_t, kEdProj, m * 256);
+  CAPY_SCRATCH(ux, uint8_t, kEdTmp56A, m * 56);
+  int rc = hasher_final_items(ctx, dc, st, h, 0, m, 56, nullptr, h->d_n1[k]);
+  if (rc) return rc;
+  rc = launch_scalar_prep(ctx, st, h->d_n1[k], 1, h->d_k[k], nullptr, m);
+  if (rc) return rc;
+  rc = launch_fixed_base(ctx, dc, st, h->d_k[k], proj, m, true);
+  if (rc) return rc;
+  rc = launch_to_affine(ctx, st, proj, m, 1, nullptr, ux);
+  if (rc) return rc;
+  KmacPass t(h->d_bits, "T", m);
+  t.job.keys = ux;
+  t.job.key_stride = t.job.key_len = 56;
+  rc = launch_kmac_state(ctx, dc, st, t, false, h->d_state[k]);
+  if (rc) return rc;
+  KmacPass n2(h->d_bits, "N", m);
+  n2.job.keys = h->d_s_be[k];
+  n2.job.key_stride = n2.job.key_len = 56;
+  rc = launch_kmac_state(ctx, dc, st, n2, false, h->d_state2[k]);
+  if (rc) return rc;
+  return hasher_restart(ctx, dc, st, h);
+}
+
+// h = the "T" output ; ok = (N2 == N1) ; z = k - h * s mod r where ok, h = z = 0 elsewhere
+int sign_stream_final(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint8_t* d_h, uint8_t* d_z,
+                      uint8_t* d_ok) {
+  const int k = dc.index;
+  const uint64_t m = h->first[k + 1] - h->first[k];
+  CAPY_SCRATCH(n2, uint8_t, kEdTmp56B, m * 56);
+  int rc = hasher_final_items(ctx, dc, st, h, 0, m, 56, nullptr, d_h);
+  if (rc) return rc;
+  rc = hasher_final_items(ctx, dc, st, h, 0, m, 56, nullptr, n2, h->d_state2[k]);
+  if (rc) return rc;
+  rc = launch_verify_compare(ctx, st, n2, h->d_n1[k], nullptr, d_ok, nullptr, m);
+  if (rc) return rc;
+  sign_finish_kernel<<<grid_for(m, 128), 128, 0, st>>>(h->d_k[k], h->d_s[k], d_h, d_z, m, d_ok);
+  ctx->launches++;
+  CAPY_CUDA(ctx, cudaGetLastError());
+  return CAPY_OK;
 }
 
 }  // namespace capy
@@ -691,6 +742,40 @@ int capy_ed448_verify_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pub_x
     if (vs.bad) CAPY_CUDA(ctx, cudaMemcpyAsync(h->d_bad[k], vs.bad, m, cudaMemcpyDeviceToDevice, st));
     KmacPass a(d_bits, "T", m);
     a.job.keys = vs.ux;
+    a.job.key_stride = a.job.key_len = 56;
+    return launch_kmac_state(ctx, dc, st, a, false, h->d_state[k]);
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+// Sign streams: s and the KMAC streams keyed by BE56(s) with S = "N" (one chunk per device: [l * items + j])
+int capy_ed448_sign_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off, uint64_t n,
+                               capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (!ctx || (n && (!pws || !pw_off))) return CAPY_ERR_BAD_ARG;
+  if (!valid_secparam(d_bits)) return CAPY_ERR_BAD_SECPARAM;
+  if (d_bits == 224) return CAPY_ERR_BAD_ARG;  // "N" and "T" absorb at the 172-byte rate (Q7): see the header
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, d_bits, kSignStream, n, &h, 448);
+  if (rc || n == 0) {
+    *out = h;
+    return rc;
+  }
+  rc = run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    const StagedPacked sp = io.in_packed(pws, pw_off);
+    if (io.rc()) return io.rc();
+    const int k = dc.index;
+    const int r = dev_secret_scalar(ctx, dc, st, d_bits, sp.d_base, sp.d_off, io.n(), h->d_s[k], h->d_s_be[k]);
+    if (r) return r;
+    KmacPass a(d_bits, "N", io.n());
+    a.job.keys = h->d_s_be[k];
     a.job.key_stride = a.job.key_len = 56;
     return launch_kmac_state(ctx, dc, st, a, false, h->d_state[k]);
   });

@@ -202,8 +202,21 @@ struct capy_ed448_pub {
 //   d_ks_pos[k]    [j] = keystream bytes used so far
 // Verification streams (capy_ed448_verify_stream_new, ed448_api.cu) are KMAC streams keyed by U'.x with S = "T", and keep
 //   d_h[k]    [j * 56 ..) the signature's h ;  d_bad[k]  [j] = V_j is off the curve
+// Sign and decryption streams read the message twice (capy_hasher_next_pass between the passes; pass[k] = 1 or 2).  Both
+// passes share d_carry and d_total, which the next pass starts from zero.
+// Sign streams (capy_ed448_sign_stream_new, ed448_api.cu): pass 1 is the KMAC stream keyed by BE56(s) with S = "N" in
+// d_state; pass 2 runs the "T" stream keyed by U.x in d_state and the second "N" stream in d_state2 (SpongeDual, dual
+// absorb), and
+//   d_s[k], d_k[k]  14 words at [w * items_k + j]: s and k ;  d_s_be[k]  [j * 56 ..) BE56(s) ;  d_n1[k]  [j * 56 ..) the
+//                   first "N" output
+// Decryption streams (capy_sponge_decrypt_stream_new / capy_ed448_key_decrypt_stream_new, ae_api.cu) hold the tag stream
+// in d_state and the keystream at the start of its current squeeze block in d_ks_state (SpongeDual, open; the keystream
+// position is d_total), and
+//   d_state0[k], d_ks_state0[k]  the two states at creation, where pass 2 starts again
+//   d_h[k]   [j * tag_bits / 8 ..) the expected tag ;  d_verdict[k]  [j] = the tag over the plaintext of pass 1 matched
+//   d_bad[k] (key_decrypt) [j] = Z_j is off the curve
 namespace capy {
-enum HasherKind { kSha3Stream, kKmacStream, kEncryptStream, kVerifyStream };
+enum HasherKind { kSha3Stream, kKmacStream, kEncryptStream, kVerifyStream, kSignStream, kDecryptStream };
 }
 struct capy_hasher {
   const capy_ctx* ctx = nullptr;
@@ -220,8 +233,17 @@ struct capy_hasher {
   std::vector<uint64_t*> d_total;
   std::vector<uint64_t*> d_ks_state;  // encryption streams only
   std::vector<uint64_t*> d_ks_pos;
-  std::vector<uint8_t*> d_h;          // verification streams only
-  std::vector<uint8_t*> d_bad;
+  std::vector<uint8_t*> d_h;          // verification and decryption streams
+  std::vector<uint8_t*> d_bad;        // verification and key_decrypt streams
+  std::vector<uint64_t*> d_state2;    // sign streams only
+  std::vector<uint32_t*> d_s;
+  std::vector<uint32_t*> d_k;
+  std::vector<uint8_t*> d_s_be;
+  std::vector<uint8_t*> d_n1;
+  std::vector<uint64_t*> d_state0;    // decryption streams only
+  std::vector<uint64_t*> d_ks_state0;
+  std::vector<uint8_t*> d_verdict;
+  std::vector<char> pass;          // [device index] sign and decryption streams: 1 or 2
   std::vector<char> finished;      // [device index] its items were finalised
 };
 
@@ -326,6 +348,20 @@ int launch_kmac_xof_dep(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const
 int launch_kmac_state(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const KmacPass& a, bool trailer, uint64_t* states);
 // a stream batch of `kind` (HasherKind) with zeroed buffers on every device that holds items (blocking; sha3_api.cu)
 int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher** out, uint32_t tag_bits = 0);
+// The final of the items [j0, j0 + n) of device dc.index: carry | T | pad, then out_bytes per item (or out_off); from
+// `state` (nullptr: d_state) with the hasher's carry and totals (sha3_api.cu)
+int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
+                       uint64_t out_bytes, const uint64_t* d_out_off, uint8_t* d_out, const uint64_t* state = nullptr);
+// the carries and totals of device dc.index back to zero: where the second pass starts
+int hasher_restart(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h);
+// capy_hasher_next_pass and the finals of sign streams (ed448_api.cu) and decryption streams (ae_api.cu), over every item
+// of device dc.index
+int sign_stream_next(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h);
+int sign_stream_final(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint8_t* d_h, uint8_t* d_z,
+                      uint8_t* d_ok);
+// second == false: the verdict of pass 1 (into d_verdict, copied to d_ok when given) and the restart; true: the final ok
+int decrypt_stream_check(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, bool second, uint8_t* d_ok,
+                         int* d_bad_flag);
 // ok[i] = (hp_i == h_i) && !bad[i] over 56-byte rows; *bad_flag |= 1 when a bad[i] is set (ed448_api.cu)
 int launch_verify_compare(capy_ctx* ctx, cudaStream_t st, const uint8_t* hp, const uint8_t* h, const uint8_t* bad, uint8_t* ok,
                           int* bad_flag, uint64_t n);

@@ -659,7 +659,7 @@ static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t
 // jobs = 1, J0 alone (and, with `resume`, as resumable streams)
 static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J0, const SpongeJob& J1,
                              bool data_dependent, uint32_t jobs = 2, const SpongeResume* resume = nullptr,
-                             const SpongeSqueeze* squeeze = nullptr) {
+                             const SpongeSqueeze* squeeze = nullptr, const SpongeDual* dual = nullptr) {
   const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
   uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
   if (!sync) return CAPY_ERR_OOM;
@@ -672,6 +672,7 @@ static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, 
   C.data_dependent = data_dependent ? 1u : 0u;
   C.resume = resume ? *resume : SpongeResume{};
   C.squeeze = squeeze ? *squeeze : SpongeSqueeze{};
+  C.dual = dual ? *dual : SpongeDual{};
   return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J0), [&](auto L) {
     sponge_chain_kernel<decltype(L)::value><<<jobs * nb, 128, 0, stream>>>(C);
     ctx->launches++;
@@ -1037,6 +1038,15 @@ static bool hasher_any_finished(const capy_hasher* h) {
     if (f) return true;
   return false;
 }
+// a stream of `kind` in `pass` on device k, not finished
+static bool hasher_dev_in_pass(const capy_hasher* h, int k, int kind, int pass) {
+  return h->kind == kind && !h->finished[k] && h->pass[k] == pass;
+}
+static bool hasher_in_pass(const capy_hasher* h, int kind, int pass) {
+  for (size_t k = 0; k < h->finished.size(); k++)
+    if (!hasher_dev_in_pass(h, (int)k, kind, pass)) return false;
+  return true;
+}
 std::vector<Range> hasher_shards(const capy_hasher* h) {
   std::vector<Range> s;
   for (size_t k = 0; k + 1 < h->first.size(); k++) s.push_back({h->first[k], h->first[k + 1]});
@@ -1102,11 +1112,47 @@ static int hasher_encrypt_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, c
   return launch_chain_jobs(ctx, dc, st, J0, J1, false, 2, &R, &S);
 }
 
-static int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
-                              uint64_t out_bytes, const uint64_t* d_out_off, uint8_t* d_out) {
+// an update of sign streams in pass 2 (A: the "T" stream, B: the second "N" stream) or of decryption streams (A: the
+// keystream, B: the tag stream; d_out in pass 2 only): one launch of the two-state path
+static int hasher_dual_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, uint64_t j0, uint64_t n,
+                             const uint8_t* d_data, const uint64_t* d_off, uint8_t* d_out) {
+  if (n == 0) return CAPY_OK;
+  const int k = dc.index;
+  SpongeResume R;
+  SpongeJob J = hasher_job(h, k, j0, n, &R);
+  SpongeDual D{};
+  if (h->kind == kDecryptStream) {
+    J.chain_out = h->d_ks_state[k] + j0;
+    D.b_state = h->d_state[k] + j0;
+    D.open = 1;
+    D.out = d_out;
+    D.verdict = h->d_verdict[k] + j0;
+  } else {
+    J.chain_out = h->d_state[k] + j0;
+    D.b_state = h->d_state2[k] + j0;
+  }
+  J.chain_in = J.chain_out;
+  J.stop_block = ~0ull;
+  J.data = d_data;
+  J.off = d_off;
+  return launch_chain_jobs(ctx, dc, st, J, J, false, 1, &R, nullptr, &D);
+}
+
+// a piece of every stream: pass 1 of sign streams is a plain KMAC stream update, pass 2 and decryption streams run two
+// states
+static int hasher_piece_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h, uint64_t j0, uint64_t n,
+                              const uint8_t* d_data, const uint64_t* d_off) {
+  if (h->kind == kDecryptStream || (h->kind == kSignStream && h->pass[dc.index] == 2))
+    return hasher_dual_items(ctx, dc, st, h, j0, n, d_data, d_off, nullptr);
+  return hasher_update_items(ctx, dc, st, h, j0, n, d_data, d_off);
+}
+
+int hasher_final_items(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t j0, uint64_t n,
+                       uint64_t out_bytes, const uint64_t* d_out_off, uint8_t* d_out, const uint64_t* state) {
   if (n == 0 || (!d_out_off && out_bytes == 0)) return CAPY_OK;
   SpongeResume R;
   SpongeJob J = hasher_job(h, dc.index, j0, n, &R);
+  if (state) J.chain_in = state + j0;
   J.out = d_out;
   J.out_off = d_out_off;
   J.out_stride = J.out_bytes = out_bytes;
@@ -1136,6 +1182,13 @@ int launch_kmac_state(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const K
   return launch_chain_jobs(ctx, dc, stream, J, J, false, 1);
 }
 
+int hasher_restart(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, capy_hasher* h) {
+  const size_t m = (size_t)hasher_items(h, dc.index);
+  CAPY_CUDA(ctx, cudaMemsetAsync(h->d_carry[dc.index], 0, m * h->rate, st));
+  CAPY_CUDA(ctx, cudaMemsetAsync(h->d_total[dc.index], 0, m * 8, st));
+  return CAPY_OK;
+}
+
 // Items are dealt out in equal contiguous ranges.
 int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher** out, uint32_t tag_bits) {
   capy_hasher* h = new (std::nothrow) capy_hasher();
@@ -1157,6 +1210,15 @@ int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher**
   h->d_ks_pos.assign(nd, nullptr);
   h->d_h.assign(nd, nullptr);
   h->d_bad.assign(nd, nullptr);
+  h->d_state2.assign(nd, nullptr);
+  h->d_s.assign(nd, nullptr);
+  h->d_k.assign(nd, nullptr);
+  h->d_s_be.assign(nd, nullptr);
+  h->d_n1.assign(nd, nullptr);
+  h->d_state0.assign(nd, nullptr);
+  h->d_ks_state0.assign(nd, nullptr);
+  h->d_verdict.assign(nd, nullptr);
+  h->pass.assign(nd, kind == kSignStream || kind == kDecryptStream ? 1 : 0);
   h->finished.assign(nd, 0);
   for (DeviceCtx& dc : ctx->devs) {
     const uint64_t m = hasher_items(h, dc.index);
@@ -1174,10 +1236,21 @@ int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher**
       int r = zeroed(h->d_state[k], (size_t)m * 200);
       if (!r) r = zeroed(h->d_carry[k], (size_t)m * h->rate);
       if (!r) r = zeroed(h->d_total[k], (size_t)m * 8);
-      if (!r && kind == kEncryptStream) r = zeroed(h->d_ks_state[k], (size_t)m * 200);
+      const bool sign = kind == kSignStream, dec = kind == kDecryptStream;
+      if (!r && (kind == kEncryptStream || dec)) r = zeroed(h->d_ks_state[k], (size_t)m * 200);
       if (!r && kind == kEncryptStream) r = zeroed(h->d_ks_pos[k], (size_t)m * 8);
       if (!r && kind == kVerifyStream) r = zeroed(h->d_h[k], (size_t)m * 56);
       if (!r && kind == kVerifyStream) r = zeroed(h->d_bad[k], (size_t)m);
+      if (!r && sign) r = zeroed(h->d_state2[k], (size_t)m * 200);
+      if (!r && sign) r = zeroed(h->d_s[k], (size_t)m * 56);
+      if (!r && sign) r = zeroed(h->d_k[k], (size_t)m * 56);
+      if (!r && sign) r = zeroed(h->d_s_be[k], (size_t)m * 56);
+      if (!r && sign) r = zeroed(h->d_n1[k], (size_t)m * 56);
+      if (!r && dec) r = zeroed(h->d_state0[k], (size_t)m * 200);
+      if (!r && dec) r = zeroed(h->d_ks_state0[k], (size_t)m * 200);
+      if (!r && dec) r = zeroed(h->d_h[k], (size_t)m * (tag_bits / 8));
+      if (!r && dec) r = zeroed(h->d_verdict[k], (size_t)m);
+      if (!r && dec && tag_bits == 448) r = zeroed(h->d_bad[k], (size_t)m);
       if (r) return r;
       CAPY_CUDA(ctx, cudaStreamSynchronize(st));
       return CAPY_OK;
@@ -1510,6 +1583,7 @@ int capy_hasher_device_range(const capy_hasher* h, int dev_index, uint64_t* i0, 
 int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const uint64_t* off) {
   if (hasher_check(ctx, h) || h->kind == kEncryptStream || hasher_any_finished(h) || (h->n && (!data || !off)))
     return CAPY_ERR_BAD_ARG;
+  if (h->kind == kDecryptStream && !hasher_in_pass(h, kDecryptStream, 1)) return CAPY_ERR_BAD_ARG;  // pass 2: decrypt_update
   if (h->n == 0) return CAPY_OK;
   auto chunks = [&](Range sh) {
     return split_items(off, 0, sh.i0, sh.i1, chunk_count(off[sh.i1] - off[sh.i0], sh.i1 - sh.i0), 200);
@@ -1517,7 +1591,7 @@ int capy_hasher_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* data, const
   return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
     const StagedPacked sp = io.in_packed(data, off);
     if (io.rc()) return io.rc();
-    return hasher_update_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), sp.d_base, sp.d_off);
+    return hasher_piece_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), sp.d_base, sp.d_off);
   });
 }
 
@@ -1525,11 +1599,12 @@ int capy_hasher_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* s
                            const uint64_t* d_off) {
   if (hasher_check(ctx, h) || h->kind == kEncryptStream || !dev_index_ok(ctx, dev_index) || h->finished[dev_index])
     return CAPY_ERR_BAD_ARG;
+  if (h->kind == kDecryptStream && h->pass[dev_index] != 1) return CAPY_ERR_BAD_ARG;
   const uint64_t m = hasher_items(h, dev_index);
   if (m && (!d_data || !d_off)) return CAPY_ERR_BAD_ARG;
   if (m == 0) return CAPY_OK;
   CAPY_DEV_PROLOGUE
-  return hasher_update_items(ctx, dc, st, h, 0, m, d_data, d_off);
+  return hasher_piece_items(ctx, dc, st, h, 0, m, d_data, d_off);
 }
 
 int capy_hasher_final(capy_ctx* ctx, capy_hasher* h, uint64_t out_bits, const uint64_t* out_off, uint8_t* out) {
@@ -1617,10 +1692,117 @@ int capy_hasher_verify_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, v
   return hasher_verify_items(ctx, dc, st, h, 0, m, d_ok, d_bad_flag);
 }
 
+// ---- sign and decryption streams: two passes (created in ed448_api.cu and ae_api.cu) ----------------------------------
+// The pass moves to 2 before the device work of next_pass runs, as `finished` does before a final: a next_pass that fails
+// (an OOM, a CUDA error) leaves its streams with half-updated states, and the only call left that is of use is
+// capy_hasher_free.
+int capy_hasher_next_pass(capy_ctx* ctx, capy_hasher* h, uint8_t* ok) {
+  if (hasher_check(ctx, h)) return CAPY_ERR_BAD_ARG;
+  const bool sign = hasher_in_pass(h, kSignStream, 1), dec = hasher_in_pass(h, kDecryptStream, 1);
+  if ((!sign && !dec) || (sign && ok)) return CAPY_ERR_BAD_ARG;
+  for (char& p : h->pass) p = 2;
+  if (h->n == 0) return CAPY_OK;
+  return run_host_call(ctx, hasher_shards(h), one_chunk, dec && h->tag_bits == 448,
+                       [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;  // (a device without items)
+    uint8_t* d_ok = ok ? io.out(ok, 1) : nullptr;
+    if (io.rc()) return io.rc();
+    return sign ? sign_stream_next(ctx, dc, st, h) : decrypt_stream_check(ctx, dc, st, h, false, d_ok, io.d_flag());
+  });
+}
+
+int capy_hasher_next_pass_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index)) return CAPY_ERR_BAD_ARG;
+  const bool sign = hasher_dev_in_pass(h, dev_index, kSignStream, 1), dec = hasher_dev_in_pass(h, dev_index, kDecryptStream, 1);
+  if ((!sign && !dec) || (sign && d_ok)) return CAPY_ERR_BAD_ARG;
+  h->pass[dev_index] = 2;
+  if (hasher_items(h, dev_index) == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return sign ? sign_stream_next(ctx, dc, st, h) : decrypt_stream_check(ctx, dc, st, h, false, d_ok, d_bad_flag);
+}
+
+int capy_hasher_decrypt_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* ct, const uint64_t* off, uint8_t* out) {
+  if (hasher_check(ctx, h) || !hasher_in_pass(h, kDecryptStream, 2) || (h->n && (!ct || !off || !out))) return CAPY_ERR_BAD_ARG;
+  if (h->n == 0) return CAPY_OK;
+  auto chunks = [&](Range sh) {
+    return split_items(off, 0, sh.i0, sh.i1, chunk_count(off[sh.i1] - off[sh.i0], sh.i1 - sh.i0), 400);
+  };
+  return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const StagedPacked sp = io.in_packed(ct, off);
+    uint8_t* d_out = io.out_packed(out, off);
+    if (io.rc()) return io.rc();
+    return hasher_dual_items(ctx, dc, st, h, io.i0() - h->first[dc.index], io.n(), sp.d_base, sp.d_off, d_out);
+  });
+}
+
+int capy_hasher_decrypt_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_ct,
+                                   const uint64_t* d_off, uint8_t* d_out) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || !hasher_dev_in_pass(h, dev_index, kDecryptStream, 2))
+    return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && (!d_ct || !d_off || !d_out)) return CAPY_ERR_BAD_ARG;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return hasher_dual_items(ctx, dc, st, h, 0, m, d_ct, d_off, d_out);
+}
+
+int capy_hasher_decrypt_final(capy_ctx* ctx, capy_hasher* h, uint8_t* ok) {
+  if (hasher_check(ctx, h) || !hasher_in_pass(h, kDecryptStream, 2) || (h->n && !ok)) return CAPY_ERR_BAD_ARG;
+  for (char& f : h->finished) f = 1;
+  if (h->n == 0) return CAPY_OK;
+  return run_host_call(ctx, hasher_shards(h), one_chunk, h->tag_bits == 448,
+                       [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return decrypt_stream_check(ctx, dc, st, h, true, d_ok, io.d_flag());
+  });
+}
+
+int capy_hasher_decrypt_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || !hasher_dev_in_pass(h, dev_index, kDecryptStream, 2))
+    return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && !d_ok) return CAPY_ERR_BAD_ARG;
+  h->finished[dev_index] = 1;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return decrypt_stream_check(ctx, dc, st, h, true, d_ok, d_bad_flag);
+}
+
+int capy_hasher_sign_final(capy_ctx* ctx, capy_hasher* h, uint8_t* h56, uint8_t* z_be56, uint8_t* ok) {
+  if (hasher_check(ctx, h) || !hasher_in_pass(h, kSignStream, 2) || (h->n && (!h56 || !z_be56 || !ok)))
+    return CAPY_ERR_BAD_ARG;
+  for (char& f : h->finished) f = 1;
+  if (h->n == 0) return CAPY_OK;
+  return run_host_call(ctx, hasher_shards(h), one_chunk, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    if (io.n() == 0) return CAPY_OK;
+    uint8_t* d_h = io.out(h56, 56);
+    uint8_t* d_z = io.out(z_be56, 56);
+    uint8_t* d_ok = io.out(ok, 1);
+    if (io.rc()) return io.rc();
+    return sign_stream_final(ctx, dc, st, h, d_h, d_z, d_ok);
+  });
+}
+
+int capy_hasher_sign_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_h56, uint8_t* d_z_be56,
+                               uint8_t* d_ok) {
+  if (hasher_check(ctx, h) || !dev_index_ok(ctx, dev_index) || !hasher_dev_in_pass(h, dev_index, kSignStream, 2))
+    return CAPY_ERR_BAD_ARG;
+  const uint64_t m = hasher_items(h, dev_index);
+  if (m && (!d_h56 || !d_z_be56 || !d_ok)) return CAPY_ERR_BAD_ARG;
+  h->finished[dev_index] = 1;
+  if (m == 0) return CAPY_OK;
+  CAPY_DEV_PROLOGUE
+  return sign_stream_final(ctx, dc, st, h, d_h56, d_z_be56, d_ok);
+}
+
 void capy_hasher_free(capy_hasher* h) {
   if (!h) return;
   for (size_t k = 0; k < h->dev.size(); k++) {
-    void* bufs[] = {h->d_state[k], h->d_carry[k], h->d_total[k], h->d_ks_state[k], h->d_ks_pos[k], h->d_h[k], h->d_bad[k]};
+    void* bufs[] = {h->d_state[k], h->d_carry[k], h->d_total[k], h->d_ks_state[k], h->d_ks_pos[k], h->d_h[k], h->d_bad[k],
+                    h->d_state2[k], h->d_s[k], h->d_k[k], h->d_s_be[k], h->d_n1[k], h->d_state0[k], h->d_ks_state0[k],
+                    h->d_verdict[k]};
     bool any = false;
     for (void* p : bufs) any = any || p;
     if (!any) continue;
@@ -1631,6 +1813,11 @@ void capy_hasher_free(capy_hasher* h) {
     if (h->d_state[k]) cudaMemset(h->d_state[k], 0, m * 200);
     if (h->d_carry[k]) cudaMemset(h->d_carry[k], 0, m * h->rate);
     if (h->d_ks_state[k]) cudaMemset(h->d_ks_state[k], 0, m * 200);
+    // sign streams: s, k, the first "N" output and the second "N" state; decryption streams: the ke / ka states
+    for (void* p : {(void*)h->d_state2[k], (void*)h->d_state0[k], (void*)h->d_ks_state0[k]})
+      if (p) cudaMemset(p, 0, m * 200);
+    for (void* p : {(void*)h->d_s[k], (void*)h->d_k[k], (void*)h->d_s_be[k], (void*)h->d_n1[k]})
+      if (p) cudaMemset(p, 0, m * 56);
     cudaDeviceSynchronize();
     for (void* p : bufs)
       if (p) cudaFree(p);

@@ -734,6 +734,7 @@ struct SpongeChain {
   uint32_t data_dependent;
   SpongeResume resume;  // carry == nullptr: the jobs are not resumable streams
   SpongeSqueeze squeeze;  // resumable streams with two jobs: job 1 is the keystream update of encryption streams
+  SpongeDual dual;        // b_state != nullptr: job 0 runs two states in lockstep (sign and decryption streams)
 };
 // resumable streams (order == nullptr: rank = item), out of line: the cut chains keep their own register allocation
 template <int LANES>
@@ -785,6 +786,89 @@ __device__ __noinline__ void sponge_squeeze_resume_ool(const SpongeJob& J, const
   S->pos[i] = p1;
 }
 
+// Two states of item i in lockstep (SpongeDual), entered at any byte of a block.  Block s of the stream is carry | piece
+// bytes; a block that the piece completes goes into B (and into A in dual absorb) and both states permute, the bytes of
+// an incomplete last block join the carry.  Lanes wholly inside the piece take the 8-byte path of
+// sponge_squeeze_resume_ool, any other lane goes byte by byte.  In the open mode the plaintext exists only in registers,
+// in the stream's own carry and in `out`: fused, because the tag depends on the keystream output, and two jobs would have
+// to pass the unverified plaintext through a buffer the stream does not own.
+template <int LANES>
+__device__ __noinline__ void sponge_dual_resume_ool(const SpongeJob& J, const SpongeResume* R, const SpongeDual* D, uint64_t i) {
+  constexpr uint64_t RATE = 8ull * LANES;
+  const uint64_t state_n = R->state_n;
+  uint64_t* bs = D->b_state;
+  Lane a[25], b[25];
+#pragma unroll
+  for (int k = 0; k < 25; k++) {
+    const uint64_t va = J.chain_in[(uint64_t)k * state_n + i], vb = bs[(uint64_t)k * state_n + i];
+    a[k].lo = (uint32_t)va;
+    a[k].hi = (uint32_t)(va >> 32);
+    b[k].lo = (uint32_t)vb;
+    b[k].hi = (uint32_t)(vb >> 32);
+  }
+  const bool open = D->open != 0;
+  const uint64_t p0 = R->totals[i], a0 = J.off[i], p1 = p0 + (J.off[i + 1] - a0);
+  const uint8_t* x = J.data + a0;  // stream byte p goes with x[p - p0] and o[p - p0]
+  uint8_t* o = D->out ? D->out + a0 : nullptr;
+  const bool release = o && D->verdict[i];
+  uint8_t* cb = R->carry + i * RATE;  // stream byte p of the current block s at cb[p - s]
+  const bool al = ((reinterpret_cast<uintptr_t>(x) - p0) & 7u) == 0 && (!o || ((reinterpret_cast<uintptr_t>(o) - p0) & 7u) == 0);
+#pragma unroll 1
+  for (uint64_t s = p0 - p0 % RATE; s < p1; s += RATE) {
+    const bool full = s + RATE <= p1;
+#pragma unroll
+    for (int j = 0; j < LANES; j++) {
+      const uint64_t l0 = s + 8ull * j, lo = l0 > p0 ? l0 : p0, hi = l0 + 8 < p1 ? l0 + 8 : p1;
+      const uint64_t ks = open ? ((uint64_t)a[j].hi << 32) | a[j].lo : 0ull;
+      uint64_t v = 0;  // the lane of block s: carry bytes below p0, piece bytes (plaintext in the open mode) from p0 on
+      if (lo < hi) {
+        if (al && hi - lo == 8) {
+          const uint2 m = *reinterpret_cast<const uint2*>(x + (lo - p0));
+          const uint64_t c = ((uint64_t)m.y << 32) | m.x;
+          v = c ^ ks;
+          if (o) {
+            const uint64_t w = release ? v : c;
+            *reinterpret_cast<uint2*>(o + (lo - p0)) = make_uint2((uint32_t)w, (uint32_t)(w >> 32));
+          }
+          if (!full) *reinterpret_cast<uint2*>(cb + 8 * j) = make_uint2((uint32_t)v, (uint32_t)(v >> 32));
+        } else {
+#pragma unroll 1
+          for (uint64_t q = lo; q < hi; q++) {
+            const uint8_t c = x[q - p0], pt = c ^ (uint8_t)(ks >> (8 * (uint32_t)(q - l0)));
+            if (o) o[q - p0] = release ? pt : c;
+            if (!full) cb[q - s] = pt;
+            v |= (uint64_t)pt << (8 * (uint32_t)(q - l0));
+          }
+        }
+      }
+      if (full) {
+#pragma unroll 1
+        for (uint64_t q = l0; q < p0 && q < l0 + 8; q++) v |= (uint64_t)cb[q - s] << (8 * (uint32_t)(q - l0));
+        b[j].lo ^= (uint32_t)v;
+        b[j].hi ^= (uint32_t)(v >> 32);
+        if (!open) {
+          a[j].lo ^= (uint32_t)v;
+          a[j].hi ^= (uint32_t)(v >> 32);
+        }
+      }
+    }
+    if (full) {
+      keccak_f1600(a);
+      keccak_f1600(b);
+    }
+  }
+#pragma unroll
+  for (int k = 0; k < 25; k++) {
+    J.chain_out[(uint64_t)k * state_n + i] = ((uint64_t)a[k].hi << 32) | a[k].lo;
+    bs[(uint64_t)k * state_n + i] = ((uint64_t)b[k].hi << 32) | b[k].lo;
+  }
+  R->totals[i] = p1;
+}
+
+// the two-state path exists at the KMAC rates of D256 / 384 / 512 only (the other instantiations keep their registers)
+template <int LANES>
+constexpr bool kDualLanes = LANES == 17 || LANES == 19 || LANES == 21;
+
 template <int LANES>
 __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(const __grid_constant__ SpongeChain C) {
   __shared__ uint32_t ticket_s;
@@ -801,6 +885,7 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(con
   const uint64_t r = (uint64_t)b * 128 + threadIdx.x;
   if (r < J.n) {
     if (job && C.data_dependent) sponge_item<LANES, true, true>(J, sponge_rank_item(J, r), r);
+    else if (kDualLanes<LANES> && C.dual.b_state) sponge_dual_resume_ool<LANES>(J, &C.resume, &C.dual, r);  // (job 0 alone)
     else if (C.resume.carry && job) sponge_squeeze_resume_ool<LANES>(J, &C.squeeze, r);  // (only encryption streams have a job 1)
     else if (C.resume.carry) sponge_item_resume_ool<LANES>(J, &C.resume, r);
     else sponge_item<LANES, true>(J, sponge_rank_item(J, r), r);

@@ -83,6 +83,23 @@ struct SpongeSqueeze {
   uint64_t state_n;
 };
 
+// Two-state resumable streams (sign and decryption streams of capy_hasher: job 0 of sponge_chain_kernel alone, beside a
+// SpongeResume).  State A at chain_in / chain_out and state B at b_state[k * state_n + i] have the same rate, 8 LANES
+// bytes (the KMAC rate, which at D256 / 384 / 512 is also the squeeze width), so they share the carry and the total of
+// the SpongeResume and permute at the same block ends.
+//   open == 0 (dual absorb, sign pass 2): every whole block of carry | X is absorbed into A and into B.
+//   open != 0 (decryption): A is a keystream at the start of squeeze block totals[i] / rate; pt = X ^ keystream, and every
+//     whole block of carry | pt is absorbed into B (the tag stream); the carry holds plaintext.  With out, item i writes
+//     out[off[i] ..) = pt when verdict[i] != 0, else X (the ciphertext); out may be data.  Without out nothing is written
+//     but the states, the carry and the total.
+// Kept out of SpongeJob, like SpongeResume.
+struct SpongeDual {
+  uint64_t* b_state;  // nullptr: not a two-state job
+  uint32_t open;
+  const uint8_t* verdict;
+  uint8_t* out;
+};
+
 // ---- rates in bytes, as the reference computes them ------------------------------------------------------------------
 // SHA3-d capacity in bits: 2d rounded up to the reference's buckets (constants.rs:38-45)
 inline uint32_t sha3_capacity(int d) {

@@ -232,6 +232,84 @@ class VerifyStream(Hasher):
         return t_ok
 
 
+class SignStream(Hasher):
+    """n signatures whose messages are fed twice (Engine.ed448_sign_stream): update() as Hasher in both passes,
+    next_pass() between them, final() -> (h, z, ok).  ok[i] = 0: pass 2 carried other bytes than pass 1, and h[i], z[i]
+    are zero."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, n: int, d: int):
+        super().__init__(engine, handle, n, d, True)
+
+    def next_pass(self) -> None:
+        """capy_hasher_next_pass (blocking)"""
+        self._engine._check(self._engine.lib.capy_hasher_next_pass(self._engine._ctx, self.handle, None))
+
+    def final(self) -> tuple[np.ndarray, np.ndarray, np.ndarray]:
+        h, z = np.zeros((self.n, 56), dtype=np.uint8), np.zeros((self.n, 56), dtype=np.uint8)
+        ok = np.zeros(self.n, dtype=np.uint8)
+        self._engine._check(self._engine.lib.capy_hasher_sign_final(self._engine._ctx, self.handle, _hp(h), _hp(z), _hp(ok)))
+        return h, z, ok
+
+    def next_pass_dev(self, dev_index: int = 0) -> None:
+        self._engine._check(self._engine.lib.capy_hasher_next_pass_dev(self._engine._ctx, self.handle, dev_index,
+                                                                       self._engine._stream(), None, None))
+
+    def final_dev(self, t_h, t_z, t_ok, dev_index: int = 0):
+        """capy_hasher_sign_final_dev on torch's current stream"""
+        self._engine._check(self._engine.lib.capy_hasher_sign_final_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), t_h.data_ptr(), t_z.data_ptr(),
+            t_ok.data_ptr()))
+
+
+class DecryptStream(Hasher):
+    """n decryptions whose ciphertexts are fed twice (Engine.sponge_decrypt_stream / Engine.ed448_key_decrypt_stream):
+    update() takes the ciphertext in pass 1 and writes nothing, next_pass() -> (rc, verdicts), decrypt() takes the same
+    ciphertext in pass 2 (plaintext out where the verdict was 1, the ciphertext elsewhere), final() -> (rc, ok).  rc is
+    CAPY_OK or, for key_decrypt with an off-curve Z, ERR_BAD_POINT."""
+
+    def __init__(self, engine: "Engine", handle: C.c_void_p, n: int, d: int):
+        super().__init__(engine, handle, n, d, True)
+
+    def next_pass(self, ok_out: np.ndarray | None = None) -> tuple[int, np.ndarray]:
+        ok = _out(ok_out, (self.n,), "verdicts")
+        rc = self._engine._check(self._engine.lib.capy_hasher_next_pass(self._engine._ctx, self.handle, _hp(ok)),
+                                 allow=(B.ERR_BAD_POINT,))
+        return rc, ok
+
+    def decrypt(self, data, off, out: np.ndarray | None = None) -> np.ndarray:
+        """capy_hasher_decrypt_update (out may be data itself: in place)"""
+        data, off = _u8(data), _u64(off)
+        if _need_packed(data, off, "stream pieces") != self.n:
+            raise ValueError(f"stream decrypt: {off.size - 1} pieces for {self.n} streams")
+        out = _out(out, (data.size,), "stream plaintext")
+        self._engine._check(self._engine.lib.capy_hasher_decrypt_update(self._engine._ctx, self.handle, _hp(data), _hp(off),
+                                                                        _hp(out)))
+        return out
+
+    def final(self, ok_out: np.ndarray | None = None) -> tuple[int, np.ndarray]:
+        ok = _out(ok_out, (self.n,), "decrypt flags")
+        rc = self._engine._check(self._engine.lib.capy_hasher_decrypt_final(self._engine._ctx, self.handle, _hp(ok)),
+                                 allow=(B.ERR_BAD_POINT,))
+        return rc, ok
+
+    def next_pass_dev(self, t_ok=None, t_bad=None, dev_index: int = 0) -> None:
+        self._engine._check(self._engine.lib.capy_hasher_next_pass_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(),
+            t_ok.data_ptr() if t_ok is not None else None, t_bad.data_ptr() if t_bad is not None else None))
+
+    def decrypt_dev(self, t_ct, t_off, t_out, dev_index: int = 0) -> None:
+        """capy_hasher_decrypt_update_dev on torch's current stream (t_out may be t_ct)"""
+        self._engine._check(self._engine.lib.capy_hasher_decrypt_update_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), t_ct.data_ptr(), t_off.data_ptr(),
+            t_out.data_ptr()))
+
+    def final_dev(self, t_ok, t_bad=None, dev_index: int = 0):
+        self._engine._check(self._engine.lib.capy_hasher_decrypt_final_dev(
+            self._engine._ctx, self.handle, dev_index, self._engine._stream(), t_ok.data_ptr(),
+            t_bad.data_ptr() if t_bad is not None else None))
+        return t_ok
+
+
 def _pub_or_key(pub):
     """(pub_xy112 bytes or None, prepared key handle or None) of a PreparedPublicKey or n x 112 key bytes"""
     if isinstance(pub, PreparedPublicKey):
@@ -410,6 +488,37 @@ class Engine:
         h = C.c_void_p()
         self._check(self.lib.capy_ed448_verify_stream_new(self._ctx, d, _hp(pub_b), key, _hp(hb), _hp(zb), n, C.byref(h)))
         return VerifyStream(self, h, n, d)
+
+    def ed448_sign_stream(self, pws, pw_off, d: int) -> SignStream:
+        """capy_ed448_sign_stream_new: one sign stream per password (blocking)"""
+        pws, pw_off = _u8(pws), _u64(pw_off)
+        n = _need_packed(pws, pw_off, "stream passwords")
+        h = C.c_void_p()
+        self._check(self.lib.capy_ed448_sign_stream_new(self._ctx, d, _hp(pws), _hp(pw_off), n, C.byref(h)))
+        return SignStream(self, h, n, d)
+
+    def sponge_decrypt_stream(self, pws, pw_off, nonces, nonce_len: int, tags64, d: int,
+                              variant: int = B.AE_SHA3) -> DecryptStream:
+        """capy_sponge_decrypt_stream_new: one open stream per password, expected tags n x 64 (blocking)"""
+        pws, pw_off, nonces, tags = _u8(pws), _u64(pw_off), _u8(nonces), _u8(tags64)
+        n = _need_packed(pws, pw_off, "stream passwords")
+        if len(nonces) != n * nonce_len or len(tags) != n * 64:
+            raise ValueError(f"sponge_decrypt_stream: need {n} x {nonce_len} nonce bytes and {n} x 64 tag bytes")
+        h = C.c_void_p()
+        self._check(self.lib.capy_sponge_decrypt_stream_new(self._ctx, d, variant, _hp(pws), _hp(pw_off), _hp(nonces),
+                                                            nonce_len, _hp(tags), n, C.byref(h)))
+        return DecryptStream(self, h, n, d)
+
+    def ed448_key_decrypt_stream(self, pws, pw_off, z_xy112, tags56, d: int) -> DecryptStream:
+        """capy_ed448_key_decrypt_stream_new: one key_decrypt stream per password and Z, expected tags n x 56 (blocking)"""
+        pws, pw_off, z, tags = _u8(pws), _u64(pw_off), _u8(z_xy112), _u8(tags56)
+        n = _need_packed(pws, pw_off, "stream passwords")
+        if len(z) != n * 112 or len(tags) != n * 56:
+            raise ValueError(f"key_decrypt_stream: need {n} x 112 Z bytes and {n} x 56 tag bytes")
+        h = C.c_void_p()
+        self._check(self.lib.capy_ed448_key_decrypt_stream_new(self._ctx, d, _hp(pws), _hp(pw_off), _hp(z), _hp(tags), n,
+                                                               C.byref(h)))
+        return DecryptStream(self, h, n, d)
 
     def ed448_fixed_base(self, scalars_be56, out: np.ndarray | None = None) -> np.ndarray:
         sc = _u8(scalars_be56)

@@ -127,7 +127,7 @@ class PreparedPublicKey {
 // before the Engine.
 class Hasher {
  public:
-  Hasher(Hasher&& o) noexcept : ctx_(o.ctx_), h_(o.h_), n_(o.n_), d_bits_(o.d_bits_) { o.h_ = nullptr; }
+  Hasher(Hasher&& o) noexcept : ctx_(o.ctx_), h_(o.h_), n_(o.n_), d_bits_(o.d_bits_), sign_(o.sign_) { o.h_ = nullptr; }
   Hasher& operator=(Hasher&& o) noexcept {
     if (this != &o) {
       capy_hasher_free(h_);
@@ -135,6 +135,7 @@ class Hasher {
       h_ = o.h_;
       n_ = o.n_;
       d_bits_ = o.d_bits_;
+      sign_ = o.sign_;
       o.h_ = nullptr;
     }
     return *this;
@@ -186,6 +187,49 @@ class Hasher {
     return ok;
   }
 
+  // sign and decryption streams (Engine::sign_stream / sha3_decrypt_stream / key_decrypt_stream): the end of pass 1.
+  // Decryption: the verdict per stream; *bad_point = a Z was off the curve.  Sign: an empty result.
+  Bytes next_pass(bool* bad_point = nullptr) {
+    Bytes ok(n_ + 1);
+    const int rc = capy_hasher_next_pass(ctx_, h_, sign_ ? nullptr : ok.data());
+    if (rc != CAPY_ERR_BAD_POINT) check(rc);
+    if (bad_point) *bad_point = rc == CAPY_ERR_BAD_POINT;
+    ok.resize(sign_ ? 0 : n_);
+    return ok;
+  }
+  // decryption pass 2: the plaintext of pieces[i] (the ciphertext where the verdict was 0)
+  std::vector<Bytes> decrypt_update(const std::vector<Bytes>& pieces) {
+    if (pieces.size() != n_) throw GpuError(CAPY_ERR_BAD_ARG, "Hasher::decrypt_update: one piece per stream");
+    Bytes data;
+    std::vector<uint64_t> off;
+    detail::pack(pieces, [](const Bytes& b) -> const Bytes& { return b; }, data, off);
+    check(capy_hasher_decrypt_update(ctx_, h_, data.data(), off.data(), data.data()));
+    std::vector<Bytes> res(n_);
+    for (size_t i = 0; i < n_; i++) res[i].assign(data.begin() + off[i], data.begin() + off[i + 1]);
+    return res;
+  }
+  Bytes decrypt_final(bool* bad_point = nullptr) {
+    Bytes ok(n_ + 1);
+    const int rc = capy_hasher_decrypt_final(ctx_, h_, ok.data());
+    if (rc != CAPY_ERR_BAD_POINT) check(rc);
+    if (bad_point) *bad_point = rc == CAPY_ERR_BAD_POINT;
+    ok.resize(n_);
+    return ok;
+  }
+  // the signatures; ok[i] = 0 where pass 2 carried other bytes than pass 1 (then sigs[i] is all zero bytes)
+  std::vector<Signature> sign_final(Bytes& ok) {
+    Bytes h(n_ * 56 + 1), z(n_ * 56 + 1);
+    ok.assign(n_ + 1, 0);
+    check(capy_hasher_sign_final(ctx_, h_, h.data(), z.data(), ok.data()));
+    ok.resize(n_);
+    std::vector<Signature> res(n_);
+    for (size_t i = 0; i < n_; i++) {
+      res[i].h.assign(h.begin() + 56 * i, h.begin() + 56 * (i + 1));
+      std::copy(z.begin() + 56 * i, z.begin() + 56 * (i + 1), res[i].z.begin());
+    }
+    return res;
+  }
+
  private:
   friend class Engine;
   Hasher(capy_ctx* ctx, capy_hasher* h, size_t n, int d_bits) : ctx_(ctx), h_(h), n_(n), d_bits_(d_bits) {}
@@ -196,6 +240,7 @@ class Hasher {
   capy_hasher* h_ = nullptr;
   size_t n_ = 0;
   int d_bits_ = 0;
+  bool sign_ = false;  // a sign stream (Engine::sign_stream): next_pass passes no ok
 };
 
 class Engine {
@@ -307,6 +352,60 @@ class Engine {
     capy_hasher* hs = nullptr;
     check(capy_ed448_verify_stream_new(ctx_, d_bits, nullptr, key.raw(), h.data(), z.data(), sigs.size(), &hs));
     return Hasher(ctx_, hs, sigs.size(), d_bits);
+  }
+
+  // sign of messages fed twice in pieces: update, next_pass, update, sign_final (blocking creation)
+  Hasher sign_stream(const std::vector<Bytes>& pws, int d_bits) {
+    Bytes pd;
+    std::vector<uint64_t> po;
+    detail::pack(pws, [](const Bytes& b) -> const Bytes& { return b; }, pd, po);
+    capy_hasher* h = nullptr;
+    check(capy_ed448_sign_stream_new(ctx_, d_bits, pd.data(), po.data(), pws.size(), &h));
+    Hasher r(ctx_, h, pws.size(), d_bits);
+    r.sign_ = true;
+    return r;
+  }
+
+  // sha3_decrypt of ciphertexts fed twice: update, next_pass, decrypt_update, decrypt_final (512-byte nonces)
+  Hasher sha3_decrypt_stream(const std::vector<Bytes>& pws, const std::vector<Bytes>& nonces, const std::vector<Bytes>& tags,
+                             int d_bits) {
+    if (nonces.size() != pws.size() || tags.size() != pws.size())
+      throw GpuError(CAPY_ERR_BAD_ARG, "sha3_decrypt_stream: one nonce and one tag per password");
+    Bytes pd, zs, ts;
+    std::vector<uint64_t> po;
+    detail::pack(pws, [](const Bytes& b) -> const Bytes& { return b; }, pd, po);
+    for (size_t i = 0; i < pws.size(); i++) {
+      if (nonces[i].size() != 512 || tags[i].size() != 64)
+        throw GpuError(CAPY_ERR_BAD_ARG, "sha3_decrypt_stream: 512-byte nonces and 64-byte tags");
+      zs.insert(zs.end(), nonces[i].begin(), nonces[i].end());
+      ts.insert(ts.end(), tags[i].begin(), tags[i].end());
+    }
+    zs.push_back(0);
+    ts.push_back(0);
+    capy_hasher* h = nullptr;
+    check(capy_sponge_decrypt_stream_new(ctx_, d_bits, CAPY_AE_SHA3, pd.data(), po.data(), zs.data(), 512, ts.data(),
+                                         pws.size(), &h));
+    return Hasher(ctx_, h, pws.size(), d_bits);
+  }
+
+  // key_decrypt of ciphertexts fed twice (z[i] = Z_i, 56-byte tags)
+  Hasher key_decrypt_stream(const std::vector<Bytes>& pws, const std::vector<AffinePoint>& z, const std::vector<Bytes>& tags,
+                            int d_bits) {
+    if (z.size() != pws.size() || tags.size() != pws.size())
+      throw GpuError(CAPY_ERR_BAD_ARG, "key_decrypt_stream: one Z and one tag per password");
+    Bytes pd, zs, ts;
+    std::vector<uint64_t> po;
+    detail::pack(pws, [](const Bytes& b) -> const Bytes& { return b; }, pd, po);
+    for (size_t i = 0; i < pws.size(); i++) {
+      if (tags[i].size() != 56) throw GpuError(CAPY_ERR_BAD_ARG, "key_decrypt_stream: 56-byte tags");
+      zs.insert(zs.end(), z[i].begin(), z[i].end());
+      ts.insert(ts.end(), tags[i].begin(), tags[i].end());
+    }
+    zs.push_back(0);
+    ts.push_back(0);
+    capy_hasher* h = nullptr;
+    check(capy_ed448_key_decrypt_stream_new(ctx_, d_bits, pd.data(), po.data(), zs.data(), ts.data(), pws.size(), &h));
+    return Hasher(ctx_, h, pws.size(), d_bits);
   }
 
   // KeyPair::new for every password

@@ -337,8 +337,8 @@ void capy_hasher_free(capy_hasher* h);
 
 /* ---- Encrypting and verifying in pieces ------------------------------------------------------------------------------
  * Two more kinds of hasher, for the operators that read their message once.  The concatenated pieces give, byte for
- * byte, what the one-shot calls give.  Sign and the decryptions stay one-shot: sign reads the message twice, and a
- * decryption must not release plaintext before the tag is checked.
+ * byte, what the one-shot calls give.  Sign and the decryptions read their message twice: see "Signing and decrypting
+ * in two passes" below.
  *  - encryption streams (sha3_encrypt, the KEM symmetric half, key_encrypt): each stream holds the tag sponge, a KMAC
  *    stream keyed by ka, and the keystream sponge KMACXOF(ke, "", ., KE), whose first |m| bytes do not depend on |m|.
  *    ke || ka is derived on the device and never leaves it.  capy_hasher_encrypt_update writes the ciphertext of each
@@ -366,6 +366,57 @@ int capy_hasher_encrypt_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index,
 /* ok[i] = 1 iff h' == h and V_i is on the curve; CAPY_ERR_BAD_POINT if any V_i was off the curve (_dev: *d_bad_flag |= 1) */
 int capy_hasher_verify_final(capy_ctx* ctx, capy_hasher* h, uint8_t* ok);
 int capy_hasher_verify_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag);
+
+/* ---- Signing and decrypting in two passes -----------------------------------------------------------------------------
+ * Sign and the decryptions read their message twice: sign needs k, from a first pass over the message, before its "T"
+ * pass; a decryption must not release plaintext before the tag is checked.  The caller feeds every message twice, cut
+ * into pieces any way it likes in each pass (empty pieces allowed), with capy_hasher_next_pass between the passes.  The
+ * engine checks that both passes carried the same bytes: without that check a sign pass 2 over other bytes would sign
+ * them with the k of pass 1, and two signatures sharing k give the private key away; a decryption would release bytes
+ * that were never authenticated.
+ *  - sign streams: s = 4 BE(KMACXOF(pw, "", 448, "SK")) mod r per item, then the "N" KMAC stream keyed by BE56(s).  Both
+ *    passes take capy_hasher_update.  capy_hasher_next_pass (ok = NULL) closes "N" -> N1, k, U = [k]G, and starts "T"
+ *    keyed by U.x and a second "N" stream; pass 2 feeds both.  capy_hasher_sign_final: ok[i] = 1 iff the second "N"
+ *    output equals N1, and then (h, z) are those of capy_ed448_sign_batch; ok[i] = 0: h and z of item i are zero bytes
+ *    and nothing derived from its k leaves the device.
+ *  - decryption streams (sha3_decrypt, the KEM symmetric half, key_decrypt): (ke || ka) is derived on the device as the
+ *    one-shot calls do, and the expected tags are taken at creation.  Pass 1 takes the ciphertext through
+ *    capy_hasher_update and writes nothing.  capy_hasher_next_pass gives the verdict, ok[i] = 1 iff the tag over the
+ *    plaintext matched (NULL allowed).  Pass 2 takes capy_hasher_decrypt_update: the plaintext for items whose verdict was
+ *    1, the ciphertext for the others.  capy_hasher_decrypt_final: ok[i] = the verdict && the tag over the plaintext of
+ *    pass 2 matched too; treat the plaintext of an item with ok[i] = 0 as unauthenticated.
+ *  - key_decrypt: an off-curve Z_i fails its item, and capy_hasher_next_pass and capy_hasher_decrypt_final return
+ *    CAPY_ERR_BAD_POINT (_dev: *d_bad_flag |= 1), as capy_ed448_key_decrypt_batch does.
+ *  - every call out of order is CAPY_ERR_BAD_ARG: a second next_pass, decrypt_update in pass 1, capy_hasher_update on a
+ *    decryption stream in pass 2, a final before next_pass, any call after the final, capy_hasher_final /
+ *    verify_final / encrypt_update on these kinds, the calls of this block on the other kinds, a hasher of another ctx.
+ *    The pass is kept per device, like the finished state.  A next_pass that fails (e.g. CAPY_ERR_OOM) leaves the
+ *    streams of its devices unusable: free them.
+ *  - d_bits = 224 is refused (CAPY_ERR_BAD_ARG) as for the other streams; a bad variant: CAPY_ERR_BAD_ARG.
+ *  - capy_hasher_free zeroes s, k, N1, the key-derived states and the carries (which hold plaintext). */
+/* sign streams, one per password; blocking */
+int capy_ed448_sign_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off, uint64_t n,
+                               capy_hasher** out);
+/* sponge AE open streams (variant CAPY_AE_SHA3 | CAPY_AE_KEM); nonces: n * nonce_len bytes; tag64: n * 64; blocking */
+int capy_sponge_decrypt_stream_new(capy_ctx* ctx, int d_bits, int variant, const uint8_t* pws, const uint64_t* pw_off,
+                                   const uint8_t* nonces, uint64_t nonce_len, const uint8_t* tag64, uint64_t n,
+                                   capy_hasher** out);
+/* key_decrypt streams: z_xy112 the Z of every message, tag56: n * 56; blocking */
+int capy_ed448_key_decrypt_stream_new(capy_ctx* ctx, int d_bits, const uint8_t* pws, const uint64_t* pw_off,
+                                      const uint8_t* z_xy112, const uint8_t* tag56, uint64_t n, capy_hasher** out);
+/* the end of pass 1 (see above) */
+int capy_hasher_next_pass(capy_ctx* ctx, capy_hasher* h, uint8_t* ok);
+int capy_hasher_next_pass_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag);
+/* decryption pass 2: out[off[i] .. off[i+1]) = the plaintext of ct[off[i] .. off[i+1]), or the ciphertext for an item
+ * whose verdict was 0; out may alias ct */
+int capy_hasher_decrypt_update(capy_ctx* ctx, capy_hasher* h, const uint8_t* ct, const uint64_t* off, uint8_t* out);
+int capy_hasher_decrypt_update_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, const uint8_t* d_ct,
+                                   const uint64_t* d_off, uint8_t* d_out);
+int capy_hasher_decrypt_final(capy_ctx* ctx, capy_hasher* h, uint8_t* ok);
+int capy_hasher_decrypt_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_ok, int* d_bad_flag);
+int capy_hasher_sign_final(capy_ctx* ctx, capy_hasher* h, uint8_t* h56, uint8_t* z_be56, uint8_t* ok);
+int capy_hasher_sign_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_h56, uint8_t* d_z_be56,
+                               uint8_t* d_ok);
 
 #ifdef __cplusplus
 }

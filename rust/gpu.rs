@@ -160,6 +160,27 @@ extern "C" {
     fn capy_hasher_verify_final(ctx: *mut CapyCtx, h: *mut CapyHasher, ok: *mut u8) -> c_int;
     fn capy_hasher_verify_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
         d_ok: *mut u8, d_bad_flag: *mut c_int) -> c_int;
+    fn capy_ed448_sign_stream_new(ctx: *mut CapyCtx, d_bits: c_int, pws: *const u8, pw_off: *const u64, n: u64,
+        out: *mut *mut CapyHasher) -> c_int;
+    fn capy_sponge_decrypt_stream_new(ctx: *mut CapyCtx, d_bits: c_int, variant: c_int, pws: *const u8,
+        pw_off: *const u64, nonces: *const u8, nonce_len: u64, tag64: *const u8, n: u64,
+        out: *mut *mut CapyHasher) -> c_int;
+    fn capy_ed448_key_decrypt_stream_new(ctx: *mut CapyCtx, d_bits: c_int, pws: *const u8, pw_off: *const u64,
+        z_xy112: *const u8, tag56: *const u8, n: u64, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_hasher_next_pass(ctx: *mut CapyCtx, h: *mut CapyHasher, ok: *mut u8) -> c_int;
+    fn capy_hasher_next_pass_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_ok: *mut u8, d_bad_flag: *mut c_int) -> c_int;
+    fn capy_hasher_decrypt_update(ctx: *mut CapyCtx, h: *mut CapyHasher, ct: *const u8, off: *const u64,
+        out: *mut u8) -> c_int;
+    fn capy_hasher_decrypt_update_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_ct: *const u8, d_off: *const u64, d_out: *mut u8) -> c_int;
+    fn capy_hasher_decrypt_final(ctx: *mut CapyCtx, h: *mut CapyHasher, ok: *mut u8) -> c_int;
+    fn capy_hasher_decrypt_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_ok: *mut u8, d_bad_flag: *mut c_int) -> c_int;
+    fn capy_hasher_sign_final(ctx: *mut CapyCtx, h: *mut CapyHasher, h56: *mut u8, z_be56: *mut u8,
+        ok: *mut u8) -> c_int;
+    fn capy_hasher_sign_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
+        d_h56: *mut u8, d_z_be56: *mut u8, d_ok: *mut u8) -> c_int;
 }
 
 const CAPY_AE_SHA3: c_int = 0;
@@ -684,6 +705,104 @@ impl Drop for VerifyStream {
     }
 }
 
+/// n signatures whose messages are fed twice in pieces (`Gpu::sign_stream`): `update` in pass 1, `next_pass`, `update`
+/// with the same bytes in pass 2, then `finish`.  An item whose two passes differ gets `OperationResultNotSet` and no
+/// signature.
+pub struct SignStream {
+    ctx: *mut CapyCtx,
+    h: *mut CapyHasher,
+    n: usize,
+}
+unsafe impl Send for SignStream {}
+
+impl SignStream {
+    pub fn update(&mut self, pieces: &[&[u8]]) -> Result<(), OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        status(unsafe { capy_hasher_update(self.ctx, self.h, data.as_ptr(), off.as_ptr()) })
+    }
+
+    pub fn next_pass(&mut self) -> Result<(), OperationError> {
+        status(unsafe { capy_hasher_next_pass(self.ctx, self.h, std::ptr::null_mut()) })
+    }
+
+    pub fn finish(&mut self) -> Vec<Result<Signature, OperationError>> {
+        let (mut h, mut z, mut ok) = (vec![0u8; self.n * 56 + 1], vec![0u8; self.n * 56 + 1], vec![0u8; self.n + 1]);
+        let rc = unsafe { capy_hasher_sign_final(self.ctx, self.h, h.as_mut_ptr(), z.as_mut_ptr(), ok.as_mut_ptr()) };
+        (0..self.n)
+            .map(|i| {
+                if rc != 0 || ok[i] == 0 {
+                    return Err(OperationError::OperationResultNotSet);
+                }
+                let z_scalar = Scalar { val: crypto_bigint::U448::from_be_slice(&z[56 * i..56 * i + 56]) };
+                Ok(Signature { h: h[56 * i..56 * i + 56].to_vec(), z: z_scalar })
+            })
+            .collect()
+    }
+}
+
+impl Drop for SignStream {
+    fn drop(&mut self) {
+        unsafe { capy_hasher_free(self.h) }
+    }
+}
+
+/// n decryptions whose ciphertexts are fed twice in pieces (`Gpu::sha3_decrypt_stream` / `key_decrypt_stream`):
+/// `update` in pass 1, `next_pass` (the verdicts), `decrypt` with the same bytes in pass 2 (plaintext where the verdict
+/// was good, the ciphertext elsewhere), then `finish`.
+pub struct DecryptStream {
+    ctx: *mut CapyCtx,
+    h: *mut CapyHasher,
+    n: usize,
+    key: bool, // key_decrypt (KeyDecryptionError) rather than sha3_decrypt (SHA3DecryptionFailure)
+}
+unsafe impl Send for DecryptStream {}
+
+impl DecryptStream {
+    pub fn update(&mut self, pieces: &[&[u8]]) -> Result<(), OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        status(unsafe { capy_hasher_update(self.ctx, self.h, data.as_ptr(), off.as_ptr()) })
+    }
+
+    fn verdicts(&self, rc: c_int, ok: &[u8]) -> Vec<Result<(), OperationError>> {
+        let err = || if self.key { OperationError::KeyDecryptionError } else { OperationError::SHA3DecryptionFailure };
+        (0..self.n).map(|i| if rc != 0 || ok[i] == 0 { Err(err()) } else { Ok(()) }).collect()
+    }
+
+    pub fn next_pass(&mut self) -> Vec<Result<(), OperationError>> {
+        let mut ok = vec![0u8; self.n + 1];
+        let rc = unsafe { capy_hasher_next_pass(self.ctx, self.h, ok.as_mut_ptr()) };
+        self.verdicts(rc, &ok)
+    }
+
+    pub fn decrypt(&mut self, pieces: &[&[u8]]) -> Result<Vec<Vec<u8>>, OperationError> {
+        if pieces.len() != self.n {
+            return Err(OperationError::OperationResultNotSet);
+        }
+        let (data, off) = pack(pieces.iter().copied());
+        let mut out = vec![0u8; data.len()];
+        status(unsafe { capy_hasher_decrypt_update(self.ctx, self.h, data.as_ptr(), off.as_ptr(), out.as_mut_ptr()) })?;
+        Ok((0..self.n).map(|i| out[off[i] as usize..off[i + 1] as usize].to_vec()).collect())
+    }
+
+    pub fn finish(&mut self) -> Vec<Result<(), OperationError>> {
+        let mut ok = vec![0u8; self.n + 1];
+        let rc = unsafe { capy_hasher_decrypt_final(self.ctx, self.h, ok.as_mut_ptr()) };
+        self.verdicts(rc, &ok)
+    }
+}
+
+impl Drop for DecryptStream {
+    fn drop(&mut self) {
+        unsafe { capy_hasher_free(self.h) }
+    }
+}
+
 impl Gpu {
     /// One `sha3_encrypt` per password whose plaintext arrives in pieces (blocking); the 512 nonce bytes per message are
     /// drawn with the reference's `get_random_bytes`.  D224 is refused (capy_gpu.h: quirk Q7).
@@ -741,5 +860,52 @@ impl Gpu {
 impl Drop for Gpu {
     fn drop(&mut self) {
         unsafe { capy_gpu_destroy(self.ctx) }
+    }
+}
+
+impl Gpu {
+    /// `sign` of messages fed twice in pieces (blocking creation).  D224 is refused (capy_gpu.h: quirk Q7).
+    pub fn sign_stream(&self, keys: &[&KeyPair], d: SecParam) -> Result<SignStream, OperationError> {
+        let (pd, po) = pack(keys.iter().map(|k| k.priv_key.as_slice()));
+        let mut h = std::ptr::null_mut();
+        status(unsafe { capy_ed448_sign_stream_new(self.ctx, d as c_int, pd.as_ptr(), po.as_ptr(), keys.len() as u64, &mut h) })?;
+        Ok(SignStream { ctx: self.ctx, h, n: keys.len() })
+    }
+
+    /// `sha3_decrypt` of ciphertexts fed twice in pieces; every nonce has `nonces[0].len()` bytes and every tag 64.
+    pub fn sha3_decrypt_stream(&self, pws: &[&[u8]], nonces: &[&[u8]], tags: &[&[u8]], d: SecParam)
+                               -> Result<DecryptStream, OperationError> {
+        let n = pws.len();
+        let nonce_len = nonces.first().map_or(0, |z| z.len());
+        if nonces.len() != n || tags.len() != n || nonces.iter().any(|z| z.len() != nonce_len) || tags.iter().any(|t| t.len() != 64) {
+            return Err(OperationError::SHA3DecryptionFailure);
+        }
+        let (pd, po) = pack(pws.iter().copied());
+        let (zd, _) = pack(nonces.iter().copied());
+        let (td, _) = pack(tags.iter().copied());
+        let mut h = std::ptr::null_mut();
+        status(unsafe {
+            capy_sponge_decrypt_stream_new(self.ctx, d as c_int, CAPY_AE_SHA3, pd.as_ptr(), po.as_ptr(), zd.as_ptr(),
+                                           nonce_len as u64, td.as_ptr(), n as u64, &mut h)
+        })?;
+        Ok(DecryptStream { ctx: self.ctx, h, n, key: false })
+    }
+
+    /// `key_decrypt` of ciphertexts fed twice in pieces; `asym_nonces[i]` is Z_i (112 bytes), every tag 56 bytes.
+    pub fn key_decrypt_stream(&self, pws: &[&[u8]], asym_nonces: &[&[u8]], tags: &[&[u8]], d: SecParam)
+                              -> Result<DecryptStream, OperationError> {
+        let n = pws.len();
+        if asym_nonces.len() != n || tags.len() != n || asym_nonces.iter().any(|z| z.len() != 112) || tags.iter().any(|t| t.len() != 56) {
+            return Err(OperationError::KeyDecryptionError);
+        }
+        let (pd, po) = pack(pws.iter().copied());
+        let (zd, _) = pack(asym_nonces.iter().copied());
+        let (td, _) = pack(tags.iter().copied());
+        let mut h = std::ptr::null_mut();
+        status(unsafe {
+            capy_ed448_key_decrypt_stream_new(self.ctx, d as c_int, pd.as_ptr(), po.as_ptr(), zd.as_ptr(), td.as_ptr(), n as u64,
+                                              &mut h)
+        })?;
+        Ok(DecryptStream { ctx: self.ctx, h, n, key: true })
     }
 }
