@@ -22,11 +22,15 @@ R = E.R
 GUARD = 4096
 
 
-def _matrix():
-    spec = importlib.util.spec_from_file_location("dispatch_matrix", os.path.join(HERE, "test_dispatch_matrix_gpu.py"))
+def _load(name):
+    spec = importlib.util.spec_from_file_location(name, os.path.join(HERE, name + ".py"))
     mod = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(mod)
     return mod
+
+
+def _matrix():
+    return _load("test_dispatch_matrix_gpu")
 
 
 @pytest.fixture(scope="module")
@@ -110,9 +114,14 @@ def test_key_encrypt_prepared_equals_key_encrypt_and_decrypts(engine, signers, d
     assert ok.all() and np.array_equal(out, msgs)
 
 
+TORSION_S = 0x1234567890ABCDEF
+# the secret scalar s of each special key and the order t of its torsion component: a signature made with s verifies iff
+# BE(h) = 0 (mod t) (quirk Q10: V is multiplied by the unreduced h)
+SIGNERS = {"G": (1, 1), "identity": (0, 1), "torsion": (TORSION_S, 4)}
+
+
 def _special_keys():
-    s = 0x1234567890ABCDEF
-    torsion = E.point_add(E.scalar_mult(s, E.GENERATOR), (1, 0))  # (1, 0) has order 4
+    torsion = E.point_add(E.scalar_mult(TORSION_S, E.GENERATOR), (1, 0))  # (1, 0) has order 4
     return {"G": (E.GENERATOR, 1), "identity": (E.IDENTITY, 1), "torsion": (torsion, 0)}
 
 
@@ -129,13 +138,10 @@ def test_special_keys_same_bytes(engine, oracle, signer, which):
     h = rnd.integers(0, 256, size=(n, 56), dtype=np.uint8)
     z = rnd.integers(0, 256, size=(n, 56), dtype=np.uint8)
     k = rnd.integers(0, 256, size=n * 56, dtype=np.uint8)
-    if which == "G":  # some valid signatures against G: the secret scalar is 1 (z = k - h mod r with U = [k]G)
-        for i in range(0, n, 3):
-            kk = int.from_bytes(k[56 * i:56 * i + 56].tobytes(), "big") % R
-            ux = E.point_to_bytes(E.scalar_mult(kk, E.GENERATOR))[:56]
-            hh = oracle.kmac_xof(ux, msgs[int(moff[i]):int(moff[i + 1])].tobytes(), 448, b"T", d)
-            h[i] = np.frombuffer(hh, np.uint8)
-            z[i] = np.frombuffer(((kk - int.from_bytes(hh, "big")) % R).to_bytes(56, "big"), np.uint8)
+    if which in SIGNERS:  # valid signatures on every third item, signed the reference's way with the key's s
+        s, t = SIGNERS[which]
+        signed = [msgs[int(moff[i]):int(moff[i + 1])].tobytes() for i in range(0, n, 3)]
+        h[::3], z[::3] = _load("test_ed448_torsion_gpu").sign_as(oracle, s, signed, d, rnd, t, range(len(signed)))
     pubs = np.frombuffer(pub * n, np.uint8)
     with engine.ed448_pub_prepare(pub) as key:
         assert key.uses_comb == bool(comb)
@@ -143,7 +149,7 @@ def test_special_keys_same_bytes(engine, oracle, signer, which):
         rc, want = engine.ed448_verify(pubs, msgs, moff, h, z, d)
         assert rc == 0 and np.array_equal(ok, want)
         assert np.array_equal(ok, oracle.verify_batch(pubs, msgs, moff, h, z, d, threads=0))
-        if which == "G":
+        if which in SIGNERS:
             assert ok[::3].all()
         ct, tag, zp = engine.ed448_key_encrypt_prepared(key, k, msgs, moff, d)
         rc, ct0, tag0, z0 = engine.ed448_key_encrypt(pubs, k, msgs, moff, d)

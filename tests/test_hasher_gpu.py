@@ -262,6 +262,10 @@ def _kernels(fn, tmp_path):
 
     torch.cuda.synchronize()
     with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        # one device activity before fn: the profiler requests its first activity buffer when the first record arrives,
+        # and device records that come before the buffer is in place are lost (fn's first kernel, at times)
+        torch.zeros(1, device="cuda")
+        torch.cuda.synchronize()
         fn()
         torch.cuda.synchronize()
     path = tmp_path / "trace.json"
