@@ -109,6 +109,11 @@ SIGNATURES = {
     "capy_hasher_decrypt_final_dev": (i32, [vp, vp, i32, vp, u8p, vp]),
     "capy_hasher_sign_final": (i32, [vp, vp, u8p, u8p, u8p]),
     "capy_hasher_sign_final_dev": (i32, [vp, vp, i32, vp, u8p, u8p, u8p]),
+    "capy_hasher_export_size": (i32, [vp, C.POINTER(u64)]),
+    "capy_hasher_export": (i32, [vp, vp, u8p, u64]),
+    "capy_hasher_blob_info": (i32, [u8p, u64, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(u64)]),
+    "capy_hasher_import": (i32, [vp, u8p, u64, C.POINTER(vp)]),
+    "capy_hasher_fork": (i32, [vp, vp, u64p, u64, C.POINTER(vp)]),
 }
 
 

@@ -135,6 +135,11 @@ class Gpu:
         kd, ko = pack(keys)
         return SpongeStream(self.engine.kmac_xof_hasher(kd, ko, s, int(d)), int(d))
 
+    def resume_stream(self, blob: bytes) -> "SpongeStream":
+        """the streams of a blob from SpongeStream.export, on this Gpu's devices"""
+        h = self.engine.import_hasher(np.frombuffer(blob, dtype=np.uint8))
+        return SpongeStream(h, h.d)
+
     def sha3_encrypt_stream(self, pws: Sequence[bytes], d: SecParam,
                             nonces: Optional[Sequence[bytes]] = None) -> "EncryptStream":
         """one sha3_encrypt per password whose plaintext arrives in pieces: update() returns the ciphertext pieces,
@@ -455,6 +460,18 @@ class SpongeStream:
         """SHA3-d: the digests (l must be None or d).  KMACXOF: l output bits per stream (default d)."""
         out = self.hasher.final(self.d if l is None else l)
         return [r.tobytes() for r in out]
+
+    def export(self) -> bytes:
+        """the streams as a blob for Gpu.resume_stream (a KMACXOF blob is as secret as its keys)"""
+        return self.hasher.export().tobytes()
+
+    def fork(self, indices: Sequence[int]) -> "SpongeStream":
+        """new streams on the same engine: stream j starts as a copy of stream indices[j] of this one, which is unchanged"""
+        return SpongeStream(self.hasher.fork(list(indices)), self.d)
+
+    def copy(self) -> "SpongeStream":
+        """fork(range(n)): copy().finish() is the digest so far, and this stream goes on"""
+        return self.fork(range(self.hasher.n))
 
     def close(self) -> None:
         self.hasher.close()

@@ -6,6 +6,7 @@
 // prefix block of cSHAKE/KMAC; every byte that is absorbed per item is produced on the device.
 #include <algorithm>
 #include <cmath>
+#include <cstring>
 #include <cstdlib>
 #include <memory>
 #include <thread>
@@ -659,7 +660,8 @@ static bool chain_cut(int sm_count, uint64_t n, uint64_t absorb_blocks, uint64_t
 // jobs = 1, J0 alone (and, with `resume`, as resumable streams)
 static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, const SpongeJob& J0, const SpongeJob& J1,
                              bool data_dependent, uint32_t jobs = 2, const SpongeResume* resume = nullptr,
-                             const SpongeSqueeze* squeeze = nullptr, const SpongeDual* dual = nullptr) {
+                             const SpongeSqueeze* squeeze = nullptr, const SpongeDual* dual = nullptr,
+                             const SpongeCopy* copy = nullptr) {
   const uint32_t nb = (uint32_t)((J0.n + 127) / 128);
   uint32_t* sync = (uint32_t*)scratch_get(dc, stream, kChainSync, ((size_t)nb + 1) * sizeof(uint32_t));
   if (!sync) return CAPY_ERR_OOM;
@@ -673,6 +675,7 @@ static int launch_chain_jobs(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t stream, 
   C.resume = resume ? *resume : SpongeResume{};
   C.squeeze = squeeze ? *squeeze : SpongeSqueeze{};
   C.dual = dual ? *dual : SpongeDual{};
+  C.copy = copy ? *copy : SpongeCopy{};
   return with_lanes<9, 13, 17, 18, 19, 21>(job_lanes(J0), [&](auto L) {
     sponge_chain_kernel<decltype(L)::value><<<jobs * nb, 128, 0, stream>>>(C);
     ctx->launches++;
@@ -1265,6 +1268,170 @@ int hasher_create(capy_ctx* ctx, int d_bits, int kind, uint64_t n, capy_hasher**
   return CAPY_OK;
 }
 
+// ---- checkpoints and forks of SHA3-d / KMACXOF streams (capy_hasher_export / _import / _fork) -------------------------
+// The blob format is decided here alone; capy_gpu.h documents it.  Header (64 bytes, little-endian): "CAPYHSTR", u32
+// version, u32 kind (0 SHA3-d, 1 KMACXOF), u32 d_bits, u32 rate, u32 record bytes, u32 zero, u64 n, zeros; then n records
+// of 208 + rate bytes (SpongeCopy).  Every copy is one launch of the copy path of sponge_chain_kernel.
+constexpr uint64_t kBlobHeader = 64;
+constexpr uint32_t kBlobVersion = 1;
+static const char kBlobMagic[8] = {'C', 'A', 'P', 'Y', 'H', 'S', 'T', 'R'};
+
+static uint64_t blob_record(uint32_t rate) { return 208ull + rate; }
+// the kinds a blob can hold, and only while no device has finished its items
+static bool hasher_portable(const capy_hasher* h) {
+  return (h->kind == kSha3Stream || h->kind == kKmacStream) && !hasher_any_finished(h);
+}
+static uint64_t get_le(const uint8_t* p, int bytes) {
+  uint64_t v = 0;
+  for (int k = bytes - 1; k >= 0; k--) v = (v << 8) | p[k];
+  return v;
+}
+static void put_le(uint8_t* p, uint64_t v, int bytes) {
+  for (int k = 0; k < bytes; k++) p[k] = (uint8_t)(v >> (8 * k));
+}
+
+struct BlobHeader {
+  int kind;  // kSha3Stream or kKmacStream
+  int d_bits;
+  uint32_t rate;
+  uint64_t n;
+};
+static int blob_parse(const uint8_t* blob, uint64_t blob_len, BlobHeader* b) {
+  if (!blob || blob_len < kBlobHeader || memcmp(blob, kBlobMagic, 8) != 0) return CAPY_ERR_BAD_ARG;
+  const uint32_t version = (uint32_t)get_le(blob + 8, 4), kind = (uint32_t)get_le(blob + 12, 4);
+  const int d = (int)get_le(blob + 16, 4);
+  const uint32_t rate = (uint32_t)get_le(blob + 20, 4), rec = (uint32_t)get_le(blob + 24, 4);
+  if (version != kBlobVersion || kind > 1 || !valid_secparam(d) || (kind == 1 && d == 224)) return CAPY_ERR_BAD_ARG;
+  const uint32_t want = kind == 1 ? cshake_rate(d) : sha3_rate(d);
+  if (rate != want || rec != blob_record(rate) || get_le(blob + 28, 4) != 0) return CAPY_ERR_BAD_ARG;
+  for (uint64_t k = 40; k < kBlobHeader; k++)
+    if (blob[k]) return CAPY_ERR_BAD_ARG;
+  const uint64_t n = get_le(blob + 32, 8);
+  if (n > (blob_len - kBlobHeader) / rec || blob_len - kBlobHeader != n * rec) return CAPY_ERR_BAD_ARG;
+  b->kind = kind == 1 ? kKmacStream : kSha3Stream;
+  b->d_bits = d;
+  b->rate = rate;
+  b->n = n;
+  return CAPY_OK;
+}
+
+// the streams of device k from item j0 on (indices on that device), as a side of a copy
+static SpongeStreams hasher_side(const capy_hasher* h, int k, uint64_t j0) {
+  SpongeStreams s{};
+  s.state = h->d_state[k] + j0;
+  s.carry = h->d_carry[k] + j0 * h->rate;
+  s.totals = h->d_total[k] + j0;
+  s.state_n = hasher_items(h, k);
+  return s;
+}
+static SpongeStreams record_side(uint8_t* rec) {
+  SpongeStreams s{};
+  s.rec = rec;
+  return s;
+}
+
+// n streams from P.from to P.to at the rate of h's operator: one launch of the copy path
+static int launch_copy(capy_ctx* ctx, DeviceCtx& dc, cudaStream_t st, const capy_hasher* h, uint64_t n, SpongeCopy P) {
+  if (n == 0) return CAPY_OK;
+  SpongeJob J = hasher_operator(h);
+  J.n = n;
+  P.on = 1;
+  return launch_chain_jobs(ctx, dc, st, J, J, false, 1, nullptr, nullptr, nullptr, &P);
+}
+
+// a device copy of v (kept alive by p) on st; v must outlive the copy
+static int upload(capy_ctx* ctx, cudaStream_t st, DevPtr<uint64_t>& p, const std::vector<uint64_t>& v) {
+  if (v.empty()) return CAPY_OK;
+  if (dev_alloc(p, v.size() * 8) != cudaSuccess) {
+    cudaGetLastError();
+    return CAPY_ERR_OOM;
+  }
+  CAPY_CUDA(ctx, cudaMemcpyAsync(p.get(), v.data(), v.size() * 8, cudaMemcpyHostToDevice, st));
+  return CAPY_OK;
+}
+
+// Item j of f starts as a copy of item src[j] of h (same ctx).  A destination device b copies the sources it holds itself
+// in one launch with both maps.  Sources on another device a are gathered there into compact records, moved to b with one
+// peer copy and scattered.  Blocking: every phase ends in stream synchronisations before the next one reads its results.
+static int fork_items(capy_ctx* ctx, const capy_hasher* h, const uint64_t* src, capy_hasher* f) {
+  const size_t nd = ctx->devs.size();
+  const uint64_t rec = blob_record(h->rate);
+  // s_loc[a][b] / d_loc[a][b]: the sources on device a of the destinations on device b, as indices on a and on b
+  std::vector<std::vector<std::vector<uint64_t>>> s_loc(nd, std::vector<std::vector<uint64_t>>(nd)), d_loc = s_loc;
+  for (size_t b = 0; b < nd; b++)
+    for (uint64_t j = f->first[b]; j < f->first[b + 1]; j++) {
+      const size_t a = (size_t)(std::upper_bound(h->first.begin(), h->first.end(), src[j]) - h->first.begin()) - 1;
+      s_loc[a][b].push_back(src[j] - h->first[a]);
+      d_loc[a][b].push_back(j - f->first[b]);
+    }
+  std::vector<std::vector<DevPtr<uint8_t>>> moved(nd);  // [a][b]: records gathered on a for b
+  std::vector<std::vector<DevPtr<uint64_t>>> maps(nd);
+  for (size_t a = 0; a < nd; a++) {
+    moved[a].resize(nd);
+    maps[a].resize(2 * nd);
+  }
+  for (size_t a = 0; a < nd; a++) {  // gather
+    DeviceCtx& dc = ctx->devs[a];
+    std::lock_guard<std::mutex> lk(*dc.mu);
+    DeviceGuard g(dc.dev);
+    const cudaStream_t st = dc.streams[0];
+    for (size_t b = 0; b < nd; b++) {
+      const uint64_t cnt = s_loc[a][b].size();
+      if (b == a || cnt == 0) continue;
+      if (dev_alloc(moved[a][b], cnt * rec) != cudaSuccess) {
+        cudaGetLastError();
+        return CAPY_ERR_OOM;
+      }
+      int rc = upload(ctx, st, maps[a][b], s_loc[a][b]);
+      SpongeCopy P{};
+      P.src = maps[a][b].get();
+      P.from = hasher_side(h, (int)a, 0);
+      P.to = record_side(moved[a][b].get());
+      if (!rc) rc = launch_copy(ctx, dc, st, h, cnt, P);
+      if (rc) return rc;
+    }
+    CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+  }
+  for (size_t b = 0; b < nd; b++) {  // move and scatter, or copy in place
+    DeviceCtx& dc = ctx->devs[b];
+    std::lock_guard<std::mutex> lk(*dc.mu);
+    DeviceGuard g(dc.dev);
+    const cudaStream_t st = dc.streams[0];
+    std::vector<DevPtr<uint8_t>> here(nd);
+    for (size_t a = 0; a < nd; a++) {
+      const uint64_t cnt = s_loc[a][b].size();
+      if (cnt == 0) continue;
+      SpongeCopy P{};
+      P.to = hasher_side(f, (int)b, 0);
+      int rc = CAPY_OK;
+      if (cnt < hasher_items(f, (int)b)) rc = upload(ctx, st, maps[b][nd + a], d_loc[a][b]);  // else the identity
+      P.dst = maps[b][nd + a].get();
+      if (a == b) {
+        if (!rc) rc = upload(ctx, st, maps[b][b], s_loc[b][b]);
+        P.src = maps[b][b].get();
+        P.from = hasher_side(h, (int)b, 0);
+      } else {
+        if (!rc && dev_alloc(here[a], cnt * rec) != cudaSuccess) {
+          cudaGetLastError();
+          rc = CAPY_ERR_OOM;
+        }
+        if (!rc) {
+          const cudaError_t e = cudaMemcpyPeerAsync(here[a].get(), dc.dev, moved[a][b].get(), ctx->devs[a].dev, cnt * rec, st);
+          if (e != cudaSuccess) rc = cuda_fail(ctx, e, "cudaMemcpyPeerAsync");
+        }
+        P.from = record_side(here[a].get());
+      }
+      if (!rc) rc = launch_copy(ctx, dc, st, h, cnt, P);
+      if (rc) {
+        cudaStreamSynchronize(st);  // (the buffers of this device go back after the work that reads them)
+        return rc;
+      }
+    }
+    CAPY_CUDA(ctx, cudaStreamSynchronize(st));
+  }
+  return CAPY_OK;
+}
+
 }  // namespace capy
 
 using namespace capy;
@@ -1795,6 +1962,98 @@ int capy_hasher_sign_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, voi
   if (m == 0) return CAPY_OK;
   CAPY_DEV_PROLOGUE
   return sign_stream_final(ctx, dc, st, h, d_h56, d_z_be56, d_ok);
+}
+
+// ---- checkpoints and forks of SHA3-d / KMACXOF streams --------------------------------------------------------------
+int capy_hasher_export_size(const capy_hasher* h, uint64_t* bytes) {
+  if (!h || !bytes || !hasher_portable(h)) return CAPY_ERR_BAD_ARG;
+  *bytes = kBlobHeader + h->n * blob_record(h->rate);
+  return CAPY_OK;
+}
+
+int capy_hasher_export(capy_ctx* ctx, const capy_hasher* h, uint8_t* blob, uint64_t blob_len) {
+  if (hasher_check(ctx, h) || !hasher_portable(h) || !blob) return CAPY_ERR_BAD_ARG;
+  const uint64_t rec = blob_record(h->rate);
+  if (blob_len < kBlobHeader + h->n * rec) return CAPY_ERR_BAD_ARG;
+  uint8_t hdr[kBlobHeader] = {};
+  memcpy(hdr, kBlobMagic, 8);
+  put_le(hdr + 8, kBlobVersion, 4);
+  put_le(hdr + 12, h->kind == kKmacStream ? 1 : 0, 4);
+  put_le(hdr + 16, (uint64_t)h->d_bits, 4);
+  put_le(hdr + 20, h->rate, 4);
+  put_le(hdr + 24, rec, 4);
+  put_le(hdr + 32, h->n, 8);
+  memcpy(blob, hdr, kBlobHeader);
+  if (h->n == 0) return CAPY_OK;
+  auto chunks = [&](Range sh) {
+    return split_items(nullptr, rec, sh.i0, sh.i1, chunk_count((sh.i1 - sh.i0) * rec, sh.i1 - sh.i0), 0);
+  };
+  return run_host_call(ctx, hasher_shards(h), chunks, false, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    uint8_t* d_rec = io.out(blob + kBlobHeader, rec);
+    if (io.rc()) return io.rc();
+    SpongeCopy P{};
+    P.from = hasher_side(h, dc.index, io.i0() - h->first[dc.index]);
+    P.to = record_side(d_rec);
+    return launch_copy(ctx, dc, st, h, io.n(), P);
+  });
+}
+
+int capy_hasher_blob_info(const uint8_t* blob, uint64_t blob_len, int* kind, int* d_bits, uint64_t* n) {
+  BlobHeader b;
+  const int rc = blob_parse(blob, blob_len, &b);
+  if (rc) return rc;
+  if (kind) *kind = b.kind == kKmacStream ? 1 : 0;
+  if (d_bits) *d_bits = b.d_bits;
+  if (n) *n = b.n;
+  return CAPY_OK;
+}
+
+int capy_hasher_import(capy_ctx* ctx, const uint8_t* blob, uint64_t blob_len, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  BlobHeader b;
+  if (!ctx || blob_parse(blob, blob_len, &b)) return CAPY_ERR_BAD_ARG;
+  capy_hasher* h = nullptr;
+  int rc = hasher_create(ctx, b.d_bits, b.kind, b.n, &h);
+  if (rc) return rc;
+  const uint64_t rec = blob_record(b.rate);
+  auto chunks = [&](Range sh) {
+    return split_items(nullptr, rec, sh.i0, sh.i1, chunk_count((sh.i1 - sh.i0) * rec, sh.i1 - sh.i0), 0);
+  };
+  // a record with a non-zero carry tail raises the chunk's flag, which run_host_call reports as a bad point
+  rc = run_host_call(ctx, hasher_shards(h), chunks, true, [&](DeviceCtx& dc, cudaStream_t st, HostChunk& io) -> int {
+    const uint8_t* d_rec = io.in(blob + kBlobHeader, rec);
+    if (io.rc()) return io.rc();
+    SpongeCopy P{};
+    P.from = record_side(const_cast<uint8_t*>(d_rec));
+    P.to = hasher_side(h, dc.index, io.i0() - h->first[dc.index]);
+    P.bad_tail = io.d_flag();
+    return launch_copy(ctx, dc, st, h, io.n(), P);
+  });
+  if (rc) {
+    capy_hasher_free(h);
+    return rc == CAPY_ERR_BAD_POINT ? CAPY_ERR_BAD_ARG : rc;
+  }
+  *out = h;
+  return CAPY_OK;
+}
+
+int capy_hasher_fork(capy_ctx* ctx, const capy_hasher* h, const uint64_t* src, uint64_t m, capy_hasher** out) {
+  if (!out) return CAPY_ERR_BAD_ARG;
+  *out = nullptr;
+  if (hasher_check(ctx, h) || !hasher_portable(h) || (m && !src)) return CAPY_ERR_BAD_ARG;
+  for (uint64_t j = 0; j < m; j++)
+    if (src[j] >= h->n) return CAPY_ERR_BAD_ARG;  // (every m > 0 with n == 0 too)
+  capy_hasher* f = nullptr;
+  int rc = hasher_create(ctx, h->d_bits, h->kind, m, &f);
+  if (rc) return rc;
+  if (m) rc = fork_items(ctx, h, src, f);
+  if (rc) {
+    capy_hasher_free(f);
+    return rc;
+  }
+  *out = f;
+  return CAPY_OK;
 }
 
 void capy_hasher_free(capy_hasher* h) {

@@ -735,6 +735,7 @@ struct SpongeChain {
   SpongeResume resume;  // carry == nullptr: the jobs are not resumable streams
   SpongeSqueeze squeeze;  // resumable streams with two jobs: job 1 is the keystream update of encryption streams
   SpongeDual dual;        // b_state != nullptr: job 0 runs two states in lockstep (sign and decryption streams)
+  SpongeCopy copy;        // on != 0: job 0 copies streams (export, import and fork of hashers)
 };
 // resumable streams (order == nullptr: rank = item), out of line: the cut chains keep their own register allocation
 template <int LANES>
@@ -869,6 +870,39 @@ __device__ __noinline__ void sponge_dual_resume_ool(const SpongeJob& J, const Sp
 template <int LANES>
 constexpr bool kDualLanes = LANES == 17 || LANES == 19 || LANES == 21;
 
+// Copy of stream t (SpongeCopy): the lanes, the total and the carry words go through one at a time, so the path needs
+// few registers.  The record of a stream is 208 + 8 LANES bytes, a multiple of 8: every access is one aligned 8-byte
+// word.  Out of line like the resume path.
+template <int LANES>
+__device__ __noinline__ void sponge_copy_ool(const SpongeCopy* P, uint64_t t) {
+  constexpr uint64_t RATE = 8ull * LANES, REC_WORDS = 26 + LANES;
+  const uint64_t s = P->src ? P->src[t] : t, d = P->dst ? P->dst[t] : t;
+  const SpongeStreams &A = P->from, &B = P->to;
+  const uint64_t* ra = A.state ? nullptr : reinterpret_cast<const uint64_t*>(A.rec) + s * REC_WORDS;
+  uint64_t* rb = B.state ? nullptr : reinterpret_cast<uint64_t*>(B.rec) + d * REC_WORDS;
+#pragma unroll 5
+  for (int k = 0; k < 25; k++) {
+    const uint64_t v = ra ? ra[k] : A.state[(uint64_t)k * A.state_n + s];
+    if (rb) rb[k] = v;
+    else B.state[(uint64_t)k * B.state_n + d] = v;
+  }
+  const uint64_t total = ra ? ra[25] : A.totals[s];
+  if (rb) rb[25] = total;
+  else B.totals[d] = total;
+  const uint64_t* ca = ra ? ra + 26 : reinterpret_cast<const uint64_t*>(A.carry + s * RATE);
+  uint64_t* cb = rb ? rb + 26 : reinterpret_cast<uint64_t*>(B.carry + d * RATE);
+  const uint32_t used = (uint32_t)(total % RATE);
+  uint64_t tail = 0;
+#pragma unroll 1
+  for (uint32_t j = 0; j < (uint32_t)LANES; j++) {
+    const uint64_t v = ca[j];
+    const uint64_t keep = 8 * j + 8 <= used ? ~0ull : 8 * j >= used ? 0ull : (1ull << (8 * (used - 8 * j))) - 1;
+    tail |= v & ~keep;
+    cb[j] = v & keep;
+  }
+  if (tail && ra && P->bad_tail) *P->bad_tail = 1;
+}
+
 template <int LANES>
 __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(const __grid_constant__ SpongeChain C) {
   __shared__ uint32_t ticket_s;
@@ -888,6 +922,7 @@ __global__ void __launch_bounds__(128, CAPY_SPONGE_MINB) sponge_chain_kernel(con
     else if (kDualLanes<LANES> && C.dual.b_state) sponge_dual_resume_ool<LANES>(J, &C.resume, &C.dual, r);  // (job 0 alone)
     else if (C.resume.carry && job) sponge_squeeze_resume_ool<LANES>(J, &C.squeeze, r);  // (only encryption streams have a job 1)
     else if (C.resume.carry) sponge_item_resume_ool<LANES>(J, &C.resume, r);
+    else if (C.copy.on) sponge_copy_ool<LANES>(&C.copy, r);  // (job 0 alone)
     else sponge_item<LANES, true>(J, sponge_rank_item(J, r), r);
   }
   if (!job) {

@@ -100,6 +100,27 @@ struct SpongeDual {
   uint8_t* out;
 };
 
+// Copies of resumable streams (export, import and fork of SHA3-d / KMACXOF capy_hasher batches: job 0 of
+// sponge_chain_kernel alone, J.n items).  Item t reads stream src ? src[t] : t of `from` and writes stream
+// dst ? dst[t] : t of `to`.  A side is either a hasher's buffers (state != nullptr: 25 lanes at state[l * state_n + j],
+// the carry at carry[j * rate ..), totals[j]) or item-major records of 208 + rate bytes at rec (the 25 lanes, the total,
+// the carry).  Carry bytes from total % rate on are written as zero, so a record does not depend on how the stream was
+// cut into pieces; a non-zero one read from records sets *bad_tail.  Kept out of SpongeJob, like SpongeResume.
+struct SpongeStreams {
+  uint64_t* state;
+  uint8_t* carry;
+  uint64_t* totals;
+  uint64_t state_n;
+  uint8_t* rec;
+};
+struct SpongeCopy {
+  const uint64_t* src;  // nullptr: identity
+  const uint64_t* dst;
+  SpongeStreams from, to;
+  int* bad_tail;        // nullptr: not checked
+  uint32_t on;          // 0: not a copy job
+};
+
 // ---- rates in bytes, as the reference computes them ------------------------------------------------------------------
 // SHA3-d capacity in bits: 2d rounded up to the reference's buckets (constants.rs:38-45)
 inline uint32_t sha3_capacity(int d) {

@@ -159,6 +159,24 @@ class Hasher:
             t_out_off.data_ptr() if t_out_off is not None else None, t_out.data_ptr()))
         return t_out
 
+    def export(self) -> np.ndarray:
+        """capy_hasher_export: the streams as a blob (capy_gpu.h: the blob format; a KMACXOF blob is as secret as its
+        keys), to be resumed by Engine.import_hasher in this or another engine (blocking)"""
+        size = C.c_uint64(0)
+        self._engine._check(self._engine.lib.capy_hasher_export_size(self.handle, C.byref(size)))
+        blob = np.zeros(int(size.value), np.uint8)
+        self._engine._check(self._engine.lib.capy_hasher_export(self._engine._ctx, self.handle, _hp(blob), blob.size))
+        return blob
+
+    def fork(self, src) -> "Hasher":
+        """capy_hasher_fork: a new hasher of len(src) streams on the same engine; stream j starts as a copy of stream
+        src[j] of this one, which is unchanged (blocking)"""
+        src = _u64(src)
+        h = C.c_void_p()
+        self._engine._check(self._engine.lib.capy_hasher_fork(self._engine._ctx, self.handle, _hp(src), src.size,
+                                                              C.byref(h)))
+        return Hasher(self._engine, h, int(src.size), self.d, self.kmac)
+
     def close(self):
         if self.handle is not None and self.handle.value:
             self._engine.lib.capy_hasher_free(self.handle)
@@ -310,6 +328,18 @@ class DecryptStream(Hasher):
         return t_ok
 
 
+def hasher_blob_info(blob, lib=None) -> tuple[int, int, int]:
+    """capy_hasher_blob_info (no GPU): (kind, d, n) of a blob from Hasher.export; kind 0 = SHA3-d, 1 = KMACXOF.
+    CapyError(ERR_BAD_ARG) for a malformed header or a length that does not match it."""
+    blob = _u8(blob)
+    lib = lib or B.load()
+    kind, d, n = C.c_int(0), C.c_int(0), C.c_uint64(0)
+    rc = lib.capy_hasher_blob_info(_hp(blob), blob.size, C.byref(kind), C.byref(d), C.byref(n))
+    if rc != B.OK:
+        raise B.CapyError(rc, lib.capy_strerror(rc).decode())
+    return int(kind.value), int(d.value), int(n.value)
+
+
 def _pub_or_key(pub):
     """(pub_xy112 bytes or None, prepared key handle or None) of a PreparedPublicKey or n x 112 key bytes"""
     if isinstance(pub, PreparedPublicKey):
@@ -452,6 +482,14 @@ class Engine:
         self._check(self.lib.capy_kmac_xof_hasher_new(self._ctx, d, _hp(keys), _hp(key_off), n, _hp(cs_a), len(cs_a),
                                                       C.byref(h)))
         return Hasher(self, h, n, d, True)
+
+    def import_hasher(self, blob) -> Hasher:
+        """capy_hasher_import: the streams of a blob from Hasher.export, dealt over this engine's devices (blocking)"""
+        blob = _u8(blob)
+        kind, d, n = hasher_blob_info(blob, self.lib)
+        h = C.c_void_p()
+        self._check(self.lib.capy_hasher_import(self._ctx, _hp(blob), blob.size, C.byref(h)))
+        return Hasher(self, h, n, d, kind == 1)
 
     def sponge_encrypt_stream(self, pws, pw_off, nonces, nonce_len: int, d: int, variant: int = B.AE_SHA3) -> EncryptStream:
         """capy_sponge_encrypt_stream_new: one seal stream per password (blocking); tags of 64 bytes"""

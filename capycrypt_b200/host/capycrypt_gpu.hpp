@@ -163,6 +163,22 @@ class Hasher {
     return res;
   }
 
+  // SHA3-d and KMACXOF streams: the blob of capy_hasher_export, for Engine::import_hasher in this or another Engine (a
+  // KMACXOF blob is as secret as its keys)
+  Bytes export_blob() {
+    uint64_t bytes = 0;
+    check(capy_hasher_export_size(h_, &bytes));
+    Bytes blob(bytes);
+    check(capy_hasher_export(ctx_, h_, blob.data(), bytes));
+    return blob;
+  }
+  // a new hasher on the same Engine: stream j starts as a copy of stream src[j] of this one, which is unchanged (blocking)
+  Hasher fork(const std::vector<uint64_t>& src) {
+    capy_hasher* f = nullptr;
+    check(capy_hasher_fork(ctx_, h_, src.data(), src.size(), &f));
+    return Hasher(ctx_, f, src.size(), d_bits_);
+  }
+
   // encryption streams (Engine::sha3_encrypt_stream / key_encrypt_stream): the ciphertext of pieces[i] for every stream;
   // final(512) (sponge AE) or final(448) (key_encrypt) then returns the tags
   std::vector<Bytes> encrypt_update(const std::vector<Bytes>& pieces) {
@@ -307,6 +323,16 @@ class Engine {
     check(capy_kmac_xof_hasher_new(ctx_, d_bits, kd.data(), ko.data(), keys.size(),
                                    reinterpret_cast<const uint8_t*>(s.data()), (uint32_t)s.size(), &h));
     return Hasher(ctx_, h, keys.size(), d_bits);
+  }
+
+  // the streams of a blob from Hasher::export_blob, dealt over this Engine's devices (blocking)
+  Hasher import_hasher(const Bytes& blob) {
+    int d_bits = 0;
+    uint64_t n = 0;
+    check(capy_hasher_blob_info(blob.data(), blob.size(), nullptr, &d_bits, &n));
+    capy_hasher* h = nullptr;
+    check(capy_hasher_import(ctx_, blob.data(), blob.size(), &h));
+    return Hasher(ctx_, h, (size_t)n, d_bits);
   }
 
   // sha3_encrypt of plaintexts fed in pieces (Hasher::encrypt_update, then final(512) for the tags): one stream per

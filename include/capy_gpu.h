@@ -418,6 +418,46 @@ int capy_hasher_sign_final(capy_ctx* ctx, capy_hasher* h, uint8_t* h56, uint8_t*
 int capy_hasher_sign_final_dev(capy_ctx* ctx, capy_hasher* h, int dev_index, void* stream, uint8_t* d_h56, uint8_t* d_z_be56,
                                uint8_t* d_ok);
 
+/* ---- Checkpoints and forks of SHA3-d and KMACXOF streams ---------------------------------------------------------------
+ * A hasher of capy_sha3_hasher_new or capy_kmac_xof_hasher_new can be written to a blob and read back into a new hasher,
+ * in this ctx or another, on any number of devices, in this process or a later one; and it can be forked into a new
+ * hasher of the same ctx whose streams start as copies of its own.  A stream so copied continues exactly as the original
+ * would: its final gives the bytes of the one-shot call on everything fed before and after the copy.  Uses: surviving a
+ * restart, the digest so far (fork, then final the fork), and a prefix shared by many streams (absorb it once, fork).
+ *  - Other kinds of hasher are refused (CAPY_ERR_BAD_ARG), and so is a hasher finished on any device:
+ *      encryption streams: a fork, or one blob imported twice, reuses keystream bytes, and two ciphertexts under one
+ *        keystream reveal the XOR of their plaintexts.
+ *      sign streams: a copy carries s and k off the device, and the pass-equality check would hold per copy only.
+ *      decryption streams: they carry the expected tags and verdicts; an imported blob would decide which plaintext is
+ *        released.
+ *      verification streams: the stored h decides the verdict; whoever writes the blob decides whether a signature
+ *        verifies.
+ *  - A KMACXOF blob is as secret as the key: whoever holds it can compute the KMAC of any extension of that stream.
+ *    Blobs are neither authenticated nor encrypted.  capy_hasher_free zeroes the device state; the page-locked buffers a
+ *    pageable blob is staged through are zeroed by capy_gpu_scrub.
+ *  - The hasher's _dev work must have completed (as before its host calls).  Fork and import are creation calls,
+ *    blocking like every *_new.  On any error *out stays NULL and nothing is left allocated.
+ * Blob format, all fields little-endian.  Header, 64 bytes: the magic "CAPYHSTR", u32 format version = 1, u32 kind
+ * (0 = SHA3-d, 1 = KMACXOF), u32 d_bits, u32 rate (SHA3-d: 144 / 136 / 104 / 72; KMACXOF: 168 / 152 / 136), u32 record
+ * bytes = 208 + rate, u32 zero, u64 n, zero bytes up to 64.  Then n records, item-major, each the 25 state lanes
+ * (200 B), the total bytes absorbed (8 B) and the carry (rate B), of which the first total % rate bytes are the stream's
+ * and the rest are zero.  So a blob is canonical: the same absorbed bytes give the same blob however they were cut into
+ * pieces and on however many devices they lived.  capy_hasher_blob_info and capy_hasher_import refuse
+ * (CAPY_ERR_BAD_ARG) a wrong magic or version, an unknown kind, an invalid d_bits or KMACXOF at 224 (see above), a rate
+ * or record size that does not match, non-zero reserved bytes, a blob_len other than 64 + n * record; import also a
+ * record whose carry tail is not zero. */
+/* bytes of capy_hasher_export's blob: 64-byte header + n records */
+int capy_hasher_export_size(const capy_hasher* h, uint64_t* bytes);
+/* blocking; blob may be pageable; blob_len < export size: CAPY_ERR_BAD_ARG */
+int capy_hasher_export(capy_ctx* ctx, const capy_hasher* h, uint8_t* blob, uint64_t blob_len);
+/* host only, no GPU: validates the header and the length; kind 0 = SHA3-d, 1 = KMACXOF; kind, d_bits, n may be NULL */
+int capy_hasher_blob_info(const uint8_t* blob, uint64_t blob_len, int* kind, int* d_bits, uint64_t* n);
+/* blocking; the items are dealt over THIS ctx's devices in equal contiguous ranges, as at creation */
+int capy_hasher_import(capy_ctx* ctx, const uint8_t* blob, uint64_t blob_len, capy_hasher** out);
+/* blocking; a new hasher of m items on the same ctx; item j starts as a copy of item src[j] of h (any order, repeats
+ * allowed, m may differ from n); h is unchanged and stays usable.  src[j] >= n (so any m > 0 with n == 0): CAPY_ERR_BAD_ARG */
+int capy_hasher_fork(capy_ctx* ctx, const capy_hasher* h, const uint64_t* src, uint64_t m, capy_hasher** out);
+
 #ifdef __cplusplus
 }
 #endif

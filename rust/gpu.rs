@@ -181,6 +181,13 @@ extern "C" {
         ok: *mut u8) -> c_int;
     fn capy_hasher_sign_final_dev(ctx: *mut CapyCtx, h: *mut CapyHasher, dev_index: c_int, stream: *mut c_void,
         d_h56: *mut u8, d_z_be56: *mut u8, d_ok: *mut u8) -> c_int;
+    fn capy_hasher_export_size(h: *const CapyHasher, bytes: *mut u64) -> c_int;
+    fn capy_hasher_export(ctx: *mut CapyCtx, h: *const CapyHasher, blob: *mut u8, blob_len: u64) -> c_int;
+    fn capy_hasher_blob_info(blob: *const u8, blob_len: u64, kind: *mut c_int, d_bits: *mut c_int,
+        n: *mut u64) -> c_int;
+    fn capy_hasher_import(ctx: *mut CapyCtx, blob: *const u8, blob_len: u64, out: *mut *mut CapyHasher) -> c_int;
+    fn capy_hasher_fork(ctx: *mut CapyCtx, h: *const CapyHasher, src: *const u64, m: u64,
+        out: *mut *mut CapyHasher) -> c_int;
 }
 
 const CAPY_AE_SHA3: c_int = 0;
@@ -604,6 +611,24 @@ impl Hasher {
         status(unsafe { capy_hasher_final(self.ctx, self.h, l_bits, std::ptr::null(), out.as_mut_ptr()) })?;
         Ok((0..self.n).map(|i| out[i * ob..(i + 1) * ob].to_vec()).collect())
     }
+
+    /// The streams as a blob (capy_gpu.h: the blob format), to be resumed by `Gpu::import_hasher` in this or another
+    /// `Gpu`.  A KMACXOF blob is as secret as its keys.
+    pub fn export(&self) -> Result<Vec<u8>, OperationError> {
+        let mut bytes = 0u64;
+        status(unsafe { capy_hasher_export_size(self.h, &mut bytes) })?;
+        let mut blob = vec![0u8; bytes as usize];
+        status(unsafe { capy_hasher_export(self.ctx, self.h, blob.as_mut_ptr(), bytes) })?;
+        Ok(blob)
+    }
+
+    /// A new hasher of `src.len()` streams on the same `Gpu`; stream j starts as a copy of stream `src[j]` of this one,
+    /// which is unchanged (blocking).
+    pub fn fork(&self, src: &[u64]) -> Result<Hasher, OperationError> {
+        let mut h = std::ptr::null_mut();
+        status(unsafe { capy_hasher_fork(self.ctx, self.h, src.as_ptr(), src.len() as u64, &mut h) })?;
+        Ok(Hasher { ctx: self.ctx, h, n: src.len() })
+    }
 }
 
 impl Drop for Hasher {
@@ -630,6 +655,17 @@ impl Gpu {
                                      s.len() as u32, &mut h)
         })?;
         Ok(Hasher { ctx: self.ctx, h, n: keys.len() })
+    }
+
+    /// The streams of a blob from `Hasher::export`, dealt over this `Gpu`'s devices (blocking).
+    pub fn import_hasher(&self, blob: &[u8]) -> Result<Hasher, OperationError> {
+        let mut n = 0u64;
+        status(unsafe {
+            capy_hasher_blob_info(blob.as_ptr(), blob.len() as u64, std::ptr::null_mut(), std::ptr::null_mut(), &mut n)
+        })?;
+        let mut h = std::ptr::null_mut();
+        status(unsafe { capy_hasher_import(self.ctx, blob.as_ptr(), blob.len() as u64, &mut h) })?;
+        Ok(Hasher { ctx: self.ctx, h, n: n as usize })
     }
 }
 
